@@ -2,6 +2,7 @@
 """bench.py -- samp_p preimages/s (+ f_a evals/s) of the B200 backend on the configurations BASELINE.json names.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c1|c2|c3|c4|c5] [--batch B] [--impl ours|reference]
+                  [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[1] (C2: PSFGPV n = 256, q = 2^24, 1M-target workload consumed in steps of
 --batch targets per GPU); the default single-GPU run also carries `extra.rows`: C1, C3 (ring f_a / samp_p), C4 (one
@@ -57,6 +58,26 @@ WORKLOADS = {
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+DUMP_BYTES = 60_000_000  # --dump-outputs data budget: the .npy files stay under 64 MB with their headers
+
+
+def dump_outputs(out_dir, rows_total, arrays):
+    """--dump-outputs: write the same fixed, seeded sample of rows of every array as out_dir/<name>.npy.
+    `arrays` maps a name to (device tensor whose first dimension is the row, numpy float dtype to store)."""
+    import torch
+
+    row_bytes = sum(t[0].numel() * np.dtype(dt).itemsize for t, dt in arrays.values())
+    k = min(rows_total, DUMP_BYTES // row_bytes)
+    rows = np.sort(np.random.default_rng(0).choice(rows_total, k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, (t, dt) in arrays.items():
+        x = t.index_select(0, torch.from_numpy(rows).to(t.device)).cpu().numpy()
+        y = x.astype(dt)
+        assert np.array_equal(y, x), f"{name}: values not exact in {np.dtype(dt).name}"
+        np.save(os.path.join(out_dir, name + ".npy"), y)
+    log(f"[dump] {k} of {rows_total} rows of {', '.join(arrays)} -> {out_dir}")
 
 
 class ClockSampler:
@@ -324,7 +345,9 @@ def compress_headline(args, torch, dev, rank, world, local, barrier):
 
     npoly = args.batch or WORKLOADS["c5"]["batch"]
     count = npoly * 256
-    x = torch.randint(0, 3329, (count,), dtype=torch.int32, device=dev).to(torch.int16)
+    gen = torch.Generator(device=dev)
+    gen.manual_seed(1000 + rank)  # the same inputs on every run, distinct per rank
+    x = torch.randint(0, 3329, (count,), dtype=torch.int32, device=dev, generator=gen).to(torch.int16)
     y = torch.empty_like(x)
     st = torch.cuda.current_stream().cuda_stream
     for _ in range(args.warmup):
@@ -341,6 +364,9 @@ def compress_headline(args, torch, dev, rank, world, local, barrier):
     barrier()
     ms = e0.elapsed_time(e1)
     clock_info = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, npoly, {"compress_in": (x.view(npoly, 256), np.float32),
+                                                "compress_out": (y.view(npoly, 256), np.float32)})
     if world > 1:
         import torch.distributed as dist
 
@@ -388,7 +414,13 @@ def main():
     ap.add_argument("--ref-targets", type=int, default=0, help="reference arm: targets per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra.rows block of the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed, seeded sample (<= 64 MB) of the last timed step's results to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the results of --impl ours")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -526,6 +558,8 @@ def main():
     # spherical law: E||e||^2 = dim (s r)^2 / (2 pi) for D_{Lambda_u^perp(A), s r}
     norm_ratio = float((e[:4096].double() ** 2).reshape(min(batch, 4096), -1).sum(1).mean().item()
                        / (dim * (s * r_par) ** 2 / (2 * math.pi)))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, batch, {"samp_p_e": (e, np.float32), "samp_p_u": (u, np.float64)})
 
     # ---- f_a evals/s (device resident; sigma = the preimages, in domain) ---------------------------------
     for _ in range(3):
