@@ -107,13 +107,21 @@ qf_status qf_set_trapdoor_perturbation(qf_ctx* ctx, const int8_t* r, const doubl
  * trapdoor R (m_bar x nk); W = digits of -A[:, :m_bar], S' column-reversed iff base^k = q.  The m_bar x nk x m_bar
  * product R W runs on the tensor cores; s_out is m x m (host), columns are the basis vectors.  Exact. */
 qf_status qf_gen_short_basis(qf_ctx* ctx, const int8_t* r, int64_t* s_out);
+/* gen_short_basis_for_trapdoor with a tag (short_basis_classical.rs:54-110): as qf_gen_short_basis for the installed
+ * A = [A_bar | H G - A_bar R] with W = digits of -H^-1 A[:, :m_bar] mod q.  tag: n x n (host), entries taken mod q;
+ * NULL means H = I (then identical to qf_gen_short_basis).  H^-1 is computed on the device by Gauss-Jordan with unit
+ * pivots (first row at or below the diagonal whose entry is a unit mod q); QF_ERR_INVALID when no such pivot exists,
+ * where the reference panics in MatZq::inverse.  Exact. */
+qf_status qf_gen_short_basis_tagged(qf_ctx* ctx, const int8_t* r, const int64_t* tag, int64_t* s_out);
 /* compute_sqrt_sigma_2 (mp_perturbation.rs:111-139) on the device: lower Cholesky factor (m x m, row-major, host)
  * of Sigma_2 = r^2/(2 pi) (Sigma - (b^2+1) [R;I][R;I]^t - I); sigma == NULL means Sigma = s^2 I.
  * QF_ERR_INVALID when Sigma_2 is not positive definite (the reference panics in the Cholesky). */
 qf_status qf_compute_sqrt_sigma_2(qf_ctx* ctx, const int8_t* r, const double* sigma, double* sqrt_sigma_2_out);
 /* PSFGPV trapdoor (gpv.rs:61): short basis S (dim x dim, columns are basis vectors) and its
  * GSO.  dim = m for QF_PSF_GPV, n*(k+2) (coefficient embedding) for QF_PSF_GPV_RING.
- * s_gso == NULL: the GSO is computed on the device (as qf_gso) and never leaves it. */
+ * s_gso == NULL: the GSO is computed on the device (as qf_gso) and never leaves it.
+ * G-trapdoor keys A = [A_bar | H G - A_bar R] with the basis of qf_gen_short_basis_tagged are recognised for the
+ * identity tag and for any tag H invertible by unit pivoting: samp_p then runs the two-phase recursion on H^-1 A. */
 qf_status qf_set_trapdoor_gpv(qf_ctx* ctx, const int64_t* s, const double* s_gso);
 /* MatQ::gso as used at gpv.rs:91: unnormalised Gram-Schmidt of the columns of S (dim x dim) in fp64 on the
  * device (blocked Gram-Schmidt with re-orthogonalisation).  gso_out: dim x dim, host. */

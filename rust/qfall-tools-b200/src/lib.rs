@@ -188,6 +188,30 @@ impl PSFGPVB200 {
         self.ctx.check(unsafe { qf_set_trapdoor_gpv(self.ctx.raw, sw.as_ptr(), gso.as_ptr()) }, "qf_set_trapdoor_gpv");
         *self.installed.borrow_mut() = Some((aw, sw));
     }
+    /// `gen_short_basis_for_trapdoor(params, tag, a, r)` (short_basis_classical.rs:54-110) on the device for the key `a`
+    /// of this context's parameters: W = digits of -tag^-1 a[:, :m_bar] with tag^-1 and the products computed on the
+    /// GPU (qf_gen_short_basis_tagged).  Panics where the reference's `MatZq::inverse(..).unwrap()` does: no unit pivot.
+    /// Installs `a` as the context key.
+    pub fn gen_short_basis_for_trapdoor(&self, tag: &MatZq, a: &MatZq, r: &MatZ) -> MatZ {
+        let (n, m) = (self.n(), self.m());
+        let m_bar = i64::try_from(&self.inner.gp.m_bar).unwrap() as usize;
+        assert_eq!((tag.get_num_rows(), tag.get_num_columns()), (n as i64, n as i64), "tag must be n x n");
+        let (aw, tw) = (matzq_to_words(a), matzq_to_words(tag));
+        let r8: Vec<i8> = matz_to_words(r).into_iter().map(|v| i8::try_from(v).expect("R entries must fit i8")).collect();
+        assert_eq!(r8.len(), m_bar * (m - m_bar), "R must be m_bar x n k");
+        *self.installed.borrow_mut() = None; // qf_set_a drops the installed trapdoor
+        self.ctx.check(unsafe { qf_set_a(self.ctx.raw, aw.as_ptr()) }, "qf_set_a");
+        let mut s = vec![0i64; m * m];
+        self.ctx.check(unsafe { qf_gen_short_basis_tagged(self.ctx.raw, r8.as_ptr(), tw.as_ptr(), s.as_mut_ptr()) },
+                       "qf_gen_short_basis_tagged");
+        let mut out = MatZ::new(m as i64, m as i64);
+        for i in 0..m {
+            for j in 0..m {
+                out.set_entry(i as i64, j as i64, Z::from(s[i * m + j])).unwrap();
+            }
+        }
+        out
+    }
 }
 
 impl PSF for PSFGPVB200 {

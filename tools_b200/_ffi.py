@@ -48,6 +48,7 @@ SIGNATURES = {
     "qf_set_trapdoor_perturbation": (_i32, [_vp, _vp, _vp, _vp, _vp]),
     "qf_compute_sqrt_sigma_2": (_i32, [_vp, _vp, _vp, _vp]),
     "qf_gen_short_basis": (_i32, [_vp, _vp, _vp]),
+    "qf_gen_short_basis_tagged": (_i32, [_vp, _vp, _vp, _vp]),
     "qf_ring_gen_short_basis": (_i32, [_vp, _vp, _vp, _vp]),
     "qf_gso": (_i32, [_vp, _vp, _vp]),
     "qf_set_trapdoor_gpv": (_i32, [_vp, _vp, _vp]),

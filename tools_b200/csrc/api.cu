@@ -172,6 +172,14 @@ struct qf_ctx {
     // digit counts / windows of the contractions (U_22 updates, the two centre maps, U_11 updates).
     bool gadget_key_ok = false, two_phase = false;
     Dev dMt1l, dMt1scale, dMpl, dMpscale;
+    // Tagged G-trapdoor key A = [A_bar | H G - A_bar R], H invertible mod q (gadget_classical.rs:56-68): the recursion runs on
+    // H^-1 A = [A_bar' | G - A_bar' R], A_bar' = H^-1 A_bar, which has the same lattice and the same short basis; a target u
+    // becomes u' = H^-1 u.  u8 digit planes of H^-1 (n x ldk_n, one set per digit group of modq_contract) and of A_bar'
+    // (n x ldk_mb); tag_ulimbs balanced digits of a residue (the split of u).  Set by detect_gpv_structure, dropped with the key.
+    bool key_tagged = false;
+    int tag_ulimbs = 0;
+    long ldk_n = 0;
+    Dev dHinvl, dAbpl, dTagU, dTagUl, dTagTmp;
     // Defaults from the error budget of DESIGN 4.2, checked at the full C2 key (scripts/ab_c2_precision.py, profiles/README_r2.md):
     // four digits everywhere; the lowest digit sum is dropped where the operand has three digits (z2), not for the
     // two-digit z1 (dropping it there moves 14 % of the preimages, keeping it 0.3 %).
@@ -376,6 +384,33 @@ cudaError_t ctx_gemm_i8(qf_ctx* ctx, const I8GemmArgs& a, bool count_ops = true)
         ctx->prof_recs.push_back(rec);
     }
     return e;
+}
+
+// out = X W^t mod q (B x N, int64, ld N) for X = lx balanced s8 digit planes of B x K (row stride ldx, plane stride xp) and a
+// key matrix W of residues in u8 digit planes (LW = ctx->a_limbs, N x K, row stride ldw).  Two pipeline stages of the
+// contraction must hold all x planes in shared memory, which allows at most MODQ_MAX_LX of them (residues up to ~2^47).
+// Wider x is taken in two digit groups, [0, MODQ_GROUP) and [MODQ_GROUP, lx): the second group multiplies the planes of
+// 256^MODQ_GROUP W mod q (wg1) and starts from the first group's result (base), so the sum is reduced mod q exactly.
+constexpr int MODQ_MAX_LX = 6, MODQ_GROUP = 4;
+inline int modq_groups(int lx) { return lx > MODQ_MAX_LX ? 2 : 1; }
+
+qf_status modq_contract(qf_ctx* ctx, const int8_t* x, long ldx, long xp, int lx, const void* wg0, const void* wg1, long ldw,
+                        int B, int N, int K, int64_t* tmp, int64_t* out) {
+    const int groups = modq_groups(lx);
+    for (int gi = 0; gi < groups; ++gi) {
+        const int l0 = gi ? MODQ_GROUP : 0, l1 = groups == 1 ? lx : (gi ? lx : MODQ_GROUP);
+        I8GemmArgs g{};
+        g.x = x + l0 * xp; g.ldx = ldx; g.x_plane = xp;
+        g.w = gi ? wg1 : wg0; g.ldw = ldw; g.w_plane = N * ldw;
+        g.LX = l1 - l0; g.LW = ctx->a_limbs; g.w_signed = 0;
+        g.B = B; g.N = N; g.K = K;
+        g.out_kind = 0; g.sign = 1; g.q = ctx->prm.q;
+        g.base = gi ? tmp : nullptr; g.ldbase = N;
+        g.out = (gi + 1 == groups) ? out : tmp; g.ldout = N;
+        g.flag = ctx->dFlag.as<int>();
+        LAUNCH(ctx_gemm_i8(ctx, g));
+    }
+    return QF_OK;
 }
 
 // ---------------------------------------------------------------------------
@@ -1001,14 +1036,30 @@ qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t se
     ctx->np_wdrop_cur = ctx->u_limbs - ctx->u22_limbs; ctx->np_dlo_cur = ctx->u22_dlo; ctx->np_lx_min = 3;
     QF_TRY(np_block(ctx, T, Z, Bc, nk, D, NP_TOP, 0, seed, first));
 
-    // ---- h = (u - A_bar z2) mod q, exact (A_bar = the first m_bar columns of the installed digit planes of A)
+    // ---- tagged key: the recursion runs on H^-1 A, so its target is u' = H^-1 u mod q (phase 1 never reads the target)
+    const int64_t* ub = dUin;
+    if (ctx->key_tagged) {
+        const long ldkn = ctx->ldk_n, tplane = C * ldkn;
+        CK(ctx->dTagUl.ensure((size_t)ctx->tag_ulimbs * tplane));
+        CK(ctx->dTagU.ensure((size_t)C * n * 8));
+        if (modq_groups(ctx->tag_ulimbs) > 1) CK(ctx->dTagTmp.ensure((size_t)C * n * 8));
+        LAUNCH(qf_launch_split_i64_limbs(dUin, n, ctx->dTagUl.as<int8_t>(), tplane, ldkn, Bc, (int)n, ctx->tag_ulimbs, flag,
+                                         ctx->stream));
+        const uint8_t* hl = ctx->dHinvl.as<uint8_t>();
+        QF_TRY(modq_contract(ctx, ctx->dTagUl.as<int8_t>(), ldkn, tplane, ctx->tag_ulimbs, hl, hl + (size_t)ctx->a_limbs * n * ldkn,
+                             ldkn, Bc, (int)n, (int)n, ctx->dTagTmp.as<int64_t>(), ctx->dTagU.as<int64_t>()));
+        ub = ctx->dTagU.as<int64_t>();
+    }
+    // ---- h = (u - A_bar z2) mod q, exact (A_bar = the first m_bar columns of the installed digit planes of A; for a tagged
+    // key u' - A_bar' z2 with the digit planes of A_bar' = H^-1 A_bar)
     {
+        const long ldw = ctx->key_tagged ? ctx->ldk_mb : ldk;
         I8GemmArgs g{};
         g.x = zp + nk; g.ldx = ldk; g.x_plane = plane;
-        g.w = ctx->dAl.p; g.ldw = ldk; g.w_plane = n * ldk;
+        g.w = ctx->key_tagged ? ctx->dAbpl.p : ctx->dAl.p; g.ldw = ldw; g.w_plane = n * ldw;
         g.LX = L; g.LW = ctx->a_limbs; g.w_signed = 0;
         g.B = Bc; g.N = (int)n; g.K = (int)mb;
-        g.out_kind = 0; g.sign = -1; g.q = ctx->prm.q; g.base = dUin; g.ldbase = n; g.out = H; g.ldout = n;
+        g.out_kind = 0; g.sign = -1; g.q = ctx->prm.q; g.base = ub; g.ldbase = n; g.out = H; g.ldout = n;
         g.flag = flag;
         g.x_nz = ctx->dNz.as<uint8_t>(); g.nz_m_tiles = nz_m; g.nz_kb_total = nz_kb; g.nz_kb_off = (int)(nk / 128);
         QF_TRY(gemm_i8_gated(ctx, g, gate_z2));
@@ -1312,10 +1363,79 @@ qf_status gso_device(qf_ctx* ctx, const double* dS, double* dG) {
     return QF_OK;
 }
 
-// Recover (R, W) from a short basis of the form gen_short_basis_for_trapdoor builds (tag = I) and verify the
+// H^-1 mod q on the device (qf_launch_mat_inverse_mod) for the n x n residues h; *ok = false when some column has no
+// unit pivot (first row at or below the diagonal whose entry is a unit mod q), and hinv is then left empty
+qf_status tag_inverse(qf_ctx* ctx, const uint64_t* h, std::vector<int64_t>& hinv, bool* ok) {
+    const long n = ctx->n;
+    std::vector<uint64_t> mm((size_t)n * 2 * n, 0);
+    for (long i = 0; i < n; ++i) {
+        for (long j = 0; j < n; ++j) mm[(size_t)i * 2 * n + j] = h[i * n + j];
+        mm[(size_t)i * 2 * n + n + i] = 1;
+    }
+    Dev dM, dF, dFail;
+    CK(dM.ensure(mm.size() * 8));
+    CK(dF.ensure((size_t)n * 8));
+    CK(dFail.ensure(sizeof(int)));
+    CK(cudaMemcpyAsync(dM.p, mm.data(), mm.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    LAUNCH(qf_launch_mat_inverse_mod(dM.as<uint64_t>(), dF.as<uint64_t>(), (int)n, ctx->prm.q, dFail.as<int>(), ctx->stream));
+    int fail = 0;
+    CK(cudaMemcpyAsync(&fail, dFail.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(mm.data(), dM.p, mm.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    *ok = fail == 0;
+    hinv.clear();
+    if (!*ok) return QF_OK;
+    hinv.resize((size_t)n * n);
+    for (long i = 0; i < n; ++i)
+        for (long j = 0; j < n; ++j) hinv[(size_t)i * n + j] = (int64_t)mm[(size_t)i * 2 * n + n + j];
+    return QF_OK;
+}
+
+// u8 digit planes of H^-1 into dHl (n x ldk_n per digit group of modq_contract: H^-1, then 256^MODQ_GROUP H^-1 mod q when a
+// residue needs two groups; the key operand of u' = H^-1 u) and A_bar'^t = (H^-1 A_bar)^t mod q (m_bar x n, A_bar = the first
+// m_bar columns of the installed A) into abt: tcgen05 with the mod-q epilogue, the "targets" being the columns of A_bar as
+// balanced digits
+qf_status tag_apply(qf_ctx* ctx, const std::vector<int64_t>& hinv, Dev& dHl, std::vector<int64_t>& abt) {
+    const long n = ctx->n, mb = ctx->m_bar, m = ctx->m, ldk = ctx->ldk_n;
+    const uint64_t q = ctx->prm.q;
+    const int lx = limbs_for((double)(q - 1));
+    const int groups = modq_groups(lx), L = ctx->a_limbs;
+    {
+        uint64_t sh = 1;
+        for (int i = 0; i < MODQ_GROUP; ++i) sh = mulmod_h(sh, 256, q);
+        std::vector<uint8_t> planes((size_t)groups * L * n * ldk, 0);
+        for (int gi = 0; gi < groups; ++gi)
+            for (long i = 0; i < n; ++i)
+                for (long j = 0; j < n; ++j) {
+                    const uint64_t h = (uint64_t)hinv[(size_t)i * n + j], v = gi ? mulmod_h(h, sh, q) : h;
+                    for (int l = 0; l < L; ++l) planes[(((size_t)gi * L + l) * n + i) * ldk + j] = (uint8_t)(v >> (8 * l));
+                }
+        CK(dHl.ensure(planes.size()));
+        CK(cudaMemcpyAsync(dHl.p, planes.data(), planes.size(), cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    std::vector<int64_t> at((size_t)mb * n);
+    for (long j = 0; j < n; ++j)
+        for (long c = 0; c < mb; ++c) at[(size_t)c * n + j] = ctx->hA[(size_t)j * m + c];
+    Dev dX, dOut, dTmp;
+    QF_TRY(upload_limbs(ctx, at.data(), mb, n, ldk, lx, true, dX));
+    CK(dOut.ensure((size_t)mb * n * 8));
+    if (groups > 1) CK(dTmp.ensure((size_t)mb * n * 8));
+    const uint8_t* hl = dHl.as<uint8_t>();
+    QF_TRY(modq_contract(ctx, dX.as<int8_t>(), ldk, mb * ldk, lx, hl, hl + (size_t)L * n * ldk, ldk, (int)mb, (int)n, (int)n,
+                         dTmp.as<int64_t>(), dOut.as<int64_t>()));
+    abt.resize((size_t)mb * n);
+    CK(cudaMemcpyAsync(abt.data(), dOut.p, abt.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return QF_OK;
+}
+
+// Recover (R, W) from a short basis of the form gen_short_basis_for_trapdoor builds (for any tag) and verify the
 // factorisation exactly; on success e = S z runs in structured form.  Any mismatch leaves the dense path in place.
-qf_status detect_gpv_structure(qf_ctx* ctx, const int64_t* s, const std::vector<int>& piv) {
+// Then check the key against the basis: [A_bar | G - A_bar R] (identity tag) or, if find_tag, [A_bar | H G - A_bar R].
+qf_status detect_gpv_structure(qf_ctx* ctx, const int64_t* s, const std::vector<int>& piv, bool find_tag) {
     ctx->gpv_struct = false;
+    ctx->key_tagged = false;
     const char* env = getenv("QF_DISABLE_GPV_STRUCT");
     if (ctx->prm.kind != QF_PSF_GPV || !ctx->use_i8 || (env && env[0] == '1')) return QF_OK;
     const long n = ctx->n, k = ctx->k, mb = ctx->m_bar, nk = ctx->nk, m = ctx->m;
@@ -1450,6 +1570,46 @@ qf_status detect_gpv_structure(qf_ctx* ctx, const int64_t* s, const std::vector<
                 if ((uint64_t)ctx->hA[(size_t)i * m + mb + j] != (gij + q - (uint64_t)art[(size_t)j * n + i]) % q) { ok = false; break; }
             }
         ctx->gadget_key_ok = ok;
+        if (!ok && find_tag) {
+            // Tagged key A = [A_bar | H G - A_bar R]?  Then Y = A[:, m_bar:] + A_bar R = H G mod q: H from the columns with
+            // gadget entry 1, Y[:, j k + t] = base^t H[:, j] for every other column.
+            auto Y = [&](long i, long j) -> uint64_t {
+                return (uint64_t)(((u128)(uint64_t)ctx->hA[(size_t)i * m + mb + j] + (uint64_t)art[(size_t)j * n + i]) % q);
+            };
+            std::vector<uint64_t> h((size_t)n * n);
+            bool tag_ok = true;
+            for (long i = 0; i < n && tag_ok; ++i)
+                for (long jb = 0; jb < n && tag_ok; ++jb) {
+                    const uint64_t hij = Y(i, jb * k);
+                    h[(size_t)i * n + jb] = hij;
+                    for (long t = 1; t < k; ++t)
+                        if (Y(i, jb * k + t) != mulmod_h(hij, gpow[t], q)) { tag_ok = false; break; }
+                }
+            // H^-1 on the device, A_bar' = H^-1 A_bar on the tensor cores, and G W = -A_bar' mod q exactly for the W of the
+            // installed basis: this one check also rejects a wrong inverse and a basis built for another tag
+            std::vector<int64_t> hinv, abt;
+            if (tag_ok) QF_TRY(tag_inverse(ctx, h.data(), hinv, &tag_ok));
+            if (tag_ok) {
+                QF_TRY(tag_apply(ctx, hinv, ctx->dHinvl, abt));
+                for (long i = 0; i < n && tag_ok; ++i)
+                    for (long c = 0; c < mb; ++c) {
+                        u128 gw = (uint64_t)abt[(size_t)c * n + i];
+                        for (long t = 0; t < k; ++t) gw += (u128)gpow[t] * (uint64_t)w64[(size_t)(i * k + t) * mb + c];
+                        if (gw % q != 0) { tag_ok = false; break; }
+                    }
+            }
+            if (tag_ok) {
+                std::vector<int64_t> ab((size_t)n * mb);
+                for (long i = 0; i < n; ++i)
+                    for (long c = 0; c < mb; ++c) ab[(size_t)i * mb + c] = abt[(size_t)c * n + i];
+                QF_TRY(upload_limbs(ctx, ab.data(), n, mb, ctx->ldk_mb, ctx->a_limbs, false, ctx->dAbpl));
+                ctx->tag_ulimbs = limbs_for((double)(q - 1));
+                ctx->key_tagged = true;
+                ctx->gadget_key_ok = true;
+            } else {
+                ctx->dHinvl.release();
+            }
+        }
     }
     return QF_OK;
 }
@@ -1471,6 +1631,8 @@ qf_status install_a(qf_ctx* ctx, const int64_t* a) {
     // a new key invalidates whatever trapdoor was installed for the old one: samp_p answers QF_ERR_NO_KEY until the
     // trapdoor is installed again (never a preimage of the new A computed from the old A^-1, pivots, S and R)
     ctx->has_a = false; ctx->has_np = false; ctx->has_pert = false;
+    ctx->key_tagged = false;
+    ctx->dHinvl.release(); ctx->dAbpl.release();
     const long n = ctx->n, m = ctx->m;
     for (long i = 0; i < n * m; ++i)
         if (a[i] < 0 || (uint64_t)a[i] >= ctx->prm.q) return ctx->fail(QF_ERR_INVALID, "A entry outside [0,q)");
@@ -1529,6 +1691,7 @@ qf_status qf_ctx_create(const qf_params* p, int device, qf_ctx** out) {
     }
     ctx->ldk_dim = (ctx->dim + 127) / 128 * 128;
     ctx->ldk_nk = (ctx->nk + 127) / 128 * 128;
+    ctx->ldk_n = (ctx->n + 127) / 128 * 128;
     ctx->x_limbs = limbs_for(std::sqrt((double)ctx->bound));
     {
         const char* env = getenv("QF_DISABLE_I8");
@@ -1760,7 +1923,9 @@ qf_status qf_ring_gen_short_basis(qf_ctx* ctx, const int32_t* r, const int32_t* 
     return QF_OK;
 }
 
-qf_status qf_gen_short_basis(qf_ctx* ctx, const int8_t* r, int64_t* s_out) {
+// gen_short_basis_for_trapdoor (short_basis_classical.rs:54-110) for the installed A and the tag H (NULL: identity):
+// W = digits of -H^-1 A[:, :m_bar] mod q, with H^-1 (qf_launch_mat_inverse_mod) and the product (tcgen05) on the device
+qf_status qf_gen_short_basis_tagged(qf_ctx* ctx, const int8_t* r, const int64_t* tag, int64_t* s_out) {
     if (!ctx || !r || !s_out) return QF_ERR_INVALID;
     if (ctx->prm.kind == QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "ring context: the ring short basis is built by the host shim");
     if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "install A first (qf_set_a / qf_trap_gen)");
@@ -1798,12 +1963,27 @@ qf_status qf_gen_short_basis(qf_ctx* ctx, const int8_t* r, int64_t* s_out) {
             for (long i = 0; i < mb; ++i) s_out[(size_t)i * m + c] += (int64_t)r[i * nk + row] * v;
         }
     }
-    // W = base-b digits of -A[:, :m_bar] mod q (short_basis_classical.rs:105-110), stored transposed for the device:
-    // Wt[c][j k + t] = digit t of (q - A[j][c]) mod q
+    // A_bar' = H^-1 A[:, :m_bar] mod q (short_basis_classical.rs:106-107), transposed; the tag as MatZq: entries reduced mod q
+    std::vector<int64_t> abt;
+    if (tag) {
+        std::vector<uint64_t> h((size_t)n * n);
+        for (long i = 0; i < n * n; ++i) {
+            const int64_t v = tag[i] % (int64_t)q;
+            h[i] = (uint64_t)(v < 0 ? v + (int64_t)q : v);
+        }
+        std::vector<int64_t> hinv;
+        bool ok = false;
+        QF_TRY(tag_inverse(ctx, h.data(), hinv, &ok));
+        if (!ok) return ctx->fail(QF_ERR_INVALID, "tag is not invertible mod q (no unit pivot)");
+        Dev dHl;
+        QF_TRY(tag_apply(ctx, hinv, dHl, abt));
+    }
+    // W = base-b digits of -A_bar' mod q (short_basis_classical.rs:105-110), stored transposed for the device:
+    // Wt[c][j k + t] = digit t of (q - A_bar'[j][c]) mod q
     std::vector<int64_t> wt((size_t)mb * nk);
     for (long j = 0; j < n; ++j)
         for (long c = 0; c < mb; ++c) {
-            uint64_t v = (q - (uint64_t)ctx->hA[(size_t)j * m + c]) % q;
+            uint64_t v = (q - (uint64_t)(tag ? abt[(size_t)c * n + j] : ctx->hA[(size_t)j * m + c])) % q;
             for (long t = 0; t < k; ++t) {
                 const int64_t d = (int64_t)(v % base);
                 v /= base;
@@ -1836,6 +2016,8 @@ qf_status qf_gen_short_basis(qf_ctx* ctx, const int8_t* r, int64_t* s_out) {
     }
     return check_flag(ctx);
 }
+
+qf_status qf_gen_short_basis(qf_ctx* ctx, const int8_t* r, int64_t* s_out) { return qf_gen_short_basis_tagged(ctx, r, nullptr, s_out); }
 
 qf_status qf_compute_sqrt_sigma_2(qf_ctx* ctx, const int8_t* r, const double* sigma, double* out) {
     if (!ctx || !r || !out) return QF_ERR_INVALID;
@@ -1964,17 +2146,18 @@ qf_status qf_set_trapdoor_gpv(qf_ctx* ctx, const int64_t* s, const double* sg) {
     if (ctx->use_i8) {
         if (ctx->z_limbs + ctx->s_limbs - 1 > 16) return ctx->fail(QF_ERR_UNSUPPORTED, "too many digits for the int8 S*z product");
         ctx->zlimit = std::min(ctx->zlimit, limb_capacity(ctx->z_limbs));
-        QF_TRY(detect_gpv_structure(ctx, s, piv));
-        if (ctx->gpv_struct) ctx->dSl.release();
-        else QF_TRY(upload_limbs(ctx, s, D, D, ctx->ldk_dim, ctx->s_limbs, true, ctx->dSl));
         const char* env = getenv("QF_DISABLE_OZAKI");
         const char* envmin = getenv("QF_OZAKI_MIN_DIM");
         const long min_dim = envmin ? atol(envmin) : 2 * NP_SIZES[2];
-        // two-phase recursion (samp_p_np2_chunk): G-trapdoor basis of a key of the form [A_bar | G - A_bar R], tensor-core
+        // two-phase recursion (samp_p_np2_chunk): G-trapdoor basis of a key of the form [A_bar | H G - A_bar R], tensor-core
         // dimensions.  z then only has to hold the phase-1 coefficients (widths s/||b~_i||, centres of the same size).
         const char* env2 = getenv("QF_DISABLE_TWO_PHASE");  // test switch: the one-pass recursion
-        ctx->two_phase = ctx->gpv_struct && ctx->gadget_key_ok && D > std::max(min_dim, NP_SIZES[2]) &&
-                         !(env && env[0] == '1') && !(env2 && env2[0] == '1');
+        const bool two_phase_allowed = D > std::max(min_dim, NP_SIZES[2]) && !(env && env[0] == '1') && !(env2 && env2[0] == '1');
+        // the tag of a tagged key is only looked for where two-phase can use it
+        QF_TRY(detect_gpv_structure(ctx, s, piv, two_phase_allowed));
+        if (ctx->gpv_struct) ctx->dSl.release();
+        else QF_TRY(upload_limbs(ctx, s, D, D, ctx->ldk_dim, ctx->s_limbs, true, ctx->dSl));
+        ctx->two_phase = ctx->gpv_struct && ctx->gadget_key_ok && two_phase_allowed;
         if (ctx->two_phase) {
             // the gadget digits g3 reach base - 1: one more digit of M' for bases above 4 (its error scales with |g3|)
             ctx->mt1g_limbs = ctx->prm.base > 4 ? 5 : 4;

@@ -833,6 +833,27 @@ __global__ void __launch_bounds__(256) range_check_i64_kernel(const int64_t* __r
         bad |= (unsigned long long)v[i] >= q;  // negative values are huge as unsigned
     if (bad) atomicOr(flag, 32);
 }
+// balanced base-256 digits of int64 values (|v| < 2^63): planes[l][b][j] = digit l of in[b][j] for j < M, zero for
+// M <= j < ldk; *flag |= 8 when a value does not fit L digits.  One thread per (row, column).
+__global__ void __launch_bounds__(256) split_i64_limbs_kernel(const int64_t* __restrict__ in, long ldin, int8_t* __restrict__ planes,
+                                                              long plane_stride, long ldk, int B, int M, int L, int* flag) {
+    const long total = (long)B * ldk;
+    bool bad = false;
+    for (long t = (long)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (long)gridDim.x * blockDim.x) {
+        const long b = t / ldk, j = t - b * ldk;
+        long long v = j < M ? in[b * ldin + j] : 0;
+        for (int l = 0; l < L; ++l) {
+            long long lo = ((v + 128) & 255) - 128;
+            if (l == L - 1) {
+                bad |= v != lo;
+                lo = v;
+            }
+            v = (v - lo) >> 8;
+            planes[l * plane_stride + b * ldk + j] = (int8_t)lo;
+        }
+    }
+    if (bad && flag) atomicOr(flag, 8);
+}
 }  // namespace
 cudaError_t qf_launch_narrow_i32_i16(const int32_t* in, int16_t* out, size_t count, int* flag, cudaStream_t stream) {
     if (count == 0) return cudaSuccess;
@@ -849,5 +870,13 @@ cudaError_t qf_launch_widen_i16_i32(const int16_t* in, int32_t* out, size_t coun
 cudaError_t qf_launch_range_check_i64(const int64_t* v, size_t count, unsigned long long q, int* flag, cudaStream_t stream) {
     if (count == 0) return cudaSuccess;
     range_check_i64_kernel<<<grid_for((long long)count, 256, 148 * 4), 256, 0, stream>>>(v, count, q, flag);
+    return cudaGetLastError();
+}
+cudaError_t qf_launch_split_i64_limbs(const int64_t* in, long ldin, int8_t* planes, long plane_stride, long ldk, int B, int M,
+                                      int L, int* flag, cudaStream_t stream) {
+    if (B <= 0) return cudaSuccess;
+    if (M > ldk || L < 1 || L > 8) return cudaErrorInvalidValue;
+    split_i64_limbs_kernel<<<grid_for((long long)B * ldk, 256, 148 * 8), 256, 0, stream>>>(in, ldin, planes, plane_stride, ldk, B, M,
+                                                                                         L, flag);
     return cudaGetLastError();
 }

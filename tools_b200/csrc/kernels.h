@@ -261,6 +261,15 @@ cudaError_t qf_launch_ozaki_prepare(const double* U, long ld, int D, int blk, in
 cudaError_t qf_launch_narrow_i32_i16(const int32_t* in, int16_t* out, size_t count, int* flag, cudaStream_t stream);
 cudaError_t qf_launch_widen_i16_i32(const int16_t* in, int32_t* out, size_t count, cudaStream_t stream);
 cudaError_t qf_launch_range_check_i64(const int64_t* v, size_t count, unsigned long long q, int* flag, cudaStream_t stream);
+// balanced s8 digit planes of int64 values (B x M, row stride ldin) into L planes of B x ldk bytes, columns [M, ldk) zeroed;
+// *flag |= 8 when a value does not fit L digits (the x operand of a contraction whose "targets" are residues, e.g. u' = H^-1 u)
+cudaError_t qf_launch_split_i64_limbs(const int64_t* in, long ldin, int8_t* planes, long plane_stride, long ldk, int B, int M,
+                                      int L, int* flag, cudaStream_t stream);
+
+// tag inverse of a G-trapdoor key (setup.cu): Gauss-Jordan over Z_q with unit pivots on M = [H | I] (n x 2n residues,
+// q < 2^62); on return *fail = 0 and the right half of M is H^-1, or *fail = c + 1 when column c has no unit pivot.
+// f: n words of device scratch.
+cudaError_t qf_launch_mat_inverse_mod(uint64_t* M, uint64_t* f, int n, unsigned long long q, int* fail, cudaStream_t stream);
 
 // polynomial arithmetic of the ring short basis (setup.cu): P[2][2][n], Q[k][2][n]
 cudaError_t qf_launch_ring_basis_polys(const int32_t* e, const int32_t* r, const int32_t* w, const int64_t* sk, int n, int k,

@@ -422,3 +422,76 @@ cudaError_t qf_launch_ring_basis_polys(const int32_t* e, const int32_t* r, const
     ring_basis_polys_kernel<<<4 + 2 * k, 256, 0, stream>>>(e, r, w, sk, n, k, P, Q);
     return cudaGetLastError();
 }
+
+// ---- tag inverse (short_basis_classical.rs:106, MatZq::inverse): Gauss-Jordan over Z_q on M = [H | I] (n x 2n residues,
+// row-major, q < 2^62, 128-bit products).  Column c takes as pivot the first row r >= c whose entry is a unit mod q -- the
+// rule of the host restatement gadget._inverse_mod, so both fail on the same tags.  On success the right half of M is H^-1 and *fail = 0;
+// without a unit pivot *fail = c + 1 and M is left part-reduced.  One CTA: n pivot steps separated by block barriers;
+// per step the factors of column c are saved in f (n words) before the rows are updated.
+namespace {
+__device__ __forceinline__ uint64_t gcd_dev(uint64_t a, uint64_t b) {
+    while (b) { const uint64_t t = a % b; a = b; b = t; }
+    return a;
+}
+// a^-1 mod q for gcd(a, q) = 1 (extended Euclid; the coefficients stay below q < 2^62 in magnitude)
+__device__ __forceinline__ uint64_t inv_mod_dev(uint64_t a, uint64_t q) {
+    long long t = 0, nt = 1;
+    uint64_t r = q, nr = a % q;
+    while (nr) {
+        const uint64_t qu = r / nr;
+        const long long tt = t - (long long)qu * nt; t = nt; nt = tt;
+        const uint64_t rr = r - qu * nr; r = nr; nr = rr;
+    }
+    return t < 0 ? (uint64_t)(t + (long long)q) : (uint64_t)t;
+}
+
+__global__ void __launch_bounds__(1024) mat_inverse_mod_kernel(uint64_t* __restrict__ M, uint64_t* __restrict__ f, int n,
+                                                               uint64_t q, int* __restrict__ fail) {
+    __shared__ int piv;
+    __shared__ uint64_t inv;
+    const long w = 2L * n;
+    const int tid = threadIdx.x, nth = blockDim.x;
+    for (int c = 0; c < n; ++c) {
+        if (tid == 0) piv = n;
+        __syncthreads();
+        for (int r = c + tid; r < n; r += nth)
+            if (gcd_dev(M[(long)r * w + c], q) == 1) atomicMin(&piv, r);
+        __syncthreads();
+        const int p = piv;
+        if (p == n) {
+            if (tid == 0) *fail = c + 1;
+            return;
+        }
+        if (tid == 0) inv = inv_mod_dev(M[(long)p * w + c], q);
+        if (p != c)
+            for (long j = c + tid; j < w; j += nth) {
+                const uint64_t t = M[(long)p * w + j];
+                M[(long)p * w + j] = M[(long)c * w + j];
+                M[(long)c * w + j] = t;
+            }
+        __syncthreads();
+        for (long j = c + tid; j < w; j += nth) M[(long)c * w + j] = mulmod_u64(M[(long)c * w + j], inv, q);
+        for (int r = tid; r < n; r += nth) f[r] = r == c ? 0 : M[(long)r * w + c];
+        __syncthreads();
+        // rows r != c: M[r][j] -= f[r] M[c][j] for j >= c (columns left of c are already zero in row c)
+        const long cols = w - c, total = (long)n * cols;
+        for (long t = tid; t < total; t += nth) {
+            const int r = (int)(t / cols);
+            const uint64_t fr = f[r];
+            if (!fr) continue;
+            const long j = c + (t - (long)r * cols);
+            const uint64_t sub = mulmod_u64(fr, M[(long)c * w + j], q);
+            const uint64_t v = M[(long)r * w + j];
+            M[(long)r * w + j] = v >= sub ? v - sub : v + (q - sub);
+        }
+        __syncthreads();
+    }
+    if (tid == 0) *fail = 0;
+}
+}  // namespace
+
+cudaError_t qf_launch_mat_inverse_mod(uint64_t* M, uint64_t* f, int n, unsigned long long q, int* fail, cudaStream_t stream) {
+    if (n < 1 || q < 2 || q >= (1ull << 62)) return cudaErrorInvalidValue;
+    mat_inverse_mod_kernel<<<1, 1024, 0, stream>>>(M, f, n, (uint64_t)q, fail);
+    return cudaGetLastError();
+}

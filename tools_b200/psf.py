@@ -168,13 +168,21 @@ class PSFGPV(_PSFBase):
             self.ctx.call("qf_set_trapdoor_gpv", _ffi.ptr(s), _ffi.ptr(sg))
             self._td_id = td
 
-    def trap_gen(self, seed=None, dense_gso: bool = None):
+    def trap_gen(self, seed=None, dense_gso: bool = None, tag=None):
         """gpv.rs:83-94: uniform A_bar, gen_trapdoor, short basis, GSO -- all on the device.  dense_gso=False
         leaves the second trapdoor component None (the backend computes the GSO when the trapdoor is installed and
         keeps it in HBM instead of moving m x m doubles through the host twice); default: the reference's
-        (S, S~) pair up to m = 2048, None above."""
+        (S, S~) pair up to m = 2048, None above.
+        tag: an n x n matrix H invertible mod q (gadget_classical.rs:56-68 with a tag): A = [A_bar | H G - A_bar R] from
+        the same device-sampled A_bar and R (qf_trap_gen_from), and the short basis for that tag.  None: H = I."""
         a, r = _trap_gen_classical(self, seed)
-        short_base = self.gen_short_basis_for_trapdoor(r)
+        if tag is not None:
+            tg = np.array(np.asarray(tag, dtype=object) % self.gp.q, dtype=np.int64)
+            assert tg.shape == (self.n, self.n)
+            ab = np.ascontiguousarray(a[:, : self.gp.m_bar])
+            a = np.empty((self.n, self.m), dtype=np.int64)
+            self.ctx.call("qf_trap_gen_from", _ffi.ptr(ab), _ffi.ptr(r), _ffi.ptr(tg), _ffi.ptr(a))
+        short_base = self.gen_short_basis_for_trapdoor(r, tag)
         if dense_gso is None:
             dense_gso = self.m <= 2048
         td = (short_base, self.gso(short_base) if dense_gso else None)
@@ -186,13 +194,20 @@ class PSFGPV(_PSFBase):
         return _gso(self, basis)
 
 
-    def gen_short_basis_for_trapdoor(self, r) -> np.ndarray:
-        """short_basis_classical.rs:54-110 for the installed A, tag = I: the integer products run on the device
-        (qf_gen_short_basis); exact.  gadget.gen_short_basis_for_trapdoor is the host restatement (tags, tests)."""
+    def gen_short_basis_for_trapdoor(self, r, tag=None) -> np.ndarray:
+        """short_basis_classical.rs:54-110 for the installed A and the tag H (n x n, entries taken mod q; None: H = I):
+        H^-1 and every integer product run on the device (qf_gen_short_basis_tagged); exact.  Raises QfError
+        (QF_ERR_INVALID) when H is not invertible by unit pivoting, where the reference panics.
+        gadget.gen_short_basis_for_trapdoor is the host restatement (tests)."""
         r8 = np.ascontiguousarray(r, dtype=np.int8)
         assert r8.shape == (self.gp.m_bar, self.gp.n * self.gp.k)
         out = np.empty((self.m, self.m), dtype=np.int64)
-        self.ctx.call("qf_gen_short_basis", _ffi.ptr(r8), _ffi.ptr(out))
+        if tag is None:
+            self.ctx.call("qf_gen_short_basis", _ffi.ptr(r8), _ffi.ptr(out))
+            return out
+        tg = np.array(np.asarray(tag, dtype=object) % self.gp.q, dtype=np.int64)
+        assert tg.shape == (self.n, self.n)
+        self.ctx.call("qf_gen_short_basis_tagged", _ffi.ptr(r8), _ffi.ptr(tg), _ffi.ptr(out))
         return out
 
 
