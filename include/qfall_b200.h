@@ -99,9 +99,22 @@ qf_status qf_set_a(qf_ctx* ctx, const int64_t* a);
  * I_n (x) S_k with its GSO (gadget_classical.rs:248-287; the shim checks block-diagonality).
  * sqrt_sigma_2 == NULL: the backend derives its own square root of the DEFAULT covariance
  * Sigma = s^2 I (what PSFPerturbation::trap_gen builds, mp_perturbation.rs:227-231) from R, s, r on the
- * device, in block form (only an m_bar x m_bar Cholesky factor is dense) -- same law, ~4x less work per target. */
+ * device, in block form (only an m_bar x m_bar Cholesky factor is dense) -- same law, ~4x less work per target.
+ * Needs an installed A (QF_ERR_NO_KEY otherwise).  Tagged keys A = [A_bar | H G - A_bar R] (gadget_classical.rs:56-68) for
+ * this R are recognised: A [R; I] = H G, so samp_p samples the gadget preimage of H^-1 (u - A p) mod q (H^-1 by
+ * Gauss-Jordan with unit pivots on the device).  For H = I the sampler is the untagged one.  A key of this form whose H
+ * has no unit pivot (singular H included) is QF_ERR_INVALID and no trapdoor is installed; a key of any other form is
+ * installed as given. */
 qf_status qf_set_trapdoor_perturbation(qf_ctx* ctx, const int8_t* r, const double* sqrt_sigma_2,
                                        const int64_t* s_block, const double* s_block_gso);
+/* Switch the tag of the installed PSFPerturbation key without re-installing the trapdoor: A = [A_bar | H G - A_bar R]
+ * becomes [A_bar | H' G - A_bar R], i.e. A[:, m_bar:] += (H' - H) G mod q, bit-identical to qf_trap_gen_from(A_bar, R, H').
+ * tag: n x n (host), entries taken mod q; NULL means H' = I.  a_out: the new A, n x m (host), may be NULL.  R, sqrt(Sigma_2)
+ * and the gadget basis stay installed; every device copy of A and H^-1 are replaced.  QF_ERR_INVALID on a context of
+ * another kind, QF_ERR_NO_KEY without key and trapdoor, QF_ERR_INVALID when the installed key was not recognised as a
+ * G-trapdoor for the installed R, and QF_ERR_INVALID for a tag H' without a unit pivot (the key and its tag then stay as
+ * they were). */
+qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out);
 /* gen_short_basis_for_trapdoor with tag = I (short_basis_classical.rs:54-110): the short basis
  * S_A = [[I,R],[0,I]] [[0,I],[S',W]] = [[R S', I + R W],[S', W]] of Lambda^perp(A) for the installed A and the
  * trapdoor R (m_bar x nk); W = digits of -A[:, :m_bar], S' column-reversed iff base^k = q.  The m_bar x nk x m_bar

@@ -47,6 +47,7 @@ extern "C" {
 
     pub fn qf_set_a(ctx: *mut qf_ctx, a: *const i64) -> i32;
     pub fn qf_set_trapdoor_perturbation(ctx: *mut qf_ctx, r: *const i8, sqrt_sigma_2: *const f64, s_block: *const i64, s_block_gso: *const f64) -> i32;
+    pub fn qf_set_tag(ctx: *mut qf_ctx, tag: *const i64, a_out: *mut i64) -> i32;
     pub fn qf_gen_short_basis(ctx: *mut qf_ctx, r: *const i8, s_out: *mut i64) -> i32;
     pub fn qf_gen_short_basis_tagged(ctx: *mut qf_ctx, r: *const i8, tag: *const i64, s_out: *mut i64) -> i32;
     pub fn qf_compute_sqrt_sigma_2(ctx: *mut qf_ctx, r: *const i8, sigma: *const f64, sqrt_sigma_2_out: *mut f64) -> i32;

@@ -111,6 +111,29 @@ impl PSFPerturbationB200 {
         self.ctx.check(st, "qf_set_trapdoor_perturbation");
         *self.installed_r.borrow_mut() = Some(key);
     }
+
+    /// Tag switch for a key `a = [A_bar | H G - A_bar R]` (gen_trapdoor with a tag, gadget_classical.rs:56-68) and its
+    /// trapdoor `td`: returns `[A_bar | H' G - A_bar R]` for `tag` = H' (n x n), equal to gen_trapdoor(A_bar, R, H'), and
+    /// installs it while R, sqrt(Sigma_2) and the gadget basis stay on the device (qf_set_tag).  Panics when `a` is not such a
+    /// key for the R of `td` or when H' has no unit pivot (the reference panics in `MatZq::inverse`).
+    pub fn set_tag(&self, a: &MatZq, td: &(MatZ, MatQ, (MatZ, MatQ)), tag: &MatZq) -> MatZq {
+        let (n, m) = (self.n(), self.m());
+        assert_eq!((tag.get_num_rows(), tag.get_num_columns()), (n as i64, n as i64), "tag must be n x n");
+        self.install_a(a);
+        self.install_td(td);
+        let tw = matzq_to_words(tag);
+        let mut aw = vec![0i64; n * m];
+        self.ctx.check(unsafe { qf_set_tag(self.ctx.raw, tw.as_ptr(), aw.as_mut_ptr()) }, "qf_set_tag");
+        let q = Z::from(&self.inner.gp.q);
+        let mut out = MatZq::new(n as i64, m as i64, &q);
+        for i in 0..n {
+            for j in 0..m {
+                out.set_entry(i as i64, j as i64, Z::from(aw[i * m + j])).unwrap();
+            }
+        }
+        *self.installed_a.borrow_mut() = Some(aw);
+        out
+    }
 }
 
 impl PSF for PSFPerturbationB200 {

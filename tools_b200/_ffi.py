@@ -46,6 +46,7 @@ SIGNATURES = {
                                C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_uint64)]),
     "qf_set_a": (_i32, [_vp, _vp]),
     "qf_set_trapdoor_perturbation": (_i32, [_vp, _vp, _vp, _vp, _vp]),
+    "qf_set_tag": (_i32, [_vp, _vp, _vp]),
     "qf_compute_sqrt_sigma_2": (_i32, [_vp, _vp, _vp, _vp]),
     "qf_gen_short_basis": (_i32, [_vp, _vp, _vp]),
     "qf_gen_short_basis_tagged": (_i32, [_vp, _vp, _vp, _vp]),

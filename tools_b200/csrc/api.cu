@@ -105,6 +105,11 @@ struct qf_ctx {
     long ld_mb = 0;
     double sqrt_beta = 0, xb_fscale = 0;
     int xb_limbs = 3;
+    // the installed key is A = [A_bar | H G - A_bar R] for the installed R (recognised by qf_set_trapdoor_perturbation,
+    // replaced by qf_set_tag): pert_tag = H mod q (n x n).  For H != I, key_tagged is set and v = u - A p becomes
+    // v' = H^-1 v before the gadget sampler (digit planes of H^-1 in dHinvl).
+    bool pert_gadget_key = false;
+    std::vector<uint64_t> pert_tag;
     // nearest-plane engine (GPV, ring)
     bool has_np = false;
     int npiv = 0;
@@ -175,7 +180,8 @@ struct qf_ctx {
     // Tagged G-trapdoor key A = [A_bar | H G - A_bar R], H invertible mod q (gadget_classical.rs:56-68): the recursion runs on
     // H^-1 A = [A_bar' | G - A_bar' R], A_bar' = H^-1 A_bar, which has the same lattice and the same short basis; a target u
     // becomes u' = H^-1 u.  u8 digit planes of H^-1 (n x ldk_n, one set per digit group of modq_contract) and of A_bar'
-    // (n x ldk_mb); tag_ulimbs balanced digits of a residue (the split of u).  Set by detect_gpv_structure, dropped with the key.
+    // (n x ldk_mb); tag_ulimbs balanced digits of a residue (the split of u).  Set by detect_gpv_structure (PSFPerturbation:
+    // key_tagged, dHinvl and tag_ulimbs by qf_set_trapdoor_perturbation / qf_set_tag), dropped with the key.
     bool key_tagged = false;
     int tag_ulimbs = 0;
     long ldk_n = 0;
@@ -410,6 +416,22 @@ qf_status modq_contract(qf_ctx* ctx, const int8_t* x, long ldx, long xp, int lx,
         g.flag = ctx->dFlag.as<int>();
         LAUNCH(ctx_gemm_i8(ctx, g));
     }
+    return QF_OK;
+}
+
+// Tagged key: v' = H^-1 v mod q for Bc residue vectors v (row stride n) -- tag_ulimbs balanced digits of v against the digit
+// planes of H^-1 (dHinvl).  *out = the device buffer holding v' (row stride n).
+qf_status tag_targets(qf_ctx* ctx, const int64_t* dV, int Bc, const int64_t** out) {
+    const long n = ctx->n, C = ctx->chunk, ldkn = ctx->ldk_n, tplane = C * ldkn;
+    CK(ctx->dTagUl.ensure((size_t)ctx->tag_ulimbs * tplane));
+    CK(ctx->dTagU.ensure((size_t)C * n * 8));
+    if (modq_groups(ctx->tag_ulimbs) > 1) CK(ctx->dTagTmp.ensure((size_t)C * n * 8));
+    LAUNCH(qf_launch_split_i64_limbs(dV, n, ctx->dTagUl.as<int8_t>(), tplane, ldkn, Bc, (int)n, ctx->tag_ulimbs,
+                                     ctx->dFlag.as<int>(), ctx->stream));
+    const uint8_t* hl = ctx->dHinvl.as<uint8_t>();
+    QF_TRY(modq_contract(ctx, ctx->dTagUl.as<int8_t>(), ldkn, tplane, ctx->tag_ulimbs, hl, hl + (size_t)ctx->a_limbs * n * ldkn,
+                         ldkn, Bc, (int)n, (int)n, ctx->dTagTmp.as<int64_t>(), ctx->dTagU.as<int64_t>()));
+    *out = ctx->dTagU.as<int64_t>();
     return QF_OK;
 }
 
@@ -649,9 +671,12 @@ qf_status samp_p_pert_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t s
         ca.nacc = ctx->a_nchunks; ca.acc_sign = -1; ca.ldacc = ldn; ca.base = dUin; ca.ldbase = ctx->n; ca.q = ctx->prm.q;
         LAUNCH(qf_launch_combine_i64(ca, V, ctx->n, Bc, (int)ctx->n, ctx->stream));
     }
+    // tagged key A = [A_bar | H G - A_bar R]: A [R; I] = H G, so z solves G z = v' = H^-1 v
+    const int64_t* Vg = V;
+    if (ctx->key_tagged) QF_TRY(tag_targets(ctx, V, Bc, &Vg));
     // z <- D_{Lambda_v^perp(G), r sqrt(b^2+1)}   (:321-326 -> :173-191)
     const double s_g = ctx->prm.r * std::sqrt((double)(ctx->prm.base * ctx->prm.base + 1));
-    LAUNCH(qf_launch_gadget_sample(V, ctx->n, Z, ldnk, Bc, (int)ctx->n, (int)ctx->k, (int)ctx->prm.base, ctx->prm.q,
+    LAUNCH(qf_launch_gadget_sample(Vg, ctx->n, Z, ldnk, Bc, (int)ctx->n, (int)ctx->k, (int)ctx->prm.base, ctx->prm.q,
                                    ctx->dSk.as<double>(), ctx->dSkGso.as<double>(), s_g, seed, first, ctx->dFlag.as<int>(),
                                    ctx->stream));
     // e = p + [R; I] z   (:328-335): top block accumulates R z into p in place (exact small integers)
@@ -1038,18 +1063,7 @@ qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t se
 
     // ---- tagged key: the recursion runs on H^-1 A, so its target is u' = H^-1 u mod q (phase 1 never reads the target)
     const int64_t* ub = dUin;
-    if (ctx->key_tagged) {
-        const long ldkn = ctx->ldk_n, tplane = C * ldkn;
-        CK(ctx->dTagUl.ensure((size_t)ctx->tag_ulimbs * tplane));
-        CK(ctx->dTagU.ensure((size_t)C * n * 8));
-        if (modq_groups(ctx->tag_ulimbs) > 1) CK(ctx->dTagTmp.ensure((size_t)C * n * 8));
-        LAUNCH(qf_launch_split_i64_limbs(dUin, n, ctx->dTagUl.as<int8_t>(), tplane, ldkn, Bc, (int)n, ctx->tag_ulimbs, flag,
-                                         ctx->stream));
-        const uint8_t* hl = ctx->dHinvl.as<uint8_t>();
-        QF_TRY(modq_contract(ctx, ctx->dTagUl.as<int8_t>(), ldkn, tplane, ctx->tag_ulimbs, hl, hl + (size_t)ctx->a_limbs * n * ldkn,
-                             ldkn, Bc, (int)n, (int)n, ctx->dTagTmp.as<int64_t>(), ctx->dTagU.as<int64_t>()));
-        ub = ctx->dTagU.as<int64_t>();
-    }
+    if (ctx->key_tagged) QF_TRY(tag_targets(ctx, dUin, Bc, &ub));
     // ---- h = (u - A_bar z2) mod q, exact (A_bar = the first m_bar columns of the installed digit planes of A; for a tagged
     // key u' - A_bar' z2 with the digit planes of A_bar' = H^-1 A_bar)
     {
@@ -1391,29 +1405,34 @@ qf_status tag_inverse(qf_ctx* ctx, const uint64_t* h, std::vector<int64_t>& hinv
     return QF_OK;
 }
 
-// u8 digit planes of H^-1 into dHl (n x ldk_n per digit group of modq_contract: H^-1, then 256^MODQ_GROUP H^-1 mod q when a
-// residue needs two groups; the key operand of u' = H^-1 u) and A_bar'^t = (H^-1 A_bar)^t mod q (m_bar x n, A_bar = the first
-// m_bar columns of the installed A) into abt: tcgen05 with the mod-q epilogue, the "targets" being the columns of A_bar as
-// balanced digits
-qf_status tag_apply(qf_ctx* ctx, const std::vector<int64_t>& hinv, Dev& dHl, std::vector<int64_t>& abt) {
+// u8 digit planes of H^-1 into dHl: n x ldk_n per digit group of modq_contract (H^-1, then 256^MODQ_GROUP H^-1 mod q when a
+// residue needs two groups), the key operand of u' = H^-1 u
+qf_status tag_planes(qf_ctx* ctx, const std::vector<int64_t>& hinv, Dev& dHl) {
+    const long n = ctx->n, ldk = ctx->ldk_n;
+    const uint64_t q = ctx->prm.q;
+    const int groups = modq_groups(limbs_for((double)(q - 1))), L = ctx->a_limbs;
+    uint64_t sh = 1;
+    for (int i = 0; i < MODQ_GROUP; ++i) sh = mulmod_h(sh, 256, q);
+    std::vector<uint8_t> planes((size_t)groups * L * n * ldk, 0);
+    for (int gi = 0; gi < groups; ++gi)
+        for (long i = 0; i < n; ++i)
+            for (long j = 0; j < n; ++j) {
+                const uint64_t h = (uint64_t)hinv[(size_t)i * n + j], v = gi ? mulmod_h(h, sh, q) : h;
+                for (int l = 0; l < L; ++l) planes[(((size_t)gi * L + l) * n + i) * ldk + j] = (uint8_t)(v >> (8 * l));
+            }
+    CK(dHl.ensure(planes.size()));
+    CK(cudaMemcpyAsync(dHl.p, planes.data(), planes.size(), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return QF_OK;
+}
+
+// A_bar'^t = (H^-1 A_bar)^t mod q (m_bar x n, A_bar = the first m_bar columns of the installed A) into abt, for the digit
+// planes dHl of H^-1 (tag_planes): tcgen05 with the mod-q epilogue, the "targets" being the columns of A_bar as balanced digits
+qf_status tag_abar(qf_ctx* ctx, const Dev& dHl, std::vector<int64_t>& abt) {
     const long n = ctx->n, mb = ctx->m_bar, m = ctx->m, ldk = ctx->ldk_n;
     const uint64_t q = ctx->prm.q;
     const int lx = limbs_for((double)(q - 1));
     const int groups = modq_groups(lx), L = ctx->a_limbs;
-    {
-        uint64_t sh = 1;
-        for (int i = 0; i < MODQ_GROUP; ++i) sh = mulmod_h(sh, 256, q);
-        std::vector<uint8_t> planes((size_t)groups * L * n * ldk, 0);
-        for (int gi = 0; gi < groups; ++gi)
-            for (long i = 0; i < n; ++i)
-                for (long j = 0; j < n; ++j) {
-                    const uint64_t h = (uint64_t)hinv[(size_t)i * n + j], v = gi ? mulmod_h(h, sh, q) : h;
-                    for (int l = 0; l < L; ++l) planes[(((size_t)gi * L + l) * n + i) * ldk + j] = (uint8_t)(v >> (8 * l));
-                }
-        CK(dHl.ensure(planes.size()));
-        CK(cudaMemcpyAsync(dHl.p, planes.data(), planes.size(), cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-    }
     std::vector<int64_t> at((size_t)mb * n);
     for (long j = 0; j < n; ++j)
         for (long c = 0; c < mb; ++c) at[(size_t)c * n + j] = ctx->hA[(size_t)j * m + c];
@@ -1427,6 +1446,85 @@ qf_status tag_apply(qf_ctx* ctx, const std::vector<int64_t>& hinv, Dev& dHl, std
     abt.resize((size_t)mb * n);
     CK(cudaMemcpyAsync(abt.data(), dOut.p, abt.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
+    return QF_OK;
+}
+
+// gadget entries base^t mod q, t < k
+std::vector<uint64_t> gadget_powers(const qf_ctx* ctx) {
+    std::vector<uint64_t> gpow(ctx->k);
+    u128 pwt = 1;
+    for (long t = 0; t < ctx->k; ++t) { gpow[t] = (uint64_t)(pwt % ctx->prm.q); pwt = pwt * (uint64_t)ctx->prm.base % ctx->prm.q; }
+    return gpow;
+}
+
+// Form of the installed key A for a trapdoor R (m_bar x nk): a G-trapdoor A = [A_bar | H G - A_bar R] (gadget_classical.rs:56-68)
+// with H = I, with an H invertible by unit pivoting, with an H that has no unit pivot (singular ones included), or none of these.
+enum KeyForm { KEY_OTHER, KEY_IDENTITY, KEY_TAGGED, KEY_TAG_SINGULAR };
+struct KeyTag {
+    KeyForm form = KEY_OTHER;
+    std::vector<uint64_t> h;     // H mod q, n x n (KEY_IDENTITY, KEY_TAGGED, KEY_TAG_SINGULAR)
+    std::vector<int64_t> hinv;   // H^-1 mod q (KEY_TAGGED)
+};
+
+// The one place that decides how a G-trapdoor key is recognised (PSFGPV and PSFPerturbation trapdoor installs).  A_bar R on
+// the tensor cores ("targets" = the columns of R, key matrix = the installed digit planes of A), compared exactly on the host:
+// Y = A[:, m_bar:] + A_bar R mod q must be H G, with H read from the columns with gadget entry 1 and Y[:, j k + t] =
+// base^t H[:, j] for every other column.  H = I is KEY_IDENTITY.  Otherwise, if find_tag, H^-1 is computed on the device
+// (unit pivots) and, for KEY_TAGGED, its digit planes are written to dHl (tag_planes); without find_tag the key is KEY_OTHER.
+qf_status match_key_tag(qf_ctx* ctx, const int8_t* R, bool find_tag, Dev& dHl, KeyTag& kt) {
+    kt = KeyTag();
+    const long n = ctx->n, k = ctx->k, mb = ctx->m_bar, nk = ctx->nk, m = ctx->m;
+    const uint64_t q = ctx->prm.q;
+    const long ldk = (mb + 127) / 128 * 128;
+    Dev dRt, dAr;
+    {
+        // R^t as one s8 plane (nk x ldk), transposed in cache blocks
+        constexpr long TB = 64;
+        std::vector<uint8_t> rt((size_t)nk * ldk, 0);
+        for (long i0 = 0; i0 < mb; i0 += TB)
+            for (long j0 = 0; j0 < nk; j0 += TB)
+                for (long i = i0; i < std::min(mb, i0 + TB); ++i)
+                    for (long j = j0; j < std::min(nk, j0 + TB); ++j) rt[(size_t)j * ldk + i] = (uint8_t)R[(size_t)i * nk + j];
+        CK(dRt.ensure(rt.size()));
+        CK(cudaMemcpyAsync(dRt.p, rt.data(), rt.size(), cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    CK(dAr.ensure((size_t)nk * n * 8));
+    I8GemmArgs g{};
+    g.x = dRt.as<int8_t>(); g.ldx = ldk; g.x_plane = nk * ldk;
+    g.w = ctx->dAl.p; g.ldw = ctx->ldk_dim; g.w_plane = n * ctx->ldk_dim;
+    g.LX = 1; g.LW = ctx->a_limbs; g.w_signed = 0;
+    g.B = (int)nk; g.N = (int)n; g.K = (int)mb;
+    g.out_kind = 0; g.sign = 1; g.q = q; g.out = dAr.p; g.ldout = n;
+    g.flag = ctx->dFlag.as<int>();
+    LAUNCH(ctx_gemm_i8(ctx, g));
+    std::vector<int64_t> art((size_t)nk * n);
+    CK(cudaMemcpyAsync(art.data(), dAr.p, art.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    const std::vector<uint64_t> gpow = gadget_powers(ctx);
+    auto Y = [&](long i, long j) -> uint64_t {
+        return (uint64_t)(((u128)(uint64_t)ctx->hA[(size_t)i * m + mb + j] + (uint64_t)art[(size_t)j * n + i]) % q);
+    };
+    std::vector<uint64_t> h((size_t)n * n);
+    bool ident = true;
+    for (long i = 0; i < n; ++i)
+        for (long jb = 0; jb < n; ++jb) {
+            const uint64_t hij = Y(i, jb * k);
+            h[(size_t)i * n + jb] = hij;
+            ident = ident && hij == (i == jb ? 1u : 0u);
+            for (long t = 1; t < k; ++t)
+                if (Y(i, jb * k + t) != mulmod_h(hij, gpow[t], q)) return QF_OK;
+        }
+    if (ident) {
+        kt.form = KEY_IDENTITY;
+    } else {
+        if (!find_tag) return QF_OK;
+        bool ok = false;
+        QF_TRY(tag_inverse(ctx, h.data(), kt.hinv, &ok));
+        kt.form = ok ? KEY_TAGGED : KEY_TAG_SINGULAR;
+        if (ok) QF_TRY(tag_planes(ctx, kt.hinv, dHl));
+    }
+    kt.h = std::move(h);
     return QF_OK;
 }
 
@@ -1537,67 +1635,27 @@ qf_status detect_gpv_structure(qf_ctx* ctx, const int64_t* s, const std::vector<
     for (int pc : piv) piv_low = piv_low || pc >= mb;
     ctx->i2_limbs = limbs_for(8.0 * ctx->prm.s + 64.0 + (piv_low ? (double)q : 0.0));
     ctx->gpv_struct = true;
-    // Does the installed key have the trapdoor form A = [A_bar | G - A_bar R] for this R (tag = identity,
-    // gadget_classical.rs:56-68)?  Then x = [R g; g] with g = digits(u) solves A x = u and the two-phase recursion applies.
-    // A_bar R on the tensor cores ("targets" = the columns of R, key matrix = the installed digit planes of A), compared
-    // exactly on the host.
+    // Does the installed key have the trapdoor form A = [A_bar | H G - A_bar R] for this R (gadget_classical.rs:56-68)?  For
+    // H = I, x = [R g; g] with g = digits(u) solves A x = u and the two-phase recursion applies; a tag H is looked for only if
+    // find_tag.
     ctx->gadget_key_ok = false;
     if (base <= 128) {
-        std::vector<int64_t> rt((size_t)nk * mb);
-        for (long i = 0; i < mb; ++i)
-            for (long j = 0; j < nk; ++j) rt[(size_t)j * mb + i] = R[(size_t)i * nk + j];
-        Dev dRt, dAr;
-        QF_TRY(upload_limbs(ctx, rt.data(), nk, mb, ctx->ldk_mb, 1, true, dRt));
-        CK(dAr.ensure((size_t)nk * n * 8));
-        I8GemmArgs g{};
-        g.x = dRt.as<int8_t>(); g.ldx = ctx->ldk_mb; g.x_plane = nk * ctx->ldk_mb;
-        g.w = ctx->dAl.p; g.ldw = ctx->ldk_dim; g.w_plane = n * ctx->ldk_dim;
-        g.LX = 1; g.LW = ctx->a_limbs; g.w_signed = 0;
-        g.B = (int)nk; g.N = (int)n; g.K = (int)mb;
-        g.out_kind = 0; g.sign = 1; g.q = q; g.out = dAr.p; g.ldout = n;
-        g.flag = ctx->dFlag.as<int>();
-        LAUNCH(ctx_gemm_i8(ctx, g));
-        std::vector<int64_t> art((size_t)nk * n);
-        CK(cudaMemcpyAsync(art.data(), dAr.p, art.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-        std::vector<uint64_t> gpow(k);
-        u128 pwt = 1;
-        for (long t = 0; t < k; ++t) { gpow[t] = (uint64_t)(pwt % q); pwt *= base; }
-        bool ok = true;
-        for (long i = 0; i < n && ok; ++i)
-            for (long j = 0; j < nk; ++j) {
-                const uint64_t gij = (j / k == i) ? gpow[j % k] : 0;
-                if ((uint64_t)ctx->hA[(size_t)i * m + mb + j] != (gij + q - (uint64_t)art[(size_t)j * n + i]) % q) { ok = false; break; }
-            }
-        ctx->gadget_key_ok = ok;
-        if (!ok && find_tag) {
-            // Tagged key A = [A_bar | H G - A_bar R]?  Then Y = A[:, m_bar:] + A_bar R = H G mod q: H from the columns with
-            // gadget entry 1, Y[:, j k + t] = base^t H[:, j] for every other column.
-            auto Y = [&](long i, long j) -> uint64_t {
-                return (uint64_t)(((u128)(uint64_t)ctx->hA[(size_t)i * m + mb + j] + (uint64_t)art[(size_t)j * n + i]) % q);
-            };
-            std::vector<uint64_t> h((size_t)n * n);
+        KeyTag kt;
+        QF_TRY(match_key_tag(ctx, R.data(), find_tag, ctx->dHinvl, kt));
+        ctx->gadget_key_ok = kt.form == KEY_IDENTITY;
+        if (kt.form == KEY_TAGGED) {
+            // A_bar' = H^-1 A_bar on the tensor cores, and G W = -A_bar' mod q exactly for the W of the installed basis: this
+            // one check also rejects a wrong inverse and a basis built for another tag
+            std::vector<int64_t> abt;
+            QF_TRY(tag_abar(ctx, ctx->dHinvl, abt));
+            const std::vector<uint64_t> gpow = gadget_powers(ctx);
             bool tag_ok = true;
             for (long i = 0; i < n && tag_ok; ++i)
-                for (long jb = 0; jb < n && tag_ok; ++jb) {
-                    const uint64_t hij = Y(i, jb * k);
-                    h[(size_t)i * n + jb] = hij;
-                    for (long t = 1; t < k; ++t)
-                        if (Y(i, jb * k + t) != mulmod_h(hij, gpow[t], q)) { tag_ok = false; break; }
+                for (long c = 0; c < mb; ++c) {
+                    u128 gw = (uint64_t)abt[(size_t)c * n + i];
+                    for (long t = 0; t < k; ++t) gw += (u128)gpow[t] * (uint64_t)w64[(size_t)(i * k + t) * mb + c];
+                    if (gw % q != 0) { tag_ok = false; break; }
                 }
-            // H^-1 on the device, A_bar' = H^-1 A_bar on the tensor cores, and G W = -A_bar' mod q exactly for the W of the
-            // installed basis: this one check also rejects a wrong inverse and a basis built for another tag
-            std::vector<int64_t> hinv, abt;
-            if (tag_ok) QF_TRY(tag_inverse(ctx, h.data(), hinv, &tag_ok));
-            if (tag_ok) {
-                QF_TRY(tag_apply(ctx, hinv, ctx->dHinvl, abt));
-                for (long i = 0; i < n && tag_ok; ++i)
-                    for (long c = 0; c < mb; ++c) {
-                        u128 gw = (uint64_t)abt[(size_t)c * n + i];
-                        for (long t = 0; t < k; ++t) gw += (u128)gpow[t] * (uint64_t)w64[(size_t)(i * k + t) * mb + c];
-                        if (gw % q != 0) { tag_ok = false; break; }
-                    }
-            }
             if (tag_ok) {
                 std::vector<int64_t> ab((size_t)n * mb);
                 for (long i = 0; i < n; ++i)
@@ -1631,7 +1689,7 @@ qf_status install_a(qf_ctx* ctx, const int64_t* a) {
     // a new key invalidates whatever trapdoor was installed for the old one: samp_p answers QF_ERR_NO_KEY until the
     // trapdoor is installed again (never a preimage of the new A computed from the old A^-1, pivots, S and R)
     ctx->has_a = false; ctx->has_np = false; ctx->has_pert = false;
-    ctx->key_tagged = false;
+    ctx->key_tagged = false; ctx->pert_gadget_key = false;
     ctx->dHinvl.release(); ctx->dAbpl.release();
     const long n = ctx->n, m = ctx->m;
     for (long i = 0; i < n * m; ++i)
@@ -1650,6 +1708,30 @@ qf_status install_a(qf_ctx* ctx, const int64_t* a) {
     ctx->a_limbs = (qbits + 7) / 8;
     QF_TRY(upload_limbs(ctx, a, n, m, ctx->ldk_dim, ctx->a_limbs, false, ctx->dAl));
     ctx->has_a = true;
+    return QF_OK;
+}
+
+// Columns [c0, m) of the host copy of A into the device representations install_a built (fp64 digit matrices and u8 digit
+// planes); the other columns are left as they are
+qf_status upload_a_cols(qf_ctx* ctx, long c0) {
+    const long n = ctx->n, m = ctx->m, w = m - c0;
+    std::vector<double> f((size_t)n * w);
+    const unsigned long long mask = (ctx->a_bits >= 64) ? ~0ull : ((1ull << ctx->a_bits) - 1);
+    for (int c = 0; c < ctx->a_nchunks; ++c) {
+        for (long i = 0; i < n; ++i)
+            for (long j = 0; j < w; ++j) f[(size_t)i * w + j] = (double)(((unsigned long long)ctx->hA[(size_t)i * m + c0 + j] >> (c * ctx->a_bits)) & mask);
+        CK(cudaMemcpy2DAsync(ctx->dA[c].as<double>() + c0, (size_t)ctx->ld_dim * 8, f.data(), (size_t)w * 8, (size_t)w * 8, (size_t)n,
+                             cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    std::vector<uint8_t> b((size_t)n * w);
+    for (int l = 0; l < ctx->a_limbs; ++l) {
+        for (long i = 0; i < n; ++i)
+            for (long j = 0; j < w; ++j) b[(size_t)i * w + j] = (uint8_t)((uint64_t)ctx->hA[(size_t)i * m + c0 + j] >> (8 * l));
+        CK(cudaMemcpy2DAsync(ctx->dAl.as<uint8_t>() + (size_t)l * n * ctx->ldk_dim + c0, (size_t)ctx->ldk_dim, b.data(), (size_t)w, (size_t)w,
+                             (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
     return QF_OK;
 }
 
@@ -1815,13 +1897,28 @@ qf_status qf_set_trapdoor_perturbation(qf_ctx* ctx, const int8_t* r, const doubl
                                        const double* skg) {
     if (!ctx || !r || !sk || !skg) return QF_ERR_INVALID;
     if (ctx->prm.kind != QF_PSF_PERTURBATION) return ctx->fail(QF_ERR_INVALID, "not a PSFPerturbation context");
+    if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "install A first (qf_set_a / qf_trap_gen)");
     ctx->has_pert = false;
+    ctx->key_tagged = false; ctx->pert_gadget_key = false;
     CK(cudaSetDevice(ctx->device));
     QF_TRY(upload_as_f64(ctx, r, ctx->m_bar, ctx->nk, ctx->ld_nk, ctx->dR));
     {
         std::vector<int64_t> r64((size_t)ctx->m_bar * ctx->nk);
         for (size_t i = 0; i < r64.size(); ++i) r64[i] = r[i];
         QF_TRY(upload_limbs(ctx, r64.data(), ctx->m_bar, ctx->nk, ctx->ldk_nk, 1, true, ctx->dRl));
+    }
+    // A = [A_bar | H G - A_bar R]: A [R; I] = H G, so samp_p samples z with G z = H^-1 (u - A p) (samp_p_pert_chunk).  A tag
+    // without a unit pivot is refused, as by qf_gen_short_basis_tagged; a key of another form is installed as it is.
+    {
+        KeyTag kt;
+        QF_TRY(match_key_tag(ctx, r, true, ctx->dHinvl, kt));
+        if (kt.form == KEY_TAG_SINGULAR)
+            return ctx->fail(QF_ERR_INVALID, "key is [A_bar | H G - A_bar R] with a tag H that is not invertible mod q (no unit pivot)");
+        if (kt.form != KEY_TAGGED) ctx->dHinvl.release();
+        ctx->pert_gadget_key = kt.form != KEY_OTHER;
+        ctx->key_tagged = kt.form == KEY_TAGGED;
+        ctx->tag_ulimbs = limbs_for((double)(ctx->prm.q - 1));
+        ctx->pert_tag = std::move(kt.h);
     }
     if (l) {
         QF_TRY(upload_as_f64(ctx, l, ctx->m, ctx->m, ctx->ld_dim, ctx->dL));
@@ -1840,6 +1937,59 @@ qf_status qf_set_trapdoor_perturbation(qf_ctx* ctx, const int8_t* r, const doubl
     QF_TRY(upload_as_f64(ctx, skg, ctx->k, ctx->k, ctx->k, ctx->dSkGso));
     QF_TRY(setup_pert_i8(ctx));
     ctx->has_pert = true;
+    return QF_OK;
+}
+
+qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out) {
+    if (!ctx) return QF_ERR_INVALID;
+    if (ctx->prm.kind != QF_PSF_PERTURBATION) return ctx->fail(QF_ERR_INVALID, "not a PSFPerturbation context");
+    if (!ctx->has_a || !ctx->has_pert) return ctx->fail(QF_ERR_NO_KEY, "PSFPerturbation: key or trapdoor missing");
+    if (!ctx->pert_gadget_key) return ctx->fail(QF_ERR_INVALID, "the installed key is not [A_bar | H G - A_bar R] for the installed R");
+    CK(cudaSetDevice(ctx->device));
+    const long n = ctx->n, k = ctx->k, mb = ctx->m_bar, m = ctx->m;
+    const uint64_t q = ctx->prm.q;
+    // the new tag H' as MatZq (entries reduced mod q); H'^-1 before anything changes, so that a tag without a unit pivot
+    // leaves the key, its tag and the outputs as they were
+    std::vector<uint64_t> h2((size_t)n * n);
+    bool ident = true;
+    for (long i = 0; i < n; ++i)
+        for (long j = 0; j < n; ++j) {
+            uint64_t v = i == j ? 1 : 0;
+            if (tag) {
+                const int64_t t = tag[i * n + j] % (int64_t)q;
+                v = (uint64_t)(t < 0 ? t + (int64_t)q : t);
+            }
+            h2[(size_t)i * n + j] = v;
+            ident = ident && v == (i == j ? 1u : 0u);
+        }
+    std::vector<int64_t> hinv;
+    if (!ident) {
+        bool ok = false;
+        QF_TRY(tag_inverse(ctx, h2.data(), hinv, &ok));
+        if (!ok) return ctx->fail(QF_ERR_INVALID, "tag is not invertible mod q (no unit pivot)");
+    }
+    // A_2 += (H' - H) G mod q: only the last nk columns of A change, R, sqrt(Sigma_2) and the gadget basis stay.  Until the
+    // device copies are consistent again the context has no key (a CUDA error on the way leaves it so).
+    ctx->has_a = false;
+    ctx->has_pert = false;
+    const std::vector<uint64_t> gpow = gadget_powers(ctx);
+    for (long i = 0; i < n; ++i)
+        for (long j = 0; j < n; ++j) {
+            const uint64_t d = (h2[(size_t)i * n + j] + q - ctx->pert_tag[(size_t)i * n + j]) % q;
+            if (!d) continue;
+            for (long t = 0; t < k; ++t) {
+                int64_t& a = ctx->hA[(size_t)i * m + mb + j * k + t];
+                a = (int64_t)(((u128)(uint64_t)a + mulmod_h(d, gpow[t], q)) % q);
+            }
+        }
+    QF_TRY(upload_a_cols(ctx, mb));
+    if (ident) ctx->dHinvl.release();
+    else QF_TRY(tag_planes(ctx, hinv, ctx->dHinvl));
+    ctx->key_tagged = !ident;
+    ctx->pert_tag = std::move(h2);
+    ctx->has_a = true;
+    ctx->has_pert = true;
+    if (a_out) memcpy(a_out, ctx->hA.data(), (size_t)n * m * sizeof(int64_t));
     return QF_OK;
 }
 
@@ -1976,7 +2126,8 @@ qf_status qf_gen_short_basis_tagged(qf_ctx* ctx, const int8_t* r, const int64_t*
         QF_TRY(tag_inverse(ctx, h.data(), hinv, &ok));
         if (!ok) return ctx->fail(QF_ERR_INVALID, "tag is not invertible mod q (no unit pivot)");
         Dev dHl;
-        QF_TRY(tag_apply(ctx, hinv, dHl, abt));
+        QF_TRY(tag_planes(ctx, hinv, dHl));
+        QF_TRY(tag_abar(ctx, dHl, abt));
     }
     // W = base-b digits of -A_bar' mod q (short_basis_classical.rs:105-110), stored transposed for the device:
     // Wt[c][j k + t] = digit t of (q - A_bar'[j][c]) mod q

@@ -278,11 +278,19 @@ class PSFPerturbation(_PSFBase):
     def randomized_nearest_plane_gadget(self, a, td, v, seed=None) -> np.ndarray:
         return self.randomized_nearest_plane_gadget_batch(a, td, np.asarray(v, dtype=np.int64).reshape(1, self.n), seed)[0]
 
-    def trap_gen(self, seed=None, full_gadget_basis: bool = None, dense_sqrt_sigma_2: bool = None):
+    def trap_gen(self, seed=None, full_gadget_basis: bool = None, dense_sqrt_sigma_2: bool = None, tag=None):
         """mp_perturbation.rs:221-244.  dense_sqrt_sigma_2=False leaves the second trapdoor component None: the
         backend then uses its block-structured square root of the default Sigma_2 (same law, ~4x less work per
-        target); default: dense (the reference's m x m matrix) up to m = 2048, structured above."""
+        target); default: dense (the reference's m x m matrix) up to m = 2048, structured above.
+        tag: an n x n matrix H invertible mod q (gadget_classical.rs:56-68 with a tag): A = [A_bar | H G - A_bar R] from
+        the same device-sampled A_bar and R (qf_trap_gen_from).  The trapdoor does not depend on H; samp_p recognises the
+        tag when the trapdoor is installed.  None: H = I."""
         a, r = _trap_gen_classical(self, seed)
+        if tag is not None:
+            tg = self._tag_words(tag)
+            ab = np.ascontiguousarray(a[:, : self.gp.m_bar])
+            a = np.empty((self.n, self.m), dtype=np.int64)
+            self.ctx.call("qf_trap_gen_from", _ffi.ptr(ab), _ffi.ptr(r), _ffi.ptr(tg), _ffi.ptr(a))
         if dense_sqrt_sigma_2 is None:
             dense_sqrt_sigma_2 = self.m <= 2048
         sqrt_sigma_2 = self.compute_sqrt_sigma_2(r) if dense_sqrt_sigma_2 else None
@@ -298,6 +306,25 @@ class PSFPerturbation(_PSFBase):
             sb, sg = blk, gblk
         self._a_id = a
         return a, (r, sqrt_sigma_2, (sb, sg))
+
+    def _tag_words(self, tag):
+        tg = np.array(np.asarray(tag, dtype=object) % self.gp.q, dtype=np.int64)
+        assert tg.shape == (self.n, self.n)
+        return tg
+
+    def set_tag(self, a, td, tag) -> np.ndarray:
+        """Tag switch without a new trapdoor install: for a key a = [A_bar | H G - A_bar R] and its trapdoor td (R, ...),
+        returns a_new = [A_bar | H' G - A_bar R] for tag = H' (n x n, entries taken mod q; None: H' = I), equal to
+        gen_trapdoor(A_bar, R, H'), and records it as the installed key; R, sqrt(Sigma_2) and the gadget basis stay on the
+        device (qf_set_tag).  Raises QfError (QF_ERR_INVALID) when a is not such a key for td's R or when H' has no unit
+        pivot; then the installed key and tag stay as they were."""
+        self._install_a(a)
+        self._install_td(a, td)
+        tg = None if tag is None else self._tag_words(tag)
+        a_new = np.empty((self.n, self.m), dtype=np.int64)
+        self.ctx.call("qf_set_tag", _ffi.ptr(tg), _ffi.ptr(a_new))
+        self._a_id = a_new
+        return a_new
 
 
 def _gso(psf, basis) -> np.ndarray:
