@@ -115,6 +115,16 @@ qf_status qf_set_trapdoor_perturbation(qf_ctx* ctx, const int8_t* r, const doubl
  * G-trapdoor for the installed R, and QF_ERR_INVALID for a tag H' without a unit pivot (the key and its tag then stay as
  * they were). */
 qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out);
+/* Tag table for samp_p with a tag per target (PSFPerturbation): one trapdoor R serves the keys
+ * A_t = [A_bar | H_t G - A_bar R] of many tags in one batch (IBE key extraction, per-message tags).  tags: ntags x n x n
+ * (host), entries taken mod q (negatives allowed), relative to the installed (A_bar, R); the installed key may itself be
+ * tagged (any H_0).  H_t^-1 is computed on the device (Gauss-Jordan with unit pivots, as qf_set_tag).  QF_ERR_INVALID on a
+ * context of another kind, for ntags < 1 or tags == NULL, when the installed key was not recognised as a G-trapdoor for
+ * the installed R, and when a tag has no unit pivot (qf_last_error names its index; the previous table then stays);
+ * QF_ERR_NO_KEY without key and trapdoor.  The table is dropped when a key or trapdoor is installed (qf_set_a,
+ * qf_trap_gen, qf_trap_gen_from, qf_set_trapdoor_perturbation) and kept by qf_set_tag.  Device memory: ntags n^2 words of
+ * 4 bytes (q <= 2^32) or 8 bytes. */
+qf_status qf_set_tag_table(qf_ctx* ctx, const int64_t* tags, int64_t ntags);
 /* gen_short_basis_for_trapdoor with tag = I (short_basis_classical.rs:54-110): the short basis
  * S_A = [[I,R],[0,I]] [[0,I],[S',W]] = [[R S', I + R W],[S', W]] of Lambda^perp(A) for the installed A and the
  * trapdoor R (m_bar x nk); W = digits of -A[:, :m_bar], S' column-reversed iff base^k = q.  The m_bar x nk x m_bar
@@ -181,6 +191,16 @@ qf_status qf_samp_p(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed,
                     int32_t* e_out);
 qf_status qf_samp_p_dev(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed, uint64_t first_index,
                         int32_t* e_out);
+/* samp_p with a tag per target: e[b] with A_t e[b] = u[b] mod q for t = tag_idx[b], the key of tag t of the installed tag
+ * table (qf_set_tag_table).  For the same seed and first_index, row b is bit-identical to what qf_set_tag(H_t) followed by
+ * qf_samp_p gives for that row.  qf_samp_p_tagged takes host pointers; targets are range-checked as in qf_samp_p and the
+ * tag indices are checked on the host before any launch (QF_ERR_INVALID outside [0, ntags)).  qf_samp_p_tagged_dev takes
+ * device pointers and is asynchronous: an index outside the table is not read, its row is unspecified and the next
+ * qf_synchronize returns QF_ERR_INVALID.  QF_ERR_NO_KEY without a tag table. */
+qf_status qf_samp_p_tagged(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, uint64_t seed,
+                           uint64_t first_index, int32_t* e_out);
+qf_status qf_samp_p_tagged_dev(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, uint64_t seed,
+                               uint64_t first_index, int32_t* e_out);
 /* Narrow Domain form: the same preimages as int16 -- |e_i| <= 6 s r is far below 2^15 for the parameter sets of the
  * reference (C2: 6 s = 8568; C3: 3135), so the device->host copy, which bounds the host-buffer path, is halved.  An entry
  * that does not fit is reported as QF_ERR_NUMERIC (then use qf_samp_p).  Targets outside [0,q) are detected on the device

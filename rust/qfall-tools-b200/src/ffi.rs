@@ -48,6 +48,7 @@ extern "C" {
     pub fn qf_set_a(ctx: *mut qf_ctx, a: *const i64) -> i32;
     pub fn qf_set_trapdoor_perturbation(ctx: *mut qf_ctx, r: *const i8, sqrt_sigma_2: *const f64, s_block: *const i64, s_block_gso: *const f64) -> i32;
     pub fn qf_set_tag(ctx: *mut qf_ctx, tag: *const i64, a_out: *mut i64) -> i32;
+    pub fn qf_set_tag_table(ctx: *mut qf_ctx, tags: *const i64, ntags: i64) -> i32;
     pub fn qf_gen_short_basis(ctx: *mut qf_ctx, r: *const i8, s_out: *mut i64) -> i32;
     pub fn qf_gen_short_basis_tagged(ctx: *mut qf_ctx, r: *const i8, tag: *const i64, s_out: *mut i64) -> i32;
     pub fn qf_compute_sqrt_sigma_2(ctx: *mut qf_ctx, r: *const i8, sigma: *const f64, sqrt_sigma_2_out: *mut f64) -> i32;
@@ -68,6 +69,8 @@ extern "C" {
     pub fn qf_samp_p(ctx: *mut qf_ctx, u: *const i64, batch: i64, seed: u64, first_index: u64, e_out: *mut i32) -> i32;
     pub fn qf_samp_p_dev(ctx: *mut qf_ctx, u: *const i64, batch: i64, seed: u64, first_index: u64, e_out: *mut i32) -> i32;
 
+    pub fn qf_samp_p_tagged(ctx: *mut qf_ctx, u: *const i64, tag_idx: *const i32, batch: i64, seed: u64, first_index: u64, e_out: *mut i32) -> i32;
+    pub fn qf_samp_p_tagged_dev(ctx: *mut qf_ctx, u: *const i64, tag_idx: *const i32, batch: i64, seed: u64, first_index: u64, e_out: *mut i32) -> i32;
     pub fn qf_samp_p_i16(ctx: *mut qf_ctx, u: *const i64, batch: i64, seed: u64, first_index: u64, e_out: *mut i16) -> i32;
     pub fn qf_f_a_i16(ctx: *mut qf_ctx, sigma: *const i16, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
     pub fn qf_narrow_i32_i16_dev(input: *const i32, out: *mut i16, count: usize, overflow: *mut i32, cuda_stream: *mut c_void) -> i32;

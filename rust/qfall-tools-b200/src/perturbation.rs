@@ -20,6 +20,8 @@ pub struct PSFPerturbationB200 {
     /// every component takes part in the comparison: the same R with another covariance (compute_sqrt_sigma_2 with a
     /// custom Sigma, mp_perturbation.rs:94-104) or another gadget basis is a different trapdoor
     installed_r: RefCell<Option<(Vec<i64>, Vec<u64>, Vec<i64>, Vec<u64>)>>,
+    /// number of tags in the table on the device (qf_set_tag_table); the device drops it with every key or trapdoor install
+    installed_tags: RefCell<Option<usize>>,
     seed: RefCell<u64>,
 }
 
@@ -45,6 +47,7 @@ impl PSFPerturbationB200 {
             ctx: Context::new(&params, device)?,
             installed_a: RefCell::new(None),
             installed_r: RefCell::new(None),
+            installed_tags: RefCell::new(None),
             seed: RefCell::new(seed),
         })
     }
@@ -73,6 +76,7 @@ impl PSFPerturbationB200 {
         self.ctx.check(unsafe { qf_set_a(self.ctx.raw, aw.as_ptr()) }, "qf_set_a");
         *self.installed_a.borrow_mut() = Some(aw);
         *self.installed_r.borrow_mut() = None;
+        *self.installed_tags.borrow_mut() = None;
     }
     /// Trapdoor `(R, sqrt(Sigma_2), (S, S~))` (mp_perturbation.rs:195).  The gadget basis must be `I_n (x) S_k`
     /// (what `short_basis_gadget` returns, gadget_classical.rs:273-286): only its first k x k block crosses the boundary.
@@ -110,6 +114,7 @@ impl PSFPerturbationB200 {
         };
         self.ctx.check(st, "qf_set_trapdoor_perturbation");
         *self.installed_r.borrow_mut() = Some(key);
+        *self.installed_tags.borrow_mut() = None;
     }
 
     /// Tag switch for a key `a = [A_bar | H G - A_bar R]` (gen_trapdoor with a tag, gadget_classical.rs:56-68) and its
@@ -134,6 +139,49 @@ impl PSFPerturbationB200 {
         *self.installed_a.borrow_mut() = Some(aw);
         out
     }
+
+    /// Installs the tag table for samp_p with a tag per target: `tags` (T matrices, n x n each, relative to the key `a` =
+    /// [A_bar | H_0 G - A_bar R] of any tag H_0 and its trapdoor `td`).  H_t^-1 is computed on the device
+    /// (qf_set_tag_table).  The table stays installed until a key or trapdoor is installed (install_a / install_td of
+    /// another `a` or `td`, trap_gen); `set_tag` keeps it.  Panics when a tag has no unit pivot (the reference panics in
+    /// `MatZq::inverse`).
+    pub fn set_tag_table(&self, a: &MatZq, td: &(MatZ, MatQ, (MatZ, MatQ)), tags: &[MatZq]) {
+        let n = self.n();
+        assert!(!tags.is_empty(), "at least one tag");
+        self.install_a(a);
+        self.install_td(td);
+        let mut tw = Vec::with_capacity(tags.len() * n * n);
+        for tag in tags {
+            assert_eq!((tag.get_num_rows(), tag.get_num_columns()), (n as i64, n as i64), "tag must be n x n");
+            tw.extend(matzq_to_words(tag));
+        }
+        self.ctx.check(unsafe { qf_set_tag_table(self.ctx.raw, tw.as_ptr(), tags.len() as i64) }, "qf_set_tag_table");
+        *self.installed_tags.borrow_mut() = Some(tags.len());
+    }
+
+    /// samp_p with a tag per target, against the table of `set_tag_table`: `us[b]` is sampled under
+    /// `[A_bar | H_t G - A_bar R]` with `H_t = tags[tag_of[b]]`, in one batch.  Row b equals what `set_tag(H_t)` followed by
+    /// `samp_p_batch` gives for it with the same seed (qf_samp_p_tagged).  The tags do not cross the boundary again, so
+    /// repeated batches cost only their targets.  Panics when no table is installed for this key and trapdoor (a key or
+    /// trapdoor install drops it: call `set_tag_table` again) or an index is out of range.
+    pub fn samp_p_tagged_batch(&self, a: &MatZq, td: &(MatZ, MatQ, (MatZ, MatQ)), us: &[MatZq], tag_of: &[usize],
+                               seed: u64) -> Vec<MatZ> {
+        let (n, m) = (self.n(), self.m());
+        assert_eq!(us.len(), tag_of.len(), "one tag index per target");
+        self.install_a(a);
+        self.install_td(td);
+        let ntags = (*self.installed_tags.borrow()).expect("no tag table installed for this key and trapdoor (set_tag_table)");
+        let mut uw = Vec::with_capacity(us.len() * n);
+        for u in us {
+            assert!(u.is_column_vector() && u.get_num_rows() as usize == n, "target must be an n x 1 vector");
+            uw.extend(matzq_to_words(u));
+        }
+        let idx: Vec<i32> = tag_of.iter().map(|t| { assert!(*t < ntags, "tag index out of range"); *t as i32 }).collect();
+        let mut e = vec![0i32; us.len() * m];
+        let st = unsafe { qf_samp_p_tagged(self.ctx.raw, uw.as_ptr(), idx.as_ptr(), us.len() as i64, seed, 0, e.as_mut_ptr()) };
+        self.ctx.check(st, "qf_samp_p_tagged");
+        e.chunks(m).map(column_from_i32).collect()
+    }
 }
 
 impl PSF for PSFPerturbationB200 {
@@ -153,6 +201,7 @@ impl PSF for PSFPerturbationB200 {
         // qf_trap_gen installed a new key (and thereby dropped the device's trapdoor): forget the cached one
         *self.installed_a.borrow_mut() = None;
         *self.installed_r.borrow_mut() = None;
+        *self.installed_tags.borrow_mut() = None;
         let mut l = vec![0f64; m * m];
         let st = unsafe { qf_compute_sqrt_sigma_2(self.ctx.raw, r.as_ptr(), std::ptr::null(), l.as_mut_ptr()) };
         self.ctx.check(st, "qf_compute_sqrt_sigma_2"); // QF_ERR_INVALID = Sigma_2 not positive definite (the reference panics)

@@ -47,6 +47,7 @@ SIGNATURES = {
     "qf_set_a": (_i32, [_vp, _vp]),
     "qf_set_trapdoor_perturbation": (_i32, [_vp, _vp, _vp, _vp, _vp]),
     "qf_set_tag": (_i32, [_vp, _vp, _vp]),
+    "qf_set_tag_table": (_i32, [_vp, _vp, _i64]),
     "qf_compute_sqrt_sigma_2": (_i32, [_vp, _vp, _vp, _vp]),
     "qf_gen_short_basis": (_i32, [_vp, _vp, _vp]),
     "qf_gen_short_basis_tagged": (_i32, [_vp, _vp, _vp, _vp]),
@@ -65,6 +66,8 @@ SIGNATURES = {
     "qf_samp_p": (_i32, [_vp, _vp, _i64, _u64, _u64, _vp]),
     "qf_samp_p_dev": (_i32, [_vp, _vp, _i64, _u64, _u64, _vp]),
     "qf_samp_p_i16": (_i32, [_vp, _vp, _i64, _u64, _u64, _vp]),
+    "qf_samp_p_tagged": (_i32, [_vp, _vp, _vp, _i64, _u64, _u64, _vp]),
+    "qf_samp_p_tagged_dev": (_i32, [_vp, _vp, _vp, _i64, _u64, _u64, _vp]),
     "qf_f_a_i16": (_i32, [_vp, _vp, _i64, _vp, _vp]),
     "qf_narrow_i32_i16_dev": (_i32, [_vp, _vp, _sz, _vp, _vp]),
     "qf_randomized_nearest_plane_gadget": (_i32, [_vp, _vp, _i64, _u64, _u64, _vp]),

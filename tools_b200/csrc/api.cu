@@ -186,6 +186,13 @@ struct qf_ctx {
     int tag_ulimbs = 0;
     long ldk_n = 0;
     Dev dHinvl, dAbpl, dTagU, dTagUl, dTagTmp;
+    // Tag table of PSFPerturbation (qf_set_tag_table): H_t^-1 mod q for tag_count tags, each n x n column-major in words
+    // of tag_word bytes (4 when q <= 2^32), relative to the installed (A_bar, R) and dropped with the key or trapdoor.
+    // dTagH0: the installed key's tag H_0 in the same layout while the key is tagged; dTagGpow: base^s mod q, s < k;
+    // io_t: tag indices of the host path's chunks (two slots, as io_b / io_b2).
+    int64_t tag_count = 0;
+    int tag_word = 8;
+    Dev dTagTab, dTagH0, dTagGpow, io_t[2];
     // Defaults from the error budget of DESIGN 4.2, checked at the full C2 key (scripts/ab_c2_precision.py, profiles/README_r2.md):
     // four digits everywhere; the lowest digit sum is dropped where the operand has three digits (z2), not for the
     // two-digit z1 (dropping it there moves 14 % of the preimages, keeping it 0.3 %).
@@ -277,6 +284,7 @@ qf_status check_flag(qf_ctx* ctx) {
         CK(cudaMemsetAsync(ctx->dFlag.p, 0, sizeof(int), ctx->stream));
         if (h & 32) return ctx->fail(QF_ERR_INVALID, "target entry outside [0,q)");
         if (h & 64) return ctx->fail(QF_ERR_NUMERIC, "a Domain entry does not fit int16: use the int32 entry point");
+        if (h & QF_FLAG_TAG_INDEX) return ctx->fail(QF_ERR_INVALID, "tag index outside the installed tag table");
         char buf[128];
         snprintf(buf, sizeof buf, "internal range check tripped (flag=%d): a value left its exact-integer range", h);
         return ctx->fail(QF_ERR_NUMERIC, buf);
@@ -594,7 +602,9 @@ qf_status ring_f_a_chunk(qf_ctx* ctx, const int32_t* dSigma, int Bc, int64_t* dU
 // ---------------------------------------------------------------------------
 qf_status pert_lg_i8(qf_ctx* ctx, const int8_t* gp, long gplane, int Bc, double* X2, long ldx, bool tri);
 
-qf_status samp_p_pert_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t seed, uint64_t first, int32_t* dE) {
+// dTidx (optional, device): the tag index of every target of the chunk in the installed tag table (qf_samp_p_tagged)
+qf_status samp_p_pert_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t seed, uint64_t first, int32_t* dE,
+                            const int32_t* dTidx = nullptr) {
     const long ldm = ctx->ld_dim, ldn = ctx->ld_n, ldnk = ctx->ld_nk;
     const long C = ctx->chunk;
     CK(ctx->w[0].ensure((size_t)C * ldm * 8));   // g, later reused
@@ -673,7 +683,18 @@ qf_status samp_p_pert_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t s
     }
     // tagged key A = [A_bar | H G - A_bar R]: A [R; I] = H G, so z solves G z = v' = H^-1 v
     const int64_t* Vg = V;
-    if (ctx->key_tagged) QF_TRY(tag_targets(ctx, V, Bc, &Vg));
+    if (dTidx) {
+        // per-target tag H_t: A_t = A + [0 | (H_t - H_0) G], so v'_t = H_t^-1 (u - A_t p) = H_t^-1 (v + H_0 y) - y with
+        // y = G p_bot (DESIGN 4.4): the same v' as after qf_set_tag(H_t)
+        CK(ctx->dTagU.ensure((size_t)C * ctx->n * 8));
+        LAUNCH(qf_launch_tag_syndrome(V, ctx->n, P, ldm, (int)ctx->m_bar, dTidx, (int)ctx->tag_count, ctx->dTagTab.p,
+                                      ctx->key_tagged ? ctx->dTagH0.p : nullptr, ctx->tag_word, ctx->dTagGpow.as<uint64_t>(),
+                                      ctx->prm.q, (int)ctx->n, (int)ctx->k, Bc, ctx->dTagU.as<int64_t>(), ctx->n,
+                                      ctx->dFlag.as<int>(), ctx->stream));
+        Vg = ctx->dTagU.as<int64_t>();
+    } else if (ctx->key_tagged) {
+        QF_TRY(tag_targets(ctx, V, Bc, &Vg));
+    }
     // z <- D_{Lambda_v^perp(G), r sqrt(b^2+1)}   (:321-326 -> :173-191)
     const double s_g = ctx->prm.r * std::sqrt((double)(ctx->prm.base * ctx->prm.base + 1));
     LAUNCH(qf_launch_gadget_sample(Vg, ctx->n, Z, ldnk, Bc, (int)ctx->n, (int)ctx->k, (int)ctx->prm.base, ctx->prm.q,
@@ -1691,6 +1712,7 @@ qf_status install_a(qf_ctx* ctx, const int64_t* a) {
     ctx->has_a = false; ctx->has_np = false; ctx->has_pert = false;
     ctx->key_tagged = false; ctx->pert_gadget_key = false;
     ctx->dHinvl.release(); ctx->dAbpl.release();
+    ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release();
     const long n = ctx->n, m = ctx->m;
     for (long i = 0; i < n * m; ++i)
         if (a[i] < 0 || (uint64_t)a[i] >= ctx->prm.q) return ctx->fail(QF_ERR_INVALID, "A entry outside [0,q)");
@@ -1732,6 +1754,28 @@ qf_status upload_a_cols(qf_ctx* ctx, long c0) {
                              (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
     }
+    return QF_OK;
+}
+
+// the installed key's tag H_0 into dTagH0 (column-major, tag_word words) for the per-target tag kernel; none for H_0 = I
+qf_status upload_tag_h0(qf_ctx* ctx) {
+    if (!ctx->key_tagged) {
+        ctx->dTagH0.release();
+        return QF_OK;
+    }
+    const long n = ctx->n;
+    std::vector<uint64_t> h((size_t)n * n);
+    for (long i = 0; i < n; ++i)
+        for (long j = 0; j < n; ++j) h[(size_t)j * n + i] = ctx->pert_tag[(size_t)i * n + j];
+    std::vector<uint32_t> h32;
+    const void* src = h.data();
+    if (ctx->tag_word == 4) {
+        h32.assign(h.begin(), h.end());
+        src = h32.data();
+    }
+    CK(ctx->dTagH0.ensure((size_t)n * n * ctx->tag_word));
+    CK(cudaMemcpyAsync(ctx->dTagH0.p, src, (size_t)n * n * ctx->tag_word, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
     return QF_OK;
 }
 
@@ -1900,6 +1944,7 @@ qf_status qf_set_trapdoor_perturbation(qf_ctx* ctx, const int8_t* r, const doubl
     if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "install A first (qf_set_a / qf_trap_gen)");
     ctx->has_pert = false;
     ctx->key_tagged = false; ctx->pert_gadget_key = false;
+    ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release();
     CK(cudaSetDevice(ctx->device));
     QF_TRY(upload_as_f64(ctx, r, ctx->m_bar, ctx->nk, ctx->ld_nk, ctx->dR));
     {
@@ -1987,9 +2032,62 @@ qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out) {
     else QF_TRY(tag_planes(ctx, hinv, ctx->dHinvl));
     ctx->key_tagged = !ident;
     ctx->pert_tag = std::move(h2);
+    if (ctx->tag_count) QF_TRY(upload_tag_h0(ctx));  // the tag table stays: it is relative to (A_bar, R)
     ctx->has_a = true;
     ctx->has_pert = true;
     if (a_out) memcpy(a_out, ctx->hA.data(), (size_t)n * m * sizeof(int64_t));
+    return QF_OK;
+}
+
+constexpr int64_t TAG_SLICE = 256;  // tags inverted per launch: 2 CTAs of 1024 threads per SM, one wave
+
+// H_t^-1 for every tag on the device: [H_t | I] built from the caller's words (reduced mod q there), Gauss-Jordan with unit
+// pivots one CTA per tag, packed column-major.  Slices of at most TAG_SLICE tags and 1 GB bound the scratch ([H | I] is
+// 16 n^2 bytes per tag, 4 MB at n = 512).  The new table replaces the old one only when every tag has been inverted.
+qf_status qf_set_tag_table(qf_ctx* ctx, const int64_t* tags, int64_t ntags) {
+    if (!ctx) return QF_ERR_INVALID;
+    if (ctx->prm.kind != QF_PSF_PERTURBATION) return ctx->fail(QF_ERR_INVALID, "not a PSFPerturbation context");
+    if (!tags || ntags < 1) return ctx->fail(QF_ERR_INVALID, "tag table: at least one tag needed");
+    if (!ctx->has_a || !ctx->has_pert) return ctx->fail(QF_ERR_NO_KEY, "PSFPerturbation: key or trapdoor missing");
+    if (!ctx->pert_gadget_key) return ctx->fail(QF_ERR_INVALID, "the installed key is not [A_bar | H G - A_bar R] for the installed R");
+    const long n = ctx->n;
+    if (ctx->k > 64 || 16 * n > 227 * 1024) return ctx->fail(QF_ERR_UNSUPPORTED, "tag table: needs k <= 64 and n <= 14528");
+    if (ntags > INT32_MAX) return ctx->fail(QF_ERR_INVALID, "tag table: more than 2^31 - 1 tags");
+    CK(cudaSetDevice(ctx->device));
+    const uint64_t q = ctx->prm.q;
+    const int word = q <= (1ull << 32) ? 4 : 8;
+    const size_t nn = (size_t)n * n;
+    const int64_t slice = std::max<int64_t>(1, std::min<int64_t>({ntags, TAG_SLICE, (int64_t)((1ull << 30) / (16 * nn))}));
+    Dev tab, dTags, dM, dF, dFail;
+    CK(tab.ensure((size_t)ntags * nn * word));
+    CK(dTags.ensure((size_t)slice * nn * 8));
+    CK(dM.ensure((size_t)slice * nn * 16));
+    CK(dF.ensure((size_t)slice * n * 8));
+    CK(dFail.ensure((size_t)slice * sizeof(int)));
+    std::vector<int> fail((size_t)slice);
+    for (int64_t t0 = 0; t0 < ntags; t0 += slice) {
+        const int cnt = (int)std::min<int64_t>(slice, ntags - t0);
+        CK(cudaMemcpyAsync(dTags.p, tags + (size_t)t0 * nn, (size_t)cnt * nn * 8, cudaMemcpyHostToDevice, ctx->stream));
+        LAUNCH(qf_launch_tag_build(dTags.as<int64_t>(), cnt, (int)n, q, dM.as<uint64_t>(), ctx->stream));
+        LAUNCH(qf_launch_mat_inverse_mod_batched(dM.as<uint64_t>(), dF.as<uint64_t>(), (int)n, q, dFail.as<int>(), cnt, ctx->stream));
+        LAUNCH(qf_launch_tag_pack(dM.as<uint64_t>(), cnt, (int)n, word, tab.as<char>() + (size_t)t0 * nn * word, ctx->stream));
+        CK(cudaMemcpyAsync(fail.data(), dFail.p, (size_t)cnt * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        for (int i = 0; i < cnt; ++i)
+            if (fail[i]) {
+                char buf[128];
+                snprintf(buf, sizeof buf, "tag %lld is not invertible mod q (no unit pivot)", (long long)(t0 + i));
+                return ctx->fail(QF_ERR_INVALID, buf);
+            }
+    }
+    const std::vector<uint64_t> gpow = gadget_powers(ctx);
+    CK(ctx->dTagGpow.ensure(gpow.size() * 8));
+    CK(cudaMemcpyAsync(ctx->dTagGpow.p, gpow.data(), gpow.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    ctx->tag_word = word;
+    QF_TRY(upload_tag_h0(ctx));
+    std::swap(ctx->dTagTab.p, tab.p);
+    std::swap(ctx->dTagTab.cap, tab.cap);
+    ctx->tag_count = ntags;
     return QF_OK;
 }
 
@@ -2765,7 +2863,9 @@ qf_status qf_samp_p_dev(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t s
 }
 
 // host-buffer samp_p; i16: results leave as int16 (half the device->host bytes)
-static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed, uint64_t first, void* e_out, bool i16) {
+// tidx (optional, host): tag index of every target in the installed tag table (qf_samp_p_tagged), copied with the targets
+static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed, uint64_t first, void* e_out, bool i16,
+                             const int32_t* tidx = nullptr) {
     if (!ctx || batch < 0 || (batch > 0 && (!u || !e_out))) return QF_ERR_INVALID;
     if (batch == 0) return QF_OK;
     CK(cudaSetDevice(ctx->device));
@@ -2774,6 +2874,7 @@ static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint6
     const size_t esz = i16 ? 2 : 4;
     CK(ctx->io_b.ensure((size_t)C * ctx->n * 8));
     CK(ctx->io_a.ensure((size_t)C * ctx->dim * 4));
+    if (tidx) CK(ctx->io_t[0].ensure((size_t)C * 4));
     if (i16) CK(ctx->io_h[0].ensure((size_t)C * ctx->dim * 2));
     // Both directions of the host traffic run on a second stream: the device->host copy of chunk i and the host->device
     // copy of the targets of chunk i+1 overlap the computation (two result buffers, two target buffers, events in both
@@ -2783,6 +2884,7 @@ static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint6
         if (i16) CK(ctx->io_h[1].ensure((size_t)C * ctx->dim * 2));
         else CK(ctx->io_a2.ensure((size_t)C * ctx->dim * 4));
         CK(ctx->io_b2.ensure((size_t)C * ctx->n * 8));
+        if (tidx) CK(ctx->io_t[1].ensure((size_t)C * 4));
         if (!ctx->copy_stream) {
             CK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
             for (int i = 0; i < 2; ++i) {
@@ -2797,9 +2899,11 @@ static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint6
     const int64_t nch = std::max<int64_t>(1, (batch + C - 1) / C);
     const int64_t per = std::min<int64_t>(C, ((batch + nch - 1) / nch + 127) / 128 * 128);
     auto u_buf = [&](int64_t i) { return (overlap && (i & 1)) ? ctx->io_b2.as<int64_t>() : ctx->io_b.as<int64_t>(); };
+    auto t_buf = [&](int64_t i) { return ctx->io_t[(overlap && (i & 1)) ? 1 : 0].as<int32_t>(); };
     auto copy_u = [&](int64_t i, cudaStream_t st) -> qf_status {
         const int64_t b0 = i * per, Bc = std::min<int64_t>(per, batch - b0);
         CK(cudaMemcpyAsync(u_buf(i), u + b0 * ctx->n, (size_t)Bc * ctx->n * 8, cudaMemcpyHostToDevice, st));
+        if (tidx) CK(cudaMemcpyAsync(t_buf(i), tidx + b0, (size_t)Bc * 4, cudaMemcpyHostToDevice, st));
         return QF_OK;
     };
     if (overlap) {
@@ -2821,14 +2925,15 @@ static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint6
                 CK(cudaEventRecord(ctx->ev_u_in[slot ^ 1], ctx->copy_stream));
             }
         } else {
-            CK(cudaMemcpyAsync(u_buf(idx), u + b0 * ctx->n, (size_t)Bc * ctx->n * 8, cudaMemcpyHostToDevice, ctx->stream));
+            QF_TRY(copy_u(idx, ctx->stream));
         }
         const int64_t* du = u_buf(idx);
         // the targets must be residues in [0, q): checked on the device (a host loop over batch x n values would sit in
         // front of every call), reported by check_flag as QF_ERR_INVALID
         LAUNCH(qf_launch_range_check_i64(du, (size_t)Bc * ctx->n, ctx->prm.q, ctx->dFlag.as<int>(), ctx->stream));
-        QF_TRY(ctx->prm.kind == QF_PSF_PERTURBATION ? samp_p_pert_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres)
-                                                    : samp_p_np_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres));
+        QF_TRY(ctx->prm.kind == QF_PSF_PERTURBATION
+                   ? samp_p_pert_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres, tidx ? t_buf(idx) : nullptr)
+                   : samp_p_np_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres));
         if (overlap) CK(cudaEventRecord(ctx->ev_u_used[slot], ctx->stream));
         const void* src = dres;
         if (i16) {
@@ -2858,6 +2963,39 @@ qf_status qf_samp_p(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed,
 }
 qf_status qf_samp_p_i16(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed, uint64_t first, int16_t* e_out) {
     return samp_p_host(ctx, u, batch, seed, first, e_out, true);
+}
+
+// ---- samp_p with a tag per target (PSFPerturbation, installed tag table) --------------------------------------------
+static qf_status samp_p_tagged_ready(qf_ctx* ctx) {
+    if (ctx->prm.kind != QF_PSF_PERTURBATION) return ctx->fail(QF_ERR_INVALID, "not a PSFPerturbation context");
+    QF_TRY(samp_p_ready(ctx));
+    if (!ctx->tag_count) return ctx->fail(QF_ERR_NO_KEY, "no tag table installed (qf_set_tag_table)");
+    return QF_OK;
+}
+
+qf_status qf_samp_p_tagged(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, uint64_t seed, uint64_t first,
+                           int32_t* e_out) {
+    if (!ctx || batch < 0 || (batch > 0 && (!u || !tag_idx || !e_out))) return QF_ERR_INVALID;
+    if (batch == 0) return QF_OK;
+    QF_TRY(samp_p_tagged_ready(ctx));
+    for (int64_t b = 0; b < batch; ++b)
+        if (tag_idx[b] < 0 || tag_idx[b] >= ctx->tag_count) {
+            char buf[128];
+            snprintf(buf, sizeof buf, "tag index outside the installed tag table (target %lld: %d)", (long long)b, (int)tag_idx[b]);
+            return ctx->fail(QF_ERR_INVALID, buf);
+        }
+    return samp_p_host(ctx, u, batch, seed, first, e_out, false, tag_idx);
+}
+
+qf_status qf_samp_p_tagged_dev(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, uint64_t seed,
+                               uint64_t first, int32_t* e_out) {
+    if (!ctx || batch < 0 || (batch > 0 && (!u || !tag_idx || !e_out))) return QF_ERR_INVALID;
+    if (batch == 0) return QF_OK;
+    CK(cudaSetDevice(ctx->device));
+    QF_TRY(samp_p_tagged_ready(ctx));
+    return for_chunks(ctx, batch, [&](int64_t b0, int Bc) -> qf_status {
+        return samp_p_pert_chunk(ctx, u + b0 * ctx->n, Bc, seed, first + (uint64_t)b0, e_out + b0 * ctx->dim, tag_idx + b0);
+    });
 }
 
 // int16 Domain input: widened on the device (the H2D copy, which dominates the host path, is halved)

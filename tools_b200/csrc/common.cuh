@@ -26,6 +26,8 @@
 #define QF_STREAM_SAMPLE_Z 9u
 // bits of the per-context numeric flag (qf_synchronize / qf_samp_p report QF_ERR_NUMERIC when any is set)
 #define QF_FLAG_DGAUSS_BAILOUT 16
+// a tag index of qf_samp_p_tagged_dev outside the installed tag table (reported by check_flag as QF_ERR_INVALID)
+#define QF_FLAG_TAG_INDEX 128
 
 struct Philox {
     uint32_t k0, k1;

@@ -880,3 +880,163 @@ cudaError_t qf_launch_split_i64_limbs(const int64_t* in, long ldin, int8_t* plan
                                                                                          L, flag);
     return cudaGetLastError();
 }
+
+// ---- per-target tag (qf_samp_p_tagged): v'_b = H_t^-1 (v_b + H_0 y_b) - y_b mod q with y_b = G p_bot_b, t = tidx[b] ----------
+// One CTA per target; thread i owns rows i, i + blockDim, ... .  The tables hold each n x n matrix column-major (word
+// [j][i] = M[i][j]), so at a fixed column the threads of a warp read consecutive words; y and w live in shared memory.
+// Exact for every q < 2^62 and n:
+//  - W = uint32_t (q <= 2^32): the shared vectors are held as 16-bit halves, so a table word times a half is < 2^48 and a
+//    row of n <= 2^14 such products stays below 2^62 in a plain 64-bit register (two IMAD.WIDE per entry, no carries);
+//    one Barrett step per half reduces the sums (mod_halves needs a0, a1 < 2^62).
+//  - W = uint64_t: a product of residues is < 2^124 and a row sum runs in three words (192 bits) before one reduction,
+//    so (q - 1)^2 n >= 2^128 cannot wrap.
+namespace {
+struct ModAcc {
+    unsigned long long lo = 0, mid = 0;
+    unsigned int hi = 0;
+    __device__ __forceinline__ void mac(uint64_t a, uint64_t b) {
+        const unsigned long long pl = a * b, ph = __umul64hi(a, b);
+        asm("add.cc.u64 %0, %0, %3;\n\taddc.cc.u64 %1, %1, %4;\n\taddc.u32 %2, %2, 0;" : "+l"(lo), "+l"(mid), "+r"(hi) : "l"(pl), "l"(ph));
+    }
+    __device__ __forceinline__ uint64_t reduce(uint64_t q) const {
+        typedef unsigned __int128 u128;
+        const uint64_t top = (uint64_t)((((u128)hi) << 64 | mid) % q);
+        return (uint64_t)((((u128)top) << 64 | lo) % q);
+    }
+};
+
+// (a1 2^16 + a0) mod q for a0, a1 < 2^62, q <= 2^32 (magic = floor(2^64 / q))
+__device__ __forceinline__ uint64_t mod_halves(uint64_t a0, uint64_t a1, uint64_t q, uint64_t magic) {
+    const uint64_t h = mod_i64_barrett((long long)a1, q, magic);
+    return mod_i64_barrett((long long)(a0 + (h << 16)), q, magic);
+}
+__device__ __forceinline__ uint2 halves(uint64_t x) { return make_uint2((unsigned)(x & 0xFFFF), (unsigned)(x >> 16)); }
+
+template <typename W>
+__global__ void __launch_bounds__(512) tag_syndrome_kernel(const int64_t* __restrict__ V, long ldv, const double* __restrict__ P,
+                                                           long ldp, int m_bar, const int32_t* __restrict__ tidx, int ntags,
+                                                           const W* __restrict__ tab, const W* __restrict__ h0,
+                                                           const uint64_t* __restrict__ gpow, uint64_t q, uint64_t magic, int n,
+                                                           int k, int64_t* __restrict__ out, long ldout, int* flag) {
+    extern __shared__ uint64_t tag_sh[];
+    const long b = blockIdx.x;
+    const int t = tidx[b];
+    if (t < 0 || t >= ntags) {  // the table is not read; the gadget sampler gets a valid residue
+        for (int i = threadIdx.x; i < n; i += blockDim.x) out[b * ldout + i] = 0;
+        if (threadIdx.x == 0 && flag) atomicOr(flag, QF_FLAG_TAG_INDEX);
+        return;
+    }
+    const double* pb = P + b * ldp + m_bar;
+    const W* hi = tab + (long)t * n * n;
+    if constexpr (sizeof(W) == 4) {
+        uint2* ys = reinterpret_cast<uint2*>(tag_sh);  // 16-bit halves of y and w
+        uint2* ws = ys + n;
+        // y_i = sum_s base^s p[m_bar + i k + s] mod q: (p mod q) times the halves of base^s mod q, k <= 64 terms < 2^48
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            uint64_t a0 = 0, a1 = 0;
+            for (int s = 0; s < k; ++s) {
+                const uint64_t pm = mod_i64_barrett((long long)pb[(long)i * k + s], q, magic), g = gpow[s];
+                a0 += pm * (g & 0xFFFF);
+                a1 += pm * (g >> 16);
+            }
+            ys[i] = halves(mod_halves(a0, a1, q, magic));
+        }
+        __syncthreads();
+        // w = v + H_0 y (v + y for H_0 = I)
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            const uint2 yi = ys[i];
+            uint64_t hy = yi.x + ((uint64_t)yi.y << 16);
+            if (h0) {
+                uint64_t a0 = 0, a1 = 0;
+#pragma unroll 8
+                for (int j = 0; j < n; ++j) {
+                    const uint64_t h = h0[(long)j * n + i];
+                    const uint2 yj = ys[j];
+                    a0 += h * yj.x;
+                    a1 += h * yj.y;
+                }
+                hy = mod_halves(a0, a1, q, magic);
+            }
+            const uint64_t sum = (uint64_t)V[b * ldv + i] + hy;
+            ws[i] = halves(sum >= q ? sum - q : sum);
+        }
+        __syncthreads();
+        // v' = H_t^-1 w - y
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            uint64_t a0 = 0, a1 = 0;
+#pragma unroll 8
+            for (int j = 0; j < n; ++j) {
+                const uint64_t h = hi[(long)j * n + i];
+                const uint2 wj = ws[j];
+                a0 += h * wj.x;
+                a1 += h * wj.y;
+            }
+            const uint64_t x = mod_halves(a0, a1, q, magic);
+            const uint2 yh = ys[i];
+            const uint64_t yi = yh.x + ((uint64_t)yh.y << 16);
+            out[b * ldout + i] = (int64_t)(x >= yi ? x - yi : x + (q - yi));
+        }
+    } else {
+        typedef __int128 i128;
+        uint64_t* y = tag_sh;
+        uint64_t* w = tag_sh + n;
+        // |p| < 2^53, base^s mod q < 2^62, k <= 64 terms fit 128 bits
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            i128 acc = 0;
+            for (int s = 0; s < k; ++s) acc += (i128)(long long)pb[(long)i * k + s] * (i128)gpow[s];
+            const i128 r = acc % (i128)q;
+            y[i] = (uint64_t)(r < 0 ? r + (i128)q : r);
+        }
+        __syncthreads();
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            uint64_t hy = y[i];
+            if (h0) {
+                ModAcc a;
+#pragma unroll 4
+                for (int j = 0; j < n; ++j) a.mac(h0[(long)j * n + i], y[j]);
+                hy = a.reduce(q);
+            }
+            const uint64_t sum = (uint64_t)V[b * ldv + i] + hy;
+            w[i] = sum >= q ? sum - q : sum;
+        }
+        __syncthreads();
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            ModAcc a;
+#pragma unroll 4
+            for (int j = 0; j < n; ++j) a.mac(hi[(long)j * n + i], w[j]);
+            const uint64_t x = a.reduce(q), yi = y[i];
+            out[b * ldout + i] = (int64_t)(x >= yi ? x - yi : x + (q - yi));
+        }
+    }
+}
+}  // namespace
+
+cudaError_t qf_launch_tag_syndrome(const int64_t* V, long ldv, const double* P, long ldp, int m_bar, const int32_t* tidx,
+                                   int ntags, const void* tab, const void* h0, int word_bytes, const uint64_t* gpow,
+                                   unsigned long long q, int n, int k, int B, int64_t* out, long ldout, int* flag,
+                                   cudaStream_t stream) {
+    if (B <= 0) return cudaSuccess;
+    if (n < 1 || k < 1 || k > 64 || q < 2 || q >= (1ull << 62) || (word_bytes != 4 && word_bytes != 8) ||
+        (word_bytes == 4 && (q > (1ull << 32) || n > (1 << 14))))
+        return cudaErrorInvalidValue;
+    const int threads = n >= 512 ? 512 : (n + 31) / 32 * 32;
+    const size_t smem = (size_t)2 * n * sizeof(uint64_t);
+    const uint64_t magic = qf_barrett_magic(q);
+    cudaError_t e;
+    if (word_bytes == 4) {
+        if (smem > 48 * 1024 &&
+            (e = cudaFuncSetAttribute(tag_syndrome_kernel<uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+            return e;
+        tag_syndrome_kernel<uint32_t><<<B, threads, smem, stream>>>(V, ldv, P, ldp, m_bar, tidx, ntags, (const uint32_t*)tab,
+                                                                    (const uint32_t*)h0, gpow, (uint64_t)q, magic, n, k, out,
+                                                                    ldout, flag);
+    } else {
+        if (smem > 48 * 1024 &&
+            (e = cudaFuncSetAttribute(tag_syndrome_kernel<uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+            return e;
+        tag_syndrome_kernel<uint64_t><<<B, threads, smem, stream>>>(V, ldv, P, ldp, m_bar, tidx, ntags, (const uint64_t*)tab,
+                                                                    (const uint64_t*)h0, gpow, (uint64_t)q, magic, n, k, out,
+                                                                    ldout, flag);
+    }
+    return cudaGetLastError();
+}

@@ -270,6 +270,20 @@ cudaError_t qf_launch_split_i64_limbs(const int64_t* in, long ldin, int8_t* plan
 // q < 2^62); on return *fail = 0 and the right half of M is H^-1, or *fail = c + 1 when column c has no unit pivot.
 // f: n words of device scratch.
 cudaError_t qf_launch_mat_inverse_mod(uint64_t* M, uint64_t* f, int n, unsigned long long q, int* fail, cudaStream_t stream);
+// the same kernel on `count` matrices at once (one CTA each): M count x n x 2n, f count x n words, fail count ints
+cudaError_t qf_launch_mat_inverse_mod_batched(uint64_t* M, uint64_t* f, int n, unsigned long long q, int* fail, int count,
+                                              cudaStream_t stream);
+// tag table (setup.cu): M_t = [H_t mod q | I] (count x n x 2n) from int64 tags (count x n x n, any sign), and the right
+// halves of inverted M_t packed column-major per tag into tab (count x n x n words of word_bytes = 4 or 8)
+cudaError_t qf_launch_tag_build(const int64_t* tags, int count, int n, unsigned long long q, uint64_t* M, cudaStream_t stream);
+cudaError_t qf_launch_tag_pack(const uint64_t* M, int count, int n, int word_bytes, void* tab, cudaStream_t stream);
+// per-target tag of samp_p (elementwise.cu): out[b] = H_{tidx[b]}^-1 (V[b] + H_0 y) - y mod q, y = G p_bot, p_bot =
+// P[b][m_bar:]; tab / h0 column-major n x n words (word_bytes 4 needs q <= 2^32 and n <= 2^14); h0 = NULL means H_0 = I; gpow: base^s mod q,
+// s < k <= 64.  A tag index outside [0, ntags) sets *flag |= QF_FLAG_TAG_INDEX and gives out[b] = 0.
+cudaError_t qf_launch_tag_syndrome(const int64_t* V, long ldv, const double* P, long ldp, int m_bar, const int32_t* tidx,
+                                   int ntags, const void* tab, const void* h0, int word_bytes, const uint64_t* gpow,
+                                   unsigned long long q, int n, int k, int B, int64_t* out, long ldout, int* flag,
+                                   cudaStream_t stream);
 
 // polynomial arithmetic of the ring short basis (setup.cu): P[2][2][n], Q[k][2][n]
 cudaError_t qf_launch_ring_basis_polys(const int32_t* e, const int32_t* r, const int32_t* w, const int64_t* sk, int n, int k,

@@ -426,8 +426,9 @@ cudaError_t qf_launch_ring_basis_polys(const int32_t* e, const int32_t* r, const
 // ---- tag inverse (short_basis_classical.rs:106, MatZq::inverse): Gauss-Jordan over Z_q on M = [H | I] (n x 2n residues,
 // row-major, q < 2^62, 128-bit products).  Column c takes as pivot the first row r >= c whose entry is a unit mod q -- the
 // rule of the host restatement gadget._inverse_mod, so both fail on the same tags.  On success the right half of M is H^-1 and *fail = 0;
-// without a unit pivot *fail = c + 1 and M is left part-reduced.  One CTA: n pivot steps separated by block barriers;
-// per step the factors of column c are saved in f (n words) before the rows are updated.
+// without a unit pivot *fail = c + 1 and M is left part-reduced.  One CTA per matrix (blockIdx.x selects one of `count`
+// matrices M_t = M + t n 2n with its own f and fail slot): n pivot steps separated by block barriers; per step the factors
+// of column c are saved in f (n words) before the rows are updated.
 namespace {
 __device__ __forceinline__ uint64_t gcd_dev(uint64_t a, uint64_t b) {
     while (b) { const uint64_t t = a % b; a = b; b = t; }
@@ -450,6 +451,9 @@ __global__ void __launch_bounds__(1024) mat_inverse_mod_kernel(uint64_t* __restr
     __shared__ int piv;
     __shared__ uint64_t inv;
     const long w = 2L * n;
+    M += (long)blockIdx.x * n * w;
+    f += (long)blockIdx.x * n;
+    fail += blockIdx.x;
     const int tid = threadIdx.x, nth = blockDim.x;
     for (int c = 0; c < n; ++c) {
         if (tid == 0) piv = n;
@@ -492,6 +496,55 @@ __global__ void __launch_bounds__(1024) mat_inverse_mod_kernel(uint64_t* __restr
 
 cudaError_t qf_launch_mat_inverse_mod(uint64_t* M, uint64_t* f, int n, unsigned long long q, int* fail, cudaStream_t stream) {
     if (n < 1 || q < 2 || q >= (1ull << 62)) return cudaErrorInvalidValue;
-    mat_inverse_mod_kernel<<<1, 1024, 0, stream>>>(M, f, n, (uint64_t)q, fail);
+    return qf_launch_mat_inverse_mod_batched(M, f, n, q, fail, 1, stream);
+}
+
+cudaError_t qf_launch_mat_inverse_mod_batched(uint64_t* M, uint64_t* f, int n, unsigned long long q, int* fail, int count,
+                                              cudaStream_t stream) {
+    if (n < 1 || q < 2 || q >= (1ull << 62) || count < 1) return cudaErrorInvalidValue;
+    mat_inverse_mod_kernel<<<count, 1024, 0, stream>>>(M, f, n, (uint64_t)q, fail);
+    return cudaGetLastError();
+}
+
+// ---- tag table (qf_set_tag_table): [H_t | I] from caller tags, and H_t^-1 column-major per tag for the per-target kernel
+namespace {
+__global__ void tag_build_kernel(const int64_t* __restrict__ tags, int count, int n, uint64_t q, uint64_t* __restrict__ M) {
+    const long nn = (long)n * n, total = (long)count * n * 2 * n;
+    for (long x = blockIdx.x * (long)blockDim.x + threadIdx.x; x < total; x += (long)gridDim.x * blockDim.x) {
+        const long t = x / (2 * nn), rem = x - t * 2 * nn, i = rem / (2 * n), j = rem - i * 2 * n;
+        uint64_t v;
+        if (j < n) {
+            const long long h = tags[t * nn + i * n + j] % (long long)q;
+            v = (uint64_t)(h < 0 ? h + (long long)q : h);
+        } else {
+            v = (j - n == i) ? 1 : 0;
+        }
+        M[x] = v;
+    }
+}
+
+// tab[t][j][i] = (H_t^-1)[i][j] = M_t[i][n + j] (32- or 64-bit words): thread i of the per-target kernel reads row i
+template <typename W>
+__global__ void tag_pack_kernel(const uint64_t* __restrict__ M, int count, int n, W* __restrict__ tab) {
+    const long nn = (long)n * n, total = (long)count * nn;
+    for (long x = blockIdx.x * (long)blockDim.x + threadIdx.x; x < total; x += (long)gridDim.x * blockDim.x) {
+        const long t = x / nn, rem = x - t * nn, j = rem / n, i = rem - j * n;
+        tab[x] = (W)M[t * 2 * nn + i * 2 * n + n + j];
+    }
+}
+inline int tag_grid(long long work) { return (int)std::min<long long>((work + 255) / 256, 148LL * 16); }
+}  // namespace
+
+cudaError_t qf_launch_tag_build(const int64_t* tags, int count, int n, unsigned long long q, uint64_t* M, cudaStream_t stream) {
+    if (n < 1 || count < 1 || q < 2) return cudaErrorInvalidValue;
+    tag_build_kernel<<<tag_grid((long long)count * n * 2 * n), 256, 0, stream>>>(tags, count, n, (uint64_t)q, M);
+    return cudaGetLastError();
+}
+
+cudaError_t qf_launch_tag_pack(const uint64_t* M, int count, int n, int word_bytes, void* tab, cudaStream_t stream) {
+    if (n < 1 || count < 1 || (word_bytes != 4 && word_bytes != 8)) return cudaErrorInvalidValue;
+    const int grid = tag_grid((long long)count * n * n);
+    if (word_bytes == 4) tag_pack_kernel<uint32_t><<<grid, 256, 0, stream>>>(M, count, n, (uint32_t*)tab);
+    else tag_pack_kernel<uint64_t><<<grid, 256, 0, stream>>>(M, count, n, (uint64_t*)tab);
     return cudaGetLastError();
 }

@@ -63,6 +63,7 @@ class _PSFBase:
         self.ctx_dim = n * (k + 2) if self.kind == _ffi.QF_PSF_GPV_RING else m_bar + n * k
         self._a_id = None
         self._td_id = None
+        self._tags_id = None  # tag table on the device (PSFPerturbation); dropped there with every key / trapdoor install
         self._keep = None
 
     # -- PSF::samp_d ------------------------------------------------------------------------
@@ -156,7 +157,7 @@ class PSFGPV(_PSFBase):
         if self._a_id is not a:
             aa = np.ascontiguousarray(a, dtype=np.int64)  # keep alive across the call
             self.ctx.call("qf_set_a", _ffi.ptr(aa))
-            self._a_id, self._td_id = a, None
+            self._a_id, self._td_id, self._tags_id = a, None, None
 
     def _install_td(self, a, td):
         if self._td_id is not td:
@@ -249,7 +250,7 @@ class PSFPerturbation(_PSFBase):
                 assert sb.shape == (k, k)
                 blk, gblk = np.ascontiguousarray(sb, dtype=np.int64), np.ascontiguousarray(sg)
             self.ctx.call("qf_set_trapdoor_perturbation", _ffi.ptr(r8), _ffi.ptr(l), _ffi.ptr(blk), _ffi.ptr(gblk))
-            self._td_id = td
+            self._td_id, self._tags_id = td, None
             self._keep = (r8, l, blk, gblk)
 
     def compute_sqrt_sigma_2(self, mat_r, mat_sigma=None) -> np.ndarray:
@@ -326,6 +327,38 @@ class PSFPerturbation(_PSFBase):
         self._a_id = a_new
         return a_new
 
+    def set_tag_table(self, a, td, tags):
+        """Installs the tag table of samp_p_tagged_batch for the key a (any tag H_0) and its trapdoor td: tags is T x n x n,
+        entries taken mod q (qf_set_tag_table: H_t^-1 on the device).  Raises QfError (QF_ERR_INVALID, naming the index)
+        when a tag has no unit pivot; the previous table then stays."""
+        self._install_a(a)
+        self._install_td(a, td)
+        t = np.asarray(tags)
+        if t.dtype == object:
+            t = np.array(t % self.gp.q, dtype=np.int64)
+        tg = np.ascontiguousarray(t, dtype=np.int64)
+        assert tg.ndim == 3 and tg.shape[1:] == (self.n, self.n) and tg.shape[0] >= 1
+        self.ctx.call("qf_set_tag_table", _ffi.ptr(tg), tg.shape[0])
+        self._tags_id = tags
+
+    def samp_p_tagged_batch(self, a, td, tags, us: np.ndarray, tag_idx, seed=None, first_index: int = 0) -> np.ndarray:
+        """samp_p with a tag per target: row b is a preimage of us[b] under [A_bar | H_t G - A_bar R], H_t = tags[tag_idx[b]],
+        for the key a = [A_bar | H_0 G - A_bar R] (any tag H_0) and its trapdoor td.  It equals what set_tag(H_t) followed
+        by samp_p_batch on the same targets gives for that row with the same seed and first_index (qf_samp_p_tagged).
+        tags: T x n x n (entries taken mod q), cached on the device by identity as keys are; tag_idx: B indices in [0, T).
+        Returns B x m int32."""
+        self._install_a(a)
+        self._install_td(a, td)
+        if self._tags_id is not tags:
+            self.set_tag_table(a, td, tags)
+        u = np.ascontiguousarray(us, dtype=np.int64)
+        assert u.ndim == 2 and u.shape[1] == self.n
+        ti = np.ascontiguousarray(tag_idx, dtype=np.int32)
+        assert ti.shape == (u.shape[0],)
+        e = np.empty((u.shape[0], self.m), dtype=np.int32)
+        self.ctx.call("qf_samp_p_tagged", _ffi.ptr(u), _ffi.ptr(ti), u.shape[0], _seed(seed), first_index, _ffi.ptr(e))
+        return e
+
 
 def _gso(psf, basis) -> np.ndarray:
     b = np.ascontiguousarray(basis, dtype=np.int64)
@@ -341,7 +374,7 @@ def _trap_gen_classical(psf, seed):
     a = np.empty((gp.n, gp.m), dtype=np.int64)
     r = np.empty((gp.m_bar, gp.n * gp.k), dtype=np.int8)
     psf.ctx.call("qf_trap_gen", _seed(seed), _ffi.ptr(a), _ffi.ptr(r))
-    psf._td_id = None
+    psf._td_id = psf._tags_id = None
     return a, r
 
 
