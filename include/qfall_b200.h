@@ -125,6 +125,15 @@ qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out);
  * qf_trap_gen, qf_trap_gen_from, qf_set_trapdoor_perturbation) and kept by qf_set_tag.  Device memory: ntags n^2 words of
  * 4 bytes (q <= 2^32) or 8 bytes. */
 qf_status qf_set_tag_table(qf_ctx* ctx, const int64_t* tags, int64_t ntags);
+/* Tag table for f_a with a tag per target (PSFGPV and PSFPerturbation): for the installed key A = [A_bar | H_0 G - A_bar R]
+ * and tags H_t, A_t := A + [0 | (H_t - H_0) G] is the key of tag t, [A_bar | H_t G - A_bar R].  tags: ntags x n x n, h0:
+ * n x n (host; entries taken mod q, negatives allowed); h0 == NULL means H_0 = I, and H_0 = 0 (the base key
+ * [A_bar | -A_bar R]) is allowed.  Needs no trapdoor and inverts nothing, so a verifier holding only A can install it and
+ * singular tags are allowed; R is not known here, so A_t is defined by the formula and not checked against A_bar.  Stores
+ * D_t = H_t - H_0 mod q on the device: ntags n^2 words of 4 bytes (q <= 2^32) or 8 bytes, plus 3 (ntags + 1) ints.
+ * QF_ERR_INVALID on a ring context and for ntags < 1 or tags == NULL; QF_ERR_NO_KEY without a key.  The table is dropped
+ * whenever A changes (qf_set_a, qf_trap_gen, qf_trap_gen_from, qf_set_tag) and is independent of qf_set_tag_table. */
+qf_status qf_set_f_a_tags(qf_ctx* ctx, const int64_t* tags, int64_t ntags, const int64_t* h0);
 /* gen_short_basis_for_trapdoor with tag = I (short_basis_classical.rs:54-110): the short basis
  * S_A = [[I,R],[0,I]] [[0,I],[S',W]] = [[R S', I + R W],[S', W]] of Lambda^perp(A) for the installed A and the
  * trapdoor R (m_bar x nk); W = digits of -A[:, :m_bar], S' column-reversed iff base^k = q.  The m_bar x nk x m_bar
@@ -180,6 +189,17 @@ qf_status qf_ring_trap_gen_from(qf_ctx* ctx, const int64_t* a_bar, const int32_t
 qf_status qf_f_a(qf_ctx* ctx, const int32_t* sigma, int64_t batch, int64_t* u_out, uint8_t* in_domain);
 qf_status qf_f_a_dev(qf_ctx* ctx, const int32_t* sigma, int64_t batch, int64_t* u_out, uint8_t* in_domain);
 qf_status qf_check_domain(qf_ctx* ctx, const int32_t* sigma, int64_t batch, uint8_t* in_domain);
+/* f_a with a tag per target: u[b] = A_t sigma[b] mod q for t = tag_idx[b], the key of tag t of the table of
+ * qf_set_f_a_tags; in_domain[b] = check_domain(sigma[b]), which does not depend on the tag.  u_out is mandatory.
+ * qf_f_a_tagged takes host pointers and works as qf_f_a (in_domain may be NULL, QF_ERR_NOT_IN_DOMAIN when a flag is 0);
+ * the tag indices are checked on the host before any launch (QF_ERR_INVALID outside [0, ntags)).  qf_f_a_tagged_dev takes
+ * device pointers and works as qf_f_a_dev (asynchronous, in_domain mandatory): an index outside the table is never used
+ * to address it, its row is unspecified and the next qf_synchronize returns QF_ERR_INVALID.  QF_ERR_NO_KEY without a
+ * table, QF_ERR_INVALID on a ring context. */
+qf_status qf_f_a_tagged(qf_ctx* ctx, const int32_t* sigma, const int32_t* tag_idx, int64_t batch, int64_t* u_out,
+                        uint8_t* in_domain);
+qf_status qf_f_a_tagged_dev(qf_ctx* ctx, const int32_t* sigma, const int32_t* tag_idx, int64_t batch, int64_t* u_out,
+                            uint8_t* in_domain);
 
 /* ---- PSF::samp_d (gpv.rs:113-116, mp_perturbation.rs:264-267, gpv_ring.rs:118-122) --- */
 qf_status qf_samp_d(qf_ctx* ctx, int64_t batch, uint64_t seed, uint64_t first_index, int32_t* out);

@@ -49,6 +49,7 @@ extern "C" {
     pub fn qf_set_trapdoor_perturbation(ctx: *mut qf_ctx, r: *const i8, sqrt_sigma_2: *const f64, s_block: *const i64, s_block_gso: *const f64) -> i32;
     pub fn qf_set_tag(ctx: *mut qf_ctx, tag: *const i64, a_out: *mut i64) -> i32;
     pub fn qf_set_tag_table(ctx: *mut qf_ctx, tags: *const i64, ntags: i64) -> i32;
+    pub fn qf_set_f_a_tags(ctx: *mut qf_ctx, tags: *const i64, ntags: i64, h0: *const i64) -> i32;
     pub fn qf_gen_short_basis(ctx: *mut qf_ctx, r: *const i8, s_out: *mut i64) -> i32;
     pub fn qf_gen_short_basis_tagged(ctx: *mut qf_ctx, r: *const i8, tag: *const i64, s_out: *mut i64) -> i32;
     pub fn qf_compute_sqrt_sigma_2(ctx: *mut qf_ctx, r: *const i8, sigma: *const f64, sqrt_sigma_2_out: *mut f64) -> i32;
@@ -64,6 +65,8 @@ extern "C" {
     pub fn qf_f_a(ctx: *mut qf_ctx, sigma: *const i32, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
     pub fn qf_f_a_dev(ctx: *mut qf_ctx, sigma: *const i32, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
     pub fn qf_check_domain(ctx: *mut qf_ctx, sigma: *const i32, batch: i64, in_domain: *mut u8) -> i32;
+    pub fn qf_f_a_tagged(ctx: *mut qf_ctx, sigma: *const i32, tag_idx: *const i32, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
+    pub fn qf_f_a_tagged_dev(ctx: *mut qf_ctx, sigma: *const i32, tag_idx: *const i32, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
     pub fn qf_samp_d(ctx: *mut qf_ctx, batch: i64, seed: u64, first_index: u64, out: *mut i32) -> i32;
     pub fn qf_samp_d_dev(ctx: *mut qf_ctx, batch: i64, seed: u64, first_index: u64, out: *mut i32) -> i32;
     pub fn qf_samp_p(ctx: *mut qf_ctx, u: *const i64, batch: i64, seed: u64, first_index: u64, e_out: *mut i32) -> i32;

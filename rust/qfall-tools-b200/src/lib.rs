@@ -142,6 +142,7 @@ pub struct PSFGPVB200 {
     pub inner: PSFGPV,
     ctx: Context,
     installed: RefCell<Option<(Vec<i64>, Vec<i64>)>>, // (A, S) words of the installed key
+    fa_tags: FaTags,
     seed: RefCell<u64>,
 }
 
@@ -161,7 +162,13 @@ impl PSFGPVB200 {
             // backend derive it from the f64-rounded s)
             norm_bound: ring::floor_u64(&(&inner.s * &inner.s * Q::from(i64::try_from(&(&gp.m_bar + &gp.n * &gp.k)).unwrap()))),
         };
-        Ok(PSFGPVB200 { inner, ctx: Context::new(&params, device)?, installed: RefCell::new(None), seed: RefCell::new(seed) })
+        Ok(PSFGPVB200 {
+            inner,
+            ctx: Context::new(&params, device)?,
+            installed: RefCell::new(None),
+            fa_tags: RefCell::new(None),
+            seed: RefCell::new(seed),
+        })
     }
     fn n(&self) -> usize {
         i64::try_from(&self.inner.gp.n).unwrap() as usize
@@ -184,6 +191,7 @@ impl PSFGPVB200 {
             }
         }
         self.ctx.check(unsafe { qf_set_a(self.ctx.raw, aw.as_ptr()) }, "qf_set_a");
+        *self.fa_tags.borrow_mut() = None;
         let gso = matq_to_f64(&td.1);
         self.ctx.check(unsafe { qf_set_trapdoor_gpv(self.ctx.raw, sw.as_ptr(), gso.as_ptr()) }, "qf_set_trapdoor_gpv");
         *self.installed.borrow_mut() = Some((aw, sw));
@@ -200,6 +208,7 @@ impl PSFGPVB200 {
         let r8: Vec<i8> = matz_to_words(r).into_iter().map(|v| i8::try_from(v).expect("R entries must fit i8")).collect();
         assert_eq!(r8.len(), m_bar * (m - m_bar), "R must be m_bar x n k");
         *self.installed.borrow_mut() = None; // qf_set_a drops the installed trapdoor
+        *self.fa_tags.borrow_mut() = None;
         self.ctx.check(unsafe { qf_set_a(self.ctx.raw, aw.as_ptr()) }, "qf_set_a");
         let mut s = vec![0i64; m * m];
         self.ctx.check(unsafe { qf_gen_short_basis_tagged(self.ctx.raw, r8.as_ptr(), tw.as_ptr(), s.as_mut_ptr()) },
@@ -212,6 +221,63 @@ impl PSFGPVB200 {
         }
         out
     }
+
+    /// f_a with a tag per target: `u[b] = A_t sigmas[b]` with `A_t = a + [0 | (H_t - H_0) G]`, `H_t = tags[tag_of[b]]`, for
+    /// a key `a = [A_bar | H_0 G - A_bar R]` (`h0` = H_0, None: I) -- the key gen_trapdoor(A_bar, R, H_t) gives, evaluated
+    /// from `a` alone (qf_set_f_a_tags, qf_f_a_tagged).  No trapdoor is needed.  The tags cross the boundary once per
+    /// table; later batches with the same `a`, `tags` and `h0` pass only sigmas and indices.  Panics like `f_a` when a
+    /// sigma is outside D_n, and when an index is out of range.
+    pub fn f_a_tagged_batch(&self, a: &MatZq, tags: &[MatZq], h0: Option<&MatZq>, sigmas: &[MatZ], tag_of: &[usize]) -> Vec<MatZq> {
+        let aw = matzq_to_words(a);
+        // the key of the cached table is on the device too: every key change drops both
+        let same = self.installed.borrow().as_ref().map(|(a0, _)| *a0 == aw).unwrap_or(false)
+            || self.fa_tags.borrow().as_ref().map(|(a0, _, _)| *a0 == aw).unwrap_or(false);
+        if !same {
+            self.ctx.check(unsafe { qf_set_a(self.ctx.raw, aw.as_ptr()) }, "qf_set_a");
+            *self.installed.borrow_mut() = None;
+            *self.fa_tags.borrow_mut() = None;
+        }
+        let q = Z::from(&self.inner.gp.q);
+        f_a_tagged_installed(&self.ctx, &self.fa_tags, aw, self.n(), self.m(), &q, tags, h0, sigmas, tag_of)
+    }
+}
+
+/// The f_a tag table on the device (qf_set_f_a_tags): (words of the key it belongs to, tag words, H_0 words; empty for
+/// H_0 = I).  The device drops it whenever the key changes, so every key install clears it here too.
+pub(crate) type FaTags = RefCell<Option<(Vec<i64>, Vec<i64>, Vec<i64>)>>;
+
+/// f_a with a tag per target against the key installed in `ctx` (qf_f_a_tagged); installs the table when it differs from
+/// the cached one.
+#[allow(clippy::too_many_arguments)]
+pub(crate) fn f_a_tagged_installed(ctx: &Context, fa_tags: &FaTags, aw: Vec<i64>, n: usize, m: usize, q: &Z, tags: &[MatZq],
+                                   h0: Option<&MatZq>, sigmas: &[MatZ], tag_of: &[usize]) -> Vec<MatZq> {
+    assert!(!tags.is_empty(), "at least one tag");
+    assert_eq!(sigmas.len(), tag_of.len(), "one tag index per sigma");
+    let square = |t: &MatZq| assert_eq!((t.get_num_rows(), t.get_num_columns()), (n as i64, n as i64), "tag must be n x n");
+    let mut tw = Vec::with_capacity(tags.len() * n * n);
+    for tag in tags {
+        square(tag);
+        tw.extend(matzq_to_words(tag));
+    }
+    let hw = h0.map(|h| { square(h); matzq_to_words(h) }).unwrap_or_default();
+    let key = (aw, tw, hw);
+    if fa_tags.borrow().as_ref() != Some(&key) {
+        let hp = if key.2.is_empty() { std::ptr::null() } else { key.2.as_ptr() };
+        ctx.check(unsafe { qf_set_f_a_tags(ctx.raw, key.1.as_ptr(), tags.len() as i64, hp) }, "qf_set_f_a_tags");
+        *fa_tags.borrow_mut() = Some(key);
+    }
+    let mut sg = Vec::with_capacity(sigmas.len() * m);
+    for sigma in sigmas {
+        assert!(sigma.is_column_vector() && sigma.get_num_rows() as usize == m, "sigma is not in D_n");
+        sg.extend(domain_to_i32(sigma).expect("sigma is not in D_n"));
+    }
+    let idx: Vec<i32> = tag_of.iter().map(|t| { assert!(*t < tags.len(), "tag index out of range"); *t as i32 }).collect();
+    let mut u = vec![0i64; sigmas.len() * n];
+    let mut ok = vec![0u8; sigmas.len()];
+    let st = unsafe { qf_f_a_tagged(ctx.raw, sg.as_ptr(), idx.as_ptr(), sigmas.len() as i64, u.as_mut_ptr(), ok.as_mut_ptr()) };
+    assert!(st != QF_ERR_NOT_IN_DOMAIN && ok.iter().all(|f| *f == 1), "sigma is not in D_n"); // gpv.rs:191
+    ctx.check(st, "qf_f_a_tagged");
+    u.chunks(n).map(|row| range_from_words(row, q)).collect()
 }
 
 impl PSF for PSFGPVB200 {
@@ -228,6 +294,7 @@ impl PSF for PSFGPVB200 {
         let (mut a, mut r) = (vec![0i64; n * m], vec![0i8; m_bar * (m - m_bar)]);
         self.ctx.check(unsafe { qf_trap_gen(self.ctx.raw, self.next_seed(), a.as_mut_ptr(), r.as_mut_ptr()) }, "qf_trap_gen");
         *self.installed.borrow_mut() = None; // qf_trap_gen installed a new key: whatever trapdoor was cached is gone
+        *self.fa_tags.borrow_mut() = None;
         let mut s = vec![0i64; m * m];
         self.ctx.check(unsafe { qf_gen_short_basis(self.ctx.raw, r.as_ptr(), s.as_mut_ptr()) }, "qf_gen_short_basis");
         let mut gso = vec![0f64; m * m];
@@ -298,6 +365,7 @@ impl PSFBatch for PSFGPVB200 {
         if !same {
             self.ctx.check(unsafe { qf_set_a(self.ctx.raw, aw.as_ptr()) }, "qf_set_a");
             *self.installed.borrow_mut() = None;
+            *self.fa_tags.borrow_mut() = None;
         }
         let (n, m) = (self.n(), self.m());
         let mut sg = Vec::with_capacity(sigmas.len() * m);

@@ -2,7 +2,8 @@
 //! `p <- D_{sqrt(Sigma_2)}`, `v = u - A p`, `z <- D_{Lambda_v^perp(G)}`, `e = p + [R; I] z` for a batch of targets.
 //! Shipped as source (see lib.rs).
 use crate::ffi::*;
-use crate::{column_from_i32, domain_to_i32, matz_to_words, matzq_to_words, range_from_words, Context, PSFBatch};
+use crate::{column_from_i32, domain_to_i32, f_a_tagged_installed, matz_to_words, matzq_to_words, range_from_words, Context, FaTags,
+            PSFBatch};
 use qfall_math::{
     integer::{MatZ, Z},
     integer_mod_q::MatZq,
@@ -22,6 +23,8 @@ pub struct PSFPerturbationB200 {
     installed_r: RefCell<Option<(Vec<i64>, Vec<u64>, Vec<i64>, Vec<u64>)>>,
     /// number of tags in the table on the device (qf_set_tag_table); the device drops it with every key or trapdoor install
     installed_tags: RefCell<Option<usize>>,
+    /// the f_a tag table on the device (qf_set_f_a_tags); the device drops it whenever the key changes
+    fa_tags: FaTags,
     seed: RefCell<u64>,
 }
 
@@ -48,6 +51,7 @@ impl PSFPerturbationB200 {
             installed_a: RefCell::new(None),
             installed_r: RefCell::new(None),
             installed_tags: RefCell::new(None),
+            fa_tags: RefCell::new(None),
             seed: RefCell::new(seed),
         })
     }
@@ -77,6 +81,7 @@ impl PSFPerturbationB200 {
         *self.installed_a.borrow_mut() = Some(aw);
         *self.installed_r.borrow_mut() = None;
         *self.installed_tags.borrow_mut() = None;
+        *self.fa_tags.borrow_mut() = None;
     }
     /// Trapdoor `(R, sqrt(Sigma_2), (S, S~))` (mp_perturbation.rs:195).  The gadget basis must be `I_n (x) S_k`
     /// (what `short_basis_gadget` returns, gadget_classical.rs:273-286): only its first k x k block crosses the boundary.
@@ -137,6 +142,7 @@ impl PSFPerturbationB200 {
             }
         }
         *self.installed_a.borrow_mut() = Some(aw);
+        *self.fa_tags.borrow_mut() = None; // qf_set_tag rewrote A
         out
     }
 
@@ -182,6 +188,16 @@ impl PSFPerturbationB200 {
         self.ctx.check(st, "qf_samp_p_tagged");
         e.chunks(m).map(column_from_i32).collect()
     }
+
+    /// f_a with a tag per target: `u[b] = A_t sigmas[b]` with `A_t = a + [0 | (H_t - H_0) G]`, `H_t = tags[tag_of[b]]`, for
+    /// a key `a = [A_bar | H_0 G - A_bar R]` (`h0` = H_0, None: I), evaluated from `a` alone (qf_set_f_a_tags,
+    /// qf_f_a_tagged): no trapdoor is needed, singular tags are allowed.  The tags cross the boundary once per table.
+    /// Independent of `set_tag_table`.  Panics like `f_a` when a sigma is outside D_n, and when an index is out of range.
+    pub fn f_a_tagged_batch(&self, a: &MatZq, tags: &[MatZq], h0: Option<&MatZq>, sigmas: &[MatZ], tag_of: &[usize]) -> Vec<MatZq> {
+        self.install_a(a);
+        let q = Z::from(&self.inner.gp.q);
+        f_a_tagged_installed(&self.ctx, &self.fa_tags, matzq_to_words(a), self.n(), self.m(), &q, tags, h0, sigmas, tag_of)
+    }
 }
 
 impl PSF for PSFPerturbationB200 {
@@ -202,6 +218,7 @@ impl PSF for PSFPerturbationB200 {
         *self.installed_a.borrow_mut() = None;
         *self.installed_r.borrow_mut() = None;
         *self.installed_tags.borrow_mut() = None;
+        *self.fa_tags.borrow_mut() = None;
         let mut l = vec![0f64; m * m];
         let st = unsafe { qf_compute_sqrt_sigma_2(self.ctx.raw, r.as_ptr(), std::ptr::null(), l.as_mut_ptr()) };
         self.ctx.check(st, "qf_compute_sqrt_sigma_2"); // QF_ERR_INVALID = Sigma_2 not positive definite (the reference panics)

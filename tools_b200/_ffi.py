@@ -48,6 +48,7 @@ SIGNATURES = {
     "qf_set_trapdoor_perturbation": (_i32, [_vp, _vp, _vp, _vp, _vp]),
     "qf_set_tag": (_i32, [_vp, _vp, _vp]),
     "qf_set_tag_table": (_i32, [_vp, _vp, _i64]),
+    "qf_set_f_a_tags": (_i32, [_vp, _vp, _i64, _vp]),
     "qf_compute_sqrt_sigma_2": (_i32, [_vp, _vp, _vp, _vp]),
     "qf_gen_short_basis": (_i32, [_vp, _vp, _vp]),
     "qf_gen_short_basis_tagged": (_i32, [_vp, _vp, _vp, _vp]),
@@ -61,6 +62,8 @@ SIGNATURES = {
     "qf_f_a": (_i32, [_vp, _vp, _i64, _vp, _vp]),
     "qf_f_a_dev": (_i32, [_vp, _vp, _i64, _vp, _vp]),
     "qf_check_domain": (_i32, [_vp, _vp, _i64, _vp]),
+    "qf_f_a_tagged": (_i32, [_vp, _vp, _vp, _i64, _vp, _vp]),
+    "qf_f_a_tagged_dev": (_i32, [_vp, _vp, _vp, _i64, _vp, _vp]),
     "qf_samp_d": (_i32, [_vp, _i64, _u64, _u64, _vp]),
     "qf_samp_d_dev": (_i32, [_vp, _i64, _u64, _u64, _vp]),
     "qf_samp_p": (_i32, [_vp, _vp, _i64, _u64, _u64, _vp]),

@@ -193,6 +193,12 @@ struct qf_ctx {
     int64_t tag_count = 0;
     int tag_word = 8;
     Dev dTagTab, dTagH0, dTagGpow, io_t[2];
+    // Tag table of f_a (qf_set_f_a_tags, PSFGPV and PSFPerturbation): D_t = H_t - H_0 mod q for fa_tag_count tags, in the
+    // layout of dTagTab, relative to the installed A and dropped whenever A changes.  dFaSort: hist / off / gstart of the
+    // counting sort by tag (3 (T + 1) ints); dFaPerm: the sorted targets of a chunk.
+    int64_t fa_tag_count = 0;
+    int fa_tag_word = 8;
+    Dev dFaTab, dFaGpow, dFaSort, dFaPerm;
     // Defaults from the error budget of DESIGN 4.2, checked at the full C2 key (scripts/ab_c2_precision.py, profiles/README_r2.md):
     // four digits everywhere; the lowest digit sum is dropped where the operand has three digits (z2), not for the
     // two-digit z1 (dropping it there moves 14 % of the preimages, keeping it 0.3 %).
@@ -1705,6 +1711,39 @@ qf_status for_chunks(qf_ctx* ctx, int64_t batch, F&& f) {
     return QF_OK;
 }
 
+// Chunks of a device-resident f_a batch.  The fused kernel needs no per-chunk workspace (8 bytes of norm per target): the
+// whole batch goes out as one grid, so only its last wave can be partial (chunks of 16 K targets are 1.7 waves each at
+// n = 256).
+template <typename F>
+qf_status f_a_dev_chunks(qf_ctx* ctx, int64_t batch, F&& run) {
+    const bool ring = ctx->prm.kind == QF_PSF_GPV_RING;
+    const bool fused = ctx->x_limbs <= 4 && (ring ? ctx->ring_dense : (ctx->use_i8 && ctx->fused_fa));
+    if (fused) {
+        constexpr int64_t kMax = 1 << 20;
+        for (int64_t b0 = 0; b0 < batch; b0 += kMax) QF_TRY(run(b0, (int)std::min<int64_t>(kMax, batch - b0)));
+        return QF_OK;
+    }
+    return for_chunks(ctx, batch, run);
+}
+
+// f_a with a tag per target (qf_f_a_tagged): A sigma from f_a_chunk, then u_b += D_t G sigma_bot_b in place, the targets
+// grouped by tag on the device (no host round trip).  dTidx: device tag indices of the chunk.
+qf_status f_a_tagged_chunk(qf_ctx* ctx, const int32_t* dSigma, const int32_t* dTidx, int Bc, int64_t* dU, uint8_t* dFlags) {
+    QF_TRY(f_a_chunk(ctx, dSigma, Bc, dU, dFlags));
+    const int T = (int)ctx->fa_tag_count;
+    int* hist = ctx->dFaSort.as<int>();
+    int *off = hist + (T + 1), *gstart = off + (T + 1), *perm = nullptr;
+    if (QF_F_A_TAG_GROUP > 1) {  // always in the library; 1 only in the benchmark's comparison build (kernels.h)
+        CK(ctx->dFaPerm.ensure((size_t)Bc * sizeof(int)));
+        perm = ctx->dFaPerm.as<int>();
+        LAUNCH(qf_launch_f_a_tag_sort(dTidx, Bc, T, hist, off, gstart, perm, ctx->dFlag.as<int>(), ctx->stream));
+    }
+    LAUNCH(qf_launch_f_a_tag_correct(dSigma, ctx->dim, (int)ctx->m_bar, dTidx, T, perm, off, gstart, ctx->dFaTab.p,
+                                     ctx->fa_tag_word, ctx->dFaGpow.as<uint64_t>(), ctx->prm.q, (int)ctx->n, (int)ctx->k, Bc,
+                                     dU, ctx->n, ctx->dFlag.as<int>(), ctx->stream));
+    return QF_OK;
+}
+
 qf_status install_a(qf_ctx* ctx, const int64_t* a) {
     if (ctx->prm.kind == QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "qf_set_a on a ring context; use qf_ring_set_a");
     // a new key invalidates whatever trapdoor was installed for the old one: samp_p answers QF_ERR_NO_KEY until the
@@ -1713,6 +1752,7 @@ qf_status install_a(qf_ctx* ctx, const int64_t* a) {
     ctx->key_tagged = false; ctx->pert_gadget_key = false;
     ctx->dHinvl.release(); ctx->dAbpl.release();
     ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release();
+    ctx->fa_tag_count = 0; ctx->dFaTab.release();
     const long n = ctx->n, m = ctx->m;
     for (long i = 0; i < n * m; ++i)
         if (a[i] < 0 || (uint64_t)a[i] >= ctx->prm.q) return ctx->fail(QF_ERR_INVALID, "A entry outside [0,q)");
@@ -2017,6 +2057,7 @@ qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out) {
     // device copies are consistent again the context has no key (a CUDA error on the way leaves it so).
     ctx->has_a = false;
     ctx->has_pert = false;
+    ctx->fa_tag_count = 0; ctx->dFaTab.release();  // the f_a table is relative to A, which changes here
     const std::vector<uint64_t> gpow = gadget_powers(ctx);
     for (long i = 0; i < n; ++i)
         for (long j = 0; j < n; ++j) {
@@ -2088,6 +2129,58 @@ qf_status qf_set_tag_table(qf_ctx* ctx, const int64_t* tags, int64_t ntags) {
     std::swap(ctx->dTagTab.p, tab.p);
     std::swap(ctx->dTagTab.cap, tab.cap);
     ctx->tag_count = ntags;
+    return QF_OK;
+}
+
+// D_t = H_t - H_0 mod q for every tag, built on the device from the caller's words in slices of at most 1 GB of int64 tags.
+// No trapdoor is needed and no tag is inverted.  The new table replaces the old one only when it is complete.
+qf_status qf_set_f_a_tags(qf_ctx* ctx, const int64_t* tags, int64_t ntags, const int64_t* h0) {
+    if (!ctx) return QF_ERR_INVALID;
+    if (ctx->prm.kind == QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "f_a tag table: not a classical context");
+    if (!tags || ntags < 1) return ctx->fail(QF_ERR_INVALID, "f_a tag table: at least one tag needed");
+    if (ntags >= INT32_MAX) return ctx->fail(QF_ERR_INVALID, "f_a tag table: more than 2^31 - 2 tags");
+    if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "no key installed");
+    const long n = ctx->n;
+    CK(cudaSetDevice(ctx->device));
+    int supported = 0;
+    CK(qf_f_a_tag_supported((int)std::min<long>(n, INT32_MAX), (int)ctx->k, &supported));
+    if (!supported)
+        return ctx->fail(QF_ERR_UNSUPPORTED, "f_a tag table: needs k <= 64 and the group's shared memory within one block's limit");
+    const uint64_t q = ctx->prm.q;
+    const int word = q <= (1ull << 32) ? 4 : 8;
+    const size_t nn = (size_t)n * n;
+    const int64_t slice = std::max<int64_t>(1, std::min<int64_t>(ntags, (int64_t)((1ull << 30) / (8 * nn))));
+    Dev tab, dTags, dH0, sort;
+    CK(tab.ensure((size_t)ntags * nn * word));
+    CK(dTags.ensure((size_t)slice * nn * 8));
+    CK(sort.ensure((size_t)3 * (ntags + 1) * sizeof(int)));
+    if (h0) {
+        std::vector<uint64_t> h((size_t)nn);
+        for (size_t x = 0; x < nn; ++x) {
+            const int64_t v = h0[x] % (int64_t)q;
+            h[x] = (uint64_t)(v < 0 ? v + (int64_t)q : v);
+        }
+        CK(dH0.ensure(nn * 8));
+        CK(cudaMemcpyAsync(dH0.p, h.data(), nn * 8, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    for (int64_t t0 = 0; t0 < ntags; t0 += slice) {
+        const int cnt = (int)std::min<int64_t>(slice, ntags - t0);
+        CK(cudaMemcpyAsync(dTags.p, tags + (size_t)t0 * nn, (size_t)cnt * nn * 8, cudaMemcpyHostToDevice, ctx->stream));
+        LAUNCH(qf_launch_tag_diff_pack(dTags.as<int64_t>(), cnt, (int)n, q, dH0.as<uint64_t>(), word,
+                                       tab.as<char>() + (size_t)t0 * nn * word, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));  // dTags is refilled by the next slice
+    }
+    const std::vector<uint64_t> gpow = gadget_powers(ctx);
+    CK(ctx->dFaGpow.ensure(gpow.size() * 8));
+    CK(cudaMemcpyAsync(ctx->dFaGpow.p, gpow.data(), gpow.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    std::swap(ctx->dFaTab.p, tab.p);
+    std::swap(ctx->dFaTab.cap, tab.cap);
+    std::swap(ctx->dFaSort.p, sort.p);
+    std::swap(ctx->dFaSort.cap, sort.cap);
+    ctx->fa_tag_word = word;
+    ctx->fa_tag_count = ntags;
     return QF_OK;
 }
 
@@ -2754,15 +2847,7 @@ qf_status qf_f_a_dev(qf_ctx* ctx, const int32_t* sigma, int64_t batch, int64_t* 
         uint8_t* f = in_domain ? in_domain + b0 : nullptr;
         return ring ? ring_f_a_chunk(ctx, s, Bc, u, f) : f_a_chunk(ctx, s, Bc, u, f);
     };
-    // The fused kernel needs no per-chunk workspace (8 bytes of norm per target): the whole device-resident batch goes out
-    // as one grid, so only its last wave can be partial (chunks of 16 K targets are 1.7 waves each at n = 256).
-    const bool fused = ctx->x_limbs <= 4 && (ring ? ctx->ring_dense : (ctx->use_i8 && ctx->fused_fa));
-    if (fused) {
-        constexpr int64_t kMax = 1 << 20;
-        for (int64_t b0 = 0; b0 < batch; b0 += kMax) QF_TRY(run(b0, (int)std::min<int64_t>(kMax, batch - b0)));
-        return QF_OK;
-    }
-    return for_chunks(ctx, batch, run);
+    return f_a_dev_chunks(ctx, batch, run);
 }
 
 qf_status qf_f_a(qf_ctx* ctx, const int32_t* sigma, int64_t batch, int64_t* u_out, uint8_t* in_domain) {
@@ -2809,6 +2894,60 @@ qf_status qf_check_domain(qf_ctx* ctx, const int32_t* sigma, int64_t batch, uint
         CK(cudaMemcpyAsync(in_domain + b0, ctx->io_c.p, (size_t)Bc, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
         return QF_OK;
+    });
+}
+
+// ---- f_a with a tag per target (installed f_a tag table) ------------------------------------------------------------
+static qf_status f_a_tagged_ready(qf_ctx* ctx) {
+    if (ctx->prm.kind == QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "f_a tag table: not a classical context");
+    if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "no key installed");
+    if (!ctx->fa_tag_count) return ctx->fail(QF_ERR_NO_KEY, "no f_a tag table installed (qf_set_f_a_tags)");
+    return QF_OK;
+}
+
+qf_status qf_f_a_tagged(qf_ctx* ctx, const int32_t* sigma, const int32_t* tag_idx, int64_t batch, int64_t* u_out,
+                        uint8_t* in_domain) {
+    if (!ctx || batch < 0 || (batch > 0 && (!sigma || !tag_idx || !u_out))) return QF_ERR_INVALID;
+    if (batch == 0) return QF_OK;
+    CK(cudaSetDevice(ctx->device));
+    QF_TRY(f_a_tagged_ready(ctx));
+    for (int64_t b = 0; b < batch; ++b)
+        if (tag_idx[b] < 0 || tag_idx[b] >= ctx->fa_tag_count) {
+            char buf[128];
+            snprintf(buf, sizeof buf, "tag index outside the installed f_a tag table (target %lld: %d)", (long long)b, (int)tag_idx[b]);
+            return ctx->fail(QF_ERR_INVALID, buf);
+        }
+    const long C = ctx->chunk;
+    CK(ctx->io_a.ensure((size_t)C * ctx->dim * 4));
+    CK(ctx->io_b.ensure((size_t)C * ctx->n * 8));
+    CK(ctx->io_c.ensure((size_t)C));
+    CK(ctx->io_t[0].ensure((size_t)C * 4));
+    std::vector<uint8_t> flags((size_t)batch);
+    QF_TRY(for_chunks(ctx, batch, [&](int64_t b0, int Bc) -> qf_status {
+        CK(cudaMemcpyAsync(ctx->io_a.p, sigma + b0 * ctx->dim, (size_t)Bc * ctx->dim * 4, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(ctx->io_t[0].p, tag_idx + b0, (size_t)Bc * 4, cudaMemcpyHostToDevice, ctx->stream));
+        QF_TRY(f_a_tagged_chunk(ctx, ctx->io_a.as<int32_t>(), ctx->io_t[0].as<int32_t>(), Bc, ctx->io_b.as<int64_t>(),
+                                ctx->io_c.as<uint8_t>()));
+        CK(cudaMemcpyAsync(u_out + b0 * ctx->n, ctx->io_b.p, (size_t)Bc * ctx->n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(flags.data() + b0, ctx->io_c.p, (size_t)Bc, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        return QF_OK;
+    }));
+    bool all = true;
+    for (int64_t b = 0; b < batch; ++b) all = all && flags[b];
+    if (in_domain) memcpy(in_domain, flags.data(), (size_t)batch);
+    if (!all) return ctx->fail(QF_ERR_NOT_IN_DOMAIN, "f_a: sigma not in the domain D_n (check_domain failed)");
+    return QF_OK;
+}
+
+qf_status qf_f_a_tagged_dev(qf_ctx* ctx, const int32_t* sigma, const int32_t* tag_idx, int64_t batch, int64_t* u_out,
+                            uint8_t* in_domain) {
+    if (!ctx || batch < 0 || (batch > 0 && (!sigma || !tag_idx || !u_out || !in_domain))) return QF_ERR_INVALID;
+    if (batch == 0) return QF_OK;
+    CK(cudaSetDevice(ctx->device));
+    QF_TRY(f_a_tagged_ready(ctx));
+    return f_a_dev_chunks(ctx, batch, [&](int64_t b0, int Bc) {
+        return f_a_tagged_chunk(ctx, sigma + b0 * ctx->dim, tag_idx + b0, Bc, u_out + b0 * ctx->n, in_domain + b0);
     });
 }
 

@@ -1040,3 +1040,289 @@ cudaError_t qf_launch_tag_syndrome(const int64_t* V, long ldv, const double* P, 
     }
     return cudaGetLastError();
 }
+
+// ---- per-target tag of f_a (qf_f_a_tagged): u_b += D_t y_b mod q with y_b = G sigma_bot_b, D_t = H_t - H_0, t = tidx[b] -------
+// The table D (T x n x n words, column-major as the samp_p table) is n^2 words per tag, far more than the n outputs of a
+// target, so the targets are grouped by tag first: a counting sort of the chunk's tag indices (histogram over T + 1 bins,
+// the last one for indices outside the table; exclusive scan; scatter into a permutation), each tag's run cut into groups of
+// at most QF_F_A_TAG_GROUP targets, one CTA per group.  Every table word a CTA loads serves all targets of its group.
+namespace {
+constexpr int FA_G = QF_F_A_TAG_GROUP;
+
+// lanes of a warp with the same bin: one atomic per distinct bin; returns the lane's rank among its peers
+__device__ __forceinline__ int fa_warp_add(int* ctr, int bin, bool active, int* base) {
+    const unsigned act = __ballot_sync(0xFFFFFFFFu, active);
+    if (!active) return 0;
+    const unsigned peers = __match_any_sync(act, bin);
+    const int lane = threadIdx.x & 31, leader = __ffs(peers) - 1;
+    int b0 = 0;
+    if (lane == leader) b0 = atomicAdd(ctr + bin, __popc(peers));
+    *base = __shfl_sync(peers, b0, leader);
+    return __popc(peers & ((1u << lane) - 1));
+}
+
+__global__ void fa_tag_hist_kernel(const int32_t* __restrict__ tidx, int B, int ntags, int* __restrict__ hist, int* flag) {
+    for (int b0 = blockIdx.x * blockDim.x; b0 < B; b0 += gridDim.x * blockDim.x) {
+        const int b = b0 + threadIdx.x;
+        int bin = ntags;
+        if (b < B) {
+            const int t = tidx[b];
+            if (t >= 0 && t < ntags) bin = t;
+            else if (flag) atomicOr(flag, QF_FLAG_TAG_INDEX);
+        }
+        int base;
+        fa_warp_add(hist, bin, b < B, &base);
+    }
+}
+
+// one CTA: off[t] = sum_{t' < t} hist[t'] (hist becomes the scatter cursor), gstart[t] = sum_{t' < t} ceil(hist[t'] / G) over
+// the valid bins, gstart[ntags] = number of groups
+__global__ void __launch_bounds__(1024) fa_tag_scan_kernel(int* __restrict__ hist, int ntags, int* __restrict__ off,
+                                                           int* __restrict__ gstart) {
+    __shared__ int wc[32], wg[32];
+    const int nb = ntags + 1, per = (nb + blockDim.x - 1) / blockDim.x;
+    const int t0 = min(nb, (int)threadIdx.x * per), t1 = min(nb, t0 + per);
+    int c = 0, g = 0;
+    for (int t = t0; t < t1; ++t) {
+        const int h = hist[t];
+        c += h;
+        if (t < ntags) g += (h + FA_G - 1) / FA_G;
+    }
+    // block-wide exclusive scan of (c, g)
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int ic = c, ig = g;
+    for (int d = 1; d < 32; d <<= 1) {
+        const int xc = __shfl_up_sync(0xFFFFFFFFu, ic, d), xg = __shfl_up_sync(0xFFFFFFFFu, ig, d);
+        if (lane >= d) { ic += xc; ig += xg; }
+    }
+    if (lane == 31) { wc[warp] = ic; wg[warp] = ig; }
+    __syncthreads();
+    if (warp == 0) {
+        const int nw = blockDim.x >> 5;
+        int vc = lane < nw ? wc[lane] : 0, vg = lane < nw ? wg[lane] : 0;
+        for (int d = 1; d < 32; d <<= 1) {
+            const int xc = __shfl_up_sync(0xFFFFFFFFu, vc, d), xg = __shfl_up_sync(0xFFFFFFFFu, vg, d);
+            if (lane >= d) { vc += xc; vg += xg; }
+        }
+        if (lane < nw) { wc[lane] = vc; wg[lane] = vg; }
+    }
+    __syncthreads();
+    int rc = ic - c + (warp ? wc[warp - 1] : 0), rg = ig - g + (warp ? wg[warp - 1] : 0);
+    for (int t = t0; t < t1; ++t) {
+        const int h = hist[t];
+        hist[t] = rc;
+        off[t] = rc;
+        if (t < ntags) gstart[t] = rg;
+        rc += h;
+        if (t < ntags) rg += (h + FA_G - 1) / FA_G;
+    }
+    if (threadIdx.x == blockDim.x - 1) gstart[ntags] = rg;
+}
+
+__global__ void fa_tag_scatter_kernel(const int32_t* __restrict__ tidx, int B, int ntags, int* __restrict__ cur,
+                                      int* __restrict__ perm) {
+    for (int b0 = blockIdx.x * blockDim.x; b0 < B; b0 += gridDim.x * blockDim.x) {
+        const int b = b0 + threadIdx.x;
+        int bin = ntags;
+        if (b < B) {
+            const int t = tidx[b];
+            if (t >= 0 && t < ntags) bin = t;
+        }
+        int base = 0;
+        const int r = fa_warp_add(cur, bin, b < B, &base);
+        if (b < B) perm[base + r] = b;
+    }
+}
+
+// One CTA per group of at most FA_G targets of one tag t.  FA_G = 1 (CTA b is target b, no sort) is not built by the
+// library: scripts/bench_f_a_tagged.py builds it to measure what the grouping gains (DESIGN 4.9).  y_g = G sigma_bot of the
+// group's targets sits in shared memory as [j][g]; thread i owns rows i, i + blockDim, ... and loads each word D_t[i][j] once
+// for all targets.  Exact for every q < 2^62 and int32 sigma (sigma is reduced mod q first):
+//  - W = uint32_t (q <= 2^32, n <= 2^14): y as 16-bit halves, a row sum of n products word x half < 2^48 stays below 2^62
+//    (mod_halves), as in tag_syndrome_kernel;
+//  - W = uint64_t: 192-bit row sums (ModAcc).
+// Unused slots of a partial group hold y = 0 and are not written.
+template <typename W>
+__global__ void __launch_bounds__(512) fa_tag_correct_kernel(const int32_t* __restrict__ sigma, long lds, int m_bar,
+                                                             const int32_t* __restrict__ tidx, int ntags,
+                                                             const int* __restrict__ perm, const int* __restrict__ off,
+                                                             const int* __restrict__ gstart, const W* __restrict__ tab,
+                                                             const uint64_t* __restrict__ gpow, uint64_t q, uint64_t magic,
+                                                             int n, int k, int64_t* __restrict__ u, long ldu, int* flag) {
+    extern __shared__ uint64_t fa_sh[];
+    __shared__ int s_t, s_cnt, s_row[FA_G];
+    if (threadIdx.x == 0) {
+        int cnt = 0, t = 0;
+        if constexpr (FA_G == 1) {
+            t = tidx[blockIdx.x];
+            if (t >= 0 && t < ntags) {
+                cnt = 1;
+                s_row[0] = blockIdx.x;
+            } else if (flag) {
+                atomicOr(flag, QF_FLAG_TAG_INDEX);
+            }
+        } else {
+            const int g = blockIdx.x;
+            if (g < gstart[ntags]) {  // the grid is an upper bound on the groups the sort made
+                int lo = 0, hi = ntags - 1;  // last t with gstart[t] <= g
+                while (lo < hi) {
+                    const int mid = (lo + hi + 1) >> 1;
+                    if (gstart[mid] <= g) lo = mid;
+                    else hi = mid - 1;
+                }
+                t = lo;
+                const int first = off[t] + (g - gstart[t]) * FA_G;
+                cnt = min(FA_G, off[t + 1] - first);
+                for (int c = 0; c < cnt; ++c) s_row[c] = perm[first + c];
+            }
+        }
+        s_t = t;
+        s_cnt = cnt;
+    }
+    __syncthreads();
+    const int cnt = s_cnt;
+    if (!cnt) return;
+    const W* d = tab + (long)s_t * n * n;
+    if constexpr (sizeof(W) == 4) {
+        uint2* ys = reinterpret_cast<uint2*>(fa_sh);
+        for (int i = threadIdx.x; i < n; i += blockDim.x)
+            for (int c = 0; c < FA_G; ++c) {
+                uint2 v = make_uint2(0, 0);
+                if (c < cnt) {
+                    const int32_t* sb = sigma + (long)s_row[c] * lds + m_bar + (long)i * k;
+                    uint64_t a0 = 0, a1 = 0;
+                    for (int s = 0; s < k; ++s) {
+                        const uint64_t sm = mod_i64_barrett((long long)sb[s], q, magic), gs = gpow[s];
+                        a0 += sm * (gs & 0xFFFF);
+                        a1 += sm * (gs >> 16);
+                    }
+                    v = halves(mod_halves(a0, a1, q, magic));
+                }
+                ys[i * FA_G + c] = v;
+            }
+        __syncthreads();
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            uint64_t a0[FA_G], a1[FA_G];
+#pragma unroll
+            for (int c = 0; c < FA_G; ++c) a0[c] = a1[c] = 0;
+#pragma unroll 4
+            for (int j = 0; j < n; ++j) {
+                const uint64_t h = d[(long)j * n + i];
+#pragma unroll
+                for (int c = 0; c < FA_G; ++c) {
+                    const uint2 yj = ys[j * FA_G + c];
+                    a0[c] += h * yj.x;
+                    a1[c] += h * yj.y;
+                }
+            }
+#pragma unroll
+            for (int c = 0; c < FA_G; ++c)
+                if (c < cnt) {
+                    int64_t* ub = u + (long)s_row[c] * ldu + i;
+                    const uint64_t sum = (uint64_t)*ub + mod_halves(a0[c], a1[c], q, magic);
+                    *ub = (int64_t)(sum >= q ? sum - q : sum);
+                }
+        }
+    } else {
+        uint64_t* ys = fa_sh;
+        for (int i = threadIdx.x; i < n; i += blockDim.x)
+            for (int c = 0; c < FA_G; ++c) {
+                uint64_t v = 0;
+                if (c < cnt) {
+                    const int32_t* sb = sigma + (long)s_row[c] * lds + m_bar + (long)i * k;
+                    ModAcc a;
+                    for (int s = 0; s < k; ++s) a.mac(sb[s] < 0 ? (uint64_t)((long long)sb[s] + (long long)q) : (uint64_t)sb[s], gpow[s]);
+                    v = a.reduce(q);
+                }
+                ys[i * FA_G + c] = v;
+            }
+        __syncthreads();
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            ModAcc a[FA_G];
+#pragma unroll 2
+            for (int j = 0; j < n; ++j) {
+                const uint64_t h = d[(long)j * n + i];
+#pragma unroll
+                for (int c = 0; c < FA_G; ++c) a[c].mac(h, ys[j * FA_G + c]);
+            }
+#pragma unroll
+            for (int c = 0; c < FA_G; ++c)
+                if (c < cnt) {
+                    int64_t* ub = u + (long)s_row[c] * ldu + i;
+                    const uint64_t sum = (uint64_t)*ub + a[c].reduce(q);
+                    *ub = (int64_t)(sum >= q ? sum - q : sum);
+                }
+        }
+    }
+}
+
+inline int fa_sort_grid(int B) { return std::max(1, std::min((B + 255) / 256, 148 * 8)); }
+
+// the y of a group (8 n bytes per target) plus the kernel's static shared memory fit what one block may opt into
+cudaError_t fa_smem_fits(int n, bool* fits) {
+    cudaFuncAttributes a4, a8;
+    cudaError_t e;
+    if ((e = cudaFuncGetAttributes(&a4, fa_tag_correct_kernel<uint32_t>)) != cudaSuccess) return e;
+    if ((e = cudaFuncGetAttributes(&a8, fa_tag_correct_kernel<uint64_t>)) != cudaSuccess) return e;
+    int dev = 0, optin = 0;
+    if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
+    if ((e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess) return e;
+    *fits = (size_t)n * FA_G * sizeof(uint64_t) + std::max(a4.sharedSizeBytes, a8.sharedSizeBytes) <= (size_t)optin;
+    return cudaSuccess;
+}
+}  // namespace
+
+cudaError_t qf_f_a_tag_supported(int n, int k, int* ok) {
+    bool fits = false;
+    cudaError_t e = fa_smem_fits(n, &fits);
+    if (e != cudaSuccess) return e;
+    *ok = n >= 1 && k >= 1 && k <= 64 && n <= (1 << 14) && fits;
+    return cudaSuccess;
+}
+
+cudaError_t qf_launch_f_a_tag_sort(const int32_t* tidx, int B, int ntags, int* hist, int* off, int* gstart, int* perm,
+                                   int* flag, cudaStream_t stream) {
+    if (B <= 0) return cudaSuccess;
+    if (ntags < 1 || ntags == INT32_MAX) return cudaErrorInvalidValue;
+    cudaError_t e = cudaMemsetAsync(hist, 0, (size_t)(ntags + 1) * sizeof(int), stream);
+    if (e != cudaSuccess) return e;
+    fa_tag_hist_kernel<<<fa_sort_grid(B), 256, 0, stream>>>(tidx, B, ntags, hist, flag);
+    fa_tag_scan_kernel<<<1, 1024, 0, stream>>>(hist, ntags, off, gstart);
+    fa_tag_scatter_kernel<<<fa_sort_grid(B), 256, 0, stream>>>(tidx, B, ntags, hist, perm);
+    return cudaGetLastError();
+}
+
+cudaError_t qf_launch_f_a_tag_correct(const int32_t* sigma, long lds, int m_bar, const int32_t* tidx, int ntags,
+                                      const int* perm, const int* off, const int* gstart, const void* tab, int word_bytes,
+                                      const uint64_t* gpow, unsigned long long q, int n, int k, int B, int64_t* u, long ldu,
+                                      int* flag, cudaStream_t stream) {
+    if (B <= 0) return cudaSuccess;
+    if (n < 1 || k < 1 || k > 64 || q < 2 || q >= (1ull << 62) || (word_bytes != 4 && word_bytes != 8) ||
+        (word_bytes == 4 && (q > (1ull << 32) || n > (1 << 14))))
+        return cudaErrorInvalidValue;
+    bool fits = false;
+    cudaError_t e = fa_smem_fits(n, &fits);
+    if (e != cudaSuccess) return e;
+    if (!fits) return cudaErrorInvalidValue;
+    const int threads = n >= 512 ? 512 : (n + 31) / 32 * 32;
+    const size_t smem = (size_t)n * FA_G * sizeof(uint64_t);
+    const uint64_t magic = qf_barrett_magic(q);
+    // groups: sum_t ceil(c_t / G) <= ceil(B / G) + (tags present) -- CTAs past the count the sort wrote exit at once
+    const long grid = FA_G == 1 ? (long)B : (long)(B + FA_G - 1) / FA_G + std::min(ntags, B);
+    if (word_bytes == 4) {
+        if (smem > 48 * 1024 &&
+            (e = cudaFuncSetAttribute(fa_tag_correct_kernel<uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+            return e;
+        fa_tag_correct_kernel<uint32_t><<<(unsigned)grid, threads, smem, stream>>>(sigma, lds, m_bar, tidx, ntags, perm, off, gstart,
+                                                                        (const uint32_t*)tab, gpow, (uint64_t)q, magic, n, k,
+                                                                        u, ldu, flag);
+    } else {
+        if (smem > 48 * 1024 &&
+            (e = cudaFuncSetAttribute(fa_tag_correct_kernel<uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+            return e;
+        fa_tag_correct_kernel<uint64_t><<<(unsigned)grid, threads, smem, stream>>>(sigma, lds, m_bar, tidx, ntags, perm, off, gstart,
+                                                                        (const uint64_t*)tab, gpow, (uint64_t)q, magic, n, k,
+                                                                        u, ldu, flag);
+    }
+    return cudaGetLastError();
+}

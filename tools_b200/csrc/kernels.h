@@ -284,6 +284,33 @@ cudaError_t qf_launch_tag_syndrome(const int64_t* V, long ldv, const double* P, 
                                    int ntags, const void* tab, const void* h0, int word_bytes, const uint64_t* gpow,
                                    unsigned long long q, int n, int k, int B, int64_t* out, long ldout, int* flag,
                                    cudaStream_t stream);
+// f_a tag table (setup.cu): tab[t] = (tags[t] - H_0) mod q column-major (count x n x n words of word_bytes = 4 or 8) from
+// int64 tags (count x n x n, any sign); h0: n x n residues row-major, NULL means H_0 = I
+cudaError_t qf_launch_tag_diff_pack(const int64_t* tags, int count, int n, unsigned long long q, const uint64_t* h0,
+                                    int word_bytes, void* tab, cudaStream_t stream);
+// per-target tag of f_a (elementwise.cu): targets are grouped by tag into groups of at most QF_F_A_TAG_GROUP, one CTA per
+// group, so that a word of the table serves every target of the group.  The library is built with 8; the value 1 (one
+// target per CTA, no sort) exists for the comparison build of scripts/bench_f_a_tagged.py.
+#ifndef QF_F_A_TAG_GROUP
+#define QF_F_A_TAG_GROUP 8
+#endif
+// Counting sort of the tag indices of B targets: hist, off and gstart hold ntags + 1 ints each; afterwards perm (B ints)
+// lists the targets tag by tag, off[t] is where tag t starts in perm (off[ntags]: indices outside the table) and gstart[t]
+// its first group (gstart[ntags]: the number of groups).  An index outside [0, ntags) sets *flag |= QF_FLAG_TAG_INDEX.
+// Not used when QF_F_A_TAG_GROUP = 1.
+// *ok = 1 when the correction kernel runs for this n and k on the current device (k <= 64, n <= 2^14, and its static plus
+// dynamic shared memory fit the per-block opt-in limit: n <= 3631 at QF_F_A_TAG_GROUP = 8 on sm_100a)
+cudaError_t qf_f_a_tag_supported(int n, int k, int* ok);
+cudaError_t qf_launch_f_a_tag_sort(const int32_t* tidx, int B, int ntags, int* hist, int* off, int* gstart, int* perm,
+                                   int* flag, cudaStream_t stream);
+// u[b] += D_t G sigma[b][m_bar:] mod q for t = tidx[b] (in place, u[b] = A sigma[b] from f_a); tab: the table of
+// qf_launch_tag_diff_pack; gpow: base^s mod q, s < k <= 64; word_bytes 4 needs q <= 2^32.  With QF_F_A_TAG_GROUP > 1 it
+// reads the output of qf_launch_f_a_tag_sort (tidx unused); with 1 it reads tidx and flags an index outside the table.
+// Rows of such indices are left as A sigma.
+cudaError_t qf_launch_f_a_tag_correct(const int32_t* sigma, long lds, int m_bar, const int32_t* tidx, int ntags,
+                                      const int* perm, const int* off, const int* gstart, const void* tab, int word_bytes,
+                                      const uint64_t* gpow, unsigned long long q, int n, int k, int B, int64_t* u, long ldu,
+                                      int* flag, cudaStream_t stream);
 
 // polynomial arithmetic of the ring short basis (setup.cu): P[2][2][n], Q[k][2][n]
 cudaError_t qf_launch_ring_basis_polys(const int32_t* e, const int32_t* r, const int32_t* w, const int64_t* sk, int n, int k,

@@ -533,7 +533,29 @@ __global__ void tag_pack_kernel(const uint64_t* __restrict__ M, int count, int n
     }
 }
 inline int tag_grid(long long work) { return (int)std::min<long long>((work + 255) / 256, 148LL * 16); }
+
+// f_a tag table (qf_set_f_a_tags): tab[t][j][i] = (tags[t][i][j] - H_0[i][j]) mod q
+template <typename W>
+__global__ void tag_diff_pack_kernel(const int64_t* __restrict__ tags, int count, int n, uint64_t q, const uint64_t* __restrict__ h0,
+                                     W* __restrict__ tab) {
+    const long nn = (long)n * n, total = (long)count * nn;
+    for (long x = blockIdx.x * (long)blockDim.x + threadIdx.x; x < total; x += (long)gridDim.x * blockDim.x) {
+        const long t = x / nn, rem = x - t * nn, j = rem / n, i = rem - j * n;
+        const long long h = tags[t * nn + i * n + j] % (long long)q;
+        const uint64_t v = (uint64_t)(h < 0 ? h + (long long)q : h), z = h0 ? h0[i * n + j] : (i == j ? 1 : 0);
+        tab[x] = (W)(v >= z ? v - z : v + (q - z));
+    }
+}
 }  // namespace
+
+cudaError_t qf_launch_tag_diff_pack(const int64_t* tags, int count, int n, unsigned long long q, const uint64_t* h0,
+                                    int word_bytes, void* tab, cudaStream_t stream) {
+    if (n < 1 || count < 1 || q < 2 || (word_bytes != 4 && word_bytes != 8)) return cudaErrorInvalidValue;
+    const int grid = tag_grid((long long)count * n * n);
+    if (word_bytes == 4) tag_diff_pack_kernel<uint32_t><<<grid, 256, 0, stream>>>(tags, count, n, (uint64_t)q, h0, (uint32_t*)tab);
+    else tag_diff_pack_kernel<uint64_t><<<grid, 256, 0, stream>>>(tags, count, n, (uint64_t)q, h0, (uint64_t*)tab);
+    return cudaGetLastError();
+}
 
 cudaError_t qf_launch_tag_build(const int64_t* tags, int count, int n, unsigned long long q, uint64_t* M, cudaStream_t stream) {
     if (n < 1 || count < 1 || q < 2) return cudaErrorInvalidValue;

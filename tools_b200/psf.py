@@ -64,6 +64,7 @@ class _PSFBase:
         self._a_id = None
         self._td_id = None
         self._tags_id = None  # tag table on the device (PSFPerturbation); dropped there with every key / trapdoor install
+        self._fa_tags_id = None  # (tags, h0) of the f_a tag table on the device; dropped there whenever A changes
         self._keep = None
 
     # -- PSF::samp_d ------------------------------------------------------------------------
@@ -105,6 +106,41 @@ class _PSFBase:
         u = np.empty((b, self.n), dtype=np.int64)
         flags = np.empty(b, dtype=np.uint8)
         st = self.ctx.status(fn, _ffi.ptr(s), b, _ffi.ptr(u), _ffi.ptr(flags))
+        if st not in (_ffi.QF_OK, _ffi.QF_ERR_NOT_IN_DOMAIN):
+            raise QfError(st, self.ctx._lib.qf_last_error(self.ctx._h).decode())
+        ok = flags.astype(bool) & ~oob
+        if strict and not ok.all():
+            raise NotInDomain(_ffi.QF_ERR_NOT_IN_DOMAIN, "sigma is not in the domain D_n")
+        return u, ok
+
+    def f_a_tagged_batch(self, a, tags, sigmas: np.ndarray, tag_idx, h0=None, strict: bool = True):
+        """f_a with a tag per target (classical contexts): u[b] = A_t sigma[b] with A_t = a + [0 | (H_t - H_0) G],
+        H_t = tags[tag_idx[b]], for a key a = [A_bar | H_0 G - A_bar R] (h0 = H_0, None: I; H_0 = 0 is allowed).  That is
+        the key gen_trapdoor(A_bar, R, H_t) gives, evaluated from a alone: no trapdoor is needed and no tag is inverted.
+        tags: T x n x n, h0: n x n (entries taken mod q); the table (qf_set_f_a_tags) is cached on the device by the
+        identity of tags and h0 until the key on the device changes: the device drops the table there, and every place
+        here that installs or rewrites A resets _fa_tags_id.  tag_idx: B indices in [0, T).  Returns (u, in_domain) as
+        f_a_batch does."""
+        self._install_a(a)
+        key = self._fa_tags_id
+        if key is None or key[0] is not tags or key[1] is not h0:
+            t = np.asarray(tags)
+            tg = np.ascontiguousarray(np.array(t % self.gp.q, dtype=np.int64) if t.dtype == object else t, dtype=np.int64)
+            assert tg.ndim == 3 and tg.shape[1:] == (self.n, self.n) and tg.shape[0] >= 1
+            hg = None
+            if h0 is not None:
+                h = np.asarray(h0)
+                hg = np.ascontiguousarray(np.array(h % self.gp.q, dtype=np.int64) if h.dtype == object else h, dtype=np.int64)
+                assert hg.shape == (self.n, self.n)
+            self.ctx.call("qf_set_f_a_tags", _ffi.ptr(tg), tg.shape[0], _ffi.ptr(hg))
+            self._fa_tags_id = (tags, h0)
+        s, oob = _domain_i32(sigmas, self._domain_shape)
+        ti = np.ascontiguousarray(tag_idx, dtype=np.int32)
+        b = s.shape[0]
+        assert ti.shape == (b,)
+        u = np.empty((b, self.n), dtype=np.int64)
+        flags = np.empty(b, dtype=np.uint8)
+        st = self.ctx.status("qf_f_a_tagged", _ffi.ptr(s), _ffi.ptr(ti), b, _ffi.ptr(u), _ffi.ptr(flags))
         if st not in (_ffi.QF_OK, _ffi.QF_ERR_NOT_IN_DOMAIN):
             raise QfError(st, self.ctx._lib.qf_last_error(self.ctx._h).decode())
         ok = flags.astype(bool) & ~oob
@@ -157,7 +193,7 @@ class PSFGPV(_PSFBase):
         if self._a_id is not a:
             aa = np.ascontiguousarray(a, dtype=np.int64)  # keep alive across the call
             self.ctx.call("qf_set_a", _ffi.ptr(aa))
-            self._a_id, self._td_id, self._tags_id = a, None, None
+            self._a_id, self._td_id, self._tags_id, self._fa_tags_id = a, None, None, None
 
     def _install_td(self, a, td):
         if self._td_id is not td:
@@ -324,7 +360,7 @@ class PSFPerturbation(_PSFBase):
         tg = None if tag is None else self._tag_words(tag)
         a_new = np.empty((self.n, self.m), dtype=np.int64)
         self.ctx.call("qf_set_tag", _ffi.ptr(tg), _ffi.ptr(a_new))
-        self._a_id = a_new
+        self._a_id, self._fa_tags_id = a_new, None  # qf_set_tag rewrote A: the f_a table is gone
         return a_new
 
     def set_tag_table(self, a, td, tags):
@@ -374,7 +410,7 @@ def _trap_gen_classical(psf, seed):
     a = np.empty((gp.n, gp.m), dtype=np.int64)
     r = np.empty((gp.m_bar, gp.n * gp.k), dtype=np.int8)
     psf.ctx.call("qf_trap_gen", _seed(seed), _ffi.ptr(a), _ffi.ptr(r))
-    psf._td_id = psf._tags_id = None
+    psf._td_id = psf._tags_id = psf._fa_tags_id = None
     return a, r
 
 
@@ -417,7 +453,7 @@ class PSFGPVRing(_PSFBase):
             aa = np.ascontiguousarray(a, dtype=np.int64)
             assert aa.shape == (self.gp.k + 2, self.gp.n)
             self.ctx.call("qf_ring_set_a", _ffi.ptr(aa))
-            self._a_id, self._td_id = a, None
+            self._a_id, self._td_id, self._fa_tags_id = a, None, None
 
     def _install_td(self, a, td):
         if self._td_id is not td:
@@ -467,5 +503,5 @@ class PSFGPVRing(_PSFBase):
         ee = np.ascontiguousarray(e, dtype=np.int32)
         assert ab.shape == (gp.n,) and rr.shape == (gp.k, gp.n) and ee.shape == (gp.k, gp.n)
         self.ctx.call("qf_ring_trap_gen_from", _ffi.ptr(ab), _ffi.ptr(rr), _ffi.ptr(ee), _ffi.ptr(a))
-        self._a_id, self._td_id = a, None
+        self._a_id, self._td_id, self._fa_tags_id = a, None, None
         return a
