@@ -113,17 +113,28 @@ qf_status qf_set_trapdoor_perturbation(qf_ctx* ctx, const int8_t* r, const doubl
  * and the gadget basis stay installed; every device copy of A and H^-1 are replaced.  QF_ERR_INVALID on a context of
  * another kind, QF_ERR_NO_KEY without key and trapdoor, QF_ERR_INVALID when the installed key was not recognised as a
  * G-trapdoor for the installed R, and QF_ERR_INVALID for a tag H' without a unit pivot (the key and its tag then stay as
- * they were). */
+ * they were).  PSFGPV contexts switch tags with qf_gpv_set_tag. */
 qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out);
-/* Tag table for samp_p with a tag per target (PSFPerturbation): one trapdoor R serves the keys
- * A_t = [A_bar | H_t G - A_bar R] of many tags in one batch (IBE key extraction, per-message tags).  tags: ntags x n x n
- * (host), entries taken mod q (negatives allowed), relative to the installed (A_bar, R); the installed key may itself be
- * tagged (any H_0).  H_t^-1 is computed on the device (Gauss-Jordan with unit pivots, as qf_set_tag).  QF_ERR_INVALID on a
- * context of another kind, for ntags < 1 or tags == NULL, when the installed key was not recognised as a G-trapdoor for
+/* Switch the tag of the installed PSFGPV key without re-installing the trapdoor: A = [A_bar | H G - A_bar R] becomes
+ * [A_bar | H' G - A_bar R] (A[:, m_bar:] += (H' - H) G mod q), bit-identical to qf_trap_gen_from(A_bar, R, H').  The GSO of
+ * the short basis does not depend on the tag, so the fp64 matrices derived from it stay on the device; everything else is
+ * what qf_set_a(A') + qf_set_trapdoor_gpv(S_H') builds.  tag: n x n (host), entries taken mod q; NULL means H' = I.
+ * a_out: the new A, n x m (host), may be NULL.  s_out: the short basis for the installed R and H', m x m (host),
+ * bit-identical to qf_gen_short_basis_tagged(R, H'), may be NULL.  Needs the two-phase recursion (a G-trapdoor key and its
+ * basis from qf_gen_short_basis_tagged, dim above the tensor-core threshold): QF_ERR_INVALID otherwise, also without a key,
+ * on a context of another kind, and for an H' without a unit pivot (nothing then changes).  Drops the f_a tag table and
+ * keeps the samp_p tag table. */
+qf_status qf_gpv_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out, int64_t* s_out);
+/* Tag table for samp_p with a tag per target (PSFPerturbation, and PSFGPV on the two-phase recursion): one trapdoor serves
+ * the keys A_t = [A_bar | H_t G - A_bar R] of many tags in one batch (IBE key extraction, per-message tags).  tags:
+ * ntags x n x n (host), entries taken mod q (negatives allowed), relative to the installed (A_bar, R); the installed key may
+ * itself be tagged (any H_0).  H_t^-1 is computed on the device (Gauss-Jordan with unit pivots, as qf_set_tag).
+ * QF_ERR_INVALID on a ring context, on a PSFGPV context whose key and trapdoor do not run the two-phase recursion (no key
+ * included), for ntags < 1 or tags == NULL, when the installed PSFPerturbation key was not recognised as a G-trapdoor for
  * the installed R, and when a tag has no unit pivot (qf_last_error names its index; the previous table then stays);
- * QF_ERR_NO_KEY without key and trapdoor.  The table is dropped when a key or trapdoor is installed (qf_set_a,
- * qf_trap_gen, qf_trap_gen_from, qf_set_trapdoor_perturbation) and kept by qf_set_tag.  Device memory: ntags n^2 words of
- * 4 bytes (q <= 2^32) or 8 bytes. */
+ * QF_ERR_NO_KEY without PSFPerturbation key and trapdoor.  The table is dropped when a key or trapdoor is installed
+ * (qf_set_a, qf_trap_gen, qf_trap_gen_from, qf_set_trapdoor_perturbation, qf_set_trapdoor_gpv) and kept by qf_set_tag and
+ * qf_gpv_set_tag.  Device memory: ntags n^2 words of 4 bytes (q <= 2^32) or 8 bytes. */
 qf_status qf_set_tag_table(qf_ctx* ctx, const int64_t* tags, int64_t ntags);
 /* Tag table for f_a with a tag per target (PSFGPV and PSFPerturbation): for the installed key A = [A_bar | H_0 G - A_bar R]
  * and tags H_t, A_t := A + [0 | (H_t - H_0) G] is the key of tag t, [A_bar | H_t G - A_bar R].  tags: ntags x n x n, h0:
@@ -132,7 +143,8 @@ qf_status qf_set_tag_table(qf_ctx* ctx, const int64_t* tags, int64_t ntags);
  * singular tags are allowed; R is not known here, so A_t is defined by the formula and not checked against A_bar.  Stores
  * D_t = H_t - H_0 mod q on the device: ntags n^2 words of 4 bytes (q <= 2^32) or 8 bytes, plus 3 (ntags + 1) ints.
  * QF_ERR_INVALID on a ring context and for ntags < 1 or tags == NULL; QF_ERR_NO_KEY without a key.  The table is dropped
- * whenever A changes (qf_set_a, qf_trap_gen, qf_trap_gen_from, qf_set_tag) and is independent of qf_set_tag_table. */
+ * whenever A changes (qf_set_a, qf_trap_gen, qf_trap_gen_from, qf_set_tag, qf_gpv_set_tag) and is independent of
+ * qf_set_tag_table. */
 qf_status qf_set_f_a_tags(qf_ctx* ctx, const int64_t* tags, int64_t ntags, const int64_t* h0);
 /* gen_short_basis_for_trapdoor with tag = I (short_basis_classical.rs:54-110): the short basis
  * S_A = [[I,R],[0,I]] [[0,I],[S',W]] = [[R S', I + R W],[S', W]] of Lambda^perp(A) for the installed A and the
@@ -153,7 +165,8 @@ qf_status qf_compute_sqrt_sigma_2(qf_ctx* ctx, const int8_t* r, const double* si
  * GSO.  dim = m for QF_PSF_GPV, n*(k+2) (coefficient embedding) for QF_PSF_GPV_RING.
  * s_gso == NULL: the GSO is computed on the device (as qf_gso) and never leaves it.
  * G-trapdoor keys A = [A_bar | H G - A_bar R] with the basis of qf_gen_short_basis_tagged are recognised for the
- * identity tag and for any tag H invertible by unit pivoting: samp_p then runs the two-phase recursion on H^-1 A. */
+ * identity tag and for any tag H invertible by unit pivoting: samp_p then runs the two-phase recursion on H^-1 A.  Drops
+ * the samp_p tag table. */
 qf_status qf_set_trapdoor_gpv(qf_ctx* ctx, const int64_t* s, const double* s_gso);
 /* MatQ::gso as used at gpv.rs:91: unnormalised Gram-Schmidt of the columns of S (dim x dim) in fp64 on the
  * device (blocked Gram-Schmidt with re-orthogonalisation).  gso_out: dim x dim, host. */
@@ -212,11 +225,12 @@ qf_status qf_samp_p(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed,
 qf_status qf_samp_p_dev(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed, uint64_t first_index,
                         int32_t* e_out);
 /* samp_p with a tag per target: e[b] with A_t e[b] = u[b] mod q for t = tag_idx[b], the key of tag t of the installed tag
- * table (qf_set_tag_table).  For the same seed and first_index, row b is bit-identical to what qf_set_tag(H_t) followed by
- * qf_samp_p gives for that row.  qf_samp_p_tagged takes host pointers; targets are range-checked as in qf_samp_p and the
+ * table (qf_set_tag_table).  For the same seed and first_index, row b is bit-identical to what qf_set_tag(H_t)
+ * (PSFGPV: qf_gpv_set_tag(H_t)) followed by qf_samp_p gives for that row.  PSFGPV needs the two-phase recursion
+ * (QF_ERR_INVALID otherwise, as for qf_set_tag_table).  qf_samp_p_tagged takes host pointers; targets are range-checked as in qf_samp_p and the
  * tag indices are checked on the host before any launch (QF_ERR_INVALID outside [0, ntags)).  qf_samp_p_tagged_dev takes
  * device pointers and is asynchronous: an index outside the table is not read, its row is unspecified and the next
- * qf_synchronize returns QF_ERR_INVALID.  QF_ERR_NO_KEY without a tag table. */
+ * qf_synchronize returns QF_ERR_INVALID.  QF_ERR_NO_KEY without a tag table; QF_ERR_INVALID on a ring context. */
 qf_status qf_samp_p_tagged(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, uint64_t seed,
                            uint64_t first_index, int32_t* e_out);
 qf_status qf_samp_p_tagged_dev(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, uint64_t seed,

@@ -48,6 +48,7 @@ extern "C" {
     pub fn qf_set_a(ctx: *mut qf_ctx, a: *const i64) -> i32;
     pub fn qf_set_trapdoor_perturbation(ctx: *mut qf_ctx, r: *const i8, sqrt_sigma_2: *const f64, s_block: *const i64, s_block_gso: *const f64) -> i32;
     pub fn qf_set_tag(ctx: *mut qf_ctx, tag: *const i64, a_out: *mut i64) -> i32;
+    pub fn qf_gpv_set_tag(ctx: *mut qf_ctx, tag: *const i64, a_out: *mut i64, s_out: *mut i64) -> i32;
     pub fn qf_set_tag_table(ctx: *mut qf_ctx, tags: *const i64, ntags: i64) -> i32;
     pub fn qf_set_f_a_tags(ctx: *mut qf_ctx, tags: *const i64, ntags: i64, h0: *const i64) -> i32;
     pub fn qf_gen_short_basis(ctx: *mut qf_ctx, r: *const i8, s_out: *mut i64) -> i32;

@@ -142,6 +142,9 @@ pub struct PSFGPVB200 {
     pub inner: PSFGPV,
     ctx: Context,
     installed: RefCell<Option<(Vec<i64>, Vec<i64>)>>, // (A, S) words of the installed key
+    /// number of tags in the samp_p tag table on the device (qf_set_tag_table); the device drops it with every key or
+    /// trapdoor install and keeps it across set_tag
+    installed_tags: RefCell<Option<usize>>,
     fa_tags: FaTags,
     seed: RefCell<u64>,
 }
@@ -166,6 +169,7 @@ impl PSFGPVB200 {
             inner,
             ctx: Context::new(&params, device)?,
             installed: RefCell::new(None),
+            installed_tags: RefCell::new(None),
             fa_tags: RefCell::new(None),
             seed: RefCell::new(seed),
         })
@@ -195,6 +199,78 @@ impl PSFGPVB200 {
         let gso = matq_to_f64(&td.1);
         self.ctx.check(unsafe { qf_set_trapdoor_gpv(self.ctx.raw, sw.as_ptr(), gso.as_ptr()) }, "qf_set_trapdoor_gpv");
         *self.installed.borrow_mut() = Some((aw, sw));
+        *self.installed_tags.borrow_mut() = None;
+    }
+
+    /// Tag switch without a new trapdoor install, for a key `a = [A_bar | H G - A_bar R]` (gen_trapdoor with a tag,
+    /// gadget_classical.rs:56-68) and its trapdoor `td = (S_H, GSO)` on the two-phase recursion: returns
+    /// `(a', (S_H', td.1))` with `a' = [A_bar | H' G - A_bar R]` for `tag` = H' (equal to gen_trapdoor(A_bar, R, H')) and
+    /// `S_H'` equal to gen_short_basis_for_trapdoor(H', a', R).  The GSO does not depend on the tag, so it is kept and
+    /// nothing is re-installed: the pair is recorded as the installed key (qf_gpv_set_tag).  The samp_p tag table stays;
+    /// the f_a tag table is dropped.  Panics off the two-phase recursion and when H' has no unit pivot (the reference
+    /// panics in `MatZq::inverse`).
+    pub fn set_tag(&self, a: &MatZq, td: &(MatZ, MatQ), tag: &MatZq) -> (MatZq, (MatZ, MatQ)) {
+        let (n, m) = (self.n(), self.m());
+        assert_eq!((tag.get_num_rows(), tag.get_num_columns()), (n as i64, n as i64), "tag must be n x n");
+        self.install(a, td);
+        let tw = matzq_to_words(tag);
+        let mut aw = vec![0i64; n * m];
+        let mut sw = vec![0i64; m * m];
+        self.ctx.check(unsafe { qf_gpv_set_tag(self.ctx.raw, tw.as_ptr(), aw.as_mut_ptr(), sw.as_mut_ptr()) }, "qf_gpv_set_tag");
+        let q = Z::from(&self.inner.gp.q);
+        let mut a_new = MatZq::new(n as i64, m as i64, &q);
+        for i in 0..n {
+            for j in 0..m {
+                a_new.set_entry(i as i64, j as i64, Z::from(aw[i * m + j])).unwrap();
+            }
+        }
+        let mut s_new = MatZ::new(m as i64, m as i64);
+        for i in 0..m {
+            for j in 0..m {
+                s_new.set_entry(i as i64, j as i64, Z::from(sw[i * m + j])).unwrap();
+            }
+        }
+        *self.installed.borrow_mut() = Some((aw, sw));
+        *self.fa_tags.borrow_mut() = None; // qf_gpv_set_tag rewrote A
+        (a_new, (s_new, td.1.clone()))
+    }
+
+    /// Installs the tag table for samp_p with a tag per target: `tags` (T matrices, n x n each, relative to the key `a` =
+    /// [A_bar | H_0 G - A_bar R] of any tag H_0 and its trapdoor `td` on the two-phase recursion).  H_t^-1 is computed on
+    /// the device (qf_set_tag_table).  The table stays installed until a key or trapdoor is installed; `set_tag` keeps
+    /// it.  Panics off the two-phase recursion and when a tag has no unit pivot.
+    pub fn set_tag_table(&self, a: &MatZq, td: &(MatZ, MatQ), tags: &[MatZq]) {
+        let n = self.n();
+        assert!(!tags.is_empty(), "at least one tag");
+        self.install(a, td);
+        let mut tw = Vec::with_capacity(tags.len() * n * n);
+        for tag in tags {
+            assert_eq!((tag.get_num_rows(), tag.get_num_columns()), (n as i64, n as i64), "tag must be n x n");
+            tw.extend(matzq_to_words(tag));
+        }
+        self.ctx.check(unsafe { qf_set_tag_table(self.ctx.raw, tw.as_ptr(), tags.len() as i64) }, "qf_set_tag_table");
+        *self.installed_tags.borrow_mut() = Some(tags.len());
+    }
+
+    /// samp_p with a tag per target, against the table of `set_tag_table`: `us[b]` is sampled under
+    /// `[A_bar | H_t G - A_bar R]` with `H_t = tags[tag_of[b]]`, in one batch.  Row b equals what `set_tag(H_t)` followed
+    /// by `samp_p_batch` gives for it with the same seed (qf_samp_p_tagged).  Panics when no table is installed for this
+    /// key and trapdoor or an index is out of range.
+    pub fn samp_p_tagged_batch(&self, a: &MatZq, td: &(MatZ, MatQ), us: &[MatZq], tag_of: &[usize], seed: u64) -> Vec<MatZ> {
+        let (n, m) = (self.n(), self.m());
+        assert_eq!(us.len(), tag_of.len(), "one tag index per target");
+        self.install(a, td);
+        let ntags = (*self.installed_tags.borrow()).expect("no tag table installed for this key and trapdoor (set_tag_table)");
+        let mut uw = Vec::with_capacity(us.len() * n);
+        for u in us {
+            assert!(u.is_column_vector() && u.get_num_rows() as usize == n, "target must be an n x 1 vector");
+            uw.extend(matzq_to_words(u));
+        }
+        let idx: Vec<i32> = tag_of.iter().map(|t| { assert!(*t < ntags, "tag index out of range"); *t as i32 }).collect();
+        let mut e = vec![0i32; us.len() * m];
+        let st = unsafe { qf_samp_p_tagged(self.ctx.raw, uw.as_ptr(), idx.as_ptr(), us.len() as i64, seed, 0, e.as_mut_ptr()) };
+        self.ctx.check(st, "qf_samp_p_tagged");
+        e.chunks(m).map(column_from_i32).collect()
     }
     /// `gen_short_basis_for_trapdoor(params, tag, a, r)` (short_basis_classical.rs:54-110) on the device for the key `a`
     /// of this context's parameters: W = digits of -tag^-1 a[:, :m_bar] with tag^-1 and the products computed on the
@@ -207,6 +283,7 @@ impl PSFGPVB200 {
         let (aw, tw) = (matzq_to_words(a), matzq_to_words(tag));
         let r8: Vec<i8> = matz_to_words(r).into_iter().map(|v| i8::try_from(v).expect("R entries must fit i8")).collect();
         assert_eq!(r8.len(), m_bar * (m - m_bar), "R must be m_bar x n k");
+        *self.installed_tags.borrow_mut() = None;
         *self.installed.borrow_mut() = None; // qf_set_a drops the installed trapdoor
         *self.fa_tags.borrow_mut() = None;
         self.ctx.check(unsafe { qf_set_a(self.ctx.raw, aw.as_ptr()) }, "qf_set_a");
@@ -234,6 +311,7 @@ impl PSFGPVB200 {
             || self.fa_tags.borrow().as_ref().map(|(a0, _, _)| *a0 == aw).unwrap_or(false);
         if !same {
             self.ctx.check(unsafe { qf_set_a(self.ctx.raw, aw.as_ptr()) }, "qf_set_a");
+            *self.installed_tags.borrow_mut() = None;
             *self.installed.borrow_mut() = None;
             *self.fa_tags.borrow_mut() = None;
         }
@@ -293,6 +371,7 @@ impl PSF for PSFGPVB200 {
         let m_bar = i64::try_from(&self.inner.gp.m_bar).unwrap() as usize;
         let (mut a, mut r) = (vec![0i64; n * m], vec![0i8; m_bar * (m - m_bar)]);
         self.ctx.check(unsafe { qf_trap_gen(self.ctx.raw, self.next_seed(), a.as_mut_ptr(), r.as_mut_ptr()) }, "qf_trap_gen");
+        *self.installed_tags.borrow_mut() = None;
         *self.installed.borrow_mut() = None; // qf_trap_gen installed a new key: whatever trapdoor was cached is gone
         *self.fa_tags.borrow_mut() = None;
         let mut s = vec![0i64; m * m];
@@ -364,6 +443,7 @@ impl PSFBatch for PSFGPVB200 {
         let same = self.installed.borrow().as_ref().map(|(a0, _)| *a0 == aw).unwrap_or(false);
         if !same {
             self.ctx.check(unsafe { qf_set_a(self.ctx.raw, aw.as_ptr()) }, "qf_set_a");
+            *self.installed_tags.borrow_mut() = None;
             *self.installed.borrow_mut() = None;
             *self.fa_tags.borrow_mut() = None;
         }

@@ -47,6 +47,7 @@ SIGNATURES = {
     "qf_set_a": (_i32, [_vp, _vp]),
     "qf_set_trapdoor_perturbation": (_i32, [_vp, _vp, _vp, _vp, _vp]),
     "qf_set_tag": (_i32, [_vp, _vp, _vp]),
+    "qf_gpv_set_tag": (_i32, [_vp, _vp, _vp, _vp]),
     "qf_set_tag_table": (_i32, [_vp, _vp, _i64]),
     "qf_set_f_a_tags": (_i32, [_vp, _vp, _i64, _vp]),
     "qf_compute_sqrt_sigma_2": (_i32, [_vp, _vp, _vp, _vp]),

@@ -105,11 +105,12 @@ struct qf_ctx {
     long ld_mb = 0;
     double sqrt_beta = 0, xb_fscale = 0;
     int xb_limbs = 3;
-    // the installed key is A = [A_bar | H G - A_bar R] for the installed R (recognised by qf_set_trapdoor_perturbation,
-    // replaced by qf_set_tag): pert_tag = H mod q (n x n).  For H != I, key_tagged is set and v = u - A p becomes
-    // v' = H^-1 v before the gadget sampler (digit planes of H^-1 in dHinvl).
+    // the installed key is A = [A_bar | H G - A_bar R] for the installed R (recognised by qf_set_trapdoor_perturbation and,
+    // on the two-phase recursion, qf_set_trapdoor_gpv; replaced by qf_set_tag / qf_gpv_set_tag): key_tag = H mod q (n x n).
+    // For H != I, key_tagged is set and v = u - A p becomes v' = H^-1 v before the gadget sampler (digit planes of H^-1 in
+    // dHinvl).
     bool pert_gadget_key = false;
-    std::vector<uint64_t> pert_tag;
+    std::vector<uint64_t> key_tag;
     // nearest-plane engine (GPV, ring)
     bool has_np = false;
     int npiv = 0;
@@ -186,8 +187,9 @@ struct qf_ctx {
     int tag_ulimbs = 0;
     long ldk_n = 0;
     Dev dHinvl, dAbpl, dTagU, dTagUl, dTagTmp;
-    // Tag table of PSFPerturbation (qf_set_tag_table): H_t^-1 mod q for tag_count tags, each n x n column-major in words
-    // of tag_word bytes (4 when q <= 2^32), relative to the installed (A_bar, R) and dropped with the key or trapdoor.
+    // Tag table of samp_p (qf_set_tag_table; PSFPerturbation, and PSFGPV on the two-phase recursion): H_t^-1 mod q for
+    // tag_count tags, each n x n column-major in words of tag_word bytes (4 when q <= 2^32), relative to the installed
+    // (A_bar, R) and dropped with the key or trapdoor.
     // dTagH0: the installed key's tag H_0 in the same layout while the key is tagged; dTagGpow: base^s mod q, s < k;
     // io_t: tag indices of the host path's chunks (two slots, as io_b / io_b2).
     int64_t tag_count = 0;
@@ -1055,7 +1057,11 @@ qf_status samp_p_np1_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t se
 // precision against a 31-bit z_1, and replaces the nk x m_bar product W z_2 by the n x m_bar product A_bar z_2:
 // 9-12 digit-pair products per useful MAC instead of 18-25.
 // ---------------------------------------------------------------------------
-qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t seed, uint64_t first, int32_t* dE) {
+// dTidx (optional, device): the tag index of every target of the chunk in the installed tag table (qf_samp_p_tagged).  The
+// tag enters only between the phases (DESIGN 4.3): for A_t = [A_bar | H_t G - A_bar R], g3 = digits(h_t) with
+// h_t = H_t^-1 (u - A_bar z2) mod q, the same integer vector as after qf_gpv_set_tag(H_t); everything else is tag-independent.
+qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t seed, uint64_t first, int32_t* dE,
+                           const int32_t* dTidx = nullptr) {
     const long D = ctx->dim, ldD = ctx->ld_dim, C = ctx->chunk, nk = ctx->nk, mb = ctx->m_bar, n = ctx->n;
     const long ldk = ctx->ldk_dim, plane = C * ldk, ldnk = ctx->ld_nk, ldk_nk = ctx->ldk_nk;
     const int nz_m = (int)((C + 127) / 128), nz_kb = (int)(ldk / 128);
@@ -1089,22 +1095,30 @@ qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t se
     QF_TRY(np_block(ctx, T, Z, Bc, nk, D, NP_TOP, 0, seed, first));
 
     // ---- tagged key: the recursion runs on H^-1 A, so its target is u' = H^-1 u mod q (phase 1 never reads the target)
+    const bool abar_tagged = ctx->key_tagged && !dTidx;
     const int64_t* ub = dUin;
-    if (ctx->key_tagged) QF_TRY(tag_targets(ctx, dUin, Bc, &ub));
+    if (abar_tagged) QF_TRY(tag_targets(ctx, dUin, Bc, &ub));
     // ---- h = (u - A_bar z2) mod q, exact (A_bar = the first m_bar columns of the installed digit planes of A; for a tagged
-    // key u' - A_bar' z2 with the digit planes of A_bar' = H^-1 A_bar)
+    // key u' - A_bar' z2 with the digit planes of A_bar' = H^-1 A_bar).  With a tag per target: w = u - A_bar z2 whatever
+    // the installed tag, then h_t = H_t^-1 w per target.
+    if (dTidx) CK(ctx->dTagU.ensure((size_t)C * n * 8));
     {
-        const long ldw = ctx->key_tagged ? ctx->ldk_mb : ldk;
+        const long ldw = abar_tagged ? ctx->ldk_mb : ldk;
         I8GemmArgs g{};
         g.x = zp + nk; g.ldx = ldk; g.x_plane = plane;
-        g.w = ctx->key_tagged ? ctx->dAbpl.p : ctx->dAl.p; g.ldw = ldw; g.w_plane = n * ldw;
+        g.w = abar_tagged ? ctx->dAbpl.p : ctx->dAl.p; g.ldw = ldw; g.w_plane = n * ldw;
         g.LX = L; g.LW = ctx->a_limbs; g.w_signed = 0;
         g.B = Bc; g.N = (int)n; g.K = (int)mb;
-        g.out_kind = 0; g.sign = -1; g.q = ctx->prm.q; g.base = ub; g.ldbase = n; g.out = H; g.ldout = n;
+        g.out_kind = 0; g.sign = -1; g.q = ctx->prm.q; g.base = ub; g.ldbase = n;
+        g.out = dTidx ? ctx->dTagU.as<int64_t>() : H; g.ldout = n;
         g.flag = flag;
         g.x_nz = ctx->dNz.as<uint8_t>(); g.nz_m_tiles = nz_m; g.nz_kb_total = nz_kb; g.nz_kb_off = (int)(nk / 128);
         QF_TRY(gemm_i8_gated(ctx, g, gate_z2));
     }
+    if (dTidx)
+        LAUNCH(qf_launch_tag_syndrome(ctx->dTagU.as<int64_t>(), n, nullptr, 0, 0, dTidx, (int)ctx->tag_count, ctx->dTagTab.p,
+                                      nullptr, ctx->tag_word, nullptr, ctx->prm.q, (int)n, (int)ctx->k, Bc, H, n, flag,
+                                      ctx->stream));
     // ---- g3 = digits(h): one s8 plane (the x operand of its centre map) and, as fp64, the start of e_bot = g3 + S' z1
     // (fused tail: e_bot is formed in one pass from z1 and the g3 plane -- needs 16-byte aligned int32 rows; otherwise e_bot is
     // accumulated in fp64 as in the one-pass form)
@@ -1174,8 +1188,11 @@ qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t se
     return QF_OK;
 }
 
-qf_status samp_p_np_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t seed, uint64_t first, int32_t* dE) {
-    return ctx->two_phase ? samp_p_np2_chunk(ctx, dUin, Bc, seed, first, dE) : samp_p_np1_chunk(ctx, dUin, Bc, seed, first, dE);
+// dTidx (tag per target) only with the two-phase recursion (samp_p_tagged_ready)
+qf_status samp_p_np_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t seed, uint64_t first, int32_t* dE,
+                          const int32_t* dTidx = nullptr) {
+    return ctx->two_phase ? samp_p_np2_chunk(ctx, dUin, Bc, seed, first, dE, dTidx)
+                          : samp_p_np1_chunk(ctx, dUin, Bc, seed, first, dE);
 }
 
 // find n columns of A (n x m) that form a matrix invertible over Z_q by unit pivoting and return
@@ -1695,6 +1712,7 @@ qf_status detect_gpv_structure(qf_ctx* ctx, const int64_t* s, const std::vector<
                 ctx->dHinvl.release();
             }
         }
+        if (ctx->gadget_key_ok) ctx->key_tag = std::move(kt.h);
     }
     return QF_OK;
 }
@@ -1797,6 +1815,29 @@ qf_status upload_a_cols(qf_ctx* ctx, long c0) {
     return QF_OK;
 }
 
+// PSFGPV takes a tag per target, and switches tags, only on the two-phase recursion: there the tag enters between the
+// phases alone, while the one-pass recursion reads U_12, which depends on the tag (DESIGN 4.3)
+qf_status gpv_tags_ready(qf_ctx* ctx) {
+    if (!ctx->has_np || !ctx->two_phase)
+        return ctx->fail(QF_ERR_INVALID, "PSFGPV tags need a G-trapdoor key and its basis on the two-phase recursion");
+    return QF_OK;
+}
+
+// A^-1 on the unit pivots of the classical key (find_unit_pivots) as fp64 digit matrices: the particular-solution map
+qf_status upload_ainv(qf_ctx* ctx, const std::vector<int64_t>& ainv) {
+    ctx->npiv = (int)ctx->n;
+    ctx->ainv_identity = false;
+    const int qbits = bitlen_u64(ctx->prm.q - 1);
+    int wb = exact_bits((double)ctx->prm.q * std::sqrt((double)ctx->n), ctx->n);
+    if (wb < 2) return ctx->fail(QF_ERR_UNSUPPORTED, "modulus too large for the exact particular-solution product");
+    wb = std::min(wb, qbits);
+    int nch = (qbits + wb - 1) / wb;
+    if (nch > 4) return ctx->fail(QF_ERR_UNSUPPORTED, "modulus needs more than 4 digit matrices (GPV)");
+    ctx->ainv_bits = wb; ctx->ainv_nchunks = nch;
+    ctx->ld_piv = pad16(ctx->npiv);
+    return upload_chunks(ctx, ainv.data(), ctx->n, ctx->n, ctx->ld_piv, nch, wb, ctx->dAinv);
+}
+
 // the installed key's tag H_0 into dTagH0 (column-major, tag_word words) for the per-target tag kernel; none for H_0 = I
 qf_status upload_tag_h0(qf_ctx* ctx) {
     if (!ctx->key_tagged) {
@@ -1806,7 +1847,7 @@ qf_status upload_tag_h0(qf_ctx* ctx) {
     const long n = ctx->n;
     std::vector<uint64_t> h((size_t)n * n);
     for (long i = 0; i < n; ++i)
-        for (long j = 0; j < n; ++j) h[(size_t)j * n + i] = ctx->pert_tag[(size_t)i * n + j];
+        for (long j = 0; j < n; ++j) h[(size_t)j * n + i] = ctx->key_tag[(size_t)i * n + j];
     std::vector<uint32_t> h32;
     const void* src = h.data();
     if (ctx->tag_word == 4) {
@@ -2003,7 +2044,7 @@ qf_status qf_set_trapdoor_perturbation(qf_ctx* ctx, const int8_t* r, const doubl
         ctx->pert_gadget_key = kt.form != KEY_OTHER;
         ctx->key_tagged = kt.form == KEY_TAGGED;
         ctx->tag_ulimbs = limbs_for((double)(ctx->prm.q - 1));
-        ctx->pert_tag = std::move(kt.h);
+        ctx->key_tag = std::move(kt.h);
     }
     if (l) {
         QF_TRY(upload_as_f64(ctx, l, ctx->m, ctx->m, ctx->ld_dim, ctx->dL));
@@ -2061,7 +2102,7 @@ qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out) {
     const std::vector<uint64_t> gpow = gadget_powers(ctx);
     for (long i = 0; i < n; ++i)
         for (long j = 0; j < n; ++j) {
-            const uint64_t d = (h2[(size_t)i * n + j] + q - ctx->pert_tag[(size_t)i * n + j]) % q;
+            const uint64_t d = (h2[(size_t)i * n + j] + q - ctx->key_tag[(size_t)i * n + j]) % q;
             if (!d) continue;
             for (long t = 0; t < k; ++t) {
                 int64_t& a = ctx->hA[(size_t)i * m + mb + j * k + t];
@@ -2072,10 +2113,114 @@ qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out) {
     if (ident) ctx->dHinvl.release();
     else QF_TRY(tag_planes(ctx, hinv, ctx->dHinvl));
     ctx->key_tagged = !ident;
-    ctx->pert_tag = std::move(h2);
+    ctx->key_tag = std::move(h2);
     if (ctx->tag_count) QF_TRY(upload_tag_h0(ctx));  // the tag table stays: it is relative to (A_bar, R)
     ctx->has_a = true;
     ctx->has_pert = true;
+    if (a_out) memcpy(a_out, ctx->hA.data(), (size_t)n * m * sizeof(int64_t));
+    return QF_OK;
+}
+
+// PSFGPV tag switch (DESIGN 4.3): for A = [A_bar | H G - A_bar R] with S_H installed on the two-phase recursion, the GSO of
+// S_H' is that of S_H, so U, Mt_1, M', D and their digit planes stay; what depends on H' is rebuilt here exactly as
+// qf_set_a(A') + qf_set_trapdoor_gpv(S_H') would build it: A' (host copy, the nk changed columns on the device), the key's
+// tag, H'^-1 and A_bar' = H'^-1 A_bar (digit planes), W = digits(-A_bar'), and the pivots of A' when they can differ.
+qf_status qf_gpv_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out, int64_t* s_out) {
+    if (!ctx) return QF_ERR_INVALID;
+    if (ctx->prm.kind != QF_PSF_GPV) return ctx->fail(QF_ERR_INVALID, "not a PSFGPV context (PSFPerturbation: qf_set_tag)");
+    QF_TRY(gpv_tags_ready(ctx));
+    CK(cudaSetDevice(ctx->device));
+    const long n = ctx->n, k = ctx->k, mb = ctx->m_bar, nk = ctx->nk, m = ctx->m;
+    const uint64_t q = ctx->prm.q, base = (uint64_t)ctx->prm.base;
+    // everything that can refuse runs before the context changes: H'^-1, the pivots of A', the basis for the caller
+    std::vector<uint64_t> h2((size_t)n * n);
+    std::vector<int64_t> h2w((size_t)n * n);
+    bool ident = true;
+    for (long i = 0; i < n; ++i)
+        for (long j = 0; j < n; ++j) {
+            uint64_t v = i == j ? 1 : 0;
+            if (tag) {
+                const int64_t t = tag[i * n + j] % (int64_t)q;
+                v = (uint64_t)(t < 0 ? t + (int64_t)q : t);
+            }
+            h2[(size_t)i * n + j] = v;
+            h2w[(size_t)i * n + j] = (int64_t)v;
+            ident = ident && v == (i == j ? 1u : 0u);
+        }
+    std::vector<int64_t> hinv;
+    Dev dHl;
+    if (!ident) {
+        bool ok = false;
+        QF_TRY(tag_inverse(ctx, h2.data(), hinv, &ok));
+        if (!ok) return ctx->fail(QF_ERR_INVALID, "tag is not invertible mod q (no unit pivot)");
+        QF_TRY(tag_planes(ctx, hinv, dHl));
+    }
+    // A' = A + [0 | (H' - H) G] mod q
+    std::vector<int64_t> a2 = ctx->hA;
+    const std::vector<uint64_t> gpow = gadget_powers(ctx);
+    for (long i = 0; i < n; ++i)
+        for (long j = 0; j < n; ++j) {
+            const uint64_t d = (h2[(size_t)i * n + j] + q - ctx->key_tag[(size_t)i * n + j]) % q;
+            if (!d) continue;
+            for (long t = 0; t < k; ++t) {
+                int64_t& a = a2[(size_t)i * m + mb + j * k + t];
+                a = (int64_t)(((u128)(uint64_t)a + mulmod_h(d, gpow[t], q)) % q);
+            }
+        }
+    // The pivot search walks the columns in order and stops at n pivots: when all of them lie in A_bar, which H' leaves
+    // unchanged, the search over A' makes the same choices.  Otherwise it runs again.
+    std::vector<int> piv((size_t)ctx->npiv);
+    CK(cudaMemcpy(piv.data(), ctx->dPiv.p, piv.size() * sizeof(int), cudaMemcpyDeviceToHost));
+    std::vector<int64_t> ainv;
+    const bool repivot = *std::max_element(piv.begin(), piv.end()) >= mb;
+    if (repivot && !find_unit_pivots(a2.data(), n, m, q, piv, ainv))
+        return ctx->fail(QF_ERR_UNSUPPORTED, "A has no n columns invertible over Z_q by unit pivoting");
+    if (s_out) {
+        // the basis reads A_bar only (the first m_bar columns of the installed A) and R, read back from its s8 plane
+        std::vector<int8_t> r((size_t)mb * nk);
+        CK(cudaMemcpy2D(r.data(), (size_t)nk, ctx->dRl.p, (size_t)ctx->ldk_nk, (size_t)nk, (size_t)mb, cudaMemcpyDeviceToHost));
+        QF_TRY(qf_gen_short_basis_tagged(ctx, r.data(), ident ? nullptr : h2w.data(), s_out));
+    }
+    // A_bar' = H'^-1 A_bar (reads the unchanged first m_bar columns of hA) and W = digits(-A_bar'), nk x m_bar
+    std::vector<int64_t> abt;
+    if (!ident) QF_TRY(tag_abar(ctx, dHl, abt));
+    std::vector<int64_t> w64((size_t)nk * mb), ab;
+    for (long j = 0; j < n; ++j)
+        for (long c = 0; c < mb; ++c) {
+            uint64_t v = (q - (uint64_t)(ident ? ctx->hA[(size_t)j * m + c] : abt[(size_t)c * n + j])) % q;
+            for (long t = 0; t < k; ++t) {
+                w64[(size_t)(j * k + t) * mb + c] = (int64_t)(v % base);
+                v /= base;
+            }
+        }
+    // commit.  Until the device copies are consistent again the context has no trapdoor (a CUDA error on the way leaves it so).
+    ctx->has_np = false;
+    ctx->fa_tag_count = 0; ctx->dFaTab.release();  // the f_a table is relative to A; the samp_p table to (A_bar, R): kept
+    ctx->hA.swap(a2);
+    QF_TRY(upload_a_cols(ctx, mb));
+    if (repivot) {
+        QF_TRY(upload_ainv(ctx, ainv));
+        CK(cudaMemcpy(ctx->dPiv.p, piv.data(), piv.size() * sizeof(int), cudaMemcpyHostToDevice));
+        bool piv_low = false;
+        for (int pc : piv) piv_low = piv_low || pc >= mb;
+        ctx->i2_limbs = limbs_for(8.0 * ctx->prm.s + 64.0 + (piv_low ? (double)q : 0.0));
+    }
+    QF_TRY(upload_limbs(ctx, w64.data(), nk, mb, ctx->ldk_mb, 1, false, ctx->dWl));
+    if (ident) {
+        ctx->dHinvl.release();
+        ctx->dAbpl.release();
+    } else {
+        std::swap(ctx->dHinvl.p, dHl.p);
+        std::swap(ctx->dHinvl.cap, dHl.cap);
+        ab.resize((size_t)n * mb);
+        for (long i = 0; i < n; ++i)
+            for (long c = 0; c < mb; ++c) ab[(size_t)i * mb + c] = abt[(size_t)c * n + i];
+        QF_TRY(upload_limbs(ctx, ab.data(), n, mb, ctx->ldk_mb, ctx->a_limbs, false, ctx->dAbpl));
+        ctx->tag_ulimbs = limbs_for((double)(q - 1));
+    }
+    ctx->key_tagged = !ident;
+    ctx->key_tag = std::move(h2);
+    ctx->has_np = true;
     if (a_out) memcpy(a_out, ctx->hA.data(), (size_t)n * m * sizeof(int64_t));
     return QF_OK;
 }
@@ -2087,10 +2232,16 @@ constexpr int64_t TAG_SLICE = 256;  // tags inverted per launch: 2 CTAs of 1024 
 // 16 n^2 bytes per tag, 4 MB at n = 512).  The new table replaces the old one only when every tag has been inverted.
 qf_status qf_set_tag_table(qf_ctx* ctx, const int64_t* tags, int64_t ntags) {
     if (!ctx) return QF_ERR_INVALID;
-    if (ctx->prm.kind != QF_PSF_PERTURBATION) return ctx->fail(QF_ERR_INVALID, "not a PSFPerturbation context");
+    if (ctx->prm.kind == QF_PSF_GPV) {
+        QF_TRY(gpv_tags_ready(ctx));
+    } else if (ctx->prm.kind != QF_PSF_PERTURBATION) {
+        return ctx->fail(QF_ERR_INVALID, "not a PSFGPV or PSFPerturbation context");
+    }
     if (!tags || ntags < 1) return ctx->fail(QF_ERR_INVALID, "tag table: at least one tag needed");
-    if (!ctx->has_a || !ctx->has_pert) return ctx->fail(QF_ERR_NO_KEY, "PSFPerturbation: key or trapdoor missing");
-    if (!ctx->pert_gadget_key) return ctx->fail(QF_ERR_INVALID, "the installed key is not [A_bar | H G - A_bar R] for the installed R");
+    if (ctx->prm.kind == QF_PSF_PERTURBATION) {
+        if (!ctx->has_a || !ctx->has_pert) return ctx->fail(QF_ERR_NO_KEY, "PSFPerturbation: key or trapdoor missing");
+        if (!ctx->pert_gadget_key) return ctx->fail(QF_ERR_INVALID, "the installed key is not [A_bar | H G - A_bar R] for the installed R");
+    }
     const long n = ctx->n;
     if (ctx->k > 64 || 16 * n > 227 * 1024) return ctx->fail(QF_ERR_UNSUPPORTED, "tag table: needs k <= 64 and n <= 14528");
     if (ntags > INT32_MAX) return ctx->fail(QF_ERR_INVALID, "tag table: more than 2^31 - 1 tags");
@@ -2125,7 +2276,7 @@ qf_status qf_set_tag_table(qf_ctx* ctx, const int64_t* tags, int64_t ntags) {
     CK(ctx->dTagGpow.ensure(gpow.size() * 8));
     CK(cudaMemcpyAsync(ctx->dTagGpow.p, gpow.data(), gpow.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
     ctx->tag_word = word;
-    QF_TRY(upload_tag_h0(ctx));
+    if (ctx->prm.kind == QF_PSF_PERTURBATION) QF_TRY(upload_tag_h0(ctx));  // PSFGPV's h_t does not involve H_0
     std::swap(ctx->dTagTab.p, tab.p);
     std::swap(ctx->dTagTab.cap, tab.cap);
     ctx->tag_count = ntags;
@@ -2402,6 +2553,7 @@ qf_status qf_set_trapdoor_gpv(qf_ctx* ctx, const int64_t* s, const double* sg) {
     if (ctx->prm.kind == QF_PSF_PERTURBATION) return ctx->fail(QF_ERR_INVALID, "not a GPV context");
     ctx->has_np = false;  // stays false if anything below fails half-way (pivots / A^-1 / U are overwritten in place)
     ctx->two_phase = false;
+    ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release();  // the tag table is relative to the old (A_bar, R)
     ctx->u_limbs = 7;
     CK(cudaSetDevice(ctx->device));
     const long D = ctx->dim, ld = ctx->ld_dim;
@@ -2422,17 +2574,7 @@ qf_status qf_set_trapdoor_gpv(qf_ctx* ctx, const int64_t* s, const double* sg) {
         std::vector<int64_t> ainv;
         if (!find_unit_pivots(ctx->hA.data(), ctx->n, ctx->m, ctx->prm.q, piv, ainv))
             return ctx->fail(QF_ERR_UNSUPPORTED, "A has no n columns invertible over Z_q by unit pivoting");
-        ctx->npiv = (int)ctx->n;
-        ctx->ainv_identity = false;
-        const int qbits = bitlen_u64(ctx->prm.q - 1);
-        int wb = exact_bits((double)ctx->prm.q * std::sqrt((double)ctx->n), ctx->n);
-        if (wb < 2) return ctx->fail(QF_ERR_UNSUPPORTED, "modulus too large for the exact particular-solution product");
-        wb = std::min(wb, qbits);
-        int nch = (qbits + wb - 1) / wb;
-        if (nch > 4) return ctx->fail(QF_ERR_UNSUPPORTED, "modulus needs more than 4 digit matrices (GPV)");
-        ctx->ainv_bits = wb; ctx->ainv_nchunks = nch;
-        ctx->ld_piv = pad16(ctx->npiv);
-        QF_TRY(upload_chunks(ctx, ainv.data(), ctx->n, ctx->n, ctx->ld_piv, nch, wb, ctx->dAinv));
+        QF_TRY(upload_ainv(ctx, ainv));
     }
     ctx->ld_piv = pad16(ctx->npiv);
     CK(ctx->dPiv.ensure(piv.size() * sizeof(int)));
@@ -2590,6 +2732,7 @@ qf_status qf_set_trapdoor_gpv(qf_ctx* ctx, const int64_t* s, const double* sg) {
                     CK(cudaStreamSynchronize(ctx->stream));
                 }
                 ctx->dMtP.release();
+                ctx->dS.release();  // read only by the one-pass fp64 form: qf_gpv_set_tag then has no copy of S to rewrite
             }
             // Mt_P as fixed-point digit planes (D rows x npiv columns, one scale per row): T = -Mt_P sol_P on tcgen05
             ctx->sol_limbs = limbs_for((double)ctx->prm.q);
@@ -3070,9 +3213,9 @@ static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint6
         // the targets must be residues in [0, q): checked on the device (a host loop over batch x n values would sit in
         // front of every call), reported by check_flag as QF_ERR_INVALID
         LAUNCH(qf_launch_range_check_i64(du, (size_t)Bc * ctx->n, ctx->prm.q, ctx->dFlag.as<int>(), ctx->stream));
-        QF_TRY(ctx->prm.kind == QF_PSF_PERTURBATION
-                   ? samp_p_pert_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres, tidx ? t_buf(idx) : nullptr)
-                   : samp_p_np_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres));
+        const int32_t* dt = tidx ? t_buf(idx) : nullptr;
+        QF_TRY(ctx->prm.kind == QF_PSF_PERTURBATION ? samp_p_pert_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres, dt)
+                                                    : samp_p_np_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres, dt));
         if (overlap) CK(cudaEventRecord(ctx->ev_u_used[slot], ctx->stream));
         const void* src = dres;
         if (i16) {
@@ -3104,9 +3247,10 @@ qf_status qf_samp_p_i16(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t s
     return samp_p_host(ctx, u, batch, seed, first, e_out, true);
 }
 
-// ---- samp_p with a tag per target (PSFPerturbation, installed tag table) --------------------------------------------
+// ---- samp_p with a tag per target (PSFPerturbation, PSFGPV on the two-phase recursion; installed tag table) -----------
 static qf_status samp_p_tagged_ready(qf_ctx* ctx) {
-    if (ctx->prm.kind != QF_PSF_PERTURBATION) return ctx->fail(QF_ERR_INVALID, "not a PSFPerturbation context");
+    if (ctx->prm.kind == QF_PSF_GPV) QF_TRY(gpv_tags_ready(ctx));
+    else if (ctx->prm.kind != QF_PSF_PERTURBATION) return ctx->fail(QF_ERR_INVALID, "not a PSFGPV or PSFPerturbation context");
     QF_TRY(samp_p_ready(ctx));
     if (!ctx->tag_count) return ctx->fail(QF_ERR_NO_KEY, "no tag table installed (qf_set_tag_table)");
     return QF_OK;
@@ -3133,7 +3277,10 @@ qf_status qf_samp_p_tagged_dev(qf_ctx* ctx, const int64_t* u, const int32_t* tag
     CK(cudaSetDevice(ctx->device));
     QF_TRY(samp_p_tagged_ready(ctx));
     return for_chunks(ctx, batch, [&](int64_t b0, int Bc) -> qf_status {
-        return samp_p_pert_chunk(ctx, u + b0 * ctx->n, Bc, seed, first + (uint64_t)b0, e_out + b0 * ctx->dim, tag_idx + b0);
+        const int64_t* uu = u + b0 * ctx->n;
+        int32_t* ee = e_out + b0 * ctx->dim;
+        return ctx->prm.kind == QF_PSF_PERTURBATION ? samp_p_pert_chunk(ctx, uu, Bc, seed, first + (uint64_t)b0, ee, tag_idx + b0)
+                                                    : samp_p_np_chunk(ctx, uu, Bc, seed, first + (uint64_t)b0, ee, tag_idx + b0);
     });
 }
 

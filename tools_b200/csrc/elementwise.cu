@@ -882,6 +882,7 @@ cudaError_t qf_launch_split_i64_limbs(const int64_t* in, long ldin, int8_t* plan
 }
 
 // ---- per-target tag (qf_samp_p_tagged): v'_b = H_t^-1 (v_b + H_0 y_b) - y_b mod q with y_b = G p_bot_b, t = tidx[b] ----------
+// PSFPerturbation passes p; PSFGPV's two-phase recursion passes P == nullptr (y = 0, h0 == nullptr): h_t = H_t^-1 w.
 // One CTA per target; thread i owns rows i, i + blockDim, ... .  The tables hold each n x n matrix column-major (word
 // [j][i] = M[i][j]), so at a fixed column the threads of a warp read consecutive words; y and w live in shared memory.
 // Exact for every q < 2^62 and n:
@@ -926,7 +927,7 @@ __global__ void __launch_bounds__(512) tag_syndrome_kernel(const int64_t* __rest
         if (threadIdx.x == 0 && flag) atomicOr(flag, QF_FLAG_TAG_INDEX);
         return;
     }
-    const double* pb = P + b * ldp + m_bar;
+    const double* pb = P ? P + b * ldp + m_bar : nullptr;
     const W* hi = tab + (long)t * n * n;
     if constexpr (sizeof(W) == 4) {
         uint2* ys = reinterpret_cast<uint2*>(tag_sh);  // 16-bit halves of y and w
@@ -934,7 +935,7 @@ __global__ void __launch_bounds__(512) tag_syndrome_kernel(const int64_t* __rest
         // y_i = sum_s base^s p[m_bar + i k + s] mod q: (p mod q) times the halves of base^s mod q, k <= 64 terms < 2^48
         for (int i = threadIdx.x; i < n; i += blockDim.x) {
             uint64_t a0 = 0, a1 = 0;
-            for (int s = 0; s < k; ++s) {
+            for (int s = 0; s < (P ? k : 0); ++s) {
                 const uint64_t pm = mod_i64_barrett((long long)pb[(long)i * k + s], q, magic), g = gpow[s];
                 a0 += pm * (g & 0xFFFF);
                 a1 += pm * (g >> 16);
@@ -983,7 +984,7 @@ __global__ void __launch_bounds__(512) tag_syndrome_kernel(const int64_t* __rest
         // |p| < 2^53, base^s mod q < 2^62, k <= 64 terms fit 128 bits
         for (int i = threadIdx.x; i < n; i += blockDim.x) {
             i128 acc = 0;
-            for (int s = 0; s < k; ++s) acc += (i128)(long long)pb[(long)i * k + s] * (i128)gpow[s];
+            for (int s = 0; s < (P ? k : 0); ++s) acc += (i128)(long long)pb[(long)i * k + s] * (i128)gpow[s];
             const i128 r = acc % (i128)q;
             y[i] = (uint64_t)(r < 0 ? r + (i128)q : r);
         }

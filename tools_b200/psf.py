@@ -63,7 +63,7 @@ class _PSFBase:
         self.ctx_dim = n * (k + 2) if self.kind == _ffi.QF_PSF_GPV_RING else m_bar + n * k
         self._a_id = None
         self._td_id = None
-        self._tags_id = None  # tag table on the device (PSFPerturbation); dropped there with every key / trapdoor install
+        self._tags_id = None  # samp_p tag table on the device; dropped there with every key / trapdoor install
         self._fa_tags_id = None  # (tags, h0) of the f_a tag table on the device; dropped there whenever A changes
         self._keep = None
 
@@ -174,7 +174,51 @@ class _PSFBase:
         return self.samp_p_batch(a, td, np.asarray(u, dtype=np.int64).reshape(1, self.n), seed)[0]
 
 
-class PSFGPV(_PSFBase):
+class _TagTable:
+    """samp_p with a tag per target for the classical PSFs whose trapdoor serves every tag of (A_bar, R): PSFPerturbation,
+    and PSFGPV on the two-phase recursion (DESIGN.md 4.3, 4.4)."""
+
+    def _tag_words(self, tag):
+        tg = np.array(np.asarray(tag, dtype=object) % self.gp.q, dtype=np.int64)
+        assert tg.shape == (self.n, self.n)
+        return tg
+
+    def set_tag_table(self, a, td, tags):
+        """Installs the tag table of samp_p_tagged_batch for the key a (any tag H_0) and its trapdoor td: tags is T x n x n,
+        entries taken mod q (qf_set_tag_table: H_t^-1 on the device).  Raises QfError (QF_ERR_INVALID, naming the index)
+        when a tag has no unit pivot; the previous table then stays.  PSFGPV: QF_ERR_INVALID unless a and td run the
+        two-phase recursion (a G-trapdoor key with its basis from gen_short_basis_for_trapdoor, m above the tensor-core
+        threshold)."""
+        self._install_a(a)
+        self._install_td(a, td)
+        t = np.asarray(tags)
+        if t.dtype == object:
+            t = np.array(t % self.gp.q, dtype=np.int64)
+        tg = np.ascontiguousarray(t, dtype=np.int64)
+        assert tg.ndim == 3 and tg.shape[1:] == (self.n, self.n) and tg.shape[0] >= 1
+        self.ctx.call("qf_set_tag_table", _ffi.ptr(tg), tg.shape[0])
+        self._tags_id = tags
+
+    def samp_p_tagged_batch(self, a, td, tags, us: np.ndarray, tag_idx, seed=None, first_index: int = 0) -> np.ndarray:
+        """samp_p with a tag per target: row b is a preimage of us[b] under [A_bar | H_t G - A_bar R], H_t = tags[tag_idx[b]],
+        for the key a = [A_bar | H_0 G - A_bar R] (any tag H_0) and its trapdoor td.  It equals what set_tag(H_t) followed
+        by samp_p_batch on the same targets gives for that row with the same seed and first_index (qf_samp_p_tagged).
+        tags: T x n x n (entries taken mod q), cached on the device by identity as keys are; tag_idx: B indices in [0, T).
+        Returns B x m int32."""
+        self._install_a(a)
+        self._install_td(a, td)
+        if self._tags_id is not tags:
+            self.set_tag_table(a, td, tags)
+        u = np.ascontiguousarray(us, dtype=np.int64)
+        assert u.ndim == 2 and u.shape[1] == self.n
+        ti = np.ascontiguousarray(tag_idx, dtype=np.int32)
+        assert ti.shape == (u.shape[0],)
+        e = np.empty((u.shape[0], self.m), dtype=np.int32)
+        self.ctx.call("qf_samp_p_tagged", _ffi.ptr(u), _ffi.ptr(ti), u.shape[0], _seed(seed), first_index, _ffi.ptr(e))
+        return e
+
+
+class PSFGPV(_TagTable, _PSFBase):
     """src/primitive/psf/gpv.rs:53-225.  Trapdoor = (short basis S_A, its GSO)."""
 
     kind = _ffi.QF_PSF_GPV
@@ -203,7 +247,7 @@ class PSFGPV(_PSFBase):
             sg = None if sg is None else np.ascontiguousarray(sg, dtype=np.float64)
             assert s.shape == (self.m, self.m) and (sg is None or sg.shape == (self.m, self.m))
             self.ctx.call("qf_set_trapdoor_gpv", _ffi.ptr(s), _ffi.ptr(sg))
-            self._td_id = td
+            self._td_id, self._tags_id = td, None
 
     def trap_gen(self, seed=None, dense_gso: bool = None, tag=None):
         """gpv.rs:83-94: uniform A_bar, gen_trapdoor, short basis, GSO -- all on the device.  dense_gso=False
@@ -230,6 +274,24 @@ class PSFGPV(_PSFBase):
         """MatQ::gso (gpv.rs:91): unnormalised Gram-Schmidt of the columns, float64, on the device."""
         return _gso(self, basis)
 
+    def set_tag(self, a, td, tag):
+        """Tag switch without a new trapdoor install: for a key a = [A_bar | H G - A_bar R] and its trapdoor td = (S_H, S~)
+        on the two-phase recursion, returns (a_new, td_new) with a_new = [A_bar | H' G - A_bar R] for tag = H' (n x n,
+        entries taken mod q; None: H' = I), equal to gen_trapdoor(A_bar, R, H'), and td_new = (S_H', td[1]) with S_H' equal
+        to gen_short_basis_for_trapdoor(R, H').  The GSO of S_H does not depend on the tag, so td[1] serves S_H' too (None:
+        it stays on the device) and nothing is re-installed: both are recorded as installed (qf_gpv_set_tag).  The tag
+        table stays; the f_a tag table is dropped.  Raises QfError (QF_ERR_INVALID) off the two-phase recursion or when H'
+        has no unit pivot; then the installed key and tag stay as they were."""
+        self._install_a(a)
+        self._install_td(a, td)
+        tg = None if tag is None else self._tag_words(tag)
+        a_new = np.empty((self.n, self.m), dtype=np.int64)
+        s_new = np.empty((self.m, self.m), dtype=np.int64)
+        self.ctx.call("qf_gpv_set_tag", _ffi.ptr(tg), _ffi.ptr(a_new), _ffi.ptr(s_new))
+        td_new = (s_new, td[1])
+        self._a_id, self._td_id, self._fa_tags_id = a_new, td_new, None
+        return a_new, td_new
+
 
     def gen_short_basis_for_trapdoor(self, r, tag=None) -> np.ndarray:
         """short_basis_classical.rs:54-110 for the installed A and the tag H (n x n, entries taken mod q; None: H = I):
@@ -248,7 +310,7 @@ class PSFGPV(_PSFBase):
         return out
 
 
-class PSFPerturbation(_PSFBase):
+class PSFPerturbation(_TagTable, _PSFBase):
     """src/primitive/psf/mp_perturbation.rs:57-403.
     Trapdoor = (R, sqrt(Sigma_2), (S, S~)) with S = I_n (x) S_k the gadget short basis."""
 
@@ -344,11 +406,6 @@ class PSFPerturbation(_PSFBase):
         self._a_id = a
         return a, (r, sqrt_sigma_2, (sb, sg))
 
-    def _tag_words(self, tag):
-        tg = np.array(np.asarray(tag, dtype=object) % self.gp.q, dtype=np.int64)
-        assert tg.shape == (self.n, self.n)
-        return tg
-
     def set_tag(self, a, td, tag) -> np.ndarray:
         """Tag switch without a new trapdoor install: for a key a = [A_bar | H G - A_bar R] and its trapdoor td (R, ...),
         returns a_new = [A_bar | H' G - A_bar R] for tag = H' (n x n, entries taken mod q; None: H' = I), equal to
@@ -362,38 +419,6 @@ class PSFPerturbation(_PSFBase):
         self.ctx.call("qf_set_tag", _ffi.ptr(tg), _ffi.ptr(a_new))
         self._a_id, self._fa_tags_id = a_new, None  # qf_set_tag rewrote A: the f_a table is gone
         return a_new
-
-    def set_tag_table(self, a, td, tags):
-        """Installs the tag table of samp_p_tagged_batch for the key a (any tag H_0) and its trapdoor td: tags is T x n x n,
-        entries taken mod q (qf_set_tag_table: H_t^-1 on the device).  Raises QfError (QF_ERR_INVALID, naming the index)
-        when a tag has no unit pivot; the previous table then stays."""
-        self._install_a(a)
-        self._install_td(a, td)
-        t = np.asarray(tags)
-        if t.dtype == object:
-            t = np.array(t % self.gp.q, dtype=np.int64)
-        tg = np.ascontiguousarray(t, dtype=np.int64)
-        assert tg.ndim == 3 and tg.shape[1:] == (self.n, self.n) and tg.shape[0] >= 1
-        self.ctx.call("qf_set_tag_table", _ffi.ptr(tg), tg.shape[0])
-        self._tags_id = tags
-
-    def samp_p_tagged_batch(self, a, td, tags, us: np.ndarray, tag_idx, seed=None, first_index: int = 0) -> np.ndarray:
-        """samp_p with a tag per target: row b is a preimage of us[b] under [A_bar | H_t G - A_bar R], H_t = tags[tag_idx[b]],
-        for the key a = [A_bar | H_0 G - A_bar R] (any tag H_0) and its trapdoor td.  It equals what set_tag(H_t) followed
-        by samp_p_batch on the same targets gives for that row with the same seed and first_index (qf_samp_p_tagged).
-        tags: T x n x n (entries taken mod q), cached on the device by identity as keys are; tag_idx: B indices in [0, T).
-        Returns B x m int32."""
-        self._install_a(a)
-        self._install_td(a, td)
-        if self._tags_id is not tags:
-            self.set_tag_table(a, td, tags)
-        u = np.ascontiguousarray(us, dtype=np.int64)
-        assert u.ndim == 2 and u.shape[1] == self.n
-        ti = np.ascontiguousarray(tag_idx, dtype=np.int32)
-        assert ti.shape == (u.shape[0],)
-        e = np.empty((u.shape[0], self.m), dtype=np.int32)
-        self.ctx.call("qf_samp_p_tagged", _ffi.ptr(u), _ffi.ptr(ti), u.shape[0], _seed(seed), first_index, _ffi.ptr(e))
-        return e
 
 
 def _gso(psf, basis) -> np.ndarray:
