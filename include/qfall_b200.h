@@ -146,6 +146,23 @@ qf_status qf_set_tag_table(qf_ctx* ctx, const int64_t* tags, int64_t ntags);
  * whenever A changes (qf_set_a, qf_trap_gen, qf_trap_gen_from, qf_set_tag, qf_gpv_set_tag) and is independent of
  * qf_set_tag_table. */
 qf_status qf_set_f_a_tags(qf_ctx* ctx, const int64_t* tags, int64_t ntags, const int64_t* h0);
+/* samp_p tag table in polynomial form: H_t = rot_f(h_t). f: n low coefficients of the monic modulus; tags: ntags x n.
+ * f = X^n + sum_{i<n} f_i X^i, and column c of rot_f(h) holds the coefficients of h X^c mod f (for f = X^n + 1 that is
+ * rot^-, rotation_matrix.rs:41-63).  Entries are taken mod q, negatives allowed.  The table then serves qf_samp_p_tagged[_dev]
+ * exactly as qf_set_tag_table with the tags rot_f(h_t) would, bit for bit, but stores h_t^-1 mod (f, q) as n words per tag
+ * and inverts each tag in O(n^2) on the device (extended Euclid mod p, Newton lifting to q = p^e).  It replaces the table
+ * installed last, of either form; contexts, refusals and lifetime are those of qf_set_tag_table, and in addition:
+ * QF_ERR_UNSUPPORTED when q is not a prime power or the kernels' shared memory exceeds one block's limit; QF_ERR_INVALID
+ * when a tag is not a unit mod (f, q) (qf_last_error names its index; the previous table then stays).  For q = p^e a tag
+ * is a unit exactly when rot_f(h_t) is invertible mod q, which is when qf_set_tag_table accepts it.  Device memory: ntags n
+ * + n^2 words of 4 bytes (q <= 2^32) or 8 bytes. */
+qf_status qf_set_tag_table_poly(qf_ctx* ctx, const int64_t* f, const int64_t* tags, int64_t ntags);
+/* f_a tag table in polynomial form: A_t = A + [0 | (rot_f(h_t) - H_0) G]; h0: n x n matrix as in qf_set_f_a_tags (NULL = I).
+ * f and tags as in qf_set_tag_table_poly.  qf_f_a_tagged[_dev] then give what qf_set_f_a_tags with the tags rot_f(h_t)
+ * gives, bit for bit.  Inverts nothing: every q < 2^62, singular tags and H_0 = 0 work.  It replaces the f_a table
+ * installed last, of either form; contexts, refusals and lifetime are those of qf_set_f_a_tags, and QF_ERR_UNSUPPORTED when
+ * the kernel's shared memory exceeds one block's limit.  Device memory: ntags n + n^2 words (+ n^2 for a dense H_0). */
+qf_status qf_set_f_a_tags_poly(qf_ctx* ctx, const int64_t* f, const int64_t* tags, int64_t ntags, const int64_t* h0);
 /* gen_short_basis_for_trapdoor with tag = I (short_basis_classical.rs:54-110): the short basis
  * S_A = [[I,R],[0,I]] [[0,I],[S',W]] = [[R S', I + R W],[S', W]] of Lambda^perp(A) for the installed A and the
  * trapdoor R (m_bar x nk); W = digits of -A[:, :m_bar], S' column-reversed iff base^k = q.  The m_bar x nk x m_bar

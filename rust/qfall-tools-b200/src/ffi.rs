@@ -51,6 +51,8 @@ extern "C" {
     pub fn qf_gpv_set_tag(ctx: *mut qf_ctx, tag: *const i64, a_out: *mut i64, s_out: *mut i64) -> i32;
     pub fn qf_set_tag_table(ctx: *mut qf_ctx, tags: *const i64, ntags: i64) -> i32;
     pub fn qf_set_f_a_tags(ctx: *mut qf_ctx, tags: *const i64, ntags: i64, h0: *const i64) -> i32;
+    pub fn qf_set_tag_table_poly(ctx: *mut qf_ctx, f: *const i64, tags: *const i64, ntags: i64) -> i32;
+    pub fn qf_set_f_a_tags_poly(ctx: *mut qf_ctx, f: *const i64, tags: *const i64, ntags: i64, h0: *const i64) -> i32;
     pub fn qf_gen_short_basis(ctx: *mut qf_ctx, r: *const i8, s_out: *mut i64) -> i32;
     pub fn qf_gen_short_basis_tagged(ctx: *mut qf_ctx, r: *const i8, tag: *const i64, s_out: *mut i64) -> i32;
     pub fn qf_compute_sqrt_sigma_2(ctx: *mut qf_ctx, r: *const i8, sigma: *const f64, sqrt_sigma_2_out: *mut f64) -> i32;

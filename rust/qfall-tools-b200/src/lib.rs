@@ -252,6 +252,20 @@ impl PSFGPVB200 {
         *self.installed_tags.borrow_mut() = Some(tags.len());
     }
 
+    /// `set_tag_table` with the tags in polynomial form: tag t is H_t = rot_f(h_t), the matrix of multiplication by
+    /// `tags[t]` (an n x 1 vector of coefficients) in Z_q[X]/(f), f = X^n + sum_{i<n} f_i X^i with `f` its n low
+    /// coefficients (n x 1).  Rows equal those of `set_tag_table` with the tags rot_f(h_t); the device stores n words per
+    /// tag and inverts each in O(n^2) (qf_set_tag_table_poly).  Panics when q is not a prime power and when a tag is not a
+    /// unit.
+    pub fn set_tag_table_poly(&self, a: &MatZq, td: &(MatZ, MatQ), f: &MatZ, tags: &[MatZq]) {
+        assert!(!tags.is_empty(), "at least one tag");
+        self.install(a, td);
+        let (fw, tw) = poly_tag_words(self.n(), f, tags);
+        self.ctx.check(unsafe { qf_set_tag_table_poly(self.ctx.raw, fw.as_ptr(), tw.as_ptr(), tags.len() as i64) },
+                       "qf_set_tag_table_poly");
+        *self.installed_tags.borrow_mut() = Some(tags.len());
+    }
+
     /// samp_p with a tag per target, against the table of `set_tag_table`: `us[b]` is sampled under
     /// `[A_bar | H_t G - A_bar R]` with `H_t = tags[tag_of[b]]`, in one batch.  Row b equals what `set_tag(H_t)` followed
     /// by `samp_p_batch` gives for it with the same seed (qf_samp_p_tagged).  Panics when no table is installed for this
@@ -308,7 +322,7 @@ impl PSFGPVB200 {
         let aw = matzq_to_words(a);
         // the key of the cached table is on the device too: every key change drops both
         let same = self.installed.borrow().as_ref().map(|(a0, _)| *a0 == aw).unwrap_or(false)
-            || self.fa_tags.borrow().as_ref().map(|(a0, _, _)| *a0 == aw).unwrap_or(false);
+            || self.fa_tags.borrow().as_ref().map(|(a0, _, _, _)| *a0 == aw).unwrap_or(false);
         if !same {
             self.ctx.check(unsafe { qf_set_a(self.ctx.raw, aw.as_ptr()) }, "qf_set_a");
             *self.installed_tags.borrow_mut() = None;
@@ -318,11 +332,41 @@ impl PSFGPVB200 {
         let q = Z::from(&self.inner.gp.q);
         f_a_tagged_installed(&self.ctx, &self.fa_tags, aw, self.n(), self.m(), &q, tags, h0, sigmas, tag_of)
     }
+
+    /// `f_a_tagged_batch` with the tags in polynomial form (`f` and `tags` as in `set_tag_table_poly`): A_t = a +
+    /// [0 | (rot_f(h_t) - H_0) G] (qf_set_f_a_tags_poly).  Works for every q, singular tags and H_0 = 0.
+    pub fn f_a_tagged_batch_poly(&self, a: &MatZq, f: &MatZ, tags: &[MatZq], h0: Option<&MatZq>, sigmas: &[MatZ],
+                                 tag_of: &[usize]) -> Vec<MatZq> {
+        let aw = matzq_to_words(a);
+        let same = self.installed.borrow().as_ref().map(|(a0, _)| *a0 == aw).unwrap_or(false)
+            || self.fa_tags.borrow().as_ref().map(|(a0, _, _, _)| *a0 == aw).unwrap_or(false);
+        if !same {
+            self.ctx.check(unsafe { qf_set_a(self.ctx.raw, aw.as_ptr()) }, "qf_set_a");
+            *self.installed_tags.borrow_mut() = None;
+            *self.installed.borrow_mut() = None;
+            *self.fa_tags.borrow_mut() = None;
+        }
+        let q = Z::from(&self.inner.gp.q);
+        f_a_tagged_installed_poly(&self.ctx, &self.fa_tags, aw, self.n(), self.m(), &q, f, tags, h0, sigmas, tag_of)
+    }
 }
 
-/// The f_a tag table on the device (qf_set_f_a_tags): (words of the key it belongs to, tag words, H_0 words; empty for
-/// H_0 = I).  The device drops it whenever the key changes, so every key install clears it here too.
-pub(crate) type FaTags = RefCell<Option<(Vec<i64>, Vec<i64>, Vec<i64>)>>;
+/// (f, tags) of tags in polynomial form as words: f is the n x 1 vector of the n low coefficients of the monic modulus,
+/// each tag an n x 1 vector of coefficients.
+pub(crate) fn poly_tag_words(n: usize, f: &MatZ, tags: &[MatZq]) -> (Vec<i64>, Vec<i64>) {
+    assert!(f.is_column_vector() && f.get_num_rows() as usize == n, "f must be the n x 1 vector of its low coefficients");
+    let mut tw = Vec::with_capacity(tags.len() * n);
+    for tag in tags {
+        assert!(tag.is_column_vector() && tag.get_num_rows() as usize == n, "a tag in polynomial form is an n x 1 vector");
+        tw.extend(matzq_to_words(tag));
+    }
+    (matz_to_words(f), tw)
+}
+
+/// The f_a tag table on the device (qf_set_f_a_tags[_poly]): (words of the key it belongs to, tag words -- f first in
+/// polynomial form, H_0 words; empty for H_0 = I, polynomial form).  The device drops it whenever the key changes, so every
+/// key install clears it here too.
+pub(crate) type FaTags = RefCell<Option<(Vec<i64>, Vec<i64>, Vec<i64>, bool)>>;
 
 /// f_a with a tag per target against the key installed in `ctx` (qf_f_a_tagged); installs the table when it differs from
 /// the cached one.
@@ -338,18 +382,45 @@ pub(crate) fn f_a_tagged_installed(ctx: &Context, fa_tags: &FaTags, aw: Vec<i64>
         tw.extend(matzq_to_words(tag));
     }
     let hw = h0.map(|h| { square(h); matzq_to_words(h) }).unwrap_or_default();
-    let key = (aw, tw, hw);
+    let key = (aw, tw, hw, false);
     if fa_tags.borrow().as_ref() != Some(&key) {
         let hp = if key.2.is_empty() { std::ptr::null() } else { key.2.as_ptr() };
         ctx.check(unsafe { qf_set_f_a_tags(ctx.raw, key.1.as_ptr(), tags.len() as i64, hp) }, "qf_set_f_a_tags");
         *fa_tags.borrow_mut() = Some(key);
     }
+    f_a_tagged_run(ctx, n, m, q, tags.len(), sigmas, tag_of)
+}
+
+/// `f_a_tagged_installed` with the tags in polynomial form (qf_set_f_a_tags_poly).
+#[allow(clippy::too_many_arguments)]
+pub(crate) fn f_a_tagged_installed_poly(ctx: &Context, fa_tags: &FaTags, aw: Vec<i64>, n: usize, m: usize, q: &Z, f: &MatZ,
+                                        tags: &[MatZq], h0: Option<&MatZq>, sigmas: &[MatZ], tag_of: &[usize]) -> Vec<MatZq> {
+    assert!(!tags.is_empty(), "at least one tag");
+    assert_eq!(sigmas.len(), tag_of.len(), "one tag index per sigma");
+    let (fw, tw) = poly_tag_words(n, f, tags);
+    let hw = h0.map(|h| {
+        assert_eq!((h.get_num_rows(), h.get_num_columns()), (n as i64, n as i64), "H_0 must be n x n");
+        matzq_to_words(h)
+    }).unwrap_or_default();
+    let key = (aw, [fw, tw].concat(), hw, true);
+    if fa_tags.borrow().as_ref() != Some(&key) {
+        let hp = if key.2.is_empty() { std::ptr::null() } else { key.2.as_ptr() };
+        let st = unsafe { qf_set_f_a_tags_poly(ctx.raw, key.1.as_ptr(), key.1[n..].as_ptr(), tags.len() as i64, hp) };
+        ctx.check(st, "qf_set_f_a_tags_poly");
+        *fa_tags.borrow_mut() = Some(key);
+    }
+    f_a_tagged_run(ctx, n, m, q, tags.len(), sigmas, tag_of)
+}
+
+/// qf_f_a_tagged against the installed f_a tag table of `ntags` tags.
+fn f_a_tagged_run(ctx: &Context, n: usize, m: usize, q: &Z, ntags: usize, sigmas: &[MatZ], tag_of: &[usize]) -> Vec<MatZq> {
+    assert_eq!(sigmas.len(), tag_of.len(), "one tag index per sigma");
     let mut sg = Vec::with_capacity(sigmas.len() * m);
     for sigma in sigmas {
         assert!(sigma.is_column_vector() && sigma.get_num_rows() as usize == m, "sigma is not in D_n");
         sg.extend(domain_to_i32(sigma).expect("sigma is not in D_n"));
     }
-    let idx: Vec<i32> = tag_of.iter().map(|t| { assert!(*t < tags.len(), "tag index out of range"); *t as i32 }).collect();
+    let idx: Vec<i32> = tag_of.iter().map(|t| { assert!(*t < ntags, "tag index out of range"); *t as i32 }).collect();
     let mut u = vec![0i64; sigmas.len() * n];
     let mut ok = vec![0u8; sigmas.len()];
     let st = unsafe { qf_f_a_tagged(ctx.raw, sg.as_ptr(), idx.as_ptr(), sigmas.len() as i64, u.as_mut_ptr(), ok.as_mut_ptr()) };

@@ -2,8 +2,8 @@
 //! `p <- D_{sqrt(Sigma_2)}`, `v = u - A p`, `z <- D_{Lambda_v^perp(G)}`, `e = p + [R; I] z` for a batch of targets.
 //! Shipped as source (see lib.rs).
 use crate::ffi::*;
-use crate::{column_from_i32, domain_to_i32, f_a_tagged_installed, matz_to_words, matzq_to_words, range_from_words, Context, FaTags,
-            PSFBatch};
+use crate::{column_from_i32, domain_to_i32, f_a_tagged_installed, f_a_tagged_installed_poly, matz_to_words, matzq_to_words,
+            poly_tag_words, range_from_words, Context, FaTags, PSFBatch};
 use qfall_math::{
     integer::{MatZ, Z},
     integer_mod_q::MatZq,
@@ -165,6 +165,20 @@ impl PSFPerturbationB200 {
         *self.installed_tags.borrow_mut() = Some(tags.len());
     }
 
+    /// `set_tag_table` with the tags in polynomial form: tag t is H_t = rot_f(h_t), the matrix of multiplication by
+    /// `tags[t]` (an n x 1 vector of coefficients) in Z_q[X]/(f), `f` the n x 1 vector of the n low coefficients of the
+    /// monic modulus (qf_set_tag_table_poly: n words per tag, O(n^2) inverse on the device).  Rows equal those of
+    /// `set_tag_table` with the tags rot_f(h_t).  Panics when q is not a prime power and when a tag is not a unit.
+    pub fn set_tag_table_poly(&self, a: &MatZq, td: &(MatZ, MatQ, (MatZ, MatQ)), f: &MatZ, tags: &[MatZq]) {
+        assert!(!tags.is_empty(), "at least one tag");
+        self.install_a(a);
+        self.install_td(td);
+        let (fw, tw) = poly_tag_words(self.n(), f, tags);
+        self.ctx.check(unsafe { qf_set_tag_table_poly(self.ctx.raw, fw.as_ptr(), tw.as_ptr(), tags.len() as i64) },
+                       "qf_set_tag_table_poly");
+        *self.installed_tags.borrow_mut() = Some(tags.len());
+    }
+
     /// samp_p with a tag per target, against the table of `set_tag_table`: `us[b]` is sampled under
     /// `[A_bar | H_t G - A_bar R]` with `H_t = tags[tag_of[b]]`, in one batch.  Row b equals what `set_tag(H_t)` followed by
     /// `samp_p_batch` gives for it with the same seed (qf_samp_p_tagged).  The tags do not cross the boundary again, so
@@ -197,6 +211,16 @@ impl PSFPerturbationB200 {
         self.install_a(a);
         let q = Z::from(&self.inner.gp.q);
         f_a_tagged_installed(&self.ctx, &self.fa_tags, matzq_to_words(a), self.n(), self.m(), &q, tags, h0, sigmas, tag_of)
+    }
+
+    /// `f_a_tagged_batch` with the tags in polynomial form (`f` and `tags` as in `set_tag_table_poly`): A_t = a +
+    /// [0 | (rot_f(h_t) - H_0) G] (qf_set_f_a_tags_poly).  Works for every q, singular tags and H_0 = 0.
+    pub fn f_a_tagged_batch_poly(&self, a: &MatZq, f: &MatZ, tags: &[MatZq], h0: Option<&MatZq>, sigmas: &[MatZ],
+                                 tag_of: &[usize]) -> Vec<MatZq> {
+        self.install_a(a);
+        let q = Z::from(&self.inner.gp.q);
+        f_a_tagged_installed_poly(&self.ctx, &self.fa_tags, matzq_to_words(a), self.n(), self.m(), &q, f, tags, h0, sigmas,
+                                  tag_of)
     }
 }
 

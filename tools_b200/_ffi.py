@@ -50,6 +50,8 @@ SIGNATURES = {
     "qf_gpv_set_tag": (_i32, [_vp, _vp, _vp, _vp]),
     "qf_set_tag_table": (_i32, [_vp, _vp, _i64]),
     "qf_set_f_a_tags": (_i32, [_vp, _vp, _i64, _vp]),
+    "qf_set_tag_table_poly": (_i32, [_vp, _vp, _vp, _i64]),
+    "qf_set_f_a_tags_poly": (_i32, [_vp, _vp, _vp, _i64, _vp]),
     "qf_compute_sqrt_sigma_2": (_i32, [_vp, _vp, _vp, _vp]),
     "qf_gen_short_basis": (_i32, [_vp, _vp, _vp]),
     "qf_gen_short_basis_tagged": (_i32, [_vp, _vp, _vp, _vp]),

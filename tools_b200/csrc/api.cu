@@ -195,12 +195,21 @@ struct qf_ctx {
     int64_t tag_count = 0;
     int tag_word = 8;
     Dev dTagTab, dTagH0, dTagGpow, io_t[2];
+    // tag_poly: dTagTab holds the tags in polynomial form instead (qf_set_tag_table_poly, DESIGN 4.10): h_t^-1 mod (f, q)
+    // as n words per tag, and dTagXr the rows X^{n+j} mod (f, q), j < n - 1, of the product.
+    bool tag_poly = false;
+    Dev dTagXr;
     // Tag table of f_a (qf_set_f_a_tags, PSFGPV and PSFPerturbation): D_t = H_t - H_0 mod q for fa_tag_count tags, in the
     // layout of dTagTab, relative to the installed A and dropped whenever A changes.  dFaSort: hist / off / gstart of the
     // counting sort by tag (3 (T + 1) ints); dFaPerm: the sorted targets of a chunk.
     int64_t fa_tag_count = 0;
     int fa_tag_word = 8;
     Dev dFaTab, dFaGpow, dFaSort, dFaPerm;
+    // fa_poly: dFaTab holds h_t mod q as n words per tag instead (qf_set_f_a_tags_poly), dFaXr the rows of the product mod
+    // (f, q) and dFaH0 H_0 column-major when fa_h0_kind = 2 (0: H_0 = 0, 1: H_0 = I).
+    bool fa_poly = false;
+    int fa_h0_kind = 1;
+    Dev dFaXr, dFaH0;
     // Defaults from the error budget of DESIGN 4.2, checked at the full C2 key (scripts/ab_c2_precision.py, profiles/README_r2.md):
     // four digits everywhere; the lowest digit sum is dropped where the operand has three digits (z2), not for the
     // two-digit z1 (dropping it there moves 14 % of the preimages, keeping it 0.3 %).
@@ -698,7 +707,7 @@ qf_status samp_p_pert_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t s
         LAUNCH(qf_launch_tag_syndrome(V, ctx->n, P, ldm, (int)ctx->m_bar, dTidx, (int)ctx->tag_count, ctx->dTagTab.p,
                                       ctx->key_tagged ? ctx->dTagH0.p : nullptr, ctx->tag_word, ctx->dTagGpow.as<uint64_t>(),
                                       ctx->prm.q, (int)ctx->n, (int)ctx->k, Bc, ctx->dTagU.as<int64_t>(), ctx->n,
-                                      ctx->dFlag.as<int>(), ctx->stream));
+                                      ctx->dFlag.as<int>(), ctx->stream, ctx->tag_poly ? ctx->dTagXr.p : nullptr));
         Vg = ctx->dTagU.as<int64_t>();
     } else if (ctx->key_tagged) {
         QF_TRY(tag_targets(ctx, V, Bc, &Vg));
@@ -1118,7 +1127,7 @@ qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t se
     if (dTidx)
         LAUNCH(qf_launch_tag_syndrome(ctx->dTagU.as<int64_t>(), n, nullptr, 0, 0, dTidx, (int)ctx->tag_count, ctx->dTagTab.p,
                                       nullptr, ctx->tag_word, nullptr, ctx->prm.q, (int)n, (int)ctx->k, Bc, H, n, flag,
-                                      ctx->stream));
+                                      ctx->stream, ctx->tag_poly ? ctx->dTagXr.p : nullptr));
     // ---- g3 = digits(h): one s8 plane (the x operand of its centre map) and, as fp64, the start of e_bot = g3 + S' z1
     // (fused tail: e_bot is formed in one pass from z1 and the g3 plane -- needs 16-byte aligned int32 rows; otherwise e_bot is
     // accumulated in fp64 as in the one-pass form)
@@ -1749,6 +1758,12 @@ qf_status f_a_dev_chunks(qf_ctx* ctx, int64_t batch, F&& run) {
 qf_status f_a_tagged_chunk(qf_ctx* ctx, const int32_t* dSigma, const int32_t* dTidx, int Bc, int64_t* dU, uint8_t* dFlags) {
     QF_TRY(f_a_chunk(ctx, dSigma, Bc, dU, dFlags));
     const int T = (int)ctx->fa_tag_count;
+    if (ctx->fa_poly) {  // n words per tag: one CTA per target, no grouping
+        LAUNCH(qf_launch_f_a_tag_poly(dSigma, ctx->dim, (int)ctx->m_bar, dTidx, T, ctx->dFaTab.p, ctx->dFaXr.p, ctx->dFaH0.p,
+                                      ctx->fa_h0_kind, ctx->fa_tag_word, ctx->dFaGpow.as<uint64_t>(), ctx->prm.q, (int)ctx->n,
+                                      (int)ctx->k, Bc, dU, ctx->n, ctx->dFlag.as<int>(), ctx->stream));
+        return QF_OK;
+    }
     int* hist = ctx->dFaSort.as<int>();
     int *off = hist + (T + 1), *gstart = off + (T + 1), *perm = nullptr;
     if (QF_F_A_TAG_GROUP > 1) {  // always in the library; 1 only in the benchmark's comparison build (kernels.h)
@@ -1769,8 +1784,8 @@ qf_status install_a(qf_ctx* ctx, const int64_t* a) {
     ctx->has_a = false; ctx->has_np = false; ctx->has_pert = false;
     ctx->key_tagged = false; ctx->pert_gadget_key = false;
     ctx->dHinvl.release(); ctx->dAbpl.release();
-    ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release();
-    ctx->fa_tag_count = 0; ctx->dFaTab.release();
+    ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release(); ctx->dTagXr.release();
+    ctx->fa_tag_count = 0; ctx->dFaTab.release(); ctx->dFaXr.release(); ctx->dFaH0.release();
     const long n = ctx->n, m = ctx->m;
     for (long i = 0; i < n * m; ++i)
         if (a[i] < 0 || (uint64_t)a[i] >= ctx->prm.q) return ctx->fail(QF_ERR_INVALID, "A entry outside [0,q)");
@@ -1860,6 +1875,79 @@ qf_status upload_tag_h0(qf_ctx* ctx) {
     return QF_OK;
 }
 
+// ---- tags in polynomial form (qf_set_tag_table_poly, qf_set_f_a_tags_poly)
+typedef unsigned __int128 u128h;
+
+uint64_t powmod_u64(uint64_t a, uint64_t e, uint64_t m) {
+    uint64_t r = 1 % m;
+    for (a %= m; e; e >>= 1, a = (uint64_t)((u128h)a * a % m))
+        if (e & 1) r = (uint64_t)((u128h)r * a % m);
+    return r;
+}
+
+// deterministic for every n < 2^64 (the first twelve primes as witnesses)
+bool is_prime_u64(uint64_t n) {
+    if (n < 2) return false;
+    static const uint64_t W[] = {2, 3, 5, 7, 11, 13, 17, 19, 23, 29, 31, 37};
+    for (uint64_t w : W)
+        if (n % w == 0) return n == w;
+    uint64_t d = n - 1;
+    int r = 0;
+    while (!(d & 1)) d >>= 1, ++r;
+    for (uint64_t w : W) {
+        uint64_t x = powmod_u64(w, d, n);
+        if (x == 1 || x == n - 1) continue;
+        bool comp = true;
+        for (int i = 1; i < r && comp; ++i) {
+            x = (uint64_t)((u128h)x * x % n);
+            comp = x != n - 1;
+        }
+        if (comp) return false;
+    }
+    return true;
+}
+
+// r^e compared with q without overflow: -1, 0, 1
+int pow_cmp(uint64_t r, int e, uint64_t q) {
+    u128h x = 1;
+    for (int i = 0; i < e; ++i) {
+        x *= r;
+        if (x > q) return 1;
+    }
+    return x == q ? 0 : -1;
+}
+
+// q = p^e with p prime: the largest e for which q is a perfect e-th power, and its root must be prime
+bool prime_power(uint64_t q, uint64_t* p, int* e) {
+    for (int ee = 63; ee >= 1; --ee) {
+        uint64_t r = (uint64_t)std::llround(std::pow((double)q, 1.0 / ee));
+        while (r > 1 && pow_cmp(r, ee, q) > 0) --r;
+        while (pow_cmp(r + 1, ee, q) <= 0) ++r;
+        if (r >= 2 && pow_cmp(r, ee, q) == 0) {
+            if (!is_prime_u64(r)) return false;
+            *p = r;
+            *e = ee;
+            return true;
+        }
+    }
+    return false;
+}
+
+// f mod q on the device and the rows X^{n+j} mod (f, q) of the product (qf_launch_poly_xpow)
+qf_status poly_modulus(qf_ctx* ctx, const int64_t* f, int word, Dev& dF, Dev& xr) {
+    const long n = ctx->n;
+    const uint64_t q = ctx->prm.q;
+    std::vector<uint64_t> fq((size_t)n);
+    for (long i = 0; i < n; ++i) {
+        const int64_t v = f[i] % (int64_t)q;
+        fq[i] = (uint64_t)(v < 0 ? v + (int64_t)q : v);
+    }
+    CK(dF.ensure((size_t)n * 8));
+    CK(xr.ensure((size_t)std::max(1L, n - 1) * n * word));
+    CK(cudaMemcpyAsync(dF.p, fq.data(), (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
+    LAUNCH(qf_launch_poly_xpow(dF.as<uint64_t>(), (int)n, q, word, xr.p, ctx->stream));
+    return QF_OK;
+}
 }  // namespace
 
 extern "C" {
@@ -2025,7 +2113,7 @@ qf_status qf_set_trapdoor_perturbation(qf_ctx* ctx, const int8_t* r, const doubl
     if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "install A first (qf_set_a / qf_trap_gen)");
     ctx->has_pert = false;
     ctx->key_tagged = false; ctx->pert_gadget_key = false;
-    ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release();
+    ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release(); ctx->dTagXr.release();
     CK(cudaSetDevice(ctx->device));
     QF_TRY(upload_as_f64(ctx, r, ctx->m_bar, ctx->nk, ctx->ld_nk, ctx->dR));
     {
@@ -2098,7 +2186,8 @@ qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out) {
     // device copies are consistent again the context has no key (a CUDA error on the way leaves it so).
     ctx->has_a = false;
     ctx->has_pert = false;
-    ctx->fa_tag_count = 0; ctx->dFaTab.release();  // the f_a table is relative to A, which changes here
+    // the f_a table is relative to A, which changes here
+    ctx->fa_tag_count = 0; ctx->dFaTab.release(); ctx->dFaXr.release(); ctx->dFaH0.release();
     const std::vector<uint64_t> gpow = gadget_powers(ctx);
     for (long i = 0; i < n; ++i)
         for (long j = 0; j < n; ++j) {
@@ -2195,7 +2284,8 @@ qf_status qf_gpv_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out, int64_
         }
     // commit.  Until the device copies are consistent again the context has no trapdoor (a CUDA error on the way leaves it so).
     ctx->has_np = false;
-    ctx->fa_tag_count = 0; ctx->dFaTab.release();  // the f_a table is relative to A; the samp_p table to (A_bar, R): kept
+    // the f_a table is relative to A; the samp_p table to (A_bar, R): kept
+    ctx->fa_tag_count = 0; ctx->dFaTab.release(); ctx->dFaXr.release(); ctx->dFaH0.release();
     ctx->hA.swap(a2);
     QF_TRY(upload_a_cols(ctx, mb));
     if (repivot) {
@@ -2279,6 +2369,8 @@ qf_status qf_set_tag_table(qf_ctx* ctx, const int64_t* tags, int64_t ntags) {
     if (ctx->prm.kind == QF_PSF_PERTURBATION) QF_TRY(upload_tag_h0(ctx));  // PSFGPV's h_t does not involve H_0
     std::swap(ctx->dTagTab.p, tab.p);
     std::swap(ctx->dTagTab.cap, tab.cap);
+    ctx->tag_poly = false;
+    ctx->dTagXr.release();
     ctx->tag_count = ntags;
     return QF_OK;
 }
@@ -2331,6 +2423,148 @@ qf_status qf_set_f_a_tags(qf_ctx* ctx, const int64_t* tags, int64_t ntags, const
     std::swap(ctx->dFaSort.p, sort.p);
     std::swap(ctx->dFaSort.cap, sort.cap);
     ctx->fa_tag_word = word;
+    ctx->fa_poly = false;
+    ctx->dFaXr.release();
+    ctx->dFaH0.release();
+    ctx->fa_tag_count = ntags;
+    return QF_OK;
+}
+
+// ---- tags in polynomial form: H_t = rot_f(h_t), column c = coeffs(h_t X^c mod f) (DESIGN 4.10) -------------------------
+
+// h_t^-1 mod (f, q) for every tag on the device (qf_launch_poly_tag_inverse, one CTA per tag), for q = p^e.  Tags are
+// copied in slices of at most 1 GB.  The new table replaces the old one, of either form, only when every tag is a unit.
+qf_status qf_set_tag_table_poly(qf_ctx* ctx, const int64_t* f, const int64_t* tags, int64_t ntags) {
+    if (!ctx) return QF_ERR_INVALID;
+    if (ctx->prm.kind == QF_PSF_GPV) {
+        QF_TRY(gpv_tags_ready(ctx));
+    } else if (ctx->prm.kind != QF_PSF_PERTURBATION) {
+        return ctx->fail(QF_ERR_INVALID, "not a PSFGPV or PSFPerturbation context");
+    }
+    if (!f || !tags || ntags < 1) return ctx->fail(QF_ERR_INVALID, "tag table: f and at least one tag needed");
+    if (ctx->prm.kind == QF_PSF_PERTURBATION) {
+        if (!ctx->has_a || !ctx->has_pert) return ctx->fail(QF_ERR_NO_KEY, "PSFPerturbation: key or trapdoor missing");
+        if (!ctx->pert_gadget_key) return ctx->fail(QF_ERR_INVALID, "the installed key is not [A_bar | H G - A_bar R] for the installed R");
+    }
+    if (ntags > INT32_MAX) return ctx->fail(QF_ERR_INVALID, "tag table: more than 2^31 - 1 tags");
+    const long n = ctx->n;
+    const uint64_t q = ctx->prm.q;
+    uint64_t p = 0;
+    int e = 0;
+    if (!prime_power(q, &p, &e))
+        return ctx->fail(QF_ERR_UNSUPPORTED, "tag table in polynomial form: q must be a prime power");
+    CK(cudaSetDevice(ctx->device));
+    int supported = 0;
+    CK(qf_poly_tag_supported((int)std::min<long>(n, INT32_MAX), (int)std::min<long>(ctx->k, INT32_MAX), 1, &supported));
+    if (!supported)
+        return ctx->fail(QF_ERR_UNSUPPORTED, "tag table in polynomial form: needs k <= 64 and the shared memory within one block's limit");
+    int lifts = 0;
+    while ((1 << lifts) < e) ++lifts;
+    const int word = q <= (1ull << 32) ? 4 : 8;
+    const int64_t slice = std::max<int64_t>(1, std::min<int64_t>(ntags, (int64_t)((1ull << 30) / (8 * n))));
+    Dev tab, xr, dF, dTags, dFail;
+    QF_TRY(poly_modulus(ctx, f, word, dF, xr));
+    CK(tab.ensure((size_t)ntags * n * word));
+    CK(dTags.ensure((size_t)slice * n * 8));
+    CK(dFail.ensure((size_t)slice * sizeof(int)));
+    std::vector<int> fail((size_t)slice);
+    for (int64_t t0 = 0; t0 < ntags; t0 += slice) {
+        const int cnt = (int)std::min<int64_t>(slice, ntags - t0);
+        CK(cudaMemcpyAsync(dTags.p, tags + (size_t)t0 * n, (size_t)cnt * n * 8, cudaMemcpyHostToDevice, ctx->stream));
+        LAUNCH(qf_launch_poly_tag_inverse(dTags.as<int64_t>(), cnt, (int)n, dF.as<uint64_t>(), xr.p, word, q, p, lifts,
+                                          tab.as<char>() + (size_t)t0 * n * word, dFail.as<int>(), ctx->stream));
+        CK(cudaMemcpyAsync(fail.data(), dFail.p, (size_t)cnt * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        for (int i = 0; i < cnt; ++i)
+            if (fail[i]) {
+                char buf[128];
+                snprintf(buf, sizeof buf, "tag %lld is not a unit mod (f, q)", (long long)(t0 + i));
+                return ctx->fail(QF_ERR_INVALID, buf);
+            }
+    }
+    const std::vector<uint64_t> gpow = gadget_powers(ctx);
+    CK(ctx->dTagGpow.ensure(gpow.size() * 8));
+    CK(cudaMemcpyAsync(ctx->dTagGpow.p, gpow.data(), gpow.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    ctx->tag_word = word;
+    if (ctx->prm.kind == QF_PSF_PERTURBATION) QF_TRY(upload_tag_h0(ctx));  // PSFGPV's h_t does not involve H_0
+    CK(cudaStreamSynchronize(ctx->stream));
+    std::swap(ctx->dTagTab.p, tab.p);
+    std::swap(ctx->dTagTab.cap, tab.cap);
+    std::swap(ctx->dTagXr.p, xr.p);
+    std::swap(ctx->dTagXr.cap, xr.cap);
+    ctx->tag_poly = true;
+    ctx->tag_count = ntags;
+    return QF_OK;
+}
+
+// h_t mod q as n words per tag and H_0 (NULL: I; all zero: 0; otherwise dense, column-major).  Nothing is inverted: every
+// q < 2^62, singular tags and H_0 = 0 work.  The new table replaces the old one, of either form, only when it is complete.
+qf_status qf_set_f_a_tags_poly(qf_ctx* ctx, const int64_t* f, const int64_t* tags, int64_t ntags, const int64_t* h0) {
+    if (!ctx) return QF_ERR_INVALID;
+    if (ctx->prm.kind == QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "f_a tag table: not a classical context");
+    if (!f || !tags || ntags < 1) return ctx->fail(QF_ERR_INVALID, "f_a tag table: f and at least one tag needed");
+    if (ntags >= INT32_MAX) return ctx->fail(QF_ERR_INVALID, "f_a tag table: more than 2^31 - 2 tags");
+    if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "no key installed");
+    const long n = ctx->n;
+    const uint64_t q = ctx->prm.q;
+    CK(cudaSetDevice(ctx->device));
+    int supported = 0;
+    CK(qf_poly_tag_supported((int)std::min<long>(n, INT32_MAX), (int)std::min<long>(ctx->k, INT32_MAX), 0, &supported));
+    if (!supported)
+        return ctx->fail(QF_ERR_UNSUPPORTED, "f_a tag table in polynomial form: needs k <= 64 and the shared memory within one block's limit");
+    const int word = q <= (1ull << 32) ? 4 : 8;
+    const size_t nn = (size_t)n * n;
+    int kind = 1;
+    std::vector<uint64_t> h;
+    if (h0) {
+        h.resize(nn);
+        bool zero = true, ident = true;
+        for (long i = 0; i < n; ++i)
+            for (long j = 0; j < n; ++j) {
+                const int64_t v = h0[(size_t)i * n + j] % (int64_t)q;
+                const uint64_t r = (uint64_t)(v < 0 ? v + (int64_t)q : v);
+                h[(size_t)j * n + i] = r;
+                zero = zero && r == 0;
+                ident = ident && r == (i == j ? 1 % q : 0);
+            }
+        kind = ident ? 1 : zero ? 0 : 2;
+    }
+    const int64_t slice = std::max<int64_t>(1, std::min<int64_t>(ntags, (int64_t)((1ull << 30) / (8 * n))));
+    Dev tab, xr, dF, dTags, dH0;
+    QF_TRY(poly_modulus(ctx, f, word, dF, xr));
+    CK(tab.ensure((size_t)ntags * n * word));
+    CK(dTags.ensure((size_t)slice * n * 8));
+    if (kind == 2) {
+        std::vector<uint32_t> h32;
+        const void* src = h.data();
+        if (word == 4) {
+            h32.assign(h.begin(), h.end());
+            src = h32.data();
+        }
+        CK(dH0.ensure(nn * word));
+        CK(cudaMemcpyAsync(dH0.p, src, nn * word, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+    }
+    for (int64_t t0 = 0; t0 < ntags; t0 += slice) {
+        const int cnt = (int)std::min<int64_t>(slice, ntags - t0);
+        CK(cudaMemcpyAsync(dTags.p, tags + (size_t)t0 * n, (size_t)cnt * n * 8, cudaMemcpyHostToDevice, ctx->stream));
+        LAUNCH(qf_launch_poly_tag_pack(dTags.as<int64_t>(), (long)cnt * n, q, word, tab.as<char>() + (size_t)t0 * n * word,
+                                       ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));  // dTags is refilled by the next slice
+    }
+    const std::vector<uint64_t> gpow = gadget_powers(ctx);
+    CK(ctx->dFaGpow.ensure(gpow.size() * 8));
+    CK(cudaMemcpyAsync(ctx->dFaGpow.p, gpow.data(), gpow.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    std::swap(ctx->dFaTab.p, tab.p);
+    std::swap(ctx->dFaTab.cap, tab.cap);
+    std::swap(ctx->dFaXr.p, xr.p);
+    std::swap(ctx->dFaXr.cap, xr.cap);
+    std::swap(ctx->dFaH0.p, dH0.p);
+    std::swap(ctx->dFaH0.cap, dH0.cap);
+    ctx->fa_tag_word = word;
+    ctx->fa_h0_kind = kind;
+    ctx->fa_poly = true;
     ctx->fa_tag_count = ntags;
     return QF_OK;
 }
@@ -2553,7 +2787,8 @@ qf_status qf_set_trapdoor_gpv(qf_ctx* ctx, const int64_t* s, const double* sg) {
     if (ctx->prm.kind == QF_PSF_PERTURBATION) return ctx->fail(QF_ERR_INVALID, "not a GPV context");
     ctx->has_np = false;  // stays false if anything below fails half-way (pivots / A^-1 / U are overwritten in place)
     ctx->two_phase = false;
-    ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release();  // the tag table is relative to the old (A_bar, R)
+    // the tag table is relative to the old (A_bar, R)
+    ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release(); ctx->dTagXr.release();
     ctx->u_limbs = 7;
     CK(cudaSetDevice(ctx->device));
     const long D = ctx->dim, ld = ctx->ld_dim;

@@ -913,12 +913,102 @@ __device__ __forceinline__ uint64_t mod_halves(uint64_t a0, uint64_t a1, uint64_
 }
 __device__ __forceinline__ uint2 halves(uint64_t x) { return make_uint2((unsigned)(x & 0xFFFF), (unsigned)(x >> 16)); }
 
+// A residue as the shared vectors of the two regimes hold it: 16-bit halves for W = uint32_t, one word for W = uint64_t.
+template <typename W> struct PolySV;
+template <> struct PolySV<uint32_t> {
+    typedef uint2 T;
+    static __device__ __forceinline__ uint2 put(uint64_t x) { return halves(x); }
+    static __device__ __forceinline__ uint64_t get(uint2 h) { return h.x + ((uint64_t)h.y << 16); }
+};
+template <> struct PolySV<uint64_t> {
+    typedef uint64_t T;
+    static __device__ __forceinline__ uint64_t put(uint64_t x) { return x; }
+    static __device__ __forceinline__ uint64_t get(uint64_t x) { return x; }
+};
+
+// ---- product of tags in polynomial form (DESIGN 4.10): r = a * b mod (f, q), f = X^n + sum_{i<n} f_i X^i monic --------
+// The one product of the inverse (poly_tag_inverse_kernel), the samp_p syndrome and the f_a correction.  a: n residues in
+// any memory; b: n residues in shared memory (PolySV<W>); c: 2n - 1 PolySV<W> of shared scratch; xr: rows X^{n+j} mod f
+// for j < n - 1, n words each (qf_launch_poly_xpow; n^2 words shared by every CTA, so L2-resident).  Schoolbook
+// c_l = sum_{i+j=l} a_i b_j for l < 2n - 1, then r_i = c_i + sum_{j < n-1} c_{n+j} xr[j][i]: no sequential chain, and one
+// code path for every f.  Exact for every q < 2^62 in the regimes of tag_syndrome_kernel: for W = uint32_t (q <= 2^32) a
+// sum of at most n <= 2^14 products word x half stays below 2^62 (mod_halves), for W = uint64_t it runs in 192 bits.
+// Every thread of the CTA calls it.  emit(i, r_i) runs after a barrier that follows the last read of a and b (so it may
+// overwrite them); c may be rewritten only after the next barrier.
+template <typename W, typename A, typename Emit>
+__device__ __forceinline__ void poly_mulmod(const A* a, const typename PolySV<W>::T* b, typename PolySV<W>::T* c,
+                                            const W* __restrict__ xr, uint64_t q, uint64_t magic, int n, Emit emit) {
+    for (int l = threadIdx.x; l < 2 * n - 1; l += blockDim.x) {
+        const int i0 = max(0, l - n + 1), i1 = min(l, n - 1);
+        if constexpr (sizeof(W) == 4) {
+            uint64_t a0 = 0, a1 = 0;
+#pragma unroll 4
+            for (int i = i0; i <= i1; ++i) {
+                const uint64_t x = a[i];
+                const uint2 y = b[l - i];
+                a0 += x * y.x;
+                a1 += x * y.y;
+            }
+            c[l] = halves(mod_halves(a0, a1, q, magic));
+        } else {
+            ModAcc s;
+#pragma unroll 2
+            for (int i = i0; i <= i1; ++i) s.mac(a[i], b[l - i]);
+            c[l] = s.reduce(q);
+        }
+    }
+    __syncthreads();
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        if constexpr (sizeof(W) == 4) {
+            const uint2 ci = c[i];
+            uint64_t a0 = ci.x, a1 = ci.y;
+#pragma unroll 4
+            for (int j = 0; j < n - 1; ++j) {
+                const uint64_t x = xr[(long)j * n + i];
+                const uint2 y = c[n + j];
+                a0 += x * y.x;
+                a1 += x * y.y;
+            }
+            emit(i, mod_halves(a0, a1, q, magic));
+        } else {
+            ModAcc s;
+            s.mac(c[i], 1);
+#pragma unroll 2
+            for (int j = 0; j < n - 1; ++j) s.mac(xr[(long)j * n + i], c[n + j]);
+            emit(i, s.reduce(q));
+        }
+    }
+}
+
+// y_i = sum_{s<k} sb[s] base^s mod q for one row of int32 entries (G sigma_bot), as fa_tag_correct_kernel forms it: (sb mod
+// q) times the halves of base^s mod q for W = uint32_t (k <= 64 terms < 2^48), 192-bit sums otherwise
 template <typename W>
+__device__ __forceinline__ uint64_t gadget_row_mod(const int32_t* sb, const uint64_t* __restrict__ gpow, uint64_t q,
+                                                   uint64_t magic, int k) {
+    if constexpr (sizeof(W) == 4) {
+        uint64_t a0 = 0, a1 = 0;
+        for (int s = 0; s < k; ++s) {
+            const uint64_t sm = mod_i64_barrett((long long)sb[s], q, magic), gs = gpow[s];
+            a0 += sm * (gs & 0xFFFF);
+            a1 += sm * (gs >> 16);
+        }
+        return mod_halves(a0, a1, q, magic);
+    } else {
+        ModAcc a;
+        for (int s = 0; s < k; ++s) a.mac(sb[s] < 0 ? (uint64_t)((long long)sb[s] + (long long)q) : (uint64_t)sb[s], gpow[s]);
+        return a.reduce(q);
+    }
+}
+
+// POLY: the table holds s_t = h_t^-1 as n words per tag and the last step is v' = s_t * w mod (f, q) - y (xr: the rows of
+// poly_mulmod); otherwise H_t^-1 as n x n words and v' = H_t^-1 w - y.  y and w are formed the same way in both.
+template <typename W, bool POLY>
 __global__ void __launch_bounds__(512) tag_syndrome_kernel(const int64_t* __restrict__ V, long ldv, const double* __restrict__ P,
                                                            long ldp, int m_bar, const int32_t* __restrict__ tidx, int ntags,
                                                            const W* __restrict__ tab, const W* __restrict__ h0,
                                                            const uint64_t* __restrict__ gpow, uint64_t q, uint64_t magic, int n,
-                                                           int k, int64_t* __restrict__ out, long ldout, int* flag) {
+                                                           int k, int64_t* __restrict__ out, long ldout, int* flag,
+                                                           const W* __restrict__ xr) {
     extern __shared__ uint64_t tag_sh[];
     const long b = blockIdx.x;
     const int t = tidx[b];
@@ -928,7 +1018,7 @@ __global__ void __launch_bounds__(512) tag_syndrome_kernel(const int64_t* __rest
         return;
     }
     const double* pb = P ? P + b * ldp + m_bar : nullptr;
-    const W* hi = tab + (long)t * n * n;
+    const W* hi = tab + (long)t * n * (POLY ? 1 : n);
     if constexpr (sizeof(W) == 4) {
         uint2* ys = reinterpret_cast<uint2*>(tag_sh);  // 16-bit halves of y and w
         uint2* ws = ys + n;
@@ -963,19 +1053,26 @@ __global__ void __launch_bounds__(512) tag_syndrome_kernel(const int64_t* __rest
         }
         __syncthreads();
         // v' = H_t^-1 w - y
-        for (int i = threadIdx.x; i < n; i += blockDim.x) {
-            uint64_t a0 = 0, a1 = 0;
+        if constexpr (POLY) {
+            poly_mulmod<W>(hi, ws, ws + n, xr, q, magic, n, [&](int i, uint64_t x) {
+                const uint64_t yi = PolySV<W>::get(ys[i]);
+                out[b * ldout + i] = (int64_t)(x >= yi ? x - yi : x + (q - yi));
+            });
+        } else {
+            for (int i = threadIdx.x; i < n; i += blockDim.x) {
+                uint64_t a0 = 0, a1 = 0;
 #pragma unroll 8
-            for (int j = 0; j < n; ++j) {
-                const uint64_t h = hi[(long)j * n + i];
-                const uint2 wj = ws[j];
-                a0 += h * wj.x;
-                a1 += h * wj.y;
+                for (int j = 0; j < n; ++j) {
+                    const uint64_t h = hi[(long)j * n + i];
+                    const uint2 wj = ws[j];
+                    a0 += h * wj.x;
+                    a1 += h * wj.y;
+                }
+                const uint64_t x = mod_halves(a0, a1, q, magic);
+                const uint2 yh = ys[i];
+                const uint64_t yi = yh.x + ((uint64_t)yh.y << 16);
+                out[b * ldout + i] = (int64_t)(x >= yi ? x - yi : x + (q - yi));
             }
-            const uint64_t x = mod_halves(a0, a1, q, magic);
-            const uint2 yh = ys[i];
-            const uint64_t yi = yh.x + ((uint64_t)yh.y << 16);
-            out[b * ldout + i] = (int64_t)(x >= yi ? x - yi : x + (q - yi));
         }
     } else {
         typedef __int128 i128;
@@ -1001,45 +1098,54 @@ __global__ void __launch_bounds__(512) tag_syndrome_kernel(const int64_t* __rest
             w[i] = sum >= q ? sum - q : sum;
         }
         __syncthreads();
-        for (int i = threadIdx.x; i < n; i += blockDim.x) {
-            ModAcc a;
+        if constexpr (POLY) {
+            poly_mulmod<W>(hi, w, w + n, xr, q, magic, n, [&](int i, uint64_t x) {
+                const uint64_t yi = y[i];
+                out[b * ldout + i] = (int64_t)(x >= yi ? x - yi : x + (q - yi));
+            });
+        } else {
+            for (int i = threadIdx.x; i < n; i += blockDim.x) {
+                ModAcc a;
 #pragma unroll 4
-            for (int j = 0; j < n; ++j) a.mac(hi[(long)j * n + i], w[j]);
-            const uint64_t x = a.reduce(q), yi = y[i];
-            out[b * ldout + i] = (int64_t)(x >= yi ? x - yi : x + (q - yi));
+                for (int j = 0; j < n; ++j) a.mac(hi[(long)j * n + i], w[j]);
+                const uint64_t x = a.reduce(q), yi = y[i];
+                out[b * ldout + i] = (int64_t)(x >= yi ? x - yi : x + (q - yi));
+            }
         }
     }
+}
+
+template <typename W, bool POLY>
+cudaError_t launch_tag_syndrome(const int64_t* V, long ldv, const double* P, long ldp, int m_bar, const int32_t* tidx,
+                                int ntags, const void* tab, const void* h0, const uint64_t* gpow, uint64_t q, int n, int k,
+                                int B, int64_t* out, long ldout, int* flag, const void* xr, cudaStream_t stream) {
+    const int threads = n >= 512 ? 512 : (n + 31) / 32 * 32;
+    // y and w; the polynomial form adds the 2n - 1 words of the product's scratch
+    const size_t smem = (size_t)(POLY ? 4 : 2) * n * sizeof(uint64_t);
+    cudaError_t e;
+    if (smem > 48 * 1024 &&
+        (e = cudaFuncSetAttribute(tag_syndrome_kernel<W, POLY>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
+        return e;
+    tag_syndrome_kernel<W, POLY><<<B, threads, smem, stream>>>(V, ldv, P, ldp, m_bar, tidx, ntags, (const W*)tab,
+                                                                         (const W*)h0, gpow, q, qf_barrett_magic(q), n, k, out,
+                                                                         ldout, flag, (const W*)xr);
+    return cudaGetLastError();
 }
 }  // namespace
 
 cudaError_t qf_launch_tag_syndrome(const int64_t* V, long ldv, const double* P, long ldp, int m_bar, const int32_t* tidx,
                                    int ntags, const void* tab, const void* h0, int word_bytes, const uint64_t* gpow,
                                    unsigned long long q, int n, int k, int B, int64_t* out, long ldout, int* flag,
-                                   cudaStream_t stream) {
+                                   cudaStream_t stream, const void* xr) {
     if (B <= 0) return cudaSuccess;
     if (n < 1 || k < 1 || k > 64 || q < 2 || q >= (1ull << 62) || (word_bytes != 4 && word_bytes != 8) ||
         (word_bytes == 4 && (q > (1ull << 32) || n > (1 << 14))))
         return cudaErrorInvalidValue;
-    const int threads = n >= 512 ? 512 : (n + 31) / 32 * 32;
-    const size_t smem = (size_t)2 * n * sizeof(uint64_t);
-    const uint64_t magic = qf_barrett_magic(q);
-    cudaError_t e;
-    if (word_bytes == 4) {
-        if (smem > 48 * 1024 &&
-            (e = cudaFuncSetAttribute(tag_syndrome_kernel<uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
-            return e;
-        tag_syndrome_kernel<uint32_t><<<B, threads, smem, stream>>>(V, ldv, P, ldp, m_bar, tidx, ntags, (const uint32_t*)tab,
-                                                                    (const uint32_t*)h0, gpow, (uint64_t)q, magic, n, k, out,
-                                                                    ldout, flag);
-    } else {
-        if (smem > 48 * 1024 &&
-            (e = cudaFuncSetAttribute(tag_syndrome_kernel<uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess)
-            return e;
-        tag_syndrome_kernel<uint64_t><<<B, threads, smem, stream>>>(V, ldv, P, ldp, m_bar, tidx, ntags, (const uint64_t*)tab,
-                                                                    (const uint64_t*)h0, gpow, (uint64_t)q, magic, n, k, out,
-                                                                    ldout, flag);
-    }
-    return cudaGetLastError();
+    if (word_bytes == 4)
+        return xr ? launch_tag_syndrome<uint32_t, true>(V, ldv, P, ldp, m_bar, tidx, ntags, tab, h0, gpow, q, n, k, B, out, ldout, flag, xr, stream)
+                  : launch_tag_syndrome<uint32_t, false>(V, ldv, P, ldp, m_bar, tidx, ntags, tab, h0, gpow, q, n, k, B, out, ldout, flag, xr, stream);
+    return xr ? launch_tag_syndrome<uint64_t, true>(V, ldv, P, ldp, m_bar, tidx, ntags, tab, h0, gpow, q, n, k, B, out, ldout, flag, xr, stream)
+              : launch_tag_syndrome<uint64_t, false>(V, ldv, P, ldp, m_bar, tidx, ntags, tab, h0, gpow, q, n, k, B, out, ldout, flag, xr, stream);
 }
 
 // ---- per-target tag of f_a (qf_f_a_tagged): u_b += D_t y_b mod q with y_b = G sigma_bot_b, D_t = H_t - H_0, t = tidx[b] -------
@@ -1324,6 +1430,347 @@ cudaError_t qf_launch_f_a_tag_correct(const int32_t* sigma, long lds, int m_bar,
         fa_tag_correct_kernel<uint64_t><<<(unsigned)grid, threads, smem, stream>>>(sigma, lds, m_bar, tidx, ntags, perm, off, gstart,
                                                                         (const uint64_t*)tab, gpow, (uint64_t)q, magic, n, k,
                                                                         u, ldu, flag);
+    }
+    return cudaGetLastError();
+}
+
+// ---- tags in polynomial form (qf_set_tag_table_poly, qf_set_f_a_tags_poly; DESIGN 4.10) ---------------------------------
+// H_t = rot_f(h_t), column c = coeffs(h_t X^c mod f).  rot_f(a) b = a * b mod f and rot_f(h)^-1 = rot_f(h^-1), so a tag is
+// n words, inverting it costs O(n^2) and applying it is one poly_mulmod.
+namespace {
+typedef unsigned __int128 u128;
+
+__device__ __forceinline__ uint64_t mulmod_p(uint64_t a, uint64_t b, uint64_t p) {
+    return p <= (1ull << 32) ? (a * b) % p : (uint64_t)((u128)a * b % p);
+}
+// a^-1 mod p for a unit a (extended Euclid on integers; |t| <= p < 2^62)
+__device__ uint64_t inv_mod_p(uint64_t a, uint64_t p) {
+    long long t = 0, nt = 1;
+    uint64_t r = p, nr = a;
+    while (nr) {
+        const uint64_t qq = r / nr;
+        const long long tt = t - (long long)qq * nt;
+        t = nt;
+        nt = tt;
+        const uint64_t rr = r - qq * nr;
+        r = nr;
+        nr = rr;
+    }
+    return t < 0 ? (uint64_t)(t + (long long)p) : (uint64_t)t;
+}
+
+// rows X^{n+j} mod (f, q), j < n - 1: row 0 = -f, row j+1 = X row j mod f = (row j shifted up) - row_j[n-1] f.  One CTA; the
+// rows are built in place in the table (a barrier per row makes row j visible to the block).
+template <typename W>
+__global__ void __launch_bounds__(512) poly_xpow_kernel(const uint64_t* __restrict__ fq, int n, uint64_t q, W* xr) {
+    for (int i = threadIdx.x; i < n; i += blockDim.x) xr[i] = (W)(fq[i] ? q - fq[i] : 0);
+    for (int j = 0; j + 1 < n - 1; ++j) {
+        __syncthreads();
+        const W* row = xr + (long)j * n;
+        const uint64_t top = row[n - 1];
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            const uint64_t lo = i ? (uint64_t)row[i - 1] : 0, d = (uint64_t)((u128)top * fq[i] % q);
+            xr[(long)(j + 1) * n + i] = (W)(lo >= d ? lo - d : lo + (q - d));
+        }
+    }
+}
+
+// tab[x] = tags[x] mod q in words of W (count words, any sign)
+template <typename W>
+__global__ void poly_tag_pack_kernel(const int64_t* __restrict__ tags, long count, uint64_t q, W* __restrict__ tab) {
+    for (long x = (long)blockIdx.x * blockDim.x + threadIdx.x; x < count; x += (long)gridDim.x * blockDim.x) {
+        const long long v = tags[x] % (long long)q;
+        tab[x] = (W)(v < 0 ? v + (long long)q : v);
+    }
+}
+
+// One CTA per tag h (count tags of n int64 coefficients, any sign), q = p^e:
+//  1. h mod q, and extended Euclid in F_p[X] against f mod p, one elimination step A -= c X^(dA - dB) B per iteration
+//     (at most 2n; thread 0 keeps the degrees and the one scalar inverse per remainder, the threads the O(n) update), with
+//     the cofactors tA, tB: tA h = A, tB h = B mod (f, p).  B a non-zero constant: s = tB / B mod p; B = 0: not a unit.
+//  2. Newton s <- s (2 - h s) mod (f, q), `lifts` = ceil(log2 e) times (the error 1 - h s squares each time).
+//  3. h s = 1 mod (f, q) is checked exactly before s is stored (n words of W per tag).
+// fail[t] = 0 on success, 1 when h is not a unit (the tag's words are then left unwritten).
+template <typename W>
+__global__ void __launch_bounds__(256) poly_tag_inverse_kernel(const int64_t* __restrict__ tags, int n,
+                                                               const uint64_t* __restrict__ fq, const W* __restrict__ xr,
+                                                               uint64_t q, uint64_t magic, uint64_t p, int lifts,
+                                                               W* __restrict__ tab, int* __restrict__ fail) {
+    typedef typename PolySV<W>::T SV;
+    extern __shared__ uint64_t pi_sh[];
+    // Euclid: two remainders and two cofactors of n + 1 coefficients; Newton: h, s (words), s and u (PolySV), product scratch
+    uint64_t* rem[2] = {pi_sh, pi_sh + (n + 1)};
+    uint64_t* cof[2] = {pi_sh + 2 * (n + 1), pi_sh + 3 * (n + 1)};
+    uint64_t* h = pi_sh + 4 * (n + 1);
+    uint64_t* s = h + n;
+    SV* s_sv = reinterpret_cast<SV*>(s + n);
+    SV* u_sv = s_sv + n;
+    SV* c = u_sv + n;
+    __shared__ int s_op, s_which, s_da, s_db, s_sh;
+    __shared__ uint64_t s_cc, s_ilc;
+    const long t = blockIdx.x;
+    const int64_t* ht = tags + t * n;
+    for (int i = threadIdx.x; i <= n; i += blockDim.x) {
+        uint64_t hv = 0;
+        if (i < n) {
+            const long long v = ht[i] % (long long)q;
+            hv = (uint64_t)(v < 0 ? v + (long long)q : v);
+            h[i] = hv;
+        }
+        rem[0][i] = i < n ? fq[i] % p : 1 % p;
+        rem[1][i] = hv % p;
+        cof[0][i] = 0;
+        cof[1][i] = i == 0;
+    }
+    __syncthreads();
+    // control (thread 0): op 0 = eliminate rem[which] -= cc X^sh rem[1 - which]; 1 = rem[1 - which] is a unit; 2 = not a unit
+    auto plan = [&](int da, int db, int which, bool fresh_b) {
+        const uint64_t* A = rem[which];
+        const uint64_t* B = rem[which ^ 1];
+        if (da < db) {  // the remainder fell below the divisor: swap roles
+            which ^= 1;
+            const int x = da;
+            da = db;
+            db = x;
+            A = rem[which];
+            B = rem[which ^ 1];
+            fresh_b = true;
+        }
+        s_which = which;
+        s_da = da;
+        s_db = db;
+        if (db <= 0) {
+            s_op = db == 0 ? 1 : 2;
+            return;
+        }
+        if (fresh_b) s_ilc = inv_mod_p(B[db], p);
+        s_cc = mulmod_p(A[da], s_ilc, p);
+        s_sh = da - db;
+        s_op = 0;
+    };
+    if (threadIdx.x == 0) {
+        int db = n - 1;
+        while (db >= 0 && rem[1][db] == 0) --db;
+        plan(n, db, 0, true);
+    }
+    for (;;) {
+        __syncthreads();
+        const int op = s_op;
+        if (op) break;
+        const int which = s_which, db = s_db, sh = s_sh;
+        const uint64_t cc = s_cc;
+        uint64_t *A = rem[which], *tA = cof[which];
+        const uint64_t *B = rem[which ^ 1], *tB = cof[which ^ 1];
+        for (int i = threadIdx.x; i + sh <= n; i += blockDim.x) {
+            if (i <= db) {
+                const uint64_t d = mulmod_p(cc, B[i], p), a = A[i + sh];
+                A[i + sh] = a >= d ? a - d : a + (p - d);
+            }
+            const uint64_t d = mulmod_p(cc, tB[i], p), a = tA[i + sh];
+            tA[i + sh] = a >= d ? a - d : a + (p - d);
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            int da = s_da - 1;  // A[s_da] is now 0
+            while (da >= 0 && A[da] == 0) --da;
+            plan(da, db, which, false);
+        }
+    }
+    const bool unit = s_op == 1;
+    if (!unit) {
+        if (threadIdx.x == 0) fail[t] = 1;
+        return;
+    }
+    {
+        const int wb = s_which ^ 1;
+        const uint64_t ib = inv_mod_p(rem[wb][0], p);
+        for (int i = threadIdx.x; i < n; i += blockDim.x) {
+            const uint64_t v = mulmod_p(cof[wb][i], ib, p);
+            s[i] = v;
+            s_sv[i] = PolySV<W>::put(v);
+        }
+    }
+    __syncthreads();
+    const uint64_t two = 2 % q;
+    for (int it = 0; it < lifts; ++it) {
+        poly_mulmod<W>(h, s_sv, c, xr, q, magic, n, [&](int i, uint64_t r) {  // u = 2 - h s
+            const uint64_t w = i == 0 ? two : 0;
+            u_sv[i] = PolySV<W>::put(w >= r ? w - r : w + (q - r));
+        });
+        __syncthreads();
+        poly_mulmod<W>(s, u_sv, c, xr, q, magic, n, [&](int i, uint64_t r) {  // s <- s u
+            s[i] = r;
+            s_sv[i] = PolySV<W>::put(r);
+        });
+        __syncthreads();
+    }
+    bool ok = true;
+    poly_mulmod<W>(h, s_sv, c, xr, q, magic, n, [&](int i, uint64_t r) { ok = ok && r == (i == 0 ? 1 % q : 0); });
+    ok = __syncthreads_and(ok);
+    for (int i = threadIdx.x; i < n; i += blockDim.x)
+        if (ok) tab[t * n + i] = (W)s[i];
+    if (threadIdx.x == 0) fail[t] = ok ? 0 : 1;
+}
+
+// f_a in polynomial form, one CTA per target b (t = tidx[b]): u_b += h_t * y_b mod (f, q) - H_0 y_b, y_b = G sigma_bot_b.
+// n words per tag need no grouping by tag.  h0_kind: 0 H_0 = 0, 1 H_0 = I, 2 dense H_0 (n x n column-major words of W, the
+// same for every target, L2-resident).  An index outside the table never addresses it: the row keeps A sigma and the flag
+// bit is set.
+template <typename W>
+__global__ void __launch_bounds__(512) fa_tag_poly_kernel(const int32_t* __restrict__ sigma, long lds, int m_bar,
+                                                          const int32_t* __restrict__ tidx, int ntags, const W* __restrict__ tab,
+                                                          const W* __restrict__ xr, const W* __restrict__ h0, int h0_kind,
+                                                          const uint64_t* __restrict__ gpow, uint64_t q, uint64_t magic, int n,
+                                                          int k, int64_t* __restrict__ u, long ldu, int* flag) {
+    typedef typename PolySV<W>::T SV;
+    extern __shared__ uint64_t fp_sh[];
+    const long b = blockIdx.x;
+    const int t = tidx[b];
+    if (t < 0 || t >= ntags) {
+        if (threadIdx.x == 0 && flag) atomicOr(flag, QF_FLAG_TAG_INDEX);
+        return;
+    }
+    SV* ys = reinterpret_cast<SV*>(fp_sh);
+    SV* c = ys + n;
+    for (int i = threadIdx.x; i < n; i += blockDim.x)
+        ys[i] = PolySV<W>::put(gadget_row_mod<W>(sigma + b * lds + m_bar + (long)i * k, gpow, q, magic, k));
+    __syncthreads();
+    poly_mulmod<W>(tab + (long)t * n, ys, c, xr, q, magic, n, [&](int i, uint64_t r) {
+        uint64_t hy = 0;
+        if (h0_kind == 1) {
+            hy = PolySV<W>::get(ys[i]);
+        } else if (h0_kind == 2) {
+            if constexpr (sizeof(W) == 4) {
+                uint64_t a0 = 0, a1 = 0;
+#pragma unroll 4
+                for (int j = 0; j < n; ++j) {
+                    const uint64_t x = h0[(long)j * n + i];
+                    const uint2 yj = ys[j];
+                    a0 += x * yj.x;
+                    a1 += x * yj.y;
+                }
+                hy = mod_halves(a0, a1, q, magic);
+            } else {
+                ModAcc a;
+#pragma unroll 2
+                for (int j = 0; j < n; ++j) a.mac(h0[(long)j * n + i], ys[j]);
+                hy = a.reduce(q);
+            }
+        }
+        int64_t* ub = u + b * ldu + i;
+        uint64_t v = (uint64_t)*ub + r;
+        v = v >= q ? v - q : v;
+        *ub = (int64_t)(v >= hy ? v - hy : v + (q - hy));
+    });
+}
+
+constexpr size_t poly_inverse_smem(int n) { return ((size_t)4 * (n + 1) + (size_t)6 * n) * sizeof(uint64_t); }
+constexpr size_t poly_syndrome_smem(int n) { return (size_t)4 * n * sizeof(uint64_t); }
+constexpr size_t poly_fa_smem(int n) { return (size_t)3 * n * sizeof(uint64_t); }
+
+cudaError_t smem_optin(int* optin) {
+    int dev = 0;
+    cudaError_t e;
+    if ((e = cudaGetDevice(&dev)) != cudaSuccess) return e;
+    return cudaDeviceGetAttribute(optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+}
+
+// static + dynamic shared memory of the kernel within one block's opt-in limit
+template <typename K>
+cudaError_t smem_fits(K kernel, size_t dyn, int optin, bool* fits) {
+    cudaFuncAttributes a;
+    cudaError_t e = cudaFuncGetAttributes(&a, kernel);
+    if (e != cudaSuccess) return e;
+    *fits = *fits && dyn + a.sharedSizeBytes <= (size_t)optin;
+    return cudaSuccess;
+}
+
+template <typename K>
+cudaError_t set_smem(K kernel, size_t dyn) {
+    return dyn > 48 * 1024 ? cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn) : cudaSuccess;
+}
+}  // namespace
+
+cudaError_t qf_poly_tag_supported(int n, int k, int samp_p, int* ok) {
+    int optin = 0;
+    cudaError_t e = smem_optin(&optin);
+    if (e != cudaSuccess) return e;
+    bool fits = n >= 1 && k >= 1 && k <= 64 && n <= (1 << 14);
+    if (samp_p) {
+        if ((e = smem_fits(poly_tag_inverse_kernel<uint32_t>, poly_inverse_smem(n), optin, &fits)) != cudaSuccess) return e;
+        if ((e = smem_fits(poly_tag_inverse_kernel<uint64_t>, poly_inverse_smem(n), optin, &fits)) != cudaSuccess) return e;
+        if ((e = smem_fits(tag_syndrome_kernel<uint32_t, true>, poly_syndrome_smem(n), optin, &fits)) != cudaSuccess) return e;
+        if ((e = smem_fits(tag_syndrome_kernel<uint64_t, true>, poly_syndrome_smem(n), optin, &fits)) != cudaSuccess) return e;
+    } else {
+        if ((e = smem_fits(fa_tag_poly_kernel<uint32_t>, poly_fa_smem(n), optin, &fits)) != cudaSuccess) return e;
+        if ((e = smem_fits(fa_tag_poly_kernel<uint64_t>, poly_fa_smem(n), optin, &fits)) != cudaSuccess) return e;
+    }
+    *ok = fits;
+    return cudaSuccess;
+}
+
+cudaError_t qf_launch_poly_xpow(const uint64_t* fq, int n, unsigned long long q, int word_bytes, void* xr, cudaStream_t stream) {
+    if (n < 2) return cudaSuccess;  // no row: a product of constants needs no reduction
+    const int threads = n >= 512 ? 512 : (n + 31) / 32 * 32;
+    if (word_bytes == 4) poly_xpow_kernel<uint32_t><<<1, threads, 0, stream>>>(fq, n, (uint64_t)q, (uint32_t*)xr);
+    else poly_xpow_kernel<uint64_t><<<1, threads, 0, stream>>>(fq, n, (uint64_t)q, (uint64_t*)xr);
+    return cudaGetLastError();
+}
+
+cudaError_t qf_launch_poly_tag_pack(const int64_t* tags, long count, unsigned long long q, int word_bytes, void* tab,
+                                    cudaStream_t stream) {
+    if (count <= 0) return cudaSuccess;
+    const int grid = grid_for(count, 256, 148 * 8);
+    if (word_bytes == 4) poly_tag_pack_kernel<uint32_t><<<grid, 256, 0, stream>>>(tags, count, (uint64_t)q, (uint32_t*)tab);
+    else poly_tag_pack_kernel<uint64_t><<<grid, 256, 0, stream>>>(tags, count, (uint64_t)q, (uint64_t*)tab);
+    return cudaGetLastError();
+}
+
+cudaError_t qf_launch_poly_tag_inverse(const int64_t* tags, int count, int n, const uint64_t* fq, const void* xr,
+                                       int word_bytes, unsigned long long q, unsigned long long p, int lifts, void* tab,
+                                       int* fail, cudaStream_t stream) {
+    if (count <= 0) return cudaSuccess;
+    if (n < 1 || q < 2 || q >= (1ull << 62) || p < 2 || q % p || (word_bytes != 4 && word_bytes != 8) ||
+        (word_bytes == 4 && (q > (1ull << 32) || n > (1 << 14))))
+        return cudaErrorInvalidValue;
+    const int threads = n >= 256 ? 256 : (n + 31) / 32 * 32;
+    const size_t smem = poly_inverse_smem(n);
+    const uint64_t magic = qf_barrett_magic(q);
+    cudaError_t e;
+    if (word_bytes == 4) {
+        if ((e = set_smem(poly_tag_inverse_kernel<uint32_t>, smem)) != cudaSuccess) return e;
+        poly_tag_inverse_kernel<uint32_t><<<count, threads, smem, stream>>>(tags, n, fq, (const uint32_t*)xr, (uint64_t)q, magic,
+                                                                            (uint64_t)p, lifts, (uint32_t*)tab, fail);
+    } else {
+        if ((e = set_smem(poly_tag_inverse_kernel<uint64_t>, smem)) != cudaSuccess) return e;
+        poly_tag_inverse_kernel<uint64_t><<<count, threads, smem, stream>>>(tags, n, fq, (const uint64_t*)xr, (uint64_t)q, magic,
+                                                                            (uint64_t)p, lifts, (uint64_t*)tab, fail);
+    }
+    return cudaGetLastError();
+}
+
+cudaError_t qf_launch_f_a_tag_poly(const int32_t* sigma, long lds, int m_bar, const int32_t* tidx, int ntags, const void* tab,
+                                   const void* xr, const void* h0, int h0_kind, int word_bytes, const uint64_t* gpow,
+                                   unsigned long long q, int n, int k, int B, int64_t* u, long ldu, int* flag,
+                                   cudaStream_t stream) {
+    if (B <= 0) return cudaSuccess;
+    if (n < 1 || k < 1 || k > 64 || q < 2 || q >= (1ull << 62) || (word_bytes != 4 && word_bytes != 8) ||
+        (word_bytes == 4 && (q > (1ull << 32) || n > (1 << 14))) || h0_kind < 0 || h0_kind > 2 || (h0_kind == 2 && !h0))
+        return cudaErrorInvalidValue;
+    const int threads = n >= 512 ? 512 : (n + 31) / 32 * 32;
+    const size_t smem = poly_fa_smem(n);
+    const uint64_t magic = qf_barrett_magic(q);
+    cudaError_t e;
+    if (word_bytes == 4) {
+        if ((e = set_smem(fa_tag_poly_kernel<uint32_t>, smem)) != cudaSuccess) return e;
+        fa_tag_poly_kernel<uint32_t><<<B, threads, smem, stream>>>(sigma, lds, m_bar, tidx, ntags, (const uint32_t*)tab,
+                                                                   (const uint32_t*)xr, (const uint32_t*)h0, h0_kind, gpow,
+                                                                   (uint64_t)q, magic, n, k, u, ldu, flag);
+    } else {
+        if ((e = set_smem(fa_tag_poly_kernel<uint64_t>, smem)) != cudaSuccess) return e;
+        fa_tag_poly_kernel<uint64_t><<<B, threads, smem, stream>>>(sigma, lds, m_bar, tidx, ntags, (const uint64_t*)tab,
+                                                                   (const uint64_t*)xr, (const uint64_t*)h0, h0_kind, gpow,
+                                                                   (uint64_t)q, magic, n, k, u, ldu, flag);
     }
     return cudaGetLastError();
 }

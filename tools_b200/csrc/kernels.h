@@ -280,10 +280,12 @@ cudaError_t qf_launch_tag_pack(const uint64_t* M, int count, int n, int word_byt
 // per-target tag of samp_p (elementwise.cu): out[b] = H_{tidx[b]}^-1 (V[b] + H_0 y) - y mod q, y = G p_bot, p_bot =
 // P[b][m_bar:]; tab / h0 column-major n x n words (word_bytes 4 needs q <= 2^32 and n <= 2^14); h0 = NULL means H_0 = I; gpow: base^s mod q,
 // s < k <= 64.  A tag index outside [0, ntags) sets *flag |= QF_FLAG_TAG_INDEX and gives out[b] = 0.
+// xr != NULL: the table is in polynomial form (n words h_t^-1 per tag, xr from qf_launch_poly_xpow) and
+// out[b] = h_t^-1 * (V[b] + H_0 y) mod (f, q) - y.
 cudaError_t qf_launch_tag_syndrome(const int64_t* V, long ldv, const double* P, long ldp, int m_bar, const int32_t* tidx,
                                    int ntags, const void* tab, const void* h0, int word_bytes, const uint64_t* gpow,
                                    unsigned long long q, int n, int k, int B, int64_t* out, long ldout, int* flag,
-                                   cudaStream_t stream);
+                                   cudaStream_t stream, const void* xr = nullptr);
 // f_a tag table (setup.cu): tab[t] = (tags[t] - H_0) mod q column-major (count x n x n words of word_bytes = 4 or 8) from
 // int64 tags (count x n x n, any sign); h0: n x n residues row-major, NULL means H_0 = I
 cudaError_t qf_launch_tag_diff_pack(const int64_t* tags, int count, int n, unsigned long long q, const uint64_t* h0,
@@ -311,6 +313,28 @@ cudaError_t qf_launch_f_a_tag_correct(const int32_t* sigma, long lds, int m_bar,
                                       const int* perm, const int* off, const int* gstart, const void* tab, int word_bytes,
                                       const uint64_t* gpow, unsigned long long q, int n, int k, int B, int64_t* u, long ldu,
                                       int* flag, cudaStream_t stream);
+
+// tags in polynomial form (elementwise.cu, DESIGN 4.10): H_t = rot_f(h_t), f = X^n + sum_{i<n} f_i X^i with fq = f_i mod q.
+// *ok = 1 when the kernels of the samp_p table (samp_p != 0: inverse and syndrome) or of the f_a table run for this n and k
+// on the current device: k <= 64, n <= 2^14, static plus dynamic shared memory within the per-block opt-in limit.
+cudaError_t qf_poly_tag_supported(int n, int k, int samp_p, int* ok);
+// xr = rows X^{n+j} mod (f, q), j < n - 1, n words of word_bytes each (nothing for n = 1)
+cudaError_t qf_launch_poly_xpow(const uint64_t* fq, int n, unsigned long long q, int word_bytes, void* xr, cudaStream_t stream);
+// tab[x] = tags[x] mod q, count words of word_bytes (any sign)
+cudaError_t qf_launch_poly_tag_pack(const int64_t* tags, long count, unsigned long long q, int word_bytes, void* tab,
+                                    cudaStream_t stream);
+// tab[t] = h_t^-1 mod (f, q) for count tags of n coefficients (any sign), q = p^e, lifts = ceil(log2 e), one CTA per tag;
+// fail[t] = 0 on success, 1 when h_t is not a unit (its words are then not written)
+cudaError_t qf_launch_poly_tag_inverse(const int64_t* tags, int count, int n, const uint64_t* fq, const void* xr,
+                                       int word_bytes, unsigned long long q, unsigned long long p, int lifts, void* tab,
+                                       int* fail, cudaStream_t stream);
+// u[b] += h_t * y_b mod (f, q) - H_0 y_b with y_b = G sigma[b][m_bar:], t = tidx[b], one CTA per target; h0_kind 0: H_0 = 0,
+// 1: H_0 = I, 2: h0 (n x n column-major words).  An index outside [0, ntags) sets *flag |= QF_FLAG_TAG_INDEX and leaves
+// the row as A sigma.
+cudaError_t qf_launch_f_a_tag_poly(const int32_t* sigma, long lds, int m_bar, const int32_t* tidx, int ntags, const void* tab,
+                                   const void* xr, const void* h0, int h0_kind, int word_bytes, const uint64_t* gpow,
+                                   unsigned long long q, int n, int k, int B, int64_t* u, long ldu, int* flag,
+                                   cudaStream_t stream);
 
 // polynomial arithmetic of the ring short basis (setup.cu): P[2][2][n], Q[k][2][n]
 cudaError_t qf_launch_ring_basis_polys(const int32_t* e, const int32_t* r, const int32_t* w, const int64_t* sk, int n, int k,

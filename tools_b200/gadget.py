@@ -211,6 +211,22 @@ def rot_minus_matrix(matrix) -> np.ndarray:
     return np.concatenate([rot_minus(m[:, c]) for c in range(m.shape[1])], axis=1)
 
 
+def rot_f(h, f, q: int) -> np.ndarray:
+    """The tag of h in polynomial form: the n x n matrix of multiplication by h in Z_q[X]/(f), f = X^n + sum_{i<n} f[i] X^i
+    monic (f: its n low coefficients).  Column c holds the coefficients of h X^c mod f, reduced mod q (int64).  For
+    f = X^n + 1 it is rot_minus(h) mod q."""
+    fv = [int(x) for x in np.asarray(f, dtype=object).reshape(-1)]
+    col = [int(x) % q for x in np.asarray(h, dtype=object).reshape(-1)]
+    n = len(fv)
+    assert len(col) == n
+    out = np.zeros((n, n), dtype=object)
+    for c in range(n):
+        out[:, c] = col
+        top = col[-1]
+        col = [((col[i - 1] if i else 0) - top * fv[i]) % q for i in range(n)]
+    return np.array(out, dtype=np.int64)
+
+
 def _rot_i64(p: np.ndarray) -> np.ndarray:
     n = len(p)
     out = np.zeros((n, n), dtype=np.int64)

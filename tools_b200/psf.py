@@ -117,22 +117,27 @@ class _PSFBase:
         """f_a with a tag per target (classical contexts): u[b] = A_t sigma[b] with A_t = a + [0 | (H_t - H_0) G],
         H_t = tags[tag_idx[b]], for a key a = [A_bar | H_0 G - A_bar R] (h0 = H_0, None: I; H_0 = 0 is allowed).  That is
         the key gen_trapdoor(A_bar, R, H_t) gives, evaluated from a alone: no trapdoor is needed and no tag is inverted.
-        tags: T x n x n, h0: n x n (entries taken mod q); the table (qf_set_f_a_tags) is cached on the device by the
+        tags: T x n x n or PolyTags, h0: n x n (entries taken mod q); the table (qf_set_f_a_tags[_poly]) is cached on the device by the
         identity of tags and h0 until the key on the device changes: the device drops the table there, and every place
         here that installs or rewrites A resets _fa_tags_id.  tag_idx: B indices in [0, T).  Returns (u, in_domain) as
         f_a_batch does."""
         self._install_a(a)
         key = self._fa_tags_id
         if key is None or key[0] is not tags or key[1] is not h0:
-            t = np.asarray(tags)
-            tg = np.ascontiguousarray(np.array(t % self.gp.q, dtype=np.int64) if t.dtype == object else t, dtype=np.int64)
-            assert tg.ndim == 3 and tg.shape[1:] == (self.n, self.n) and tg.shape[0] >= 1
             hg = None
             if h0 is not None:
                 h = np.asarray(h0)
                 hg = np.ascontiguousarray(np.array(h % self.gp.q, dtype=np.int64) if h.dtype == object else h, dtype=np.int64)
                 assert hg.shape == (self.n, self.n)
-            self.ctx.call("qf_set_f_a_tags", _ffi.ptr(tg), tg.shape[0], _ffi.ptr(hg))
+            if isinstance(tags, PolyTags):
+                fw, tw = tags.words(self.gp.q)
+                assert fw.shape == (self.n,)
+                self.ctx.call("qf_set_f_a_tags_poly", _ffi.ptr(fw), _ffi.ptr(tw), tw.shape[0], _ffi.ptr(hg))
+            else:
+                t = np.asarray(tags)
+                tg = np.ascontiguousarray(np.array(t % self.gp.q, dtype=np.int64) if t.dtype == object else t, dtype=np.int64)
+                assert tg.ndim == 3 and tg.shape[1:] == (self.n, self.n) and tg.shape[0] >= 1
+                self.ctx.call("qf_set_f_a_tags", _ffi.ptr(tg), tg.shape[0], _ffi.ptr(hg))
             self._fa_tags_id = (tags, h0)
         s, oob = _domain_i32(sigmas, self._domain_shape)
         ti = np.ascontiguousarray(tag_idx, dtype=np.int32)
@@ -174,6 +179,33 @@ class _PSFBase:
         return self.samp_p_batch(a, td, np.asarray(u, dtype=np.int64).reshape(1, self.n), seed)[0]
 
 
+class PolyTags:
+    """T tags in polynomial form: tag t is H_t = rot_f(tags[t]) (gadget.rot_f), the matrix of multiplication by the ring
+    element tags[t] in Z_q[X]/(f), f = X^n + sum_{i<n} f[i] X^i.  f: n low coefficients of the monic modulus; tags: T x n.
+    Entries are taken mod q (negatives allowed).  Accepted wherever a T x n x n tag array is (set_tag_table,
+    samp_p_tagged_batch, f_a_tagged_batch) and cached on the device by identity as that is; the device stores n words per
+    tag instead of n^2 (DESIGN.md 4.10)."""
+
+    def __init__(self, f, tags):
+        self.f = np.asarray(f)
+        self.tags = np.asarray(tags)
+        assert self.f.ndim == 1 and self.tags.ndim == 2 and self.tags.shape[1] == self.f.shape[0] and len(self.tags) >= 1
+
+    def __len__(self):
+        return len(self.tags)
+
+    def matrices(self, q: int) -> np.ndarray:
+        """The T x n x n tags rot_f(tags[t]) mod q."""
+        return np.stack([gadget.rot_f(h, self.f, q) for h in self.tags])
+
+    def words(self, q: int):
+        """(f, tags) as contiguous int64 for the C ABI (object entries are reduced mod q first)."""
+        def w(x):
+            return np.ascontiguousarray(np.array(x % q, dtype=np.int64) if x.dtype == object else x, dtype=np.int64)
+
+        return w(self.f), w(self.tags)
+
+
 class _TagTable:
     """samp_p with a tag per target for the classical PSFs whose trapdoor serves every tag of (A_bar, R): PSFPerturbation,
     and PSFGPV on the two-phase recursion (DESIGN.md 4.3, 4.4)."""
@@ -185,12 +217,19 @@ class _TagTable:
 
     def set_tag_table(self, a, td, tags):
         """Installs the tag table of samp_p_tagged_batch for the key a (any tag H_0) and its trapdoor td: tags is T x n x n,
-        entries taken mod q (qf_set_tag_table: H_t^-1 on the device).  Raises QfError (QF_ERR_INVALID, naming the index)
+        entries taken mod q (qf_set_tag_table: H_t^-1 on the device), or PolyTags (qf_set_tag_table_poly: h_t^-1 mod (f, q)
+        on the device; QfError QF_ERR_UNSUPPORTED unless q is a prime power).  Raises QfError (QF_ERR_INVALID, naming the index)
         when a tag has no unit pivot; the previous table then stays.  PSFGPV: QF_ERR_INVALID unless a and td run the
         two-phase recursion (a G-trapdoor key with its basis from gen_short_basis_for_trapdoor, m above the tensor-core
         threshold)."""
         self._install_a(a)
         self._install_td(a, td)
+        if isinstance(tags, PolyTags):
+            fw, tw = tags.words(self.gp.q)
+            assert fw.shape == (self.n,)
+            self.ctx.call("qf_set_tag_table_poly", _ffi.ptr(fw), _ffi.ptr(tw), tw.shape[0])
+            self._tags_id = tags
+            return
         t = np.asarray(tags)
         if t.dtype == object:
             t = np.array(t % self.gp.q, dtype=np.int64)
@@ -203,7 +242,7 @@ class _TagTable:
         """samp_p with a tag per target: row b is a preimage of us[b] under [A_bar | H_t G - A_bar R], H_t = tags[tag_idx[b]],
         for the key a = [A_bar | H_0 G - A_bar R] (any tag H_0) and its trapdoor td.  It equals what set_tag(H_t) followed
         by samp_p_batch on the same targets gives for that row with the same seed and first_index (qf_samp_p_tagged).
-        tags: T x n x n (entries taken mod q), cached on the device by identity as keys are; tag_idx: B indices in [0, T).
+        tags: T x n x n (entries taken mod q) or PolyTags, cached on the device by identity as keys are; tag_idx: B indices in [0, T).
         Returns B x m int32."""
         self._install_a(a)
         self._install_td(a, td)
