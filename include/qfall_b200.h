@@ -264,6 +264,50 @@ qf_status qf_f_a_i16(qf_ctx* ctx, const int16_t* sigma, int64_t batch, int64_t* 
  * the caller) gets bit 64 set when a value does not fit.  in / out 16-byte aligned. */
 qf_status qf_narrow_i32_i16_dev(const int32_t* in, int16_t* out, size_t count, int* overflow, void* cuda_stream);
 
+/* ---- packed Domain values: a lossless Golomb-Rice code of preimages (DESIGN 4.11) ---------------------------------------
+ * Entries of a preimage are close to D_{Z,w} (w = s, or s r for PSFPerturbation), about 11 bits of entropy at n = 256,
+ * q = 2^24; this code stores them in about 11.3 bits instead of int16's 16, for any int32 value but INT32_MIN.
+ * Format.  One row x_0 .. x_{dim-1} (dim = m, or n (k+2) for the ring) is stored in a slot of slot_bytes bytes, a multiple
+ * of 16.  Streams are LSB-first: bit j is bit j % 8 of byte j / 8.  Parameter k, 0 <= k <= 30; for each entry a = |x_i|,
+ * h_i = floor(a / 2^k), sign = (x_i < 0).
+ *  1. Fixed part: entry i is the (k+1)-bit field (a mod 2^k) | sign << k at bit offset i (k+1); it ends at byte
+ *     H0 = 16 ceil(dim (k+1) / 128); bits dim (k+1) .. 8 H0 - 1 are zero.
+ *  2. High stream from byte H0: for i = 0 .. dim-1 in order, h_i zero bits and then one 1 bit; every bit after the
+ *     dim-th 1 bit, to the end of the slot, is zero.
+ *  3. Length: nbytes = H0 + ceil(sum_i (h_i + 1) / 8).  A caller may keep the first nbytes bytes and pad with zeros to
+ *     read the row back.
+ * Canonical form: the decoder rejects a row with an entry of sign 1 and magnitude 0, fewer than dim 1 bits in the high
+ * stream, a non-zero padding bit (fixed part or tail), or a magnitude above INT32_MAX.  Every other slot decodes to exactly
+ * one row, and encoding that row gives the same bytes back.
+ * Overflow: a row whose code does not fit its slot, or that holds INT32_MIN, gets nbytes = -1 and an all-zero slot; the
+ * other rows are written and the call returns QF_ERR_NUMERIC.  Samplers are keyed by (seed, index), so qf_samp_p (or
+ * qf_samp_p_tagged) with first_index + b and batch 1 returns the int32 preimage of an overflowed row b: nothing is lost.
+ * Argument errors are QF_ERR_INVALID before any launch: k outside [0, 30], slot_bytes not a multiple of 16 or below
+ * H0 + ceil(dim / 8), NULL pointers. */
+/* Recommended parameters for the context's width w and dim: k minimises E[k + 2 + h] for X ~ D_{Z,w} (summed over
+ * |x| <= 20 w); slot_bytes = H0 + ceil((dim E[h+1] + 12 sqrt(dim Var[h+1])) / 8), rounded up to 16 (n = 256, q = 2^24
+ * PSFGPV: k = 8, 17 696 bytes against 24 704 as int16). */
+qf_status qf_domain_code_params(qf_ctx* ctx, int* k, int64_t* slot_bytes);
+/* samp_p with packed output (host pointers): out is batch x slot_bytes, nbytes batch lengths.  Row b is byte-identical to
+ * the code of row b of qf_samp_p (tag_idx == NULL) or qf_samp_p_tagged (tag_idx: host, as there: same contexts, readiness
+ * checks, and indices checked before any launch) for the same seed and first_index.  All three PSF kinds. */
+qf_status qf_samp_p_packed(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, uint64_t seed,
+                           uint64_t first_index, int k, int64_t slot_bytes, uint8_t* out, int32_t* nbytes);
+/* f_a / check_domain on packed Domain values (host pointers): the slots are decoded on the device, then f_a as qf_f_a
+ * (tag_idx == NULL) or qf_f_a_tagged (tag_idx: classical contexts, as there).  in_domain[b] = check_domain(sigma[b]) AND
+ * slot b is canonical; any 0 gives QF_ERR_NOT_IN_DOMAIN -- a malformed encoding is a rejected signature, not an error of
+ * the call.  u_out may be NULL (flags only), in_domain too. */
+qf_status qf_f_a_packed(qf_ctx* ctx, const uint8_t* packed, const int32_t* tag_idx, int64_t batch, int k, int64_t slot_bytes,
+                        int64_t* u_out, uint8_t* in_domain);
+/* Context-free device forms (asynchronous on cuda_stream, NULL = default stream): encode rows x dim int32 into rows slots
+ * (nbytes: rows lengths, -1 on overflow -- reported only there), and decode slots into int32 rows with ok[row] = 1 iff the
+ * slot is canonical (a rejected row's values are unspecified).  Slots (out / in) 16-byte aligned, int32 rows 4-byte
+ * aligned, else QF_ERR_INVALID. */
+qf_status qf_domain_encode_dev(const int32_t* in, int64_t rows, int64_t dim, int k, int64_t slot_bytes, uint8_t* out,
+                               int32_t* nbytes, void* cuda_stream);
+qf_status qf_domain_decode_dev(const uint8_t* in, int64_t rows, int64_t dim, int k, int64_t slot_bytes, int32_t* out,
+                               uint8_t* ok, void* cuda_stream);
+
 /* ---- PSFPerturbation::randomized_nearest_plane_gadget (mp_perturbation.rs:173-191), the public helper samp_p calls:
  * z[b] = x0 + SampleD(S, S~, -x0, r sqrt(base^2 + 1)) with x0 = find_solution_gadget_mat(v[b]) -- a preimage of v[b]
  * under the gadget matrix G, Gaussian over the coset Lambda_v^perp(G).  v: B x n residues, z_out: B x (n k).  The gadget

@@ -80,6 +80,11 @@ extern "C" {
     pub fn qf_samp_p_i16(ctx: *mut qf_ctx, u: *const i64, batch: i64, seed: u64, first_index: u64, e_out: *mut i16) -> i32;
     pub fn qf_f_a_i16(ctx: *mut qf_ctx, sigma: *const i16, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
     pub fn qf_narrow_i32_i16_dev(input: *const i32, out: *mut i16, count: usize, overflow: *mut i32, cuda_stream: *mut c_void) -> i32;
+    pub fn qf_domain_code_params(ctx: *mut qf_ctx, k: *mut i32, slot_bytes: *mut i64) -> i32;
+    pub fn qf_samp_p_packed(ctx: *mut qf_ctx, u: *const i64, tag_idx: *const i32, batch: i64, seed: u64, first_index: u64, k: i32, slot_bytes: i64, out: *mut u8, nbytes: *mut i32) -> i32;
+    pub fn qf_f_a_packed(ctx: *mut qf_ctx, packed: *const u8, tag_idx: *const i32, batch: i64, k: i32, slot_bytes: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
+    pub fn qf_domain_encode_dev(input: *const i32, rows: i64, dim: i64, k: i32, slot_bytes: i64, out: *mut u8, nbytes: *mut i32, cuda_stream: *mut c_void) -> i32;
+    pub fn qf_domain_decode_dev(input: *const u8, rows: i64, dim: i64, k: i32, slot_bytes: i64, out: *mut i32, ok: *mut u8, cuda_stream: *mut c_void) -> i32;
     pub fn qf_randomized_nearest_plane_gadget(ctx: *mut qf_ctx, v: *const i64, batch: i64, seed: u64, first_index: u64, z_out: *mut i32) -> i32;
 
     pub fn qf_compress_u16(input: *const u16, out: *mut u16, count: usize, q: u32, d: u32, device_ptrs: i32, cuda_stream: *mut c_void) -> i32;

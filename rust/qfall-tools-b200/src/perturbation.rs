@@ -3,7 +3,7 @@
 //! Shipped as source (see lib.rs).
 use crate::ffi::*;
 use crate::{column_from_i32, domain_to_i32, f_a_tagged_installed, f_a_tagged_installed_poly, matz_to_words, matzq_to_words,
-            poly_tag_words, range_from_words, Context, FaTags, PSFBatch};
+            f_a_packed_run, poly_tag_words, range_from_words, samp_p_packed_run, Context, FaTags, PSFBatch, PackedDomain};
 use qfall_math::{
     integer::{MatZ, Z},
     integer_mod_q::MatZq,
@@ -328,5 +328,23 @@ impl PSFBatch for PSFPerturbationB200 {
         self.ctx.check(st, "qf_f_a");
         let q = Z::from(&self.inner.gp.q);
         u.chunks(n).map(|row| range_from_words(row, &q)).collect()
+    }
+
+    fn samp_p_batch_packed(&self, a: &MatZq, td: &Self::Trapdoor, us: &[MatZq], seed: u64, first_index: u64) -> PackedDomain {
+        self.install_a(a);
+        self.install_td(td);
+        let n = self.n();
+        let mut uw = Vec::with_capacity(us.len() * n);
+        for u in us {
+            assert!(u.is_column_vector() && u.get_num_rows() as usize == n, "target must be an n x 1 vector");
+            uw.extend(matzq_to_words(u));
+        }
+        samp_p_packed_run(&self.ctx, &uw, us.len(), seed, first_index)
+    }
+
+    fn f_a_batch_packed(&self, a: &MatZq, packed: &PackedDomain) -> Vec<MatZq> {
+        self.install_a(a);
+        let q = Z::from(&self.inner.gp.q);
+        f_a_packed_run(&self.ctx, self.n(), packed).chunks(self.n()).map(|row| range_from_words(row, &q)).collect()
     }
 }

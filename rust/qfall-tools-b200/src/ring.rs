@@ -7,7 +7,7 @@
 //! built once per trapdoor (`qf_ring_gen_short_basis` + `qf_set_trapdoor_gpv` with the GSO computed on the device).
 //! Shipped as source (see lib.rs).
 use crate::ffi::*;
-use crate::{Context, PSFBatch};
+use crate::{f_a_packed_run, samp_p_packed_run, Context, PSFBatch, PackedDomain};
 use qfall_math::{
     integer::{MatPolyOverZ, PolyOverZ, Z},
     integer_mod_q::{MatPolynomialRingZq, PolynomialRingZq},
@@ -248,6 +248,24 @@ impl PSFBatch for PSFGPVRingB200 {
         assert!(st != QF_ERR_NOT_IN_DOMAIN && ok.iter().all(|f| *f == 1), "sigma is not in D_n");
         self.ctx.check(st, "qf_f_a");
         u.chunks(n).map(|row| self.range_from_words(row)).collect()
+    }
+
+    fn samp_p_batch_packed(&self, a: &MatPolynomialRingZq, td: &Self::Trapdoor, us: &[MatPolynomialRingZq], seed: u64,
+                           first_index: u64) -> PackedDomain {
+        self.install_a(a);
+        self.install_td(td);
+        let n = self.n();
+        let mut uw = Vec::with_capacity(us.len() * n);
+        for u in us {
+            assert!(u.get_num_rows() == 1 && u.get_num_columns() == 1, "the syndrome is one ring element");
+            uw.extend(Self::polys_to_words(&u.get_representative_least_nonnegative_residue(), n));
+        }
+        samp_p_packed_run(&self.ctx, &uw, us.len(), seed, first_index)
+    }
+
+    fn f_a_batch_packed(&self, a: &MatPolynomialRingZq, packed: &PackedDomain) -> Vec<MatPolynomialRingZq> {
+        self.install_a(a);
+        f_a_packed_run(&self.ctx, self.n(), packed).chunks(self.n()).map(|row| self.range_from_words(row)).collect()
     }
 }
 

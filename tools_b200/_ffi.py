@@ -76,6 +76,11 @@ SIGNATURES = {
     "qf_samp_p_tagged_dev": (_i32, [_vp, _vp, _vp, _i64, _u64, _u64, _vp]),
     "qf_f_a_i16": (_i32, [_vp, _vp, _i64, _vp, _vp]),
     "qf_narrow_i32_i16_dev": (_i32, [_vp, _vp, _sz, _vp, _vp]),
+    "qf_domain_code_params": (_i32, [_vp, C.POINTER(_i32), C.POINTER(_i64)]),
+    "qf_samp_p_packed": (_i32, [_vp, _vp, _vp, _i64, _u64, _u64, _i32, _i64, _vp, _vp]),
+    "qf_f_a_packed": (_i32, [_vp, _vp, _vp, _i64, _i32, _i64, _vp, _vp]),
+    "qf_domain_encode_dev": (_i32, [_vp, _i64, _i64, _i32, _i64, _vp, _vp, _vp]),
+    "qf_domain_decode_dev": (_i32, [_vp, _i64, _i64, _i32, _i64, _vp, _vp, _vp]),
     "qf_randomized_nearest_plane_gadget": (_i32, [_vp, _vp, _i64, _u64, _u64, _vp]),
     "qf_compress_u16": (_i32, [_vp, _vp, _sz, _u32, _u32, _i32, _vp]),
     "qf_decompress_u16": (_i32, [_vp, _vp, _sz, _u32, _u32, _i32, _vp]),

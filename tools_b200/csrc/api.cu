@@ -134,6 +134,7 @@ struct qf_ctx {
     // workspace
     Dev w[12];  // (w[10]: digit planes of the particular solution)
     Dev dNorm, dFlag, dRetry, io_a, io_b, io_b2, io_c, io_a2, io_h[2];
+    Dev io_p[2], io_n[2];  // packed Domain rows and their lengths (qf_samp_p_packed, qf_f_a_packed)
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t ev_done[2] = {nullptr, nullptr}, ev_copied[2] = {nullptr, nullptr};
     cudaEvent_t ev_u_in[2] = {nullptr, nullptr}, ev_u_used[2] = {nullptr, nullptr};
@@ -3276,6 +3277,17 @@ qf_status qf_check_domain(qf_ctx* ctx, const int32_t* sigma, int64_t batch, uint
 }
 
 // ---- f_a with a tag per target (installed f_a tag table) ------------------------------------------------------------
+// host tag indices of a batch against a table of ntags tags, checked before any launch
+static qf_status check_tag_idx(qf_ctx* ctx, const int32_t* tag_idx, int64_t batch, int64_t ntags, const char* table) {
+    for (int64_t b = 0; b < batch; ++b)
+        if (tag_idx[b] < 0 || tag_idx[b] >= ntags) {
+            char buf[128];
+            snprintf(buf, sizeof buf, "tag index outside the installed %s (target %lld: %d)", table, (long long)b, (int)tag_idx[b]);
+            return ctx->fail(QF_ERR_INVALID, buf);
+        }
+    return QF_OK;
+}
+
 static qf_status f_a_tagged_ready(qf_ctx* ctx) {
     if (ctx->prm.kind == QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "f_a tag table: not a classical context");
     if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "no key installed");
@@ -3289,12 +3301,7 @@ qf_status qf_f_a_tagged(qf_ctx* ctx, const int32_t* sigma, const int32_t* tag_id
     if (batch == 0) return QF_OK;
     CK(cudaSetDevice(ctx->device));
     QF_TRY(f_a_tagged_ready(ctx));
-    for (int64_t b = 0; b < batch; ++b)
-        if (tag_idx[b] < 0 || tag_idx[b] >= ctx->fa_tag_count) {
-            char buf[128];
-            snprintf(buf, sizeof buf, "tag index outside the installed f_a tag table (target %lld: %d)", (long long)b, (int)tag_idx[b]);
-            return ctx->fail(QF_ERR_INVALID, buf);
-        }
+    QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->fa_tag_count, "f_a tag table"));
     const long C = ctx->chunk;
     CK(ctx->io_a.ensure((size_t)C * ctx->dim * 4));
     CK(ctx->io_b.ensure((size_t)C * ctx->n * 8));
@@ -3379,27 +3386,44 @@ qf_status qf_samp_p_dev(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t s
     });
 }
 
-// host-buffer samp_p; i16: results leave as int16 (half the device->host bytes)
+// Output form of the host-buffer samp_p: int32, int16 (half the device->host bytes) or the packed code of DESIGN 4.11
+struct SampOut {
+    enum Kind { I32, I16, PACKED } kind = I32;
+    int k = 0;              // PACKED: code parameter and slot size; nbytes: host, batch lengths
+    int64_t slot_bytes = 0;
+    int32_t* nbytes = nullptr;
+    size_t row_bytes(long dim) const { return kind == I32 ? (size_t)dim * 4 : kind == I16 ? (size_t)dim * 2 : (size_t)slot_bytes; }
+};
+
+// host-buffer samp_p in one of the SampOut forms
 // tidx (optional, host): tag index of every target in the installed tag table (qf_samp_p_tagged), copied with the targets
-static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed, uint64_t first, void* e_out, bool i16,
-                             const int32_t* tidx = nullptr) {
+static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed, uint64_t first, void* e_out,
+                             const SampOut& fmt, const int32_t* tidx = nullptr) {
     if (!ctx || batch < 0 || (batch > 0 && (!u || !e_out))) return QF_ERR_INVALID;
     if (batch == 0) return QF_OK;
     CK(cudaSetDevice(ctx->device));
     QF_TRY(samp_p_ready(ctx));
     const long C = ctx->chunk;
-    const size_t esz = i16 ? 2 : 4;
+    const bool i16 = fmt.kind == SampOut::I16, packed = fmt.kind == SampOut::PACKED;
+    const size_t esz = fmt.row_bytes(ctx->dim);  // bytes per result row on the host
     CK(ctx->io_b.ensure((size_t)C * ctx->n * 8));
     CK(ctx->io_a.ensure((size_t)C * ctx->dim * 4));
     if (tidx) CK(ctx->io_t[0].ensure((size_t)C * 4));
     if (i16) CK(ctx->io_h[0].ensure((size_t)C * ctx->dim * 2));
+    if (packed) {
+        CK(ctx->io_p[0].ensure((size_t)C * esz));
+        CK(ctx->io_n[0].ensure((size_t)C * 4));
+    }
     // Both directions of the host traffic run on a second stream: the device->host copy of chunk i and the host->device
     // copy of the targets of chunk i+1 overlap the computation (two result buffers, two target buffers, events in both
     // directions); only the first chunk's targets and the last chunk's results are exposed.
     const bool overlap = batch > C;
     if (overlap) {
         if (i16) CK(ctx->io_h[1].ensure((size_t)C * ctx->dim * 2));
-        else CK(ctx->io_a2.ensure((size_t)C * ctx->dim * 4));
+        else if (packed) {
+            CK(ctx->io_p[1].ensure((size_t)C * esz));
+            CK(ctx->io_n[1].ensure((size_t)C * 4));
+        } else CK(ctx->io_a2.ensure((size_t)C * ctx->dim * 4));
         CK(ctx->io_b2.ensure((size_t)C * ctx->n * 8));
         if (tidx) CK(ctx->io_t[1].ensure((size_t)C * 4));
         if (!ctx->copy_stream) {
@@ -3430,9 +3454,9 @@ static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint6
     int64_t idx = 0;
     QF_TRY(for_chunks(ctx, batch, [&](int64_t b0, int Bc) -> qf_status {
         const int slot = (int)(idx & 1);
-        // int32 results of the chunk: with int16 output they are narrowed into the slot's int16 buffer, so one int32
-        // buffer serves both slots
-        int32_t* dres = (!i16 && overlap && slot) ? ctx->io_a2.as<int32_t>() : ctx->io_a.as<int32_t>();
+        // int32 results of the chunk: with int16 or packed output they are converted into the slot's own buffer, so one
+        // int32 buffer serves both slots
+        int32_t* dres = (fmt.kind == SampOut::I32 && overlap && slot) ? ctx->io_a2.as<int32_t>() : ctx->io_a.as<int32_t>();
         if (overlap && idx >= 2) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_copied[slot], 0));  // buffer free again?
         if (overlap) {
             CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_u_in[slot], 0));  // this chunk's targets have arrived
@@ -3452,34 +3476,52 @@ static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint6
         QF_TRY(ctx->prm.kind == QF_PSF_PERTURBATION ? samp_p_pert_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres, dt)
                                                     : samp_p_np_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres, dt));
         if (overlap) CK(cudaEventRecord(ctx->ev_u_used[slot], ctx->stream));
+        const int bs = overlap ? slot : 0;
         const void* src = dres;
         if (i16) {
-            int16_t* d16 = ctx->io_h[overlap ? slot : 0].as<int16_t>();
+            int16_t* d16 = ctx->io_h[bs].as<int16_t>();
             LAUNCH(qf_launch_narrow_i32_i16(dres, d16, (size_t)Bc * ctx->dim, ctx->dFlag.as<int>(), ctx->stream));
             src = d16;
+        } else if (packed) {
+            LAUNCH(qf_launch_domain_encode(dres, Bc, (int)ctx->dim, fmt.k, fmt.slot_bytes, ctx->io_p[bs].as<uint8_t>(),
+                                           ctx->io_n[bs].as<int32_t>(), ctx->stream));
+            src = ctx->io_p[bs].p;
         }
-        char* dst = (char*)e_out + (size_t)b0 * ctx->dim * esz;
+        char* dst = (char*)e_out + (size_t)b0 * esz;
+        cudaStream_t cs = overlap ? ctx->copy_stream : ctx->stream;
         if (overlap) {
             CK(cudaEventRecord(ctx->ev_done[slot], ctx->stream));
             CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_done[slot], 0));
-            CK(cudaMemcpyAsync(dst, src, (size_t)Bc * ctx->dim * esz, cudaMemcpyDeviceToHost, ctx->copy_stream));
-            CK(cudaEventRecord(ctx->ev_copied[slot], ctx->copy_stream));
-        } else {
-            CK(cudaMemcpyAsync(dst, src, (size_t)Bc * ctx->dim * esz, cudaMemcpyDeviceToHost, ctx->stream));
-            CK(cudaStreamSynchronize(ctx->stream));
         }
+        CK(cudaMemcpyAsync(dst, src, (size_t)Bc * esz, cudaMemcpyDeviceToHost, cs));
+        if (packed) CK(cudaMemcpyAsync(fmt.nbytes + b0, ctx->io_n[bs].p, (size_t)Bc * 4, cudaMemcpyDeviceToHost, cs));
+        if (overlap) CK(cudaEventRecord(ctx->ev_copied[slot], ctx->copy_stream));
+        else CK(cudaStreamSynchronize(ctx->stream));
         ++idx;
         return QF_OK;
     }));
     if (overlap) CK(cudaStreamSynchronize(ctx->copy_stream));
-    return check_flag(ctx);
+    QF_TRY(check_flag(ctx));
+    if (packed) {
+        for (int64_t b = 0; b < batch; ++b)
+            if (fmt.nbytes[b] < 0) {
+                char buf[192];
+                snprintf(buf, sizeof buf, "packed samp_p: the code of target %lld does not fit its slot of %lld bytes (its row is "
+                         "zero, nbytes -1; qf_samp_p at first_index + %lld gives its preimage)", (long long)b,
+                         (long long)fmt.slot_bytes, (long long)b);
+                return ctx->fail(QF_ERR_NUMERIC, buf);
+            }
+    }
+    return QF_OK;
 }
 
 qf_status qf_samp_p(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed, uint64_t first, int32_t* e_out) {
-    return samp_p_host(ctx, u, batch, seed, first, e_out, false);
+    return samp_p_host(ctx, u, batch, seed, first, e_out, SampOut{});
 }
 qf_status qf_samp_p_i16(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed, uint64_t first, int16_t* e_out) {
-    return samp_p_host(ctx, u, batch, seed, first, e_out, true);
+    SampOut f;
+    f.kind = SampOut::I16;
+    return samp_p_host(ctx, u, batch, seed, first, e_out, f);
 }
 
 // ---- samp_p with a tag per target (PSFPerturbation, PSFGPV on the two-phase recursion; installed tag table) -----------
@@ -3496,13 +3538,8 @@ qf_status qf_samp_p_tagged(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx
     if (!ctx || batch < 0 || (batch > 0 && (!u || !tag_idx || !e_out))) return QF_ERR_INVALID;
     if (batch == 0) return QF_OK;
     QF_TRY(samp_p_tagged_ready(ctx));
-    for (int64_t b = 0; b < batch; ++b)
-        if (tag_idx[b] < 0 || tag_idx[b] >= ctx->tag_count) {
-            char buf[128];
-            snprintf(buf, sizeof buf, "tag index outside the installed tag table (target %lld: %d)", (long long)b, (int)tag_idx[b]);
-            return ctx->fail(QF_ERR_INVALID, buf);
-        }
-    return samp_p_host(ctx, u, batch, seed, first, e_out, false, tag_idx);
+    QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->tag_count, "tag table"));
+    return samp_p_host(ctx, u, batch, seed, first, e_out, SampOut{}, tag_idx);
 }
 
 qf_status qf_samp_p_tagged_dev(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, uint64_t seed,
@@ -3553,6 +3590,105 @@ qf_status qf_f_a_i16(qf_ctx* ctx, const int16_t* sigma, int64_t batch, int64_t* 
 qf_status qf_narrow_i32_i16_dev(const int32_t* in, int16_t* out, size_t count, int* overflow, void* cuda_stream) {
     if ((!in || !out) && count) return QF_ERR_INVALID;
     cudaError_t e = qf_launch_narrow_i32_i16(in, out, count, overflow, (cudaStream_t)cuda_stream);
+    return e == cudaSuccess ? QF_OK : (e == cudaErrorMisalignedAddress ? QF_ERR_INVALID : QF_ERR_CUDA);
+}
+
+// ---- packed Domain values (DESIGN 4.11) ---------------------------------------------------------------------------
+static bool packed_args_ok(int64_t dim, int k, int64_t slot_bytes) {
+    return dim > 0 && dim <= INT32_MAX && k >= 0 && k <= 30 && slot_bytes % 16 == 0 &&
+           slot_bytes >= qf_domain_h0(dim, k) + (dim + 7) / 8;
+}
+
+qf_status qf_domain_code_params(qf_ctx* ctx, int* k, int64_t* slot_bytes) {
+    if (!ctx || !k || !slot_bytes) return QF_ERR_INVALID;
+    long long sb = 0;
+    qf_domain_code_recommend(ctx->s_samp_d, ctx->dim, k, &sb);
+    *slot_bytes = sb;
+    return QF_OK;
+}
+
+qf_status qf_samp_p_packed(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, uint64_t seed, uint64_t first,
+                           int k, int64_t slot_bytes, uint8_t* out, int32_t* nbytes) {
+    if (!ctx || batch < 0 || (batch > 0 && (!u || !out || !nbytes))) return QF_ERR_INVALID;
+    if (!packed_args_ok(ctx->dim, k, slot_bytes))
+        return ctx->fail(QF_ERR_INVALID, "packed Domain code: k outside [0, 30] or slot_bytes not a multiple of 16 of at least "
+                                         "H0 + ceil(dim / 8)");
+    if (batch == 0) return QF_OK;
+    if (tag_idx) {
+        QF_TRY(samp_p_tagged_ready(ctx));
+        QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->tag_count, "tag table"));
+    }
+    SampOut f;
+    f.kind = SampOut::PACKED;
+    f.k = k;
+    f.slot_bytes = slot_bytes;
+    f.nbytes = nbytes;
+    return samp_p_host(ctx, u, batch, seed, first, out, f, tag_idx);
+}
+
+qf_status qf_f_a_packed(qf_ctx* ctx, const uint8_t* packed, const int32_t* tag_idx, int64_t batch, int k, int64_t slot_bytes,
+                        int64_t* u_out, uint8_t* in_domain) {
+    if (!ctx || batch < 0 || (batch > 0 && !packed)) return QF_ERR_INVALID;
+    if (!packed_args_ok(ctx->dim, k, slot_bytes))
+        return ctx->fail(QF_ERR_INVALID, "packed Domain code: k outside [0, 30] or slot_bytes not a multiple of 16 of at least "
+                                         "H0 + ceil(dim / 8)");
+    if (batch == 0) return QF_OK;
+    CK(cudaSetDevice(ctx->device));
+    const bool ring = ctx->prm.kind == QF_PSF_GPV_RING;
+    if (tag_idx) {
+        QF_TRY(f_a_tagged_ready(ctx));
+        QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->fa_tag_count, "f_a tag table"));
+    } else if (ring ? !ctx->has_ring : !ctx->has_a) {
+        return ctx->fail(QF_ERR_NO_KEY, "no key installed");
+    }
+    const long C = ctx->chunk;
+    CK(ctx->io_p[0].ensure((size_t)C * slot_bytes));
+    CK(ctx->io_n[0].ensure((size_t)C));
+    CK(ctx->io_a.ensure((size_t)C * ctx->dim * 4));
+    CK(ctx->io_c.ensure((size_t)C));
+    if (u_out) CK(ctx->io_b.ensure((size_t)C * ctx->n * 8));
+    if (tag_idx) CK(ctx->io_t[0].ensure((size_t)C * 4));
+    std::vector<uint8_t> flags((size_t)batch), canon((size_t)batch);
+    QF_TRY(for_chunks(ctx, batch, [&](int64_t b0, int Bc) -> qf_status {
+        CK(cudaMemcpyAsync(ctx->io_p[0].p, packed + b0 * slot_bytes, (size_t)Bc * slot_bytes, cudaMemcpyHostToDevice, ctx->stream));
+        LAUNCH(qf_launch_domain_decode(ctx->io_p[0].as<uint8_t>(), Bc, (int)ctx->dim, k, slot_bytes, ctx->io_a.as<int32_t>(),
+                                       ctx->io_n[0].as<uint8_t>(), ctx->stream));
+        int64_t* du = u_out ? ctx->io_b.as<int64_t>() : nullptr;
+        if (tag_idx && u_out) {  // the tag changes u only: flags alone come from the untagged f_a
+            CK(cudaMemcpyAsync(ctx->io_t[0].p, tag_idx + b0, (size_t)Bc * 4, cudaMemcpyHostToDevice, ctx->stream));
+            QF_TRY(f_a_tagged_chunk(ctx, ctx->io_a.as<int32_t>(), ctx->io_t[0].as<int32_t>(), Bc, du, ctx->io_c.as<uint8_t>()));
+        } else {
+            QF_TRY(ring ? ring_f_a_chunk(ctx, ctx->io_a.as<int32_t>(), Bc, du, ctx->io_c.as<uint8_t>())
+                        : f_a_chunk(ctx, ctx->io_a.as<int32_t>(), Bc, du, ctx->io_c.as<uint8_t>()));
+        }
+        if (u_out) CK(cudaMemcpyAsync(u_out + b0 * ctx->n, du, (size_t)Bc * ctx->n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(flags.data() + b0, ctx->io_c.p, (size_t)Bc, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(canon.data() + b0, ctx->io_n[0].p, (size_t)Bc, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        return QF_OK;
+    }));
+    QF_TRY(check_flag(ctx));
+    bool all = true;
+    for (int64_t b = 0; b < batch; ++b) {
+        flags[b] = flags[b] && canon[b];
+        all = all && flags[b];
+    }
+    if (in_domain) memcpy(in_domain, flags.data(), (size_t)batch);
+    if (!all) return ctx->fail(QF_ERR_NOT_IN_DOMAIN, "f_a: a packed sigma is not canonical or not in the domain D_n");
+    return QF_OK;
+}
+
+qf_status qf_domain_encode_dev(const int32_t* in, int64_t rows, int64_t dim, int k, int64_t slot_bytes, uint8_t* out,
+                               int32_t* nbytes, void* cuda_stream) {
+    if (rows < 0 || !packed_args_ok(dim, k, slot_bytes) || (rows > 0 && (!in || !out || !nbytes))) return QF_ERR_INVALID;
+    cudaError_t e = qf_launch_domain_encode(in, rows, (int)dim, k, slot_bytes, out, nbytes, (cudaStream_t)cuda_stream);
+    return e == cudaSuccess ? QF_OK : (e == cudaErrorMisalignedAddress ? QF_ERR_INVALID : QF_ERR_CUDA);
+}
+
+qf_status qf_domain_decode_dev(const uint8_t* in, int64_t rows, int64_t dim, int k, int64_t slot_bytes, int32_t* out, uint8_t* ok,
+                               void* cuda_stream) {
+    if (rows < 0 || !packed_args_ok(dim, k, slot_bytes) || (rows > 0 && (!in || !out || !ok))) return QF_ERR_INVALID;
+    cudaError_t e = qf_launch_domain_decode(in, rows, (int)dim, k, slot_bytes, out, ok, (cudaStream_t)cuda_stream);
     return e == cudaSuccess ? QF_OK : (e == cudaErrorMisalignedAddress ? QF_ERR_INVALID : QF_ERR_CUDA);
 }
 

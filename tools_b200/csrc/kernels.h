@@ -261,6 +261,18 @@ cudaError_t qf_launch_ozaki_prepare(const double* U, long ld, int D, int blk, in
 cudaError_t qf_launch_narrow_i32_i16(const int32_t* in, int16_t* out, size_t count, int* flag, cudaStream_t stream);
 cudaError_t qf_launch_widen_i16_i32(const int16_t* in, int32_t* out, size_t count, cudaStream_t stream);
 cudaError_t qf_launch_range_check_i64(const int64_t* v, size_t count, unsigned long long q, int* flag, cudaStream_t stream);
+
+// packed Domain values (domain_code.cu, DESIGN 4.11): rows x dim int32 <-> rows slots of slot_bytes bytes (k in [0, 30],
+// slot_bytes a multiple of 16 and at least H0 + ceil(dim / 8); checked by the callers).  Encode: nbytes[row], -1 and a zero
+// slot when the code does not fit or the row holds INT32_MIN.  Decode: ok[row] = 1 iff the slot is canonical.
+// out (encode) / in (decode) 16-byte aligned, else cudaErrorMisalignedAddress.
+long long qf_domain_h0(long long dim, int k);
+cudaError_t qf_launch_domain_encode(const int32_t* in, long long rows, int dim, int k, long long slot_bytes, uint8_t* out,
+                                    int32_t* nbytes, cudaStream_t stream);
+cudaError_t qf_launch_domain_decode(const uint8_t* in, long long rows, int dim, int k, long long slot_bytes, int32_t* out,
+                                    uint8_t* ok, cudaStream_t stream);
+// recommended (k, slot_bytes) for entries ~ D_{Z,w} (qf_domain_code_params)
+void qf_domain_code_recommend(double w, long long dim, int* k, long long* slot_bytes);
 // balanced s8 digit planes of int64 values (B x M, row stride ldin) into L planes of B x ldk bytes, columns [M, ldk) zeroed;
 // *flag |= 8 when a value does not fit L digits (the x operand of a contraction whose "targets" are residues, e.g. u' = H^-1 u)
 cudaError_t qf_launch_split_i64_limbs(const int64_t* in, long ldin, int8_t* planes, long plane_stride, long ldk, int B, int M,

@@ -10,6 +10,7 @@ Values cross the boundary as numpy arrays:
 """
 from __future__ import annotations
 
+import ctypes
 import math
 import os
 from fractions import Fraction
@@ -122,6 +123,23 @@ class _PSFBase:
         here that installs or rewrites A resets _fa_tags_id.  tag_idx: B indices in [0, T).  Returns (u, in_domain) as
         f_a_batch does."""
         self._install_a(a)
+        self._install_fa_tags(tags, h0)
+        s, oob = _domain_i32(sigmas, self._domain_shape)
+        ti = np.ascontiguousarray(tag_idx, dtype=np.int32)
+        b = s.shape[0]
+        assert ti.shape == (b,)
+        u = np.empty((b, self.n), dtype=np.int64)
+        flags = np.empty(b, dtype=np.uint8)
+        st = self.ctx.status("qf_f_a_tagged", _ffi.ptr(s), _ffi.ptr(ti), b, _ffi.ptr(u), _ffi.ptr(flags))
+        if st not in (_ffi.QF_OK, _ffi.QF_ERR_NOT_IN_DOMAIN):
+            raise QfError(st, self.ctx._lib.qf_last_error(self.ctx._h).decode())
+        ok = flags.astype(bool) & ~oob
+        if strict and not ok.all():
+            raise NotInDomain(_ffi.QF_ERR_NOT_IN_DOMAIN, "sigma is not in the domain D_n")
+        return u, ok
+
+    def _install_fa_tags(self, tags, h0):
+        """The f_a tag table of f_a_tagged_batch (qf_set_f_a_tags[_poly]), unless it is on the device already."""
         key = self._fa_tags_id
         if key is None or key[0] is not tags or key[1] is not h0:
             hg = None
@@ -139,19 +157,6 @@ class _PSFBase:
                 assert tg.ndim == 3 and tg.shape[1:] == (self.n, self.n) and tg.shape[0] >= 1
                 self.ctx.call("qf_set_f_a_tags", _ffi.ptr(tg), tg.shape[0], _ffi.ptr(hg))
             self._fa_tags_id = (tags, h0)
-        s, oob = _domain_i32(sigmas, self._domain_shape)
-        ti = np.ascontiguousarray(tag_idx, dtype=np.int32)
-        b = s.shape[0]
-        assert ti.shape == (b,)
-        u = np.empty((b, self.n), dtype=np.int64)
-        flags = np.empty(b, dtype=np.uint8)
-        st = self.ctx.status("qf_f_a_tagged", _ffi.ptr(s), _ffi.ptr(ti), b, _ffi.ptr(u), _ffi.ptr(flags))
-        if st not in (_ffi.QF_OK, _ffi.QF_ERR_NOT_IN_DOMAIN):
-            raise QfError(st, self.ctx._lib.qf_last_error(self.ctx._h).decode())
-        ok = flags.astype(bool) & ~oob
-        if strict and not ok.all():
-            raise NotInDomain(_ffi.QF_ERR_NOT_IN_DOMAIN, "sigma is not in the domain D_n")
-        return u, ok
 
     def f_a(self, a, sigma) -> np.ndarray:
         sigma = np.asarray(sigma)
@@ -177,6 +182,73 @@ class _PSFBase:
 
     def samp_p(self, a, td, u, seed=None) -> np.ndarray:
         return self.samp_p_batch(a, td, np.asarray(u, dtype=np.int64).reshape(1, self.n), seed)[0]
+
+    # -- packed Domain values (DESIGN 4.11) -----------------------------------------------------------------------------
+    def domain_code_params(self):
+        """(k, slot_bytes) recommended for this context's Gaussian width and dim (qf_domain_code_params)."""
+        k, sb = ctypes.c_int(), ctypes.c_int64()
+        self.ctx.call("qf_domain_code_params", ctypes.byref(k), ctypes.byref(sb))
+        return k.value, sb.value
+
+    def _code_params(self, k, slot_bytes):
+        if k is None or slot_bytes is None:
+            k0, s0 = self.domain_code_params()
+            k, slot_bytes = (k0 if k is None else k), (s0 if slot_bytes is None else slot_bytes)
+        return int(k), int(slot_bytes)
+
+    def samp_p_packed_batch(self, a, td, us: np.ndarray, seed=None, first_index: int = 0, tags=None, tag_idx=None, k=None,
+                            slot_bytes=None):
+        """samp_p with packed output (qf_samp_p_packed): returns (packed uint8 B x slot_bytes, nbytes int32 B).  Row b is the
+        code of row b of samp_p_batch (tags: samp_p_tagged_batch, same tags and tag_idx) for the same seed and first_index.
+        k / slot_bytes default to domain_code_params().  A row whose code does not fit its slot has nbytes -1 and a zero
+        slot; samp_p_batch(a, td, us[b:b+1], seed, first_index + b) gives its preimage."""
+        self._install_a(a)
+        self._install_td(a, td)
+        k, slot_bytes = self._code_params(k, slot_bytes)
+        u = np.ascontiguousarray(us, dtype=np.int64)
+        assert u.ndim == 2 and u.shape[1] == self.n
+        b = u.shape[0]
+        ti = None
+        if tags is not None:
+            if not isinstance(self, _TagTable):
+                raise QfError(_ffi.QF_ERR_INVALID, "tags need a classical context")
+            if self._tags_id is not tags:
+                self.set_tag_table(a, td, tags)
+            ti = np.ascontiguousarray(tag_idx, dtype=np.int32)
+            assert ti.shape == (b,)
+        out = np.empty((b, slot_bytes), dtype=np.uint8)
+        nbytes = np.empty(b, dtype=np.int32)
+        st = self.ctx.status("qf_samp_p_packed", _ffi.ptr(u), _ffi.ptr(ti), b, _seed(seed), first_index, k, slot_bytes,
+                             _ffi.ptr(out), _ffi.ptr(nbytes))
+        if st != _ffi.QF_OK and not (st == _ffi.QF_ERR_NUMERIC and (nbytes < 0).any()):
+            raise QfError(st, self.ctx._lib.qf_last_error(self.ctx._h).decode())
+        return out, nbytes
+
+    def f_a_packed_batch(self, a, packed: np.ndarray, k=None, tags=None, tag_idx=None, h0=None, strict: bool = True):
+        """f_a on packed Domain values (qf_f_a_packed): packed is B x slot_bytes; returns (u, in_domain) as f_a_batch, with
+        in_domain[b] False also when slot b is not a canonical code.  tags / tag_idx / h0 as in f_a_tagged_batch
+        (classical contexts).  k defaults to domain_code_params()."""
+        self._install_a(a)
+        p = np.ascontiguousarray(packed, dtype=np.uint8)
+        assert p.ndim == 2
+        b, slot_bytes = p.shape
+        k, _ = self._code_params(k, slot_bytes)
+        ti = None
+        if tags is not None:
+            if not isinstance(self, _TagTable):
+                raise QfError(_ffi.QF_ERR_INVALID, "tags need a classical context")
+            self._install_fa_tags(tags, h0)
+            ti = np.ascontiguousarray(tag_idx, dtype=np.int32)
+            assert ti.shape == (b,)
+        u = np.empty((b, self.n), dtype=np.int64)
+        flags = np.empty(b, dtype=np.uint8)
+        st = self.ctx.status("qf_f_a_packed", _ffi.ptr(p), _ffi.ptr(ti), b, k, slot_bytes, _ffi.ptr(u), _ffi.ptr(flags))
+        if st not in (_ffi.QF_OK, _ffi.QF_ERR_NOT_IN_DOMAIN):
+            raise QfError(st, self.ctx._lib.qf_last_error(self.ctx._h).decode())
+        ok = flags.astype(bool)
+        if strict and not ok.all():
+            raise NotInDomain(_ffi.QF_ERR_NOT_IN_DOMAIN, "sigma is not canonical or not in the domain D_n")
+        return u, ok
 
 
 class PolyTags:
