@@ -252,6 +252,40 @@ qf_status qf_samp_p_tagged(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx
                            uint64_t first_index, int32_t* e_out);
 qf_status qf_samp_p_tagged_dev(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, uint64_t seed,
                                uint64_t first_index, int32_t* e_out);
+/* ---- offline / online samp_p (DESIGN 4.12): PSFPerturbation, and PSFGPV on the two-phase recursion -------------------
+ * Most of samp_p does not read the target: the perturbation p and A p (PSFPerturbation), phase 1 of the recursion and the
+ * products of its z2 (PSFGPV).  qf_samp_p_offline computes that half ahead of time into a device pool of the context; the
+ * online calls then do only the target-dependent half.  Row b of an online call that consumed the pool entry of sampler
+ * index j is bit-identical to row 0 of qf_samp_p(ctx, u_b, 1, seed, j, ...) (with tag_idx: of qf_samp_p_tagged), for any
+ * split into fill calls, online calls and chunks.
+ * Caller's responsibility: every entry is served at most once, but refilling an index range already used under the same
+ * seed serves the same perturbations / phase-1 draws again -- exactly as calling qf_samp_p twice with one (seed, index).
+ * Two preimages that share such a draw leak information about the trapdoor through their difference.
+ * Lifetime: one pool per context.  It is dropped by every call that changes A or the trapdoor (qf_set_a, qf_trap_gen,
+ * qf_trap_gen_from, qf_set_trapdoor_perturbation, qf_set_trapdoor_gpv, qf_set_tag, qf_gpv_set_tag) and kept by the tag
+ * table installs of either form (samp_p and f_a).
+ * Device memory per entry: PSFPerturbation 4 m + 8 n bytes (p as int32, A p mod q); PSFGPV 4 m_bar + 8 n + 8 n k bytes
+ * (z2 as int32, A_bar z2 mod q, the centre product Mt_1 z2 in fp64). */
+/* Fill the pool with the target-independent half of samp_p for the sampler indices first_index .. first_index + count - 1
+ * under `seed`; replaces any previous pool (also when the fill fails: there is then no pool).  Synchronous.
+ * QF_ERR_UNSUPPORTED on a ring context and on a PSFGPV key that runs the one-pass recursion (its first step, A_P^-1 u,
+ * reads the target); QF_ERR_NO_KEY without key or trapdoor; QF_ERR_INVALID for count < 0; QF_ERR_CUDA when the pool does
+ * not fit in device memory (nothing is launched). */
+qf_status qf_samp_p_offline(qf_ctx* ctx, int64_t count, uint64_t seed, uint64_t first_index);
+/* Entries not yet consumed, and the sampler index the next online call starts at (0 and 0 without a pool).  Either
+ * pointer may be NULL. */
+qf_status qf_samp_p_pool_info(const qf_ctx* ctx, int64_t* remaining, uint64_t* next_index);
+/* Consume the next `batch` entries of the pool, in index order, for the targets u (batch x n).  tag_idx == NULL: as
+ * qf_samp_p; otherwise as qf_samp_p_tagged (same readiness checks and tag-index checks).  first_index_out (may be NULL)
+ * receives the sampler index of row 0.  QF_ERR_NO_KEY without a pool; QF_ERR_INVALID when batch exceeds the remaining
+ * entries, before any launch and with nothing consumed.  batch == 0 is valid.  Once the checks pass the entries are
+ * consumed, even if the call fails later.  qf_samp_p_online takes host pointers and range-checks the targets as qf_samp_p;
+ * qf_samp_p_online_dev takes device pointers and is asynchronous like the other _dev forms (its entries are consumed at
+ * enqueue). */
+qf_status qf_samp_p_online(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, int32_t* e_out,
+                           uint64_t* first_index_out);
+qf_status qf_samp_p_online_dev(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, int32_t* e_out,
+                               uint64_t* first_index_out);
 /* Narrow Domain form: the same preimages as int16 -- |e_i| <= 6 s r is far below 2^15 for the parameter sets of the
  * reference (C2: 6 s = 8568; C3: 3135), so the device->host copy, which bounds the host-buffer path, is halved.  An entry
  * that does not fit is reported as QF_ERR_NUMERIC (then use qf_samp_p).  Targets outside [0,q) are detected on the device

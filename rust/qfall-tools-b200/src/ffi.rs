@@ -77,6 +77,10 @@ extern "C" {
 
     pub fn qf_samp_p_tagged(ctx: *mut qf_ctx, u: *const i64, tag_idx: *const i32, batch: i64, seed: u64, first_index: u64, e_out: *mut i32) -> i32;
     pub fn qf_samp_p_tagged_dev(ctx: *mut qf_ctx, u: *const i64, tag_idx: *const i32, batch: i64, seed: u64, first_index: u64, e_out: *mut i32) -> i32;
+    pub fn qf_samp_p_offline(ctx: *mut qf_ctx, count: i64, seed: u64, first_index: u64) -> i32;
+    pub fn qf_samp_p_pool_info(ctx: *const qf_ctx, remaining: *mut i64, next_index: *mut u64) -> i32;
+    pub fn qf_samp_p_online(ctx: *mut qf_ctx, u: *const i64, tag_idx: *const i32, batch: i64, e_out: *mut i32, first_index_out: *mut u64) -> i32;
+    pub fn qf_samp_p_online_dev(ctx: *mut qf_ctx, u: *const i64, tag_idx: *const i32, batch: i64, e_out: *mut i32, first_index_out: *mut u64) -> i32;
     pub fn qf_samp_p_i16(ctx: *mut qf_ctx, u: *const i64, batch: i64, seed: u64, first_index: u64, e_out: *mut i16) -> i32;
     pub fn qf_f_a_i16(ctx: *mut qf_ctx, sigma: *const i16, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
     pub fn qf_narrow_i32_i16_dev(input: *const i32, out: *mut i16, count: usize, overflow: *mut i32, cuda_stream: *mut c_void) -> i32;

@@ -154,6 +154,24 @@ pub struct PackedDomain {
 }
 
 /// qf_samp_p_packed for the targets `uw` (batch x n words) with the key and trapdoor installed in `ctx`.
+/// Online half of samp_p from the context's pool (qf_samp_p_online, DESIGN 4.12): `batch` rows of `m` entries and the
+/// sampler index of row 0.  `tag_idx`: one index per target into the installed tag table (qf_samp_p_tagged).
+pub(crate) fn samp_p_online_run(ctx: &Context, uw: &[i64], tag_idx: Option<&[i32]>, batch: usize, m: usize) -> (Vec<i32>, u64) {
+    let mut e = vec![0i32; batch * m];
+    let mut first = 0u64;
+    let ti = tag_idx.map(|t| t.as_ptr()).unwrap_or(std::ptr::null());
+    let st = unsafe { qf_samp_p_online(ctx.raw, uw.as_ptr(), ti, batch as i64, e.as_mut_ptr(), &mut first) };
+    ctx.check(st, "qf_samp_p_online");
+    (e, first)
+}
+
+/// Remaining entries of the context's pool and the sampler index of the next one (qf_samp_p_pool_info).
+pub fn samp_p_pool_info(ctx: &Context) -> (i64, u64) {
+    let (mut rem, mut next) = (0i64, 0u64);
+    ctx.check(unsafe { qf_samp_p_pool_info(ctx.raw, &mut rem, &mut next) }, "qf_samp_p_pool_info");
+    (rem, next)
+}
+
 pub(crate) fn samp_p_packed_run(ctx: &Context, uw: &[i64], batch: usize, seed: u64, first_index: u64) -> PackedDomain {
     let (mut k, mut slot) = (0i32, 0i64);
     ctx.check(unsafe { qf_domain_code_params(ctx.raw, &mut k, &mut slot) }, "qf_domain_code_params");
@@ -339,6 +357,36 @@ impl PSFGPVB200 {
         self.ctx.check(st, "qf_samp_p_tagged");
         e.chunks(m).map(column_from_i32).collect()
     }
+
+    /// Fills the pool with the target-independent half of samp_p (phase 1 of the two-phase recursion and the products of its
+    /// z2) for the sampler indices `first_index .. first_index + count` under `seed` (qf_samp_p_offline).  A new key,
+    /// trapdoor or key tag drops the pool; tag tables keep it.  Never refill an index range already served under the same
+    /// seed: two preimages sharing a draw leak trapdoor information.  Panics on a one-pass key (QF_ERR_UNSUPPORTED).
+    pub fn samp_p_offline(&self, a: &MatZq, td: &(MatZ, MatQ), count: usize, seed: u64, first_index: u64) {
+        self.install(a, td);
+        self.ctx.check(unsafe { qf_samp_p_offline(self.ctx.raw, count as i64, seed, first_index) }, "qf_samp_p_offline");
+    }
+
+    /// Online half for the next `us.len()` pool entries (qf_samp_p_online): row b equals `samp_p_batch` (with `tag_of`:
+    /// `samp_p_tagged_batch`) at sampler index `first + b` under the pool's seed; returns the rows and `first`.  Panics
+    /// without a pool or when the batch exceeds the remaining entries.
+    pub fn samp_p_online_batch(&self, a: &MatZq, td: &(MatZ, MatQ), us: &[MatZq], tag_of: Option<&[usize]>) -> (Vec<MatZ>, u64) {
+        let (n, m) = (self.n(), self.m());
+        self.install(a, td);
+        let mut uw = Vec::with_capacity(us.len() * n);
+        for u in us {
+            assert!(u.is_column_vector() && u.get_num_rows() as usize == n, "target must be an n x 1 vector");
+            uw.extend(matzq_to_words(u));
+        }
+        let idx: Option<Vec<i32>> = tag_of.map(|t| {
+            assert_eq!(us.len(), t.len(), "one tag index per target");
+            let ntags = (*self.installed_tags.borrow()).expect("no tag table installed for this key and trapdoor (set_tag_table)");
+            t.iter().map(|x| { assert!(*x < ntags, "tag index out of range"); *x as i32 }).collect()
+        });
+        let (e, first) = samp_p_online_run(&self.ctx, &uw, idx.as_deref(), us.len(), m);
+        (e.chunks(m).map(column_from_i32).collect(), first)
+    }
+
     /// `gen_short_basis_for_trapdoor(params, tag, a, r)` (short_basis_classical.rs:54-110) on the device for the key `a`
     /// of this context's parameters: W = digits of -tag^-1 a[:, :m_bar] with tag^-1 and the products computed on the
     /// GPU (qf_gen_short_basis_tagged).  Panics where the reference's `MatZq::inverse(..).unwrap()` does: no unit pivot.

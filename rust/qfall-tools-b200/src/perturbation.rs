@@ -3,7 +3,7 @@
 //! Shipped as source (see lib.rs).
 use crate::ffi::*;
 use crate::{column_from_i32, domain_to_i32, f_a_tagged_installed, f_a_tagged_installed_poly, matz_to_words, matzq_to_words,
-            f_a_packed_run, poly_tag_words, range_from_words, samp_p_packed_run, Context, FaTags, PSFBatch, PackedDomain};
+            f_a_packed_run, poly_tag_words, range_from_words, samp_p_online_run, samp_p_packed_run, Context, FaTags, PSFBatch, PackedDomain};
 use qfall_math::{
     integer::{MatZ, Z},
     integer_mod_q::MatZq,
@@ -201,6 +201,38 @@ impl PSFPerturbationB200 {
         let st = unsafe { qf_samp_p_tagged(self.ctx.raw, uw.as_ptr(), idx.as_ptr(), us.len() as i64, seed, 0, e.as_mut_ptr()) };
         self.ctx.check(st, "qf_samp_p_tagged");
         e.chunks(m).map(column_from_i32).collect()
+    }
+
+    /// Fills the pool with the target-independent half of samp_p (the perturbation p and A p) for the sampler indices
+    /// `first_index .. first_index + count` under `seed` (qf_samp_p_offline).  A new key, trapdoor or key tag drops the
+    /// pool; tag tables keep it.  Never refill an index range already served under the same seed: two preimages sharing a
+    /// perturbation leak trapdoor information.
+    pub fn samp_p_offline(&self, a: &MatZq, td: &(MatZ, MatQ, (MatZ, MatQ)), count: usize, seed: u64, first_index: u64) {
+        self.install_a(a);
+        self.install_td(td);
+        self.ctx.check(unsafe { qf_samp_p_offline(self.ctx.raw, count as i64, seed, first_index) }, "qf_samp_p_offline");
+    }
+
+    /// Online half for the next `us.len()` pool entries (qf_samp_p_online): row b equals `samp_p_batch` (with `tag_of`:
+    /// `samp_p_tagged_batch`) at sampler index `first + b` under the pool's seed; returns the rows and `first`.  Panics
+    /// without a pool or when the batch exceeds the remaining entries.
+    pub fn samp_p_online_batch(&self, a: &MatZq, td: &(MatZ, MatQ, (MatZ, MatQ)), us: &[MatZq], tag_of: Option<&[usize]>)
+                               -> (Vec<MatZ>, u64) {
+        let (n, m) = (self.n(), self.m());
+        self.install_a(a);
+        self.install_td(td);
+        let mut uw = Vec::with_capacity(us.len() * n);
+        for u in us {
+            assert!(u.is_column_vector() && u.get_num_rows() as usize == n, "target must be an n x 1 vector");
+            uw.extend(matzq_to_words(u));
+        }
+        let idx: Option<Vec<i32>> = tag_of.map(|t| {
+            assert_eq!(us.len(), t.len(), "one tag index per target");
+            let ntags = (*self.installed_tags.borrow()).expect("no tag table installed for this key and trapdoor (set_tag_table)");
+            t.iter().map(|x| { assert!(*x < ntags, "tag index out of range"); *x as i32 }).collect()
+        });
+        let (e, first) = samp_p_online_run(&self.ctx, &uw, idx.as_deref(), us.len(), m);
+        (e.chunks(m).map(column_from_i32).collect(), first)
     }
 
     /// f_a with a tag per target: `u[b] = A_t sigmas[b]` with `A_t = a + [0 | (H_t - H_0) G]`, `H_t = tags[tag_of[b]]`, for

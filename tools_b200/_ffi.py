@@ -74,6 +74,10 @@ SIGNATURES = {
     "qf_samp_p_i16": (_i32, [_vp, _vp, _i64, _u64, _u64, _vp]),
     "qf_samp_p_tagged": (_i32, [_vp, _vp, _vp, _i64, _u64, _u64, _vp]),
     "qf_samp_p_tagged_dev": (_i32, [_vp, _vp, _vp, _i64, _u64, _u64, _vp]),
+    "qf_samp_p_offline": (_i32, [_vp, _i64, _u64, _u64]),
+    "qf_samp_p_pool_info": (_i32, [_vp, _vp, _vp]),
+    "qf_samp_p_online": (_i32, [_vp, _vp, _vp, _i64, _vp, _vp]),
+    "qf_samp_p_online_dev": (_i32, [_vp, _vp, _vp, _i64, _vp, _vp]),
     "qf_f_a_i16": (_i32, [_vp, _vp, _i64, _vp, _vp]),
     "qf_narrow_i32_i16_dev": (_i32, [_vp, _vp, _sz, _vp, _vp]),
     "qf_domain_code_params": (_i32, [_vp, C.POINTER(_i32), C.POINTER(_i64)]),

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libqfall_b200.so")
-SOURCES = ["api.cu", "gemm_f64.cu", "elementwise.cu", "lattice.cu", "compress.cu", "ring_ntt.cu", "setup.cu", "gemm_i8.cu", "ring_small.cu", "gemm_i8_fused.cu", "encodings.cu", "domain_code.cu"]
+SOURCES = ["api.cu", "gemm_f64.cu", "elementwise.cu", "lattice.cu", "compress.cu", "ring_ntt.cu", "setup.cu", "gemm_i8.cu", "ring_small.cu", "gemm_i8_fused.cu", "encodings.cu", "domain_code.cu", "offline_online.cu"]
 HEADERS = ["common.cuh", "kernels.h", "tc05.cuh", os.path.join("..", "..", "include", "qfall_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

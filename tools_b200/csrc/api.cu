@@ -211,6 +211,15 @@ struct qf_ctx {
     bool fa_poly = false;
     int fa_h0_kind = 1;
     Dev dFaXr, dFaH0;
+    // Pool of the target-independent half of samp_p (qf_samp_p_offline, DESIGN 4.12): entries pool_first ..
+    // pool_first + pool_count - 1 under pool_seed, entry j in slot j - pool_first; pool_next slots are consumed.
+    // PSFPerturbation: dPoolX = p (m int32), dPoolAx = -A p mod q (n words).  PSFGPV two-phase: dPoolX = z2 (m_bar int32),
+    // dPoolAx = -A_bar z2 mod q, dPoolT = -V 256^mt1_dlo of the Mt_1 z2 contraction (nk fp64, unit scale: dOnes).
+    // Dropped whenever A or the trapdoor changes (drop_pool).
+    bool pool = false;
+    int64_t pool_count = 0, pool_next = 0;
+    uint64_t pool_seed = 0, pool_first = 0;
+    Dev dPoolX, dPoolAx, dPoolT, dOnes;
     // Defaults from the error budget of DESIGN 4.2, checked at the full C2 key (scripts/ab_c2_precision.py, profiles/README_r2.md):
     // four digits everywhere; the lowest digit sum is dropped where the operand has three digits (z2), not for the
     // two-digit z1 (dropping it there moves 14 % of the preimages, keeping it 0.3 %).
@@ -228,6 +237,11 @@ struct qf_ctx {
     qf_status fail(qf_status st, const std::string& msg) {
         err = msg;
         return st;
+    }
+    void drop_pool() {
+        pool = false;
+        pool_count = pool_next = 0;
+        dPoolX.release(); dPoolAx.release(); dPoolT.release();
     }
 };
 
@@ -620,21 +634,26 @@ qf_status ring_f_a_chunk(qf_ctx* ctx, const int32_t* dSigma, int Bc, int64_t* dU
 // ---------------------------------------------------------------------------
 qf_status pert_lg_i8(qf_ctx* ctx, const int8_t* gp, long gplane, int Bc, double* X2, long ldx, bool tri);
 
-// dTidx (optional, device): the tag index of every target of the chunk in the installed tag table (qf_samp_p_tagged)
-qf_status samp_p_pert_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t seed, uint64_t first, int32_t* dE,
-                            const int32_t* dTidx = nullptr) {
-    const long ldm = ctx->ld_dim, ldn = ctx->ld_n, ldnk = ctx->ld_nk;
-    const long C = ctx->chunk;
+// The chunk is split at the first read of the target (DESIGN 4.12): pert_perturbation and pert_ap (p and A p) are the
+// offline half, pert_finish (from v = u - A p on) the online half.
+qf_status pert_workspace(qf_ctx* ctx) {
+    const long ldm = ctx->ld_dim, C = ctx->chunk;
     CK(ctx->w[0].ensure((size_t)C * ldm * 8));   // g, later reused
     CK(ctx->w[1].ensure((size_t)C * ldm * 8));   // x2 = sqrt(Sigma2) g
     CK(ctx->w[2].ensure((size_t)C * ldm * 8));   // p
-    CK(ctx->w[3].ensure((size_t)C * ldnk * 8));  // z
+    CK(ctx->w[3].ensure((size_t)C * ctx->ld_nk * 8));  // z
     CK(ctx->w[4].ensure((size_t)C * ctx->n * 8));  // v (int64)
+    return QF_OK;
+}
+
+// p <- D_{Z^m, r sqrt(Sigma_2)} into P (w[2])
+qf_status pert_perturbation(qf_ctx* ctx, int Bc, uint64_t seed, uint64_t first) {
+    const long ldm = ctx->ld_dim;
+    const long C = ctx->chunk;
+    QF_TRY(pert_workspace(ctx));
     double* G = ctx->w[0].as<double>();
     double* X2 = ctx->w[1].as<double>();
     double* P = ctx->w[2].as<double>();
-    double* Z = ctx->w[3].as<double>();
-    int64_t* V = ctx->w[4].as<int64_t>();
     // p <- D_{Z^m, r sqrt(Sigma_2)} : x2 = sqrt(Sigma_2) * N(0,I), p_i <- D_{Z, r, x2_i}   (:315)
     const bool st = ctx->pert_structured;
     if (st) CK(ctx->w[5].ensure((size_t)ctx->xb_limbs * C * ctx->ldk_nk));
@@ -672,7 +691,13 @@ qf_status samp_p_pert_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t s
     }
     LAUNCH(qf_launch_dgauss(X2, ldm, P, ldm, nullptr, 0, Bc, (int)ctx->m, ctx->prm.r, seed, first, QF_STREAM_PERT_ROUND,
                             ctx->dFlag.as<int>(), ctx->stream));
-    // v = u - A p   (:318)
+    return QF_OK;
+}
+
+// V = (base - A p) mod q for the p in P (base == nullptr: -A p mod q)   (:318)
+qf_status pert_ap(qf_ctx* ctx, const int64_t* dUin, int Bc, int64_t* V) {
+    const long ldm = ctx->ld_dim, ldn = ctx->ld_n, C = ctx->chunk;
+    double* P = ctx->w[2].as<double>();
     if (ctx->use_i8) {
         const long ldk = ctx->ldk_dim, plane = C * ldk;
         CK(ctx->w[0].ensure((size_t)ctx->x_limbs * plane));  // g is dead: reuse as digit planes of p
@@ -699,6 +724,16 @@ qf_status samp_p_pert_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t s
         ca.nacc = ctx->a_nchunks; ca.acc_sign = -1; ca.ldacc = ldn; ca.base = dUin; ca.ldbase = ctx->n; ca.q = ctx->prm.q;
         LAUNCH(qf_launch_combine_i64(ca, V, ctx->n, Bc, (int)ctx->n, ctx->stream));
     }
+    return QF_OK;
+}
+
+// from v = u - A p (V, w[4]) and p (P, w[2]) on: the gadget preimage z and e = p + [R; I] z
+// dTidx (optional, device): the tag index of every target of the chunk in the installed tag table (qf_samp_p_tagged)
+qf_status pert_finish(qf_ctx* ctx, int Bc, uint64_t seed, uint64_t first, int32_t* dE, const int32_t* dTidx) {
+    const long ldm = ctx->ld_dim, ldnk = ctx->ld_nk, C = ctx->chunk;
+    double* P = ctx->w[2].as<double>();
+    double* Z = ctx->w[3].as<double>();
+    const int64_t* V = ctx->w[4].as<int64_t>();
     // tagged key A = [A_bar | H G - A_bar R]: A [R; I] = H G, so z solves G z = v' = H^-1 v
     const int64_t* Vg = V;
     if (dTidx) {
@@ -739,6 +774,13 @@ qf_status samp_p_pert_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t s
     LAUNCH(qf_launch_finalize_pert(P, ldm, Z, ldnk, dE, ctx->m, Bc, (int)ctx->m, (int)ctx->m_bar, ctx->dFlag.as<int>(),
                                    ctx->stream));
     return QF_OK;
+}
+
+qf_status samp_p_pert_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t seed, uint64_t first, int32_t* dE,
+                            const int32_t* dTidx = nullptr) {
+    QF_TRY(pert_perturbation(ctx, Bc, seed, first));
+    QF_TRY(pert_ap(ctx, dUin, Bc, ctx->w[4].as<int64_t>()));
+    return pert_finish(ctx, Bc, seed, first, dE, dTidx);
 }
 
 // ---------------------------------------------------------------------------
@@ -1070,18 +1112,19 @@ qf_status samp_p_np1_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t se
 // dTidx (optional, device): the tag index of every target of the chunk in the installed tag table (qf_samp_p_tagged).  The
 // tag enters only between the phases (DESIGN 4.3): for A_t = [A_bar | H_t G - A_bar R], g3 = digits(h_t) with
 // h_t = H_t^-1 (u - A_bar z2) mod q, the same integer vector as after qf_gpv_set_tag(H_t); everything else is tag-independent.
-qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t seed, uint64_t first, int32_t* dE,
-                           const int32_t* dTidx = nullptr) {
-    const long D = ctx->dim, ldD = ctx->ld_dim, C = ctx->chunk, nk = ctx->nk, mb = ctx->m_bar, n = ctx->n;
-    const long ldk = ctx->ldk_dim, plane = C * ldk, ldnk = ctx->ld_nk, ldk_nk = ctx->ldk_nk;
+// The chunk is split at the first read of the target (DESIGN 4.12): np2_workspace + np2_phase1 and the products of z2
+// (np2_abar_z2, np2_mt1_z2) are the offline half, np2_finish (from h on) the online half.
+qf_status np2_workspace(qf_ctx* ctx) {
+    const long D = ctx->dim, ldD = ctx->ld_dim, C = ctx->chunk, n = ctx->n;
+    const long ldk = ctx->ldk_dim, plane = C * ldk;
     const int nz_m = (int)((C + 127) / 128), nz_kb = (int)(ldk / 128);
     const int L = ctx->z_limbs;
     CK(ctx->w[0].ensure((size_t)C * n * 8));     // h = u - A_bar z2 mod q
     CK(ctx->w[2].ensure((size_t)C * ldD * 8));   // T
     CK(ctx->w[3].ensure((size_t)C * ldD * 8));   // Z
-    CK(ctx->w[4].ensure((size_t)C * ldnk * 8));  // e_bot = g3 + S' z1
+    CK(ctx->w[4].ensure((size_t)C * ctx->ld_nk * 8));  // e_bot = g3 + S' z1
     CK(ctx->w[8].ensure((size_t)L * plane));     // digit planes of z
-    CK(ctx->w[10].ensure((size_t)C * ldk_nk));   // g3 (one digit plane)
+    CK(ctx->w[10].ensure((size_t)C * ctx->ldk_nk));   // g3 (one digit plane)
     const size_t nzb = (size_t)L * nz_m * nz_kb;
     CK(ctx->dNz.ensure(nzb));
     CK(cudaMemsetAsync(ctx->dNz.p, 0, nzb, ctx->stream));
@@ -1091,44 +1134,63 @@ qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t se
     const size_t gb = (size_t)(ctx->gate_n256 + ctx->gate_n1024 + ctx->gate_n4096 + 1) * sizeof(int);
     CK(ctx->dGate.ensure(gb));
     CK(cudaMemsetAsync(ctx->dGate.p, 0, gb, ctx->stream));
+    return QF_OK;
+}
+
+// ---- phase 1: coordinates m-1 .. nk, centres start at 0 (never reads the target)
+qf_status np2_phase1(qf_ctx* ctx, int Bc, uint64_t seed, uint64_t first) {
+    const long D = ctx->dim, ldD = ctx->ld_dim, nk = ctx->nk;
+    double* T = ctx->w[2].as<double>();
+    CK(cudaMemset2DAsync(T + nk, (size_t)ldD * 8, 0, (size_t)ctx->m_bar * 8, (size_t)Bc, ctx->stream));
+    ctx->np_wdrop_cur = ctx->u_limbs - ctx->u22_limbs; ctx->np_dlo_cur = ctx->u22_dlo; ctx->np_lx_min = 3;
+    return np_block(ctx, T, ctx->w[3].as<double>(), Bc, nk, D, NP_TOP, 0, seed, first);
+}
+
+// out = (base - A_bar z2) mod q, exact (base == nullptr: -A_bar z2 mod q).  A_bar = the first m_bar columns of the installed
+// digit planes of A, or (abar_tagged) the digit planes of A_bar' = H^-1 A_bar of a tagged key.
+qf_status np2_abar_z2(qf_ctx* ctx, const int64_t* base, bool abar_tagged, int Bc, int64_t* out) {
+    const long C = ctx->chunk, nk = ctx->nk, n = ctx->n, ldk = ctx->ldk_dim;
+    const long ldw = abar_tagged ? ctx->ldk_mb : ldk;
+    I8GemmArgs g{};
+    g.x = ctx->w[8].as<int8_t>() + nk; g.ldx = ldk; g.x_plane = C * ldk;
+    g.w = abar_tagged ? ctx->dAbpl.p : ctx->dAl.p; g.ldw = ldw; g.w_plane = n * ldw;
+    g.LX = ctx->z_limbs; g.LW = ctx->a_limbs; g.w_signed = 0;
+    g.B = Bc; g.N = (int)n; g.K = (int)ctx->m_bar;
+    g.out_kind = 0; g.sign = -1; g.q = ctx->prm.q; g.base = base; g.ldbase = n;
+    g.out = out; g.ldout = n;
+    g.flag = ctx->dFlag.as<int>();
+    g.x_nz = ctx->dNz.as<uint8_t>(); g.nz_m_tiles = (int)((C + 127) / 128); g.nz_kb_total = (int)(ldk / 128);
+    g.nz_kb_off = (int)(nk / 128);
+    return gemm_i8_gated(ctx, g, ctx->dGate.as<int>() + ctx->gate_n256 + ctx->gate_n1024 + ctx->gate_n4096);
+}
+
+// Mt_1 z2: the digit planes of z2 written by phase 1 against all digits of Mt_1; out -= V * scale (overwrite: out = -V * scale)
+qf_status np2_mt1_z2(qf_ctx* ctx, int Bc, double* out, long ldout, const double* scale, int overwrite) {
+    const long C = ctx->chunk, nk = ctx->nk, ldk = ctx->ldk_dim;
+    I8GemmArgs g{};
+    g.x = ctx->w[8].as<int8_t>() + nk; g.ldx = ldk; g.x_plane = C * ldk;
+    g.w = ctx->dMt1l.p; g.ldw = ctx->ldk_mb; g.w_plane = nk * ctx->ldk_mb;
+    g.LX = ctx->z_limbs; g.LW = ctx->mt1_limbs; g.w_signed = 1;
+    g.B = Bc; g.N = (int)nk; g.K = (int)ctx->m_bar;
+    g.out_kind = 3; g.sign = 1; g.q = 0; g.out = out; g.ldout = ldout;
+    g.flag = ctx->dFlag.as<int>();
+    g.scale = scale;
+    g.d_lo = ctx->mt1_dlo; g.overwrite = overwrite;
+    g.x_nz = ctx->dNz.as<uint8_t>(); g.nz_m_tiles = (int)((C + 127) / 128); g.nz_kb_total = (int)(ldk / 128);
+    g.nz_kb_off = (int)(nk / 128);
+    return gemm_i8_gated(ctx, g, ctx->dGate.as<int>() + ctx->gate_n256 + ctx->gate_n1024 + ctx->gate_n4096);
+}
+
+// From h = digits source (H: the residues (u - A_bar z2) mod q of the recursion's target) on: g3, the centres of phase 2,
+// phase 2 and e.  z2 in Z[:, nk:].  Tpool == nullptr: Mt_1 z2 is contracted here from the digit planes of z2; otherwise
+// Tpool holds its store-only unit-scale output (a pool entry, row stride nk).
+qf_status np2_finish(qf_ctx* ctx, const int64_t* H, int Bc, uint64_t seed, uint64_t first, int32_t* dE, const double* Tpool) {
+    const long D = ctx->dim, ldD = ctx->ld_dim, C = ctx->chunk, nk = ctx->nk, mb = ctx->m_bar, n = ctx->n;
+    const long ldnk = ctx->ld_nk, ldk_nk = ctx->ldk_nk;
     double* T = ctx->w[2].as<double>();
     double* Z = ctx->w[3].as<double>();
-    int64_t* H = ctx->w[0].as<int64_t>();
-    int8_t* zp = ctx->w[8].as<int8_t>();
     int8_t* gp = ctx->w[10].as<int8_t>();
     int* flag = ctx->dFlag.as<int>();
-    int* gate_z2 = ctx->dGate.as<int>() + ctx->gate_n256 + ctx->gate_n1024 + ctx->gate_n4096;
-
-    // ---- phase 1: coordinates m-1 .. nk, centres start at 0
-    CK(cudaMemset2DAsync(T + nk, (size_t)ldD * 8, 0, (size_t)mb * 8, (size_t)Bc, ctx->stream));
-    ctx->np_wdrop_cur = ctx->u_limbs - ctx->u22_limbs; ctx->np_dlo_cur = ctx->u22_dlo; ctx->np_lx_min = 3;
-    QF_TRY(np_block(ctx, T, Z, Bc, nk, D, NP_TOP, 0, seed, first));
-
-    // ---- tagged key: the recursion runs on H^-1 A, so its target is u' = H^-1 u mod q (phase 1 never reads the target)
-    const bool abar_tagged = ctx->key_tagged && !dTidx;
-    const int64_t* ub = dUin;
-    if (abar_tagged) QF_TRY(tag_targets(ctx, dUin, Bc, &ub));
-    // ---- h = (u - A_bar z2) mod q, exact (A_bar = the first m_bar columns of the installed digit planes of A; for a tagged
-    // key u' - A_bar' z2 with the digit planes of A_bar' = H^-1 A_bar).  With a tag per target: w = u - A_bar z2 whatever
-    // the installed tag, then h_t = H_t^-1 w per target.
-    if (dTidx) CK(ctx->dTagU.ensure((size_t)C * n * 8));
-    {
-        const long ldw = abar_tagged ? ctx->ldk_mb : ldk;
-        I8GemmArgs g{};
-        g.x = zp + nk; g.ldx = ldk; g.x_plane = plane;
-        g.w = abar_tagged ? ctx->dAbpl.p : ctx->dAl.p; g.ldw = ldw; g.w_plane = n * ldw;
-        g.LX = L; g.LW = ctx->a_limbs; g.w_signed = 0;
-        g.B = Bc; g.N = (int)n; g.K = (int)mb;
-        g.out_kind = 0; g.sign = -1; g.q = ctx->prm.q; g.base = ub; g.ldbase = n;
-        g.out = dTidx ? ctx->dTagU.as<int64_t>() : H; g.ldout = n;
-        g.flag = flag;
-        g.x_nz = ctx->dNz.as<uint8_t>(); g.nz_m_tiles = nz_m; g.nz_kb_total = nz_kb; g.nz_kb_off = (int)(nk / 128);
-        QF_TRY(gemm_i8_gated(ctx, g, gate_z2));
-    }
-    if (dTidx)
-        LAUNCH(qf_launch_tag_syndrome(ctx->dTagU.as<int64_t>(), n, nullptr, 0, 0, dTidx, (int)ctx->tag_count, ctx->dTagTab.p,
-                                      nullptr, ctx->tag_word, nullptr, ctx->prm.q, (int)n, (int)ctx->k, Bc, H, n, flag,
-                                      ctx->stream, ctx->tag_poly ? ctx->dTagXr.p : nullptr));
     // ---- g3 = digits(h): one s8 plane (the x operand of its centre map) and, as fp64, the start of e_bot = g3 + S' z1
     // (fused tail: e_bot is formed in one pass from z1 and the g3 plane -- needs 16-byte aligned int32 rows; otherwise e_bot is
     // accumulated in fp64 as in the one-pass form)
@@ -1139,7 +1201,7 @@ qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t se
     // ---- centres of phase 2 in GSO coordinates: T[:, 0:nk] = -M' g3 - Mt_1 z2, two launches:
     // (a) M' g3 (M' = U_11 S'^-1, entries <= 1/2, block triangular: the k blocks outside the triangle are skipped
     //     in-kernel), one digit of 0 .. base-1 against four digits: store-only epilogue;
-    // (b) Mt_1 z2: the three digit planes of z2 written by phase 1 against all digits of Mt_1, accumulated onto (a).
+    // (b) Mt_1 z2, accumulated onto (a) (from a pool entry: the same fma, pool_centre).
     {
         I8GemmArgs g{};
         g.x = gp; g.ldx = ldk_nk; g.x_plane = C * ldk_nk;
@@ -1153,19 +1215,11 @@ qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t se
         g.tri_mode = ctx->gpv_rev ? 3 : 4; g.tri_slack = (int)ctx->k;
         LAUNCH(ctx_gemm_i8(ctx, g));
     }
-    {
-        I8GemmArgs g{};
-        g.x = zp + nk; g.ldx = ldk; g.x_plane = plane;
-        g.w = ctx->dMt1l.p; g.ldw = ctx->ldk_mb; g.w_plane = nk * ctx->ldk_mb;
-        g.LX = L; g.LW = ctx->mt1_limbs; g.w_signed = 1;
-        g.B = Bc; g.N = (int)nk; g.K = (int)mb;
-        g.out_kind = 3; g.sign = 1; g.q = 0; g.out = T; g.ldout = ldD;
-        g.flag = flag;
-        g.scale = ctx->dMt1scale.as<double>();
-        g.d_lo = ctx->mt1_dlo; g.overwrite = 0;
-        g.x_nz = ctx->dNz.as<uint8_t>(); g.nz_m_tiles = nz_m; g.nz_kb_total = nz_kb; g.nz_kb_off = (int)(nk / 128);
-        QF_TRY(gemm_i8_gated(ctx, g, gate_z2));
-    }
+    if (Tpool)
+        LAUNCH(qf_launch_pool_centre(Tpool, nk, T, ldD, ctx->dMt1scale.as<double>(), std::ldexp(1.0, 8 * ctx->mt1_dlo), (int)nk,
+                                     Bc, ctx->stream));
+    else
+        QF_TRY(np2_mt1_z2(ctx, Bc, T, ldD, ctx->dMt1scale.as<double>(), 0));
     // ---- phase 2: coordinates nk-1 .. 0
     ctx->np_wdrop_cur = ctx->u_limbs - ctx->u11_limbs; ctx->np_dlo_cur = ctx->u11_dlo; ctx->np_lx_min = 2;
     QF_TRY(np_block(ctx, T, Z, Bc, 0, nk, NP_TOP, 0, seed, first));
@@ -1198,11 +1252,92 @@ qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t se
     return QF_OK;
 }
 
+// Per-target tag (dTidx): h_t = H_t^-1 w for w = u - A_bar z2 in dTagU (any installed tag), written to H (w[0])
+qf_status np2_tag_syndrome(qf_ctx* ctx, const int32_t* dTidx, int Bc) {
+    const long n = ctx->n;
+    LAUNCH(qf_launch_tag_syndrome(ctx->dTagU.as<int64_t>(), n, nullptr, 0, 0, dTidx, (int)ctx->tag_count, ctx->dTagTab.p,
+                                  nullptr, ctx->tag_word, nullptr, ctx->prm.q, (int)n, (int)ctx->k, Bc, ctx->w[0].as<int64_t>(), n,
+                                  ctx->dFlag.as<int>(), ctx->stream, ctx->tag_poly ? ctx->dTagXr.p : nullptr));
+    return QF_OK;
+}
+
+qf_status samp_p_np2_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t seed, uint64_t first, int32_t* dE,
+                           const int32_t* dTidx = nullptr) {
+    QF_TRY(np2_workspace(ctx));
+    QF_TRY(np2_phase1(ctx, Bc, seed, first));
+    // ---- tagged key: the recursion runs on H^-1 A, so its target is u' = H^-1 u mod q (phase 1 never reads the target)
+    const bool abar_tagged = ctx->key_tagged && !dTidx;
+    const int64_t* ub = dUin;
+    if (abar_tagged) QF_TRY(tag_targets(ctx, dUin, Bc, &ub));
+    // ---- h = (u - A_bar z2) mod q (for a tagged key u' - A_bar' z2).  With a tag per target: w = u - A_bar z2 whatever the
+    // installed tag, then h_t = H_t^-1 w per target.
+    int64_t* H = ctx->w[0].as<int64_t>();
+    if (dTidx) CK(ctx->dTagU.ensure((size_t)ctx->chunk * ctx->n * 8));
+    QF_TRY(np2_abar_z2(ctx, ub, abar_tagged, Bc, dTidx ? ctx->dTagU.as<int64_t>() : H));
+    if (dTidx) QF_TRY(np2_tag_syndrome(ctx, dTidx, Bc));
+    return np2_finish(ctx, H, Bc, seed, first, dE, nullptr);
+}
+
 // dTidx (tag per target) only with the two-phase recursion (samp_p_tagged_ready)
 qf_status samp_p_np_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t seed, uint64_t first, int32_t* dE,
                           const int32_t* dTidx = nullptr) {
     return ctx->two_phase ? samp_p_np2_chunk(ctx, dUin, Bc, seed, first, dE, dTidx)
                           : samp_p_np1_chunk(ctx, dUin, Bc, seed, first, dE);
+}
+
+// ---------------------------------------------------------------------------
+// samp_p in two halves over the context's pool (DESIGN 4.12).  Pool slot j holds the offline state of sampler index
+// pool_first + j; both halves run the launches of the composed chunk functions above, so an online row is bit-identical to
+// qf_samp_p (qf_samp_p_tagged) at its index.
+// ---------------------------------------------------------------------------
+long pool_xdim(const qf_ctx* ctx) { return ctx->prm.kind == QF_PSF_PERTURBATION ? ctx->m : ctx->m_bar; }
+long pool_tdim(const qf_ctx* ctx) { return ctx->prm.kind == QF_PSF_PERTURBATION ? 0 : ctx->nk; }
+
+// offline half of Bc entries into slots slot0 .. slot0 + Bc - 1 (sampler indices first ..)
+qf_status samp_p_offline_chunk(qf_ctx* ctx, int Bc, uint64_t seed, uint64_t first, int64_t slot0) {
+    const long xd = pool_xdim(ctx), n = ctx->n;
+    int32_t* X = ctx->dPoolX.as<int32_t>() + slot0 * xd;
+    int64_t* Ax = ctx->dPoolAx.as<int64_t>() + slot0 * n;
+    if (ctx->prm.kind == QF_PSF_PERTURBATION) {
+        QF_TRY(pert_perturbation(ctx, Bc, seed, first));
+        QF_TRY(pert_ap(ctx, nullptr, Bc, Ax));
+        LAUNCH(qf_launch_f64_to_i32(ctx->w[2].as<double>(), ctx->ld_dim, X, xd, Bc, (int)xd, ctx->dFlag.as<int>(), ctx->stream));
+        return QF_OK;
+    }
+    const long nk = ctx->nk;
+    QF_TRY(np2_workspace(ctx));
+    QF_TRY(np2_phase1(ctx, Bc, seed, first));
+    // A_bar z2 on the untagged planes of A (their first m_bar columns are A_bar whatever the installed tag): the online half
+    // applies H^-1 to u - A_bar z2, the same residues as u' - A_bar' z2
+    QF_TRY(np2_abar_z2(ctx, nullptr, false, Bc, Ax));
+    QF_TRY(np2_mt1_z2(ctx, Bc, ctx->dPoolT.as<double>() + slot0 * nk, nk, ctx->dOnes.as<double>(), 1));
+    LAUNCH(qf_launch_f64_to_i32(ctx->w[3].as<double>() + nk, ctx->ld_dim, X, xd, Bc, (int)xd, ctx->dFlag.as<int>(), ctx->stream));
+    return QF_OK;
+}
+
+// online half for the targets dUin of Bc entries from slot slot0 on
+qf_status samp_p_online_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, int64_t slot0, int32_t* dE, const int32_t* dTidx) {
+    const long xd = pool_xdim(ctx), n = ctx->n;
+    const uint64_t seed = ctx->pool_seed, first = ctx->pool_first + (uint64_t)slot0;
+    const int32_t* X = ctx->dPoolX.as<int32_t>() + slot0 * xd;
+    const int64_t* Ax = ctx->dPoolAx.as<int64_t>() + slot0 * n;
+    if (ctx->prm.kind == QF_PSF_PERTURBATION) {
+        QF_TRY(pert_workspace(ctx));
+        LAUNCH(qf_launch_pool_expand(X, xd, ctx->w[2].as<double>(), ctx->ld_dim, (int)xd, dUin, n, Ax, n, ctx->w[4].as<int64_t>(),
+                                     n, (int)n, Bc, ctx->prm.q, ctx->stream));
+        return pert_finish(ctx, Bc, seed, first, dE, dTidx);
+    }
+    const long nk = ctx->nk;
+    QF_TRY(np2_workspace(ctx));
+    int64_t* H = ctx->w[0].as<int64_t>();
+    if (dTidx) CK(ctx->dTagU.ensure((size_t)ctx->chunk * n * 8));
+    // z2 into Z[:, nk:], w = u - A_bar z2 mod q
+    LAUNCH(qf_launch_pool_expand(X, xd, ctx->w[3].as<double>() + nk, ctx->ld_dim, (int)xd, dUin, n, Ax, n,
+                                 dTidx ? ctx->dTagU.as<int64_t>() : H, n, (int)n, Bc, ctx->prm.q, ctx->stream));
+    const int64_t* h = H;
+    if (dTidx) QF_TRY(np2_tag_syndrome(ctx, dTidx, Bc));
+    else if (ctx->key_tagged) QF_TRY(tag_targets(ctx, H, Bc, &h));
+    return np2_finish(ctx, h, Bc, seed, first, dE, ctx->dPoolT.as<double>() + slot0 * nk);
 }
 
 // find n columns of A (n x m) that form a matrix invertible over Z_q by unit pivoting and return
@@ -1787,6 +1922,7 @@ qf_status install_a(qf_ctx* ctx, const int64_t* a) {
     ctx->dHinvl.release(); ctx->dAbpl.release();
     ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release(); ctx->dTagXr.release();
     ctx->fa_tag_count = 0; ctx->dFaTab.release(); ctx->dFaXr.release(); ctx->dFaH0.release();
+    ctx->drop_pool();
     const long n = ctx->n, m = ctx->m;
     for (long i = 0; i < n * m; ++i)
         if (a[i] < 0 || (uint64_t)a[i] >= ctx->prm.q) return ctx->fail(QF_ERR_INVALID, "A entry outside [0,q)");
@@ -2115,6 +2251,7 @@ qf_status qf_set_trapdoor_perturbation(qf_ctx* ctx, const int8_t* r, const doubl
     ctx->has_pert = false;
     ctx->key_tagged = false; ctx->pert_gadget_key = false;
     ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release(); ctx->dTagXr.release();
+    ctx->drop_pool();
     CK(cudaSetDevice(ctx->device));
     QF_TRY(upload_as_f64(ctx, r, ctx->m_bar, ctx->nk, ctx->ld_nk, ctx->dR));
     {
@@ -2189,6 +2326,7 @@ qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out) {
     ctx->has_pert = false;
     // the f_a table is relative to A, which changes here
     ctx->fa_tag_count = 0; ctx->dFaTab.release(); ctx->dFaXr.release(); ctx->dFaH0.release();
+    ctx->drop_pool();
     const std::vector<uint64_t> gpow = gadget_powers(ctx);
     for (long i = 0; i < n; ++i)
         for (long j = 0; j < n; ++j) {
@@ -2287,6 +2425,7 @@ qf_status qf_gpv_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out, int64_
     ctx->has_np = false;
     // the f_a table is relative to A; the samp_p table to (A_bar, R): kept
     ctx->fa_tag_count = 0; ctx->dFaTab.release(); ctx->dFaXr.release(); ctx->dFaH0.release();
+    ctx->drop_pool();
     ctx->hA.swap(a2);
     QF_TRY(upload_a_cols(ctx, mb));
     if (repivot) {
@@ -2790,6 +2929,7 @@ qf_status qf_set_trapdoor_gpv(qf_ctx* ctx, const int64_t* s, const double* sg) {
     ctx->two_phase = false;
     // the tag table is relative to the old (A_bar, R)
     ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release(); ctx->dTagXr.release();
+    ctx->drop_pool();
     ctx->u_limbs = 7;
     CK(cudaSetDevice(ctx->device));
     const long D = ctx->dim, ld = ctx->ld_dim;
@@ -3397,8 +3537,9 @@ struct SampOut {
 
 // host-buffer samp_p in one of the SampOut forms
 // tidx (optional, host): tag index of every target in the installed tag table (qf_samp_p_tagged), copied with the targets
+// pool_slot0 >= 0: the online half of the pool entries from that slot on (qf_samp_p_online; seed and first unused)
 static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed, uint64_t first, void* e_out,
-                             const SampOut& fmt, const int32_t* tidx = nullptr) {
+                             const SampOut& fmt, const int32_t* tidx = nullptr, int64_t pool_slot0 = -1) {
     if (!ctx || batch < 0 || (batch > 0 && (!u || !e_out))) return QF_ERR_INVALID;
     if (batch == 0) return QF_OK;
     CK(cudaSetDevice(ctx->device));
@@ -3473,8 +3614,9 @@ static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint6
         // front of every call), reported by check_flag as QF_ERR_INVALID
         LAUNCH(qf_launch_range_check_i64(du, (size_t)Bc * ctx->n, ctx->prm.q, ctx->dFlag.as<int>(), ctx->stream));
         const int32_t* dt = tidx ? t_buf(idx) : nullptr;
-        QF_TRY(ctx->prm.kind == QF_PSF_PERTURBATION ? samp_p_pert_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres, dt)
-                                                    : samp_p_np_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres, dt));
+        if (pool_slot0 >= 0) QF_TRY(samp_p_online_chunk(ctx, du, Bc, pool_slot0 + b0, dres, dt));
+        else QF_TRY(ctx->prm.kind == QF_PSF_PERTURBATION ? samp_p_pert_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres, dt)
+                                                         : samp_p_np_chunk(ctx, du, Bc, seed, first + (uint64_t)b0, dres, dt));
         if (overlap) CK(cudaEventRecord(ctx->ev_u_used[slot], ctx->stream));
         const int bs = overlap ? slot : 0;
         const void* src = dres;
@@ -3553,6 +3695,101 @@ qf_status qf_samp_p_tagged_dev(qf_ctx* ctx, const int64_t* u, const int32_t* tag
         int32_t* ee = e_out + b0 * ctx->dim;
         return ctx->prm.kind == QF_PSF_PERTURBATION ? samp_p_pert_chunk(ctx, uu, Bc, seed, first + (uint64_t)b0, ee, tag_idx + b0)
                                                     : samp_p_np_chunk(ctx, uu, Bc, seed, first + (uint64_t)b0, ee, tag_idx + b0);
+    });
+}
+
+// ---- offline / online samp_p (DESIGN 4.12) ---------------------------------------------------------------------------
+qf_status qf_samp_p_offline(qf_ctx* ctx, int64_t count, uint64_t seed, uint64_t first) {
+    if (!ctx || count < 0) return QF_ERR_INVALID;
+    CK(cudaSetDevice(ctx->device));
+    if (ctx->prm.kind == QF_PSF_GPV_RING) return ctx->fail(QF_ERR_UNSUPPORTED, "samp_p pool: not on a ring context");
+    QF_TRY(samp_p_ready(ctx));
+    if (ctx->prm.kind == QF_PSF_GPV && !ctx->two_phase)
+        return ctx->fail(QF_ERR_UNSUPPORTED, "samp_p pool: PSFGPV needs the two-phase recursion (the one-pass form reads the "
+                                             "target first)");
+    ctx->drop_pool();
+    const long xd = pool_xdim(ctx), td = pool_tdim(ctx);
+    const size_t per = (size_t)xd * 4 + (size_t)ctx->n * 8 + (size_t)td * 8;
+    if ((uint64_t)count > (uint64_t)(SIZE_MAX / 2) / per) return ctx->fail(QF_ERR_INVALID, "samp_p pool: count too large");
+    const size_t c = (size_t)std::max<int64_t>(count, 1);
+    cudaError_t e = ctx->dPoolX.ensure(c * xd * 4);
+    if (e == cudaSuccess) e = ctx->dPoolAx.ensure(c * ctx->n * 8);
+    if (e == cudaSuccess && td) e = ctx->dPoolT.ensure(c * td * 8);
+    if (e == cudaSuccess && td && ctx->dOnes.cap < (size_t)td * 8) {
+        std::vector<double> ones((size_t)td, 1.0);
+        e = ctx->dOnes.ensure((size_t)td * 8);
+        if (e == cudaSuccess) e = cudaMemcpy(ctx->dOnes.p, ones.data(), (size_t)td * 8, cudaMemcpyHostToDevice);
+    }
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        ctx->drop_pool();
+        char buf[192];
+        snprintf(buf, sizeof buf, "samp_p pool: %lld entries of %zu bytes do not fit in device memory (%s)", (long long)count, per,
+                 cudaGetErrorString(e));
+        return ctx->fail(QF_ERR_CUDA, buf);
+    }
+    qf_status st = for_chunks(ctx, count, [&](int64_t b0, int Bc) -> qf_status {
+        return samp_p_offline_chunk(ctx, Bc, seed, first + (uint64_t)b0, b0);
+    });
+    if (st == QF_OK) {
+        CK(cudaStreamSynchronize(ctx->stream));
+        st = check_flag(ctx);
+    }
+    if (st != QF_OK) {
+        ctx->drop_pool();
+        return st;
+    }
+    ctx->pool = true;
+    ctx->pool_count = count;
+    ctx->pool_next = 0;
+    ctx->pool_seed = seed;
+    ctx->pool_first = first;
+    return QF_OK;
+}
+
+qf_status qf_samp_p_pool_info(const qf_ctx* ctx, int64_t* remaining, uint64_t* next_index) {
+    if (!ctx) return QF_ERR_INVALID;
+    if (remaining) *remaining = ctx->pool ? ctx->pool_count - ctx->pool_next : 0;
+    if (next_index) *next_index = ctx->pool ? ctx->pool_first + (uint64_t)ctx->pool_next : 0;
+    return QF_OK;
+}
+
+// checks of an online call; on success the call owns slots *slot0 .. *slot0 + batch - 1 (the cursor has moved)
+static qf_status samp_p_online_accept(qf_ctx* ctx, const int32_t* tag_idx, int64_t batch, bool host_idx, int64_t* slot0,
+                                      uint64_t* first_index_out) {
+    CK(cudaSetDevice(ctx->device));
+    if (!ctx->pool) return ctx->fail(QF_ERR_NO_KEY, "no samp_p pool installed (qf_samp_p_offline)");
+    if (tag_idx) QF_TRY(samp_p_tagged_ready(ctx));
+    else QF_TRY(samp_p_ready(ctx));
+    if (batch > ctx->pool_count - ctx->pool_next) {
+        char buf[160];
+        snprintf(buf, sizeof buf, "samp_p pool: batch %lld exceeds the %lld remaining entries", (long long)batch,
+                 (long long)(ctx->pool_count - ctx->pool_next));
+        return ctx->fail(QF_ERR_INVALID, buf);
+    }
+    if (tag_idx && host_idx && batch > 0) QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->tag_count, "tag table"));
+    *slot0 = ctx->pool_next;
+    if (first_index_out) *first_index_out = ctx->pool_first + (uint64_t)ctx->pool_next;
+    ctx->pool_next += batch;
+    return QF_OK;
+}
+
+qf_status qf_samp_p_online(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, int32_t* e_out,
+                           uint64_t* first_index_out) {
+    if (!ctx || batch < 0 || (batch > 0 && (!u || !e_out))) return QF_ERR_INVALID;
+    int64_t slot0 = 0;
+    QF_TRY(samp_p_online_accept(ctx, tag_idx, batch, true, &slot0, first_index_out));
+    if (batch == 0) return QF_OK;
+    return samp_p_host(ctx, u, batch, 0, 0, e_out, SampOut{}, tag_idx, slot0);
+}
+
+qf_status qf_samp_p_online_dev(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx, int64_t batch, int32_t* e_out,
+                               uint64_t* first_index_out) {
+    if (!ctx || batch < 0 || (batch > 0 && (!u || !e_out))) return QF_ERR_INVALID;
+    int64_t slot0 = 0;
+    QF_TRY(samp_p_online_accept(ctx, tag_idx, batch, false, &slot0, first_index_out));
+    return for_chunks(ctx, batch, [&](int64_t b0, int Bc) -> qf_status {
+        return samp_p_online_chunk(ctx, u + b0 * ctx->n, Bc, slot0 + b0, e_out + b0 * ctx->dim, tag_idx ? tag_idx + b0 : nullptr);
     });
 }
 

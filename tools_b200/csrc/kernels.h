@@ -262,6 +262,15 @@ cudaError_t qf_launch_narrow_i32_i16(const int32_t* in, int16_t* out, size_t cou
 cudaError_t qf_launch_widen_i16_i32(const int16_t* in, int32_t* out, size_t count, cudaStream_t stream);
 cudaError_t qf_launch_range_check_i64(const int64_t* v, size_t count, unsigned long long q, int* flag, cudaStream_t stream);
 
+// online half of samp_p from a pool entry (offline_online.cu, DESIGN 4.12): out[b][0:M] = x[b] as fp64 and
+// v[b] = (u[b] + a[b]) mod q (u, a residues); T[b][n] = fma(X[b][n] / mul, scale[n] * mul, T[b][n]) with X the store-only
+// unit-scale output of the contraction (-dv mul): the same value as the accumulating epilogue of that contraction
+cudaError_t qf_launch_pool_expand(const int32_t* x, long ldx, double* out, long ldo, int M, const int64_t* u, long ldu,
+                                  const int64_t* a, long lda, int64_t* v, long ldv, int N, int B, unsigned long long q,
+                                  cudaStream_t stream);
+cudaError_t qf_launch_pool_centre(const double* X, long ldx, double* T, long ldt, const double* scale, double mul, int N, int B,
+                                  cudaStream_t stream);
+
 // packed Domain values (domain_code.cu, DESIGN 4.11): rows x dim int32 <-> rows slots of slot_bytes bytes (k in [0, 30],
 // slot_bytes a multiple of 16 and at least H0 + ceil(dim / 8); checked by the callers).  Encode: nbytes[row], -1 and a zero
 // slot when the code does not fit or the row holds INT32_MIN.  Decode: ok[row] = 1 iff the slot is canonical.

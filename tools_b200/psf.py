@@ -328,6 +328,43 @@ class _TagTable:
         self.ctx.call("qf_samp_p_tagged", _ffi.ptr(u), _ffi.ptr(ti), u.shape[0], _seed(seed), first_index, _ffi.ptr(e))
         return e
 
+    # -- offline / online samp_p (DESIGN.md 4.12) --------------------------------------------------------------------
+    def samp_p_offline(self, a, td, count: int, seed=None, first_index: int = 0):
+        """Fills the context's pool with the target-independent half of samp_p for the sampler indices first_index ..
+        first_index + count - 1 under seed (qf_samp_p_offline), replacing any previous pool.  Installing another key or
+        trapdoor, or switching the key's tag, drops the pool; tag tables keep it.  Refilling an index range already used
+        under the same seed serves the same perturbations again: the caller must not do that.  PSFGPV needs the two-phase
+        recursion (QfError QF_ERR_UNSUPPORTED otherwise)."""
+        self._install_a(a)
+        self._install_td(a, td)
+        self.ctx.call("qf_samp_p_offline", int(count), _seed(seed), int(first_index))
+
+    def pool_info(self):
+        """(remaining entries, sampler index of the next one) of the pool; (0, 0) without a pool."""
+        rem, nxt = ctypes.c_int64(), ctypes.c_uint64()
+        self.ctx.call("qf_samp_p_pool_info", ctypes.byref(rem), ctypes.byref(nxt))
+        return rem.value, nxt.value
+
+    def samp_p_online_batch(self, a, td, us: np.ndarray, tags=None, tag_idx=None):
+        """Online half of samp_p for the targets us (B x n) from the next B pool entries (qf_samp_p_online).  Returns
+        (e, first_index): row b equals row b of samp_p_batch(a, td, us, seed, first_index) for the pool's seed, or of
+        samp_p_tagged_batch with tags / tag_idx as there (matrices or PolyTags).  QfError QF_ERR_INVALID when B exceeds the
+        remaining entries (nothing is consumed), QF_ERR_NO_KEY without a pool."""
+        self._install_a(a)
+        self._install_td(a, td)
+        u = np.ascontiguousarray(us, dtype=np.int64)
+        assert u.ndim == 2 and u.shape[1] == self.n
+        ti = None
+        if tags is not None:
+            if self._tags_id is not tags:
+                self.set_tag_table(a, td, tags)
+            ti = np.ascontiguousarray(tag_idx, dtype=np.int32)
+            assert ti.shape == (u.shape[0],)
+        e = np.empty((u.shape[0], self.m), dtype=np.int32)
+        first = ctypes.c_uint64()
+        self.ctx.call("qf_samp_p_online", _ffi.ptr(u), _ffi.ptr(ti), u.shape[0], _ffi.ptr(e), ctypes.byref(first))
+        return e, first.value
+
 
 class PSFGPV(_TagTable, _PSFBase):
     """src/primitive/psf/gpv.rs:53-225.  Trapdoor = (short basis S_A, its GSO)."""
