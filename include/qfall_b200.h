@@ -231,6 +231,40 @@ qf_status qf_f_a_tagged(qf_ctx* ctx, const int32_t* sigma, const int32_t* tag_id
 qf_status qf_f_a_tagged_dev(qf_ctx* ctx, const int32_t* sigma, const int32_t* tag_idx, int64_t batch, int64_t* u_out,
                             uint8_t* in_domain);
 
+/* ---- ring f_a with a key per target (ring contexts only; QF_ERR_INVALID on a classical context), DESIGN 4.13 ----------
+ * A ring public key is (k+2) polynomials of n coefficients, so every signer may hold their own: these calls verify one
+ * batch across many keys, as PSF::f_a(&self, a, sigma) takes the key with every call (psf.rs:39-81, gpv_ring.rs:243-247).
+ * Install a table of nkeys keys (host, nkeys x (k+2) x n residues in the layout of qf_ring_set_a).  Every coefficient is
+ * checked to lie in [0, q) before anything changes: QF_ERR_INVALID names the first bad key and keeps the previous table.
+ * QF_ERR_INVALID also for keys == NULL and nkeys outside [1, 2^31 - 1).  Keys need not have a_0 = 1 (f_a reads them only
+ * as polynomials); no trapdoor and no installed key are needed, so a verifier-only context works.  The table is
+ * independent of qf_ring_set_a (neither call drops the other's state), replaced by the next install and freed with the
+ * context.  The keyed calls never use the dense tensor-core path of qf_f_a; the kernel family is chosen at install with
+ * the rules of qf_ring_set_a and does not depend on an installed key.  Device memory per key: (k+2) n words of
+ *   4 bytes  for primes q < 2^16 with n | q - 1, n a power of two in [64, 2048] (NTT mod q; not with QF_DISABLE_SMALL_NTT=1),
+ *   8 bytes  otherwise, for n a power of two in [64, 2048] with (k+2) n (q/2) sqrt(norm bound) < 2^63 (Goldilocks NTT),
+ *   8 bytes  for every other n and q (raw residues, schoolbook product);
+ * C3 (n = 256, q = 3329, k = 12): 14 336 bytes per key. */
+qf_status qf_ring_set_key_table(qf_ctx* ctx, const int64_t* keys, int64_t nkeys);
+/* u[b] = sum_j a^(t)_j sigma[b][j] mod (X^n + 1, q) for t = key_idx[b], key t of the table, and in_domain[b] =
+ * check_domain(sigma[b]).  For sigma[b] in the domain, row b is bit-identical to qf_f_a on the same context after
+ * qf_ring_set_a(key t), for any split into calls and chunks; rows outside the domain have the unspecified u of qf_f_a.
+ * u_out is mandatory.  qf_ring_f_a_keyed takes host pointers and works as qf_f_a_tagged: key indices are checked on the
+ * host before any launch (QF_ERR_INVALID outside [0, nkeys)), in_domain may be NULL, QF_ERR_NOT_IN_DOMAIN when a flag is
+ * 0.  qf_ring_f_a_keyed_dev takes device pointers and is asynchronous (in_domain mandatory): an index outside the table
+ * is never used to address it, its row is unspecified and the next qf_synchronize returns QF_ERR_INVALID.  QF_ERR_NO_KEY
+ * without a table.  An empty batch is valid.  For int16 or packed sigma, decode first (qf_domain_decode_dev). */
+qf_status qf_ring_f_a_keyed(qf_ctx* ctx, const int32_t* sigma, const int32_t* key_idx, int64_t batch, int64_t* u_out,
+                            uint8_t* in_domain);
+qf_status qf_ring_f_a_keyed_dev(qf_ctx* ctx, const int32_t* sigma, const int32_t* key_idx, int64_t batch, int64_t* u_out,
+                                uint8_t* in_domain);
+/* count ring TrapGen keys at once (host pointers): a_bar count x n residues in [0, q) (QF_ERR_INVALID otherwise), r and e
+ * count x k x n small coefficients; a_out count x (k+2) x n.  Key t is bit-identical to qf_ring_trap_gen_from(a_bar_t,
+ * r_t, e_t).  Unlike that call it installs nothing: the context key, its trapdoor and the key table stay as they were.
+ * The products a_bar_t r_{t,j} run as one keyed ring product (count k rows, one polynomial per key). */
+qf_status qf_ring_trap_gen_batch_from(qf_ctx* ctx, int64_t count, const int64_t* a_bar, const int32_t* r, const int32_t* e,
+                                      int64_t* a_out);
+
 /* ---- PSF::samp_d (gpv.rs:113-116, mp_perturbation.rs:264-267, gpv_ring.rs:118-122) --- */
 qf_status qf_samp_d(qf_ctx* ctx, int64_t batch, uint64_t seed, uint64_t first_index, int32_t* out);
 qf_status qf_samp_d_dev(qf_ctx* ctx, int64_t batch, uint64_t seed, uint64_t first_index, int32_t* out);

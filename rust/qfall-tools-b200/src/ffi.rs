@@ -70,6 +70,10 @@ extern "C" {
     pub fn qf_check_domain(ctx: *mut qf_ctx, sigma: *const i32, batch: i64, in_domain: *mut u8) -> i32;
     pub fn qf_f_a_tagged(ctx: *mut qf_ctx, sigma: *const i32, tag_idx: *const i32, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
     pub fn qf_f_a_tagged_dev(ctx: *mut qf_ctx, sigma: *const i32, tag_idx: *const i32, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
+    pub fn qf_ring_set_key_table(ctx: *mut qf_ctx, keys: *const i64, nkeys: i64) -> i32;
+    pub fn qf_ring_f_a_keyed(ctx: *mut qf_ctx, sigma: *const i32, key_idx: *const i32, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
+    pub fn qf_ring_f_a_keyed_dev(ctx: *mut qf_ctx, sigma: *const i32, key_idx: *const i32, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
+    pub fn qf_ring_trap_gen_batch_from(ctx: *mut qf_ctx, count: i64, a_bar: *const i64, r: *const i32, e: *const i32, a_out: *mut i64) -> i32;
     pub fn qf_samp_d(ctx: *mut qf_ctx, batch: i64, seed: u64, first_index: u64, out: *mut i32) -> i32;
     pub fn qf_samp_d_dev(ctx: *mut qf_ctx, batch: i64, seed: u64, first_index: u64, out: *mut i32) -> i32;
     pub fn qf_samp_p(ctx: *mut qf_ctx, u: *const i64, batch: i64, seed: u64, first_index: u64, e_out: *mut i32) -> i32;

@@ -22,6 +22,8 @@ pub struct PSFGPVRingB200 {
     ctx: Context,
     installed_a: RefCell<Option<Vec<i64>>>,
     installed_td: RefCell<Option<(Vec<i32>, Vec<i32>)>>,
+    // words of the key table on the device (qf_ring_set_key_table); independent of the installed key
+    installed_keys: RefCell<Option<Vec<i64>>>,
     seed: RefCell<u64>,
 }
 
@@ -53,6 +55,7 @@ impl PSFGPVRingB200 {
             ctx: Context::new(&params, device)?,
             installed_a: RefCell::new(None),
             installed_td: RefCell::new(None),
+            installed_keys: RefCell::new(None),
             seed: RefCell::new(seed),
         })
     }
@@ -266,6 +269,79 @@ impl PSFBatch for PSFGPVRingB200 {
     fn f_a_batch_packed(&self, a: &MatPolynomialRingZq, packed: &PackedDomain) -> Vec<MatPolynomialRingZq> {
         self.install_a(a);
         f_a_packed_run(&self.ctx, self.n(), packed).chunks(self.n()).map(|row| self.range_from_words(row)).collect()
+    }
+}
+
+impl PSFGPVRingB200 {
+    /// f_a with a key per target: `f_a(keys[key_of[b]], sigmas[b])` for every b in one call, e.g. signatures of many
+    /// signers (qf_ring_set_key_table + qf_ring_f_a_keyed).  The table is uploaded once and kept while the same keys come
+    /// back; the installed key of `f_a` / `samp_p` is not touched.  Panics like `f_a` when a sigma is outside D_n.
+    pub fn f_a_keyed_batch(&self, keys: &[MatPolynomialRingZq], sigmas: &[MatPolyOverZ], key_of: &[usize]) -> Vec<MatPolynomialRingZq> {
+        assert_eq!(sigmas.len(), key_of.len(), "one key index per sigma");
+        let mut kw = Vec::with_capacity(keys.len() * self.n() * (self.k() + 2));
+        for a in keys {
+            kw.extend(self.key_words(a));
+        }
+        if self.installed_keys.borrow().as_ref() != Some(&kw) {
+            let st = unsafe { qf_ring_set_key_table(self.ctx.raw, kw.as_ptr(), keys.len() as i64) };
+            self.ctx.check(st, "qf_ring_set_key_table");
+            *self.installed_keys.borrow_mut() = Some(kw);
+        }
+        let (n, d) = (self.n(), self.n() * (self.k() + 2));
+        let mut sg = Vec::with_capacity(sigmas.len() * d);
+        for sigma in sigmas {
+            sg.extend(self.domain_to_words(sigma).expect("sigma is not in D_n")); // gpv_ring.rs:244
+        }
+        let idx: Vec<i32> = key_of.iter().map(|&t| i32::try_from(t).expect("key index below 2^31")).collect();
+        let mut u = vec![0i64; sigmas.len() * n];
+        let mut ok = vec![0u8; sigmas.len()];
+        let st = unsafe {
+            qf_ring_f_a_keyed(self.ctx.raw, sg.as_ptr(), idx.as_ptr(), sigmas.len() as i64, u.as_mut_ptr(), ok.as_mut_ptr())
+        };
+        assert!(st != QF_ERR_NOT_IN_DOMAIN && ok.iter().all(|f| *f == 1), "sigma is not in D_n");
+        self.ctx.check(st, "qf_ring_f_a_keyed");
+        u.chunks(n).map(|row| self.range_from_words(row)).collect()
+    }
+
+    /// gen_trapdoor_ring_lwe (gadget_ring.rs:62-81) for many (a_bar, r, e) in one call (qf_ring_trap_gen_batch_from): key t
+    /// equals the single-key result bit for bit.  Installs nothing.
+    pub fn gen_trapdoor_ring_lwe_batch(&self, a_bars: &[PolyOverZ], rs: &[MatPolyOverZ], es: &[MatPolyOverZ]) -> Vec<MatPolynomialRingZq> {
+        assert!(a_bars.len() == rs.len() && rs.len() == es.len(), "one (a_bar, r, e) per key");
+        let (n, k) = (self.n(), self.k());
+        let q = self.inner.gp.modulus.get_q();
+        let mut abw = Vec::with_capacity(a_bars.len() * n);
+        for a_bar in a_bars {
+            let mut ab = MatPolyOverZ::new(1, 1);
+            ab.set_entry(0, 0, a_bar).unwrap();
+            abw.extend(Self::polys_to_words(&ab, n).into_iter().map(|v| {
+                let r = Z::from(v) % &q; // least non-negative residue, as the reference reduces a_bar
+                i64::try_from(&r).unwrap()
+            }));
+        }
+        let to32 = |ms: &[MatPolyOverZ]| -> Vec<i32> {
+            ms.iter().flat_map(|m| Self::polys_to_words(m, n).into_iter().map(|v| i32::try_from(v).expect("small coefficients"))).collect()
+        };
+        let (rw, ew) = (to32(rs), to32(es));
+        let mut a = vec![0i64; a_bars.len() * (k + 2) * n];
+        let st = unsafe {
+            qf_ring_trap_gen_batch_from(self.ctx.raw, a_bars.len() as i64, abw.as_ptr(), rw.as_ptr(), ew.as_ptr(), a.as_mut_ptr())
+        };
+        self.ctx.check(st, "qf_ring_trap_gen_batch_from");
+        a.chunks((k + 2) * n)
+            .map(|key| {
+                let mut am = MatPolyOverZ::new(1, (k + 2) as i64);
+                for j in 0..k + 2 {
+                    let mut poly = PolyOverZ::default();
+                    for t in 0..n {
+                        if key[j * n + t] != 0 {
+                            poly.set_coeff(t as i64, Z::from(key[j * n + t])).unwrap();
+                        }
+                    }
+                    am.set_entry(0, j as i64, &poly).unwrap();
+                }
+                MatPolynomialRingZq::from((&am, &self.inner.gp.modulus))
+            })
+            .collect()
     }
 }
 

@@ -67,6 +67,10 @@ SIGNATURES = {
     "qf_check_domain": (_i32, [_vp, _vp, _i64, _vp]),
     "qf_f_a_tagged": (_i32, [_vp, _vp, _vp, _i64, _vp, _vp]),
     "qf_f_a_tagged_dev": (_i32, [_vp, _vp, _vp, _i64, _vp, _vp]),
+    "qf_ring_set_key_table": (_i32, [_vp, _vp, _i64]),
+    "qf_ring_f_a_keyed": (_i32, [_vp, _vp, _vp, _i64, _vp, _vp]),
+    "qf_ring_f_a_keyed_dev": (_i32, [_vp, _vp, _vp, _i64, _vp, _vp]),
+    "qf_ring_trap_gen_batch_from": (_i32, [_vp, _i64, _vp, _vp, _vp, _vp]),
     "qf_samp_d": (_i32, [_vp, _i64, _u64, _u64, _vp]),
     "qf_samp_d_dev": (_i32, [_vp, _i64, _u64, _u64, _vp]),
     "qf_samp_p": (_i32, [_vp, _vp, _i64, _u64, _u64, _vp]),

@@ -35,6 +35,10 @@ struct Dev {
         if (e == cudaSuccess) cap = bytes;
         return e;
     }
+    void swap(Dev& o) {
+        std::swap(p, o.p);
+        std::swap(cap, o.cap);
+    }
     void release() {
         if (p) cudaFree(p);
         p = nullptr;
@@ -131,6 +135,14 @@ struct qf_ctx {
     int ring_limbs = 0;
     Dev dRotl;
     std::vector<int64_t> hAring;
+    // ring key table (qf_ring_set_key_table, DESIGN 4.13): key_count keys of (k+2) polynomials, independent of the installed
+    // key.  key_family 2: ring_small transforms (uint32, d = key_d, np^-1 = key_np_inv, tables in dKeyTw); 1: Goldilocks
+    // transforms (uint64, tables in dKeyTw); 0: the raw residues (int64, schoolbook).  dKeyIdx: key indices of the host
+    // path's chunks.
+    int64_t key_count = 0;
+    int key_family = 0, key_d = 1;
+    uint32_t key_np_inv = 0;
+    Dev dKeyTab, dKeyTw, dKeyIdx;
     // workspace
     Dev w[12];  // (w[10]: digit planes of the particular solution)
     Dev dNorm, dFlag, dRetry, io_a, io_b, io_b2, io_c, io_a2, io_h[2];
@@ -317,6 +329,7 @@ qf_status check_flag(qf_ctx* ctx) {
         if (h & 32) return ctx->fail(QF_ERR_INVALID, "target entry outside [0,q)");
         if (h & 64) return ctx->fail(QF_ERR_NUMERIC, "a Domain entry does not fit int16: use the int32 entry point");
         if (h & QF_FLAG_TAG_INDEX) return ctx->fail(QF_ERR_INVALID, "tag index outside the installed tag table");
+        if (h & QF_FLAG_KEY_INDEX) return ctx->fail(QF_ERR_INVALID, "key index outside the installed ring key table");
         char buf[128];
         snprintf(buf, sizeof buf, "internal range check tripped (flag=%d): a value left its exact-integer range", h);
         return ctx->fail(QF_ERR_NUMERIC, buf);
@@ -626,6 +639,85 @@ qf_status ring_f_a_chunk(qf_ctx* ctx, const int32_t* dSigma, int Bc, int64_t* dU
                                              Bc, npoly, (int)ctx->n, ctx->prm.q, ctx->stream));
     if (dFlags)
         LAUNCH(qf_launch_domain_flags(ctx->dNorm.as<unsigned long long>(), ctx->bound, dFlags, Bc, ctx->stream));
+    return QF_OK;
+}
+
+// Family of the NTT kernels for a ring key table (qf_ring_set_key_table) or a batch of ring TrapGen products, by the rules
+// of qf_ring_set_a: ring_small (2) for word-size NTT-friendly primes unless QF_DISABLE_SMALL_NTT=1, else Goldilocks (1)
+// when n is a power of two in [64, 2048] and npoly n (q/2) max|sigma| < 2^63, else schoolbook (0).  Never the dense path.
+int ring_key_family(unsigned long long q, long n, long npoly, double max_abs, int* d, std::vector<uint32_t>* tables,
+                    uint32_t* np_inv) {
+    const char* env = getenv("QF_DISABLE_SMALL_NTT");
+    if (!(env && env[0] == '1') && qf_ring_small_plan(q, (int)n, d, tables, np_inv) != 0) return 2;
+    if (n >= 64 && (n & (n - 1)) == 0 && n <= 2048 && (double)npoly * (double)n * ((double)q / 2) * max_abs < 9.0e18) return 1;
+    return 0;
+}
+
+// Build the transforms of npolys key polynomials (raw residues, host) into tab (device) for a family, in slices of at
+// most 2^16 polynomials through the staging buffer stage.  Family 0 copies the residues.  Enqueued on ctx->stream.
+qf_status ring_key_transform(qf_ctx* ctx, const int64_t* keys, long npolys, int family, int d, const Dev& tw, Dev& tab,
+                             Dev& stage) {
+    const long n = ctx->n;
+    const unsigned long long q = ctx->prm.q;
+    if (family == 0) {
+        CK(cudaMemcpyAsync(tab.p, keys, (size_t)npolys * n * 8, cudaMemcpyHostToDevice, ctx->stream));
+        return QF_OK;
+    }
+    const long slice = std::min<long>(npolys, 1L << 16);
+    CK(stage.ensure((size_t)slice * n * 8));
+    for (long p0 = 0; p0 < npolys; p0 += slice) {
+        const long np = std::min(slice, npolys - p0);
+        CK(cudaMemcpyAsync(stage.p, keys + p0 * n, (size_t)np * n * 8, cudaMemcpyHostToDevice, ctx->stream));
+        if (family == 2)
+            LAUNCH(qf_launch_ring_small_key(stage.as<int64_t>(), tab.as<uint32_t>() + p0 * n, np, (int)n, d, q,
+                                            tw.as<uint32_t>(), ctx->stream));
+        else
+            LAUNCH(qf_launch_ring_prepare(stage.as<int64_t>(), tab.as<uint64_t>() + p0 * n, np, (int)n, q, tw.as<uint64_t>(),
+                                          ctx->stream));
+    }
+    return QF_OK;
+}
+
+// Tables of a family (device): ring_small 3 np words, Goldilocks 2n + 1 words
+qf_status ring_key_tables(qf_ctx* ctx, int family, const std::vector<uint32_t>& small, Dev& tw) {
+    if (family == 2) {
+        CK(tw.ensure(small.size() * 4));
+        CK(cudaMemcpy(tw.p, small.data(), small.size() * 4, cudaMemcpyHostToDevice));
+    } else if (family == 1) {
+        std::vector<uint64_t> t(2 * ctx->n + 1);
+        qf_ring_make_tables((int)ctx->n, t.data());
+        CK(tw.ensure(t.size() * 8));
+        CK(cudaMemcpy(tw.p, t.data(), t.size() * 8, cudaMemcpyHostToDevice));
+    }
+    return QF_OK;
+}
+
+// Keyed ring product: out[b] = sum_j a^(t)_j sigma[b][j] mod (X^n + 1, q) for t = dKidx[b], keys of npoly polynomials
+// in tab (family, d, np_inv, tw as built by ring_key_transform); norm2 optional.
+qf_status ring_keyed_launch(qf_ctx* ctx, int family, int d, uint32_t np_inv, const Dev& tw, const Dev& tab, int64_t nkeys,
+                            const int32_t* dSigma, const int32_t* dKidx, int Bc, int npoly, int64_t* dU,
+                            unsigned long long* norm2) {
+    const int n = (int)ctx->n;
+    const unsigned long long q = ctx->prm.q;
+    int* flag = ctx->dFlag.as<int>();
+    if (family == 2)
+        LAUNCH(qf_launch_ring_small(dSigma, tab.as<uint32_t>(), dU, norm2, Bc, npoly, n, d, q, np_inv, tw.as<uint32_t>(),
+                                    ctx->stream, dKidx, (int)nkeys, flag));
+    else if (family == 1)
+        LAUNCH(qf_launch_ring_f_a(dSigma, tab.as<uint64_t>(), dU, norm2, Bc, npoly, n, q, tw.as<uint64_t>(), ctx->stream, dKidx,
+                                  (int)nkeys, flag));
+    else
+        LAUNCH(qf_launch_ring_f_a_schoolbook(dSigma, tab.as<int64_t>(), dU, norm2, Bc, npoly, n, q, ctx->stream, dKidx,
+                                             (int)nkeys, flag));
+    return QF_OK;
+}
+
+// ring f_a with a key per target (qf_ring_f_a_keyed): one keyed NTT-family launch, then the domain flags
+qf_status ring_f_a_keyed_chunk(qf_ctx* ctx, const int32_t* dSigma, const int32_t* dKidx, int Bc, int64_t* dU, uint8_t* dFlags) {
+    CK(ctx->dNorm.ensure((size_t)std::max<int64_t>(ctx->chunk, Bc) * 8));
+    QF_TRY(ring_keyed_launch(ctx, ctx->key_family, ctx->key_d, ctx->key_np_inv, ctx->dKeyTw, ctx->dKeyTab, ctx->key_count,
+                             dSigma, dKidx, Bc, (int)(ctx->k + 2), dU, ctx->dNorm.as<unsigned long long>()));
+    LAUNCH(qf_launch_domain_flags(ctx->dNorm.as<unsigned long long>(), ctx->bound, dFlags, Bc, ctx->stream));
     return QF_OK;
 }
 
@@ -3474,6 +3566,167 @@ qf_status qf_f_a_tagged_dev(qf_ctx* ctx, const int32_t* sigma, const int32_t* ta
     return f_a_dev_chunks(ctx, batch, [&](int64_t b0, int Bc) {
         return f_a_tagged_chunk(ctx, sigma + b0 * ctx->dim, tag_idx + b0, Bc, u_out + b0 * ctx->n, in_domain + b0);
     });
+}
+
+// ---- ring f_a with a key per target (DESIGN 4.13) ---------------------------------------------------------------------
+qf_status qf_ring_set_key_table(qf_ctx* ctx, const int64_t* keys, int64_t nkeys) {
+    if (!ctx) return QF_ERR_INVALID;
+    if (ctx->prm.kind != QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "ring key table: not a ring context");
+    if (!keys || nkeys < 1 || nkeys >= 0x7fffffffLL) return ctx->fail(QF_ERR_INVALID, "ring key table: keys == NULL or nkeys outside [1, 2^31 - 1)");
+    CK(cudaSetDevice(ctx->device));
+    const long n = ctx->n, np = ctx->k + 2, per = n * np;
+    const unsigned long long q = ctx->prm.q;
+    for (int64_t t = 0; t < nkeys; ++t) {
+        const int64_t* a = keys + t * per;
+        bool bad = false;
+        for (long i = 0; i < per; ++i) bad |= (uint64_t)a[i] >= q;  // negatives wrap to >= q
+        if (bad) {
+            char buf[128];
+            snprintf(buf, sizeof buf, "ring key table: key %lld has a coefficient outside [0,q)", (long long)t);
+            return ctx->fail(QF_ERR_INVALID, buf);
+        }
+    }
+    std::vector<uint32_t> small;
+    int d = 1;
+    uint32_t np_inv = 0;
+    const int family = ring_key_family(q, n, np, std::sqrt((double)ctx->bound), &d, &small, &np_inv);
+    const long npolys = (long)nkeys * np;
+    if (family == 1 && npolys > 0x7fffffffL) return ctx->fail(QF_ERR_UNSUPPORTED, "ring key table: more than 2^31 - 1 polynomials");
+    // the new table is built beside the old one, which stays installed until the build has finished
+    Dev tab, tw, stage;
+    {
+        cudaError_t e = tab.ensure((size_t)npolys * n * (family == 2 ? 4 : 8));
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            return ctx->fail(QF_ERR_CUDA, std::string("ring key table does not fit in device memory: ") + cudaGetErrorString(e));
+        }
+    }
+    QF_TRY(ring_key_tables(ctx, family, small, tw));
+    QF_TRY(ring_key_transform(ctx, keys, npolys, family, d, tw, tab, stage));
+    CK(cudaStreamSynchronize(ctx->stream));
+    ctx->dKeyTab.swap(tab);
+    ctx->dKeyTw.swap(tw);
+    ctx->key_count = nkeys;
+    ctx->key_family = family;
+    ctx->key_d = d;
+    ctx->key_np_inv = np_inv;
+    return QF_OK;
+}
+
+static qf_status ring_keyed_ready(qf_ctx* ctx) {
+    if (ctx->prm.kind != QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "ring f_a with a key per target: not a ring context");
+    if (!ctx->key_count) return ctx->fail(QF_ERR_NO_KEY, "no ring key table installed (qf_ring_set_key_table)");
+    return QF_OK;
+}
+
+qf_status qf_ring_f_a_keyed(qf_ctx* ctx, const int32_t* sigma, const int32_t* key_idx, int64_t batch, int64_t* u_out,
+                            uint8_t* in_domain) {
+    if (!ctx || batch < 0 || (batch > 0 && (!sigma || !key_idx || !u_out))) return QF_ERR_INVALID;
+    if (ctx->prm.kind != QF_PSF_GPV_RING) return ring_keyed_ready(ctx);
+    if (batch == 0) return QF_OK;
+    CK(cudaSetDevice(ctx->device));
+    QF_TRY(ring_keyed_ready(ctx));
+    for (int64_t b = 0; b < batch; ++b)
+        if (key_idx[b] < 0 || key_idx[b] >= ctx->key_count) {
+            char buf[128];
+            snprintf(buf, sizeof buf, "key index outside the installed ring key table (target %lld: %d)", (long long)b,
+                     (int)key_idx[b]);
+            return ctx->fail(QF_ERR_INVALID, buf);
+        }
+    const long C = ctx->chunk;
+    CK(ctx->io_a.ensure((size_t)C * ctx->dim * 4));
+    CK(ctx->io_b.ensure((size_t)C * ctx->n * 8));
+    CK(ctx->io_c.ensure((size_t)C));
+    CK(ctx->dKeyIdx.ensure((size_t)C * 4));
+    std::vector<uint8_t> flags((size_t)batch);
+    QF_TRY(for_chunks(ctx, batch, [&](int64_t b0, int Bc) -> qf_status {
+        CK(cudaMemcpyAsync(ctx->io_a.p, sigma + b0 * ctx->dim, (size_t)Bc * ctx->dim * 4, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(ctx->dKeyIdx.p, key_idx + b0, (size_t)Bc * 4, cudaMemcpyHostToDevice, ctx->stream));
+        QF_TRY(ring_f_a_keyed_chunk(ctx, ctx->io_a.as<int32_t>(), ctx->dKeyIdx.as<int32_t>(), Bc, ctx->io_b.as<int64_t>(),
+                                    ctx->io_c.as<uint8_t>()));
+        CK(cudaMemcpyAsync(u_out + b0 * ctx->n, ctx->io_b.p, (size_t)Bc * ctx->n * 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(flags.data() + b0, ctx->io_c.p, (size_t)Bc, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        return QF_OK;
+    }));
+    bool all = true;
+    for (int64_t b = 0; b < batch; ++b) all = all && flags[b];
+    if (in_domain) memcpy(in_domain, flags.data(), (size_t)batch);
+    if (!all) return ctx->fail(QF_ERR_NOT_IN_DOMAIN, "f_a: sigma not in the domain D_n (check_domain failed)");
+    return QF_OK;
+}
+
+qf_status qf_ring_f_a_keyed_dev(qf_ctx* ctx, const int32_t* sigma, const int32_t* key_idx, int64_t batch, int64_t* u_out,
+                                uint8_t* in_domain) {
+    if (!ctx || batch < 0 || (batch > 0 && (!sigma || !key_idx || !u_out || !in_domain))) return QF_ERR_INVALID;
+    if (ctx->prm.kind != QF_PSF_GPV_RING) return ring_keyed_ready(ctx);
+    if (batch == 0) return QF_OK;
+    CK(cudaSetDevice(ctx->device));
+    QF_TRY(ring_keyed_ready(ctx));
+    return for_chunks(ctx, batch, [&](int64_t b0, int Bc) {
+        return ring_f_a_keyed_chunk(ctx, sigma + b0 * ctx->dim, key_idx + b0, Bc, u_out + b0 * ctx->n, in_domain + b0);
+    });
+}
+
+qf_status qf_ring_trap_gen_batch_from(qf_ctx* ctx, int64_t count, const int64_t* a_bar, const int32_t* r, const int32_t* e,
+                                      int64_t* a_out) {
+    if (!ctx) return QF_ERR_INVALID;
+    if (ctx->prm.kind != QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "not a ring context");
+    if (count < 1 || count >= 0x7fffffffLL || !a_bar || !r || !e || !a_out)
+        return ctx->fail(QF_ERR_INVALID, "ring TrapGen batch: count outside [1, 2^31 - 1) or a NULL pointer");
+    const long n = ctx->n, k = ctx->k;
+    const unsigned long long q = ctx->prm.q;
+    if ((long long)count * k > 0x7fffffffLL) return ctx->fail(QF_ERR_INVALID, "ring TrapGen batch: count k >= 2^31");
+    CK(cudaSetDevice(ctx->device));
+    for (int64_t i = 0; i < count * n; ++i)
+        if ((uint64_t)a_bar[i] >= q) {
+            char buf[128];
+            snprintf(buf, sizeof buf, "ring TrapGen batch: a_bar of key %lld has a coefficient outside [0,q)", (long long)(i / n));
+            return ctx->fail(QF_ERR_INVALID, buf);
+        }
+    double rmax = 1;
+    for (int64_t i = 0; i < count * k * n; ++i) rmax = std::max(rmax, std::fabs((double)r[i]));
+    // a_bar_t r_{t,j}: a keyed ring product with one polynomial per key, B = count k rows, row t k + j -> key t
+    std::vector<uint32_t> small;
+    int d = 1;
+    uint32_t np_inv = 0;
+    const int family = ring_key_family(q, n, 1, rmax, &d, &small, &np_inv);
+    const int B = (int)(count * k);
+    Dev tab, tw, stage, dR, dE, dIdx, dAr, dAbar, dG, dOut;
+    CK(tab.ensure((size_t)count * n * (family == 2 ? 4 : 8)));
+    QF_TRY(ring_key_tables(ctx, family, small, tw));
+    QF_TRY(ring_key_transform(ctx, a_bar, (long)count, family, d, tw, tab, stage));
+    CK(dR.ensure((size_t)B * n * 4));
+    CK(cudaMemcpyAsync(dR.p, r, (size_t)B * n * 4, cudaMemcpyHostToDevice, ctx->stream));
+    {
+        std::vector<int32_t> idx((size_t)B);
+        for (int b = 0; b < B; ++b) idx[b] = (int32_t)(b / k);
+        CK(dIdx.ensure((size_t)B * 4));
+        CK(cudaMemcpyAsync(dIdx.p, idx.data(), (size_t)B * 4, cudaMemcpyHostToDevice, ctx->stream));
+        CK(dAr.ensure((size_t)B * n * 8));
+        QF_TRY(ring_keyed_launch(ctx, family, d, np_inv, tw, tab, count, dR.as<int32_t>(), dIdx.as<int32_t>(), B, 1,
+                                 dAr.as<int64_t>(), nullptr));
+        CK(cudaStreamSynchronize(ctx->stream));  // idx leaves scope
+    }
+    // A_t = [1 | a_bar_t | g^t - (a_bar_t r_t + e_t)]   (gadget_ring.rs:74-78)
+    std::vector<uint64_t> gpow((size_t)k);
+    {
+        u128 pw = 1;
+        for (long j = 0; j < k; ++j) { gpow[j] = (uint64_t)(pw % q); pw = (pw * (uint64_t)ctx->prm.base) % q; }
+    }
+    CK(dE.ensure((size_t)B * n * 4));
+    CK(cudaMemcpyAsync(dE.p, e, (size_t)B * n * 4, cudaMemcpyHostToDevice, ctx->stream));
+    CK(dAbar.ensure((size_t)count * n * 8));
+    CK(cudaMemcpyAsync(dAbar.p, a_bar, (size_t)count * n * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(dG.ensure((size_t)k * 8));
+    CK(cudaMemcpyAsync(dG.p, gpow.data(), (size_t)k * 8, cudaMemcpyHostToDevice, ctx->stream));
+    const size_t out_bytes = (size_t)count * (k + 2) * n * 8;
+    CK(dOut.ensure(out_bytes));
+    LAUNCH(qf_launch_ring_trap_assemble(dAbar.as<int64_t>(), dAr.as<int64_t>(), dE.as<int32_t>(), dG.as<uint64_t>(),
+                                        dOut.as<int64_t>(), (long)count, (int)k, (int)n, q, ctx->stream));
+    CK(cudaMemcpyAsync(a_out, dOut.p, out_bytes, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return QF_OK;
 }
 
 // ---- samp_d ------------------------------------------------------------------

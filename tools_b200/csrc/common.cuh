@@ -28,6 +28,8 @@
 #define QF_FLAG_DGAUSS_BAILOUT 16
 // a tag index of qf_samp_p_tagged_dev outside the installed tag table (reported by check_flag as QF_ERR_INVALID)
 #define QF_FLAG_TAG_INDEX 128
+// a key index of qf_ring_f_a_keyed_dev outside the installed ring key table (reported by check_flag as QF_ERR_INVALID)
+#define QF_FLAG_KEY_INDEX 256
 
 struct Philox {
     uint32_t k0, k1;

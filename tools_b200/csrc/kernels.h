@@ -146,16 +146,25 @@ cudaError_t qf_launch_decode_bits_u16(const uint16_t* coeffs, uint8_t* msg, size
 // a_hat: npoly x n precomputed transforms of the key polynomials (centred lift of a mod q).
 // tw: device table of 2n+1 words (psi powers bit-reversed, inverse powers, 1/n) from qf_ring_make_tables.
 void qf_ring_make_tables(int n, uint64_t* host_out);
-cudaError_t qf_launch_ring_prepare(const int64_t* a, uint64_t* a_hat, int npoly, int n, unsigned long long q,
+// one CTA per polynomial: npoly may be every polynomial of a key table (< 2^31)
+cudaError_t qf_launch_ring_prepare(const int64_t* a, uint64_t* a_hat, long npoly, int n, unsigned long long q,
                                    const uint64_t* tw, cudaStream_t stream);
 // out[b] = sum_j a_j * sigma[b][j] mod (X^n+1, q);  sigma: B x npoly x n (int32), out: B x n
+// key_idx != NULL (device, B ints): keyed form, row b uses the key a_hat + key_idx[b] npoly n of a table of nkeys keys;
+// an index outside [0, nkeys) is not used to address the table, sets *flag |= QF_FLAG_KEY_INDEX, and its row gets u = 0
+// and norm2 = ~0 (not in the domain).  The same holds for the keyed forms of the two launchers below.
 cudaError_t qf_launch_ring_f_a(const int32_t* sigma, const uint64_t* a_hat, int64_t* out, unsigned long long* norm2,
                                int B, int npoly, int n, unsigned long long q, const uint64_t* tw,
-                               cudaStream_t stream);
+                               cudaStream_t stream, const int32_t* key_idx = nullptr, int nkeys = 0, int* flag = nullptr);
 // Schoolbook fallback for degrees that are not a power of two (or < 64): a is the raw key, npoly x n in [0,q).
 cudaError_t qf_launch_ring_f_a_schoolbook(const int32_t* sigma, const int64_t* a, int64_t* out,
                                           unsigned long long* norm2, int B, int npoly, int n, unsigned long long q,
-                                          cudaStream_t stream);
+                                          cudaStream_t stream, const int32_t* key_idx = nullptr, int nkeys = 0,
+                                          int* flag = nullptr);
+// count ring TrapGen keys [1 | a_bar_t | g^t - (a_bar_t r_t + e_t)] mod q from ar = a_bar_t r_{t,j} mod q (count x k x n),
+// e (count x k x n) and gpow[j] = base^j mod q; out: count x (k+2) x n
+cudaError_t qf_launch_ring_trap_assemble(const int64_t* a_bar, const int64_t* ar, const int32_t* e, const uint64_t* gpow,
+                                         int64_t* out, long count, int k, int n, unsigned long long q, cudaStream_t stream);
 
 // ---- setup.cu (per-key, not per-target) --------------------------------------
 cudaError_t qf_launch_colnorm2(const double* G, long ld, int rows, int cols, double* d, cudaStream_t stream);
@@ -370,4 +379,8 @@ void qf_ring_small_key(const int64_t* a, int npoly, int n, int d, unsigned long 
                        uint32_t* a_hat);
 cudaError_t qf_launch_ring_small(const int32_t* sigma, const uint32_t* a_hat, int64_t* out, unsigned long long* norm2,
                                  int B, int npoly, int n, int d, unsigned long long q, uint32_t np_inv,
-                                 const uint32_t* tw, cudaStream_t stream);
+                                 const uint32_t* tw, cudaStream_t stream, const int32_t* key_idx = nullptr, int nkeys = 0,
+                                 int* flag = nullptr);
+// qf_ring_small_key on the device for npolys polynomials (one warp each): bit-identical words
+cudaError_t qf_launch_ring_small_key(const int64_t* a, uint32_t* a_hat, long npolys, int n, int d, unsigned long long q,
+                                     const uint32_t* tw, cudaStream_t stream);

@@ -107,9 +107,13 @@ __global__ void ring_prepare_kernel(const int64_t* __restrict__ a, uint64_t* __r
     for (int i = t_id; i < n; i += nh) a_hat[(long)poly * n + i] = sm[i];
 }
 
+// KEYED: target b reads the key at a_hat + key_idx[b] npoly n (a table of nkeys keys); an index outside [0, nkeys) sets
+// *flag |= QF_FLAG_KEY_INDEX and gives a zero row that is not in the domain, without reading the table.
+template <bool KEYED>
 __global__ void ring_f_a_kernel(const int32_t* __restrict__ sigma, const uint64_t* __restrict__ a_hat,
                                 int64_t* __restrict__ out, unsigned long long* __restrict__ norm2, int B, int npoly,
-                                int n, unsigned long long q, const uint64_t* __restrict__ tw) {
+                                int n, unsigned long long q, const uint64_t* __restrict__ tw,
+                                const int32_t* __restrict__ key_idx, int nkeys, int* flag) {
     extern __shared__ uint64_t sm[];
     const int PP = blockDim.y, nh = n >> 1;
     const int t_id = threadIdx.x, y = threadIdx.y;
@@ -120,6 +124,21 @@ __global__ void ring_f_a_kernel(const int32_t* __restrict__ sigma, const uint64_
     const uint64_t* psi_rev = tw;
     const uint64_t* psi_inv_rev = tw + n;
     for (int b = blockIdx.x; b < B; b += gridDim.x) {
+        const uint64_t* key = a_hat;
+        if (KEYED) {  // block-uniform branch
+            const int t = key_idx[b];
+            if (t < 0 || t >= nkeys) {
+                if (y == 0) {
+                    for (int i = t_id; i < n; i += nh) out[(long)b * n + i] = 0;
+                    if (t_id == 0) {
+                        if (flag) atomicOr(flag, QF_FLAG_KEY_INDEX);
+                        if (norm2) norm2[b] = ~0ull;
+                    }
+                }
+                continue;
+            }
+            key = a_hat + (long)t * npoly * n;
+        }
         if (t_id == 0 && y == 0) { nrm_s = 0; nrm_ovf = 0; }
         for (int i = t_id; i < n; i += nh) acc[i] = 0;
         NormAcc nrm;  // saturating squared norm (common.cuh)
@@ -140,7 +159,7 @@ __global__ void ring_f_a_kernel(const int32_t* __restrict__ sigma, const uint64_
             __syncthreads();
             ntt_forward(work, psi_rev, n, t_id, active);
             if (active) {
-                const uint64_t* ah = a_hat + (long)j * n;
+                const uint64_t* ah = key + (long)j * n;
                 for (int i = t_id; i < n; i += nh) acc[i] = gl_add(acc[i], gl_mul(work[i], ah[i]));
             }
         }
@@ -183,19 +202,35 @@ __global__ void ring_f_a_kernel(const int32_t* __restrict__ sigma, const uint64_
 }
 
 // O(n^2) fallback: thread per (target, output coefficient), 128-bit accumulation.
+// KEYED: as ring_f_a_kernel, with the raw keys at a + key_idx[b] npoly n.
+template <bool KEYED>
 __global__ void ring_schoolbook_kernel(const int32_t* __restrict__ sigma, const int64_t* __restrict__ a,
                                        int64_t* __restrict__ out, unsigned long long* __restrict__ norm2, int B,
-                                       int npoly, int n, unsigned long long q) {
+                                       int npoly, int n, unsigned long long q, const int32_t* __restrict__ key_idx,
+                                       int nkeys, int* flag) {
     long total = (long)B * n;
     for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
         long b = idx / n;
         int i = (int)(idx - b * n);
+        const int64_t* key = a;
+        if (KEYED) {
+            const int t = key_idx[b];
+            if (t < 0 || t >= nkeys) {
+                out[b * n + i] = 0;
+                if (i == 0) {
+                    if (flag) atomicOr(flag, QF_FLAG_KEY_INDEX);
+                    if (norm2) norm2[b] = ~0ull;
+                }
+                continue;
+            }
+            key = a + (long)t * npoly * n;
+        }
         __int128 acc = 0;
         NormAcc nrm;
         nrm.clear();
         for (int j = 0; j < npoly; ++j) {
             const int32_t* s = sigma + ((long)b * npoly + j) * n;
-            const int64_t* aj = a + (long)j * n;
+            const int64_t* aj = key + (long)j * n;
             for (int t = 0; t < n; ++t) {
                 // coefficient i gets a[t] * s[i-t] (t <= i) and -a[t] * s[n+i-t] (t > i)
                 long long sv = (t <= i) ? (long long)s[i - t] : -(long long)s[n + i - t];
@@ -209,16 +244,55 @@ __global__ void ring_schoolbook_kernel(const int32_t* __restrict__ sigma, const 
     }
 }
 
+// Keys of ring TrapGen (gadget_ring.rs:74-78), count at once: A_t = [1 | a_bar_t | g^t - (a_bar_t r_t + e_t)] with
+// ar = a_bar_t r_{t,j} mod q (count x k x n), e (count x k x n), gpow[j] = base^j mod q; out count x (k+2) x n.
+__global__ void ring_trap_assemble_kernel(const int64_t* __restrict__ a_bar, const int64_t* __restrict__ ar,
+                                          const int32_t* __restrict__ e, const uint64_t* __restrict__ gpow,
+                                          int64_t* __restrict__ out, long count, int k, int n, unsigned long long q) {
+    const long per = (long)(k + 2) * n, total = count * per;
+    for (long idx = (long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += (long)gridDim.x * blockDim.x) {
+        const long t = idx / per;
+        const long rem = idx - t * per;
+        const int row = (int)(rem / n), i = (int)(rem - (long)row * n);
+        unsigned long long v;
+        if (row == 0) {
+            v = (i == 0) ? 1 % q : 0;
+        } else if (row == 1) {
+            v = (unsigned long long)a_bar[t * n + i] % q;
+        } else {
+            const long src = (t * k + (row - 2)) * n + i;
+            // g_j - ar - e with ar in [0, q), |e| < 2^31: |value| < 2^63
+            long long x = (i == 0 ? (long long)gpow[row - 2] : 0) - ar[src] - (long long)e[src];
+            long long m = x % (long long)q;
+            v = (unsigned long long)(m < 0 ? m + (long long)q : m);
+        }
+        out[idx] = (int64_t)v;
+    }
+}
+
 }  // namespace
 
 cudaError_t qf_launch_ring_f_a_schoolbook(const int32_t* sigma, const int64_t* a, int64_t* out,
                                           unsigned long long* norm2, int B, int npoly, int n, unsigned long long q,
-                                          cudaStream_t stream) {
+                                          cudaStream_t stream, const int32_t* key_idx, int nkeys, int* flag) {
     if (B <= 0) return cudaSuccess;
     long long total = (long long)B * n;
     long long g = (total + 127) / 128;
     if (g > 148 * 16) g = 148 * 16;
-    ring_schoolbook_kernel<<<(int)g, 128, 0, stream>>>(sigma, a, out, norm2, B, npoly, n, q);
+    if (key_idx)
+        ring_schoolbook_kernel<true><<<(int)g, 128, 0, stream>>>(sigma, a, out, norm2, B, npoly, n, q, key_idx, nkeys, flag);
+    else
+        ring_schoolbook_kernel<false><<<(int)g, 128, 0, stream>>>(sigma, a, out, norm2, B, npoly, n, q, nullptr, 0, nullptr);
+    return cudaGetLastError();
+}
+
+cudaError_t qf_launch_ring_trap_assemble(const int64_t* a_bar, const int64_t* ar, const int32_t* e, const uint64_t* gpow,
+                                         int64_t* out, long count, int k, int n, unsigned long long q, cudaStream_t stream) {
+    if (count <= 0) return cudaSuccess;
+    long long total = (long long)count * (k + 2) * n;
+    long long g = (total + 255) / 256;
+    if (g > 148 * 16) g = 148 * 16;
+    ring_trap_assemble_kernel<<<(int)g, 256, 0, stream>>>(a_bar, ar, e, gpow, out, count, k, n, q);
     return cudaGetLastError();
 }
 
@@ -237,17 +311,18 @@ void qf_ring_make_tables(int n, uint64_t* host_out) {
     host_out[2 * n] = gl_pow_host((uint64_t)n, GP - 2);
 }
 
-cudaError_t qf_launch_ring_prepare(const int64_t* a, uint64_t* a_hat, int npoly, int n, unsigned long long q,
+cudaError_t qf_launch_ring_prepare(const int64_t* a, uint64_t* a_hat, long npoly, int n, unsigned long long q,
                                    const uint64_t* tw, cudaStream_t stream) {
     if (npoly <= 0) return cudaSuccess;
     if (n < 2 || n > 2048 || (n & (n - 1))) return cudaErrorInvalidValue;
-    ring_prepare_kernel<<<npoly, n / 2, (size_t)n * 8, stream>>>(a, a_hat, n, q, tw);
+    if (npoly > 0x7fffffffL) return cudaErrorInvalidValue;
+    ring_prepare_kernel<<<(unsigned)npoly, n / 2, (size_t)n * 8, stream>>>(a, a_hat, n, q, tw);
     return cudaGetLastError();
 }
 
 cudaError_t qf_launch_ring_f_a(const int32_t* sigma, const uint64_t* a_hat, int64_t* out, unsigned long long* norm2,
                                int B, int npoly, int n, unsigned long long q, const uint64_t* tw,
-                               cudaStream_t stream) {
+                               cudaStream_t stream, const int32_t* key_idx, int nkeys, int* flag) {
     if (B <= 0) return cudaSuccess;
     if (n < 2 || n > 2048 || (n & (n - 1))) return cudaErrorInvalidValue;
     int nh = n / 2;
@@ -257,14 +332,18 @@ cudaError_t qf_launch_ring_f_a(const int32_t* sigma, const uint64_t* a_hat, int6
     if (pp > 8) pp = 8;
     dim3 block(nh, pp);
     size_t smem = (size_t)2 * pp * n * 8;
-    static size_t configured_dev[QF_MAX_DEVICES] = {};
-    size_t& configured = configured_dev[qf_device_slot()];
+    static size_t configured_dev[QF_MAX_DEVICES][2] = {};
+    size_t& configured = configured_dev[qf_device_slot()][key_idx ? 1 : 0];
     if (smem > 48 * 1024 && smem > configured) {
-        cudaError_t e = cudaFuncSetAttribute(ring_f_a_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = key_idx ? cudaFuncSetAttribute(ring_f_a_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                                : cudaFuncSetAttribute(ring_f_a_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
         configured = smem;
     }
     int grid = B < 148 * 8 ? B : 148 * 8;
-    ring_f_a_kernel<<<grid, block, smem, stream>>>(sigma, a_hat, out, norm2, B, npoly, n, q, tw);
+    if (key_idx)
+        ring_f_a_kernel<true><<<grid, block, smem, stream>>>(sigma, a_hat, out, norm2, B, npoly, n, q, tw, key_idx, nkeys, flag);
+    else
+        ring_f_a_kernel<false><<<grid, block, smem, stream>>>(sigma, a_hat, out, norm2, B, npoly, n, q, tw, nullptr, 0, nullptr);
     return cudaGetLastError();
 }

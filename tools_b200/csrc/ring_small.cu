@@ -95,15 +95,31 @@ __device__ __forceinline__ void ntt_inv(uint32_t (&v)[EPL], const uint32_t* __re
     }
 }
 
-template <int EPL, int D>
-__global__ void __launch_bounds__(128)
+// KEYED: row b reads the key at a_hat + key_idx[b] npoly n (a table of nkeys keys); an index outside [0, nkeys) sets
+// *flag |= QF_FLAG_KEY_INDEX and gives a zero row that is not in the domain, without reading the table.  The keyed form
+// asks for 4 blocks per SM at 128-point tiles (the 3329 / n = 256 case): without that bound ptxas spills a register.
+template <int EPL, int D, bool KEYED = false>
+__global__ void __launch_bounds__(128, (KEYED && EPL * D == 8) ? 4 : 0)
 ring_small_kernel(const int32_t* __restrict__ sigma, const uint32_t* __restrict__ a_hat, int64_t* __restrict__ out,
-                  unsigned long long* __restrict__ norm2, int B, int npoly, SmallRing R, const uint32_t* __restrict__ tw) {
+                  unsigned long long* __restrict__ norm2, int B, int npoly, SmallRing R, const uint32_t* __restrict__ tw,
+                  const int32_t* __restrict__ key_idx = nullptr, int nkeys = 0, int* flag = nullptr) {
     const int lane = threadIdx.x & 31;
     const int wpb = blockDim.x >> 5;
     constexpr int NP = EPL * 32;
     const int n = NP * D;
     for (long b = (long)blockIdx.x * wpb + (threadIdx.x >> 5); b < B; b += (long)gridDim.x * wpb) {
+        int t = 0;
+        if (KEYED) {
+            t = key_idx[b];
+            if (t < 0 || t >= nkeys) {
+                for (int i = lane; i < n; i += 32) out[b * n + i] = 0;
+                if (lane == 0) {
+                    if (flag) atomicOr(flag, QF_FLAG_KEY_INDEX);
+                    if (norm2) norm2[b] = ~0ull;
+                }
+                continue;
+            }
+        }
         uint32_t acc[D][EPL];
 #pragma unroll
         for (int c = 0; c < D; ++c)
@@ -134,7 +150,9 @@ ring_small_kernel(const int32_t* __restrict__ sigma, const uint32_t* __restrict_
             }
 #pragma unroll
             for (int c = 0; c < D; ++c) ntt_fwd<EPL>(v[c], tw, lane, R);
-            const uint32_t* ah = a_hat + (long)j * n;
+            // (the largest tile re-reads its index from L1 instead of keeping it live: no spill at 255 registers)
+            const int kt = (KEYED && EPL * D == 32) ? __ldg(key_idx + b) : t;
+            const uint32_t* ah = a_hat + ((long)kt * npoly + j) * n;
 #pragma unroll
             for (int r = 0; r < EPL; ++r) {
                 const int e = r * 32 + lane;
@@ -171,6 +189,38 @@ ring_small_kernel(const int32_t* __restrict__ sigma, const uint32_t* __restrict_
             nrm.warp_reduce();
             if (lane == 0) norm2[b] = nrm.value();
         }
+    }
+}
+
+// Forward transform of npolys key polynomials on the device, one warp per polynomial: the words qf_ring_small_key writes
+// (same butterflies, exact mod q), for a table of many keys.
+template <int EPL, int D>
+__global__ void __launch_bounds__(128)
+ring_small_key_kernel(const int64_t* __restrict__ a, uint32_t* __restrict__ a_hat, long npolys, SmallRing R,
+                      const uint32_t* __restrict__ tw) {
+    const int lane = threadIdx.x & 31;
+    const int wpb = blockDim.x >> 5;
+    constexpr int NP = EPL * 32;
+    const int n = NP * D;
+    const uint32_t p32 = (uint32_t)((1ull << 32) - (unsigned long long)R.barrett * R.q);  // 2^32 mod q (q odd)
+    for (long p = (long)blockIdx.x * wpb + (threadIdx.x >> 5); p < npolys; p += (long)gridDim.x * wpb) {
+        const int64_t* src = a + p * n;
+        uint32_t v[D][EPL];
+#pragma unroll
+        for (int r = 0; r < EPL; ++r)
+#pragma unroll
+            for (int c = 0; c < D; ++c) {
+                // x mod q in 32-bit arithmetic: (hi mod q) (2^32 mod q) + (lo mod q) < q^2 <= 2^32
+                const unsigned long long x = (unsigned long long)src[D * (r * 32 + lane) + c];
+                v[c][r] = ((uint32_t)(x >> 32) % R.q * p32 + (uint32_t)x % R.q) % R.q;
+            }
+#pragma unroll
+        for (int c = 0; c < D; ++c) ntt_fwd<EPL>(v[c], tw, lane, R);
+        uint32_t* dst = a_hat + p * n;
+#pragma unroll
+        for (int r = 0; r < EPL; ++r)
+#pragma unroll
+            for (int c = 0; c < D; ++c) dst[D * (r * 32 + lane) + c] = v[c][r];
     }
 }
 
@@ -255,19 +305,29 @@ void qf_ring_small_key(const int64_t* a, int npoly, int n, int d, unsigned long 
         }
 }
 
-cudaError_t qf_launch_ring_small(const int32_t* sigma, const uint32_t* a_hat, int64_t* out, unsigned long long* norm2,
-                                 int B, int npoly, int n, int d, unsigned long long q, uint32_t np_inv,
-                                 const uint32_t* tw, cudaStream_t stream) {
-    if (B <= 0) return cudaSuccess;
+namespace {
+SmallRing small_ring(int n, int d, unsigned long long q, uint32_t np_inv) {
     SmallRing R;
     R.q = (uint32_t)q;
     R.barrett = (uint32_t)((1ull << 32) / q);
     R.n = n; R.d = d; R.np = n / d; R.np_inv = np_inv;
+    return R;
+}
+}  // namespace
+
+cudaError_t qf_launch_ring_small(const int32_t* sigma, const uint32_t* a_hat, int64_t* out, unsigned long long* norm2,
+                                 int B, int npoly, int n, int d, unsigned long long q, uint32_t np_inv,
+                                 const uint32_t* tw, cudaStream_t stream, const int32_t* key_idx, int nkeys, int* flag) {
+    if (B <= 0) return cudaSuccess;
+    const SmallRing R = small_ring(n, d, q, np_inv);
     const int wpb = 4;
     long long g = ((long long)B + wpb - 1) / wpb;
     if (g > 148 * 16) g = 148 * 16;
     const int epl = R.np / 32;
-#define QF_RS(E, DD) ring_small_kernel<E, DD><<<(int)g, 32 * wpb, 0, stream>>>(sigma, a_hat, out, norm2, B, npoly, R, tw)
+#define QF_RS(E, DD)                                                                                                    \
+    (key_idx ? ring_small_kernel<E, DD, true><<<(int)g, 32 * wpb, 0, stream>>>(sigma, a_hat, out, norm2, B, npoly, R, tw, \
+                                                                                key_idx, nkeys, flag)                  \
+             : ring_small_kernel<E, DD><<<(int)g, 32 * wpb, 0, stream>>>(sigma, a_hat, out, norm2, B, npoly, R, tw))
     if (d == 1) {
         switch (epl) {
             case 2: QF_RS(2, 1); break;
@@ -288,5 +348,37 @@ cudaError_t qf_launch_ring_small(const int32_t* sigma, const uint32_t* a_hat, in
         }
     }
 #undef QF_RS
+    return cudaGetLastError();
+}
+
+cudaError_t qf_launch_ring_small_key(const int64_t* a, uint32_t* a_hat, long npolys, int n, int d, unsigned long long q,
+                                     const uint32_t* tw, cudaStream_t stream) {
+    if (npolys <= 0) return cudaSuccess;
+    const SmallRing R = small_ring(n, d, q, 0);
+    const int wpb = 4;
+    long long g = ((long long)npolys + wpb - 1) / wpb;
+    if (g > 148 * 16) g = 148 * 16;
+    const int epl = R.np / 32;
+#define QF_RK(E, DD) ring_small_key_kernel<E, DD><<<(int)g, 32 * wpb, 0, stream>>>(a, a_hat, npolys, R, tw)
+    if (d == 1) {
+        switch (epl) {
+            case 2: QF_RK(2, 1); break;
+            case 4: QF_RK(4, 1); break;
+            case 8: QF_RK(8, 1); break;
+            case 16: QF_RK(16, 1); break;
+            case 32: QF_RK(32, 1); break;
+            default: return cudaErrorInvalidValue;
+        }
+    } else {
+        switch (epl) {
+            case 1: QF_RK(1, 2); break;
+            case 2: QF_RK(2, 2); break;
+            case 4: QF_RK(4, 2); break;
+            case 8: QF_RK(8, 2); break;
+            case 16: QF_RK(16, 2); break;
+            default: return cudaErrorInvalidValue;
+        }
+    }
+#undef QF_RK
     return cudaGetLastError();
 }

@@ -616,6 +616,7 @@ class PSFGPVRing(_PSFBase):
         self._domain_shape = (gp.k + 2, gp.n)
         bound = _exact_bound(s, s, gp.n * (gp.k + 2))  # gpv_ring.rs:281-282
         self._make_ctx(gp.n, gp.k, gp.k + 2, gp.base, gp.q, s, 1.0, bound, device)
+        self._keys_id = None  # the ring key table on the device (qf_ring_set_key_table); independent of the installed key
 
     def _shape_ok(self, sigma):
         # a column vector of k+2 polynomials, each given by (at most) n coefficients
@@ -677,4 +678,43 @@ class PSFGPVRing(_PSFBase):
         assert ab.shape == (gp.n,) and rr.shape == (gp.k, gp.n) and ee.shape == (gp.k, gp.n)
         self.ctx.call("qf_ring_trap_gen_from", _ffi.ptr(ab), _ffi.ptr(rr), _ffi.ptr(ee), _ffi.ptr(a))
         self._a_id, self._td_id, self._fa_tags_id = a, None, None
+        return a
+
+    def f_a_keyed_batch(self, keys, sigmas: np.ndarray, key_idx, strict: bool = True):
+        """f_a with a key per target: u[b] = f_a(keys[key_idx[b]], sigmas[b]), for batches that hold signatures of many
+        signers.  keys: T x (k+2) x n residues in [0, q) (any a_0); installed as one device table
+        (qf_ring_set_key_table) and cached by the identity of `keys`, so pass the same array again to skip the upload.
+        key_idx: B indices in [0, T).  Returns (u, in_domain) as f_a_batch does; rows in the domain equal f_a_batch with
+        that row's key, bit for bit."""
+        if self._keys_id is not keys:
+            kk = np.ascontiguousarray(keys, dtype=np.int64)
+            assert kk.ndim == 3 and kk.shape[1:] == self._domain_shape and kk.shape[0] >= 1
+            self.ctx.call("qf_ring_set_key_table", _ffi.ptr(kk), kk.shape[0])
+            self._keys_id = keys
+        s, oob = _domain_i32(sigmas, self._domain_shape)
+        ki = np.ascontiguousarray(key_idx, dtype=np.int32)
+        b = s.shape[0]
+        assert ki.shape == (b,)
+        u = np.empty((b, self.n), dtype=np.int64)
+        flags = np.empty(b, dtype=np.uint8)
+        st = self.ctx.status("qf_ring_f_a_keyed", _ffi.ptr(s), _ffi.ptr(ki), b, _ffi.ptr(u), _ffi.ptr(flags))
+        if st not in (_ffi.QF_OK, _ffi.QF_ERR_NOT_IN_DOMAIN):
+            raise QfError(st, self.ctx._lib.qf_last_error(self.ctx._h).decode())
+        ok = flags.astype(bool) & ~oob
+        if strict and not ok.all():
+            raise NotInDomain(_ffi.QF_ERR_NOT_IN_DOMAIN, "sigma is not in the domain D_n")
+        return u, ok
+
+    def gen_trapdoor_ring_lwe_batch(self, a_bars, rs, es) -> np.ndarray:
+        """gen_trapdoor_ring_lwe for T keys in one call (qf_ring_trap_gen_batch_from): a_bars T x n residues in [0, q),
+        rs and es T x k x n.  Key t equals gen_trapdoor_ring_lwe(a_bars[t], rs[t], es[t]) bit for bit; nothing is
+        installed on the context."""
+        gp = self.gp
+        ab = np.ascontiguousarray(a_bars, dtype=np.int64)
+        rr = np.ascontiguousarray(rs, dtype=np.int32)
+        ee = np.ascontiguousarray(es, dtype=np.int32)
+        t = ab.shape[0]
+        assert ab.shape == (t, gp.n) and rr.shape == (t, gp.k, gp.n) and ee.shape == (t, gp.k, gp.n)
+        a = np.empty((t, gp.k + 2, gp.n), dtype=np.int64)
+        self.ctx.call("qf_ring_trap_gen_batch_from", t, _ffi.ptr(ab), _ffi.ptr(rr), _ffi.ptr(ee), _ffi.ptr(a))
         return a
