@@ -197,7 +197,7 @@ qf_status qf_ring_set_a(qf_ctx* ctx, const int64_t* a);
 
 /* ---- TrapGen (gadget_classical.rs:56-68, gadget_ring.rs:62-81) ------------ */
 /* A = [A_bar | tag*G - A_bar*R] mod q from supplied A_bar (n x m_bar), R (m_bar x nk) and
- * tag (n x n, NULL = identity).  Bit-exact against the reference given the same inputs.
+ * tag (n x n, entries taken mod q, NULL = identity).  Bit-exact against the reference given the same inputs.
  * Writes A (n x m) and installs it as the context key. */
 qf_status qf_trap_gen_from(qf_ctx* ctx, const int64_t* a_bar, const int8_t* r, const int64_t* tag, int64_t* a_out);
 /* Samples A_bar uniform (gpv.rs:84) and R from PlusMinusOneZero (trapdoor_distribution.rs:82-86)

@@ -320,6 +320,13 @@ def test_set_tag(T):
     assert np.array_equal(a4, a1)
     e4 = tg.samp_p_batch(a4, td4, u, seed=6)
     assert np.array_equal(O.f_a_classical_batch(a4, e4, q), u)
+    # ... and so does qf_trap_gen_from itself for a tag with negative entries (h1 - q), which it takes mod q
+    # (the arrays are named: _ffi.ptr does not keep its argument alive through the call)
+    ab, r8, neg = np.ascontiguousarray(a_bar), np.ascontiguousarray(rm, dtype=np.int8), np.ascontiguousarray(h1 - q)
+    assert neg.min() < 0
+    a5 = np.empty_like(a1)
+    tg.ctx.call("qf_trap_gen_from", _ffi.ptr(ab), _ffi.ptr(r8), _ffi.ptr(neg), _ffi.ptr(a5))
+    assert np.array_equal(a5, a1)
     # refusals: a GPV context, no trapdoor, no key
     g = T.PSFGPV(gp, 90.0)
     assert g.ctx.status("qf_set_tag", None, None) == _ffi.QF_ERR_INVALID

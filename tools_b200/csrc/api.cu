@@ -26,6 +26,9 @@ typedef __int128 i128;
 struct Dev {
     void* p = nullptr;
     size_t cap = 0;
+    Dev() = default;
+    Dev(const Dev&) = delete;  // the destructor frees p: a copy would free it twice
+    Dev& operator=(const Dev&) = delete;
     cudaError_t ensure(size_t bytes) {
         if (bytes <= cap) return cudaSuccess;
         if (p) cudaFree(p);
@@ -47,6 +50,40 @@ struct Dev {
     ~Dev() { release(); }
     template <typename T>
     T* as() const { return reinterpret_cast<T*>(p); }
+};
+
+// A device tag table, one per kind on a context, built in full and then swapped in.
+// samp_p table (qf_set_tag_table[_poly]; PSFPerturbation, and PSFGPV on the two-phase recursion): H_t^-1 mod q for count
+// tags, relative to the installed (A_bar, R) and dropped with the key or trapdoor.  h0: the installed key's tag H_0 in the
+// layout of tab while a PSFPerturbation key is tagged.
+// f_a table (qf_set_f_a_tags[_poly]; PSFGPV and PSFPerturbation): D_t = H_t - H_0 mod q (matrix form) or h_t mod q (poly
+// form), relative to the installed A and dropped whenever A changes.
+struct TagTable {
+    int64_t count = 0;  // 0: no table
+    int word = 8;       // bytes of a table word: 4 when q <= 2^32
+    // matrix form: tab holds n x n words per tag, column-major.  poly form (DESIGN 4.10): n words per tag (samp_p: h_t^-1
+    // mod (f, q); f_a: h_t mod q), and xr the rows X^{n+j} mod (f, q), j < n - 1, of the product.
+    bool poly = false;
+    int h0_kind = 1;    // f_a poly form: H_0 = 0 (0), H_0 = I (1), or H_0 column-major in h0 (2)
+    Dev tab, xr;
+    Dev gpow;           // base^s mod q, s < k
+    Dev h0;
+    // f_a matrix form: hist / off / gstart of the counting sort by tag (3 (count + 1) ints), and the sorted targets of a chunk
+    Dev sort, perm;
+
+    TagTable() = default;
+    explicit TagTable(uint64_t q) : word(q <= (1ull << 32) ? 4 : 8) {}
+    void swap(TagTable& o) {
+        std::swap(count, o.count);
+        std::swap(word, o.word);
+        std::swap(poly, o.poly);
+        std::swap(h0_kind, o.h0_kind);
+        tab.swap(o.tab); xr.swap(o.xr); gpow.swap(o.gpow); h0.swap(o.h0); sort.swap(o.sort); perm.swap(o.perm);
+    }
+    void drop() {
+        TagTable none;
+        swap(none);
+    }
 };
 
 inline long pad16(long x) { return (x + 15) / 16 * 16; }
@@ -200,34 +237,13 @@ struct qf_ctx {
     int tag_ulimbs = 0;
     long ldk_n = 0;
     Dev dHinvl, dAbpl, dTagU, dTagUl, dTagTmp;
-    // Tag table of samp_p (qf_set_tag_table; PSFPerturbation, and PSFGPV on the two-phase recursion): H_t^-1 mod q for
-    // tag_count tags, each n x n column-major in words of tag_word bytes (4 when q <= 2^32), relative to the installed
-    // (A_bar, R) and dropped with the key or trapdoor.
-    // dTagH0: the installed key's tag H_0 in the same layout while the key is tagged; dTagGpow: base^s mod q, s < k;
-    // io_t: tag indices of the host path's chunks (two slots, as io_b / io_b2).
-    int64_t tag_count = 0;
-    int tag_word = 8;
-    Dev dTagTab, dTagH0, dTagGpow, io_t[2];
-    // tag_poly: dTagTab holds the tags in polynomial form instead (qf_set_tag_table_poly, DESIGN 4.10): h_t^-1 mod (f, q)
-    // as n words per tag, and dTagXr the rows X^{n+j} mod (f, q), j < n - 1, of the product.
-    bool tag_poly = false;
-    Dev dTagXr;
-    // Tag table of f_a (qf_set_f_a_tags, PSFGPV and PSFPerturbation): D_t = H_t - H_0 mod q for fa_tag_count tags, in the
-    // layout of dTagTab, relative to the installed A and dropped whenever A changes.  dFaSort: hist / off / gstart of the
-    // counting sort by tag (3 (T + 1) ints); dFaPerm: the sorted targets of a chunk.
-    int64_t fa_tag_count = 0;
-    int fa_tag_word = 8;
-    Dev dFaTab, dFaGpow, dFaSort, dFaPerm;
-    // fa_poly: dFaTab holds h_t mod q as n words per tag instead (qf_set_f_a_tags_poly), dFaXr the rows of the product mod
-    // (f, q) and dFaH0 H_0 column-major when fa_h0_kind = 2 (0: H_0 = 0, 1: H_0 = I).
-    bool fa_poly = false;
-    int fa_h0_kind = 1;
-    Dev dFaXr, dFaH0;
+    TagTable samp_tags, fa_tags;
+    Dev io_t[2];  // tag indices of the host path's chunks (two slots, as io_b / io_b2)
     // Pool of the target-independent half of samp_p (qf_samp_p_offline, DESIGN 4.12): entries pool_first ..
     // pool_first + pool_count - 1 under pool_seed, entry j in slot j - pool_first; pool_next slots are consumed.
     // PSFPerturbation: dPoolX = p (m int32), dPoolAx = -A p mod q (n words).  PSFGPV two-phase: dPoolX = z2 (m_bar int32),
     // dPoolAx = -A_bar z2 mod q, dPoolT = -V 256^mt1_dlo of the Mt_1 z2 contraction (nk fp64, unit scale: dOnes).
-    // Dropped whenever A or the trapdoor changes (drop_pool).
+    // Dropped whenever A or the trapdoor changes (a_changed, trapdoor_changed).
     bool pool = false;
     int64_t pool_count = 0, pool_next = 0;
     uint64_t pool_seed = 0, pool_first = 0;
@@ -254,6 +270,16 @@ struct qf_ctx {
         pool = false;
         pool_count = pool_next = 0;
         dPoolX.release(); dPoolAx.release(); dPoolT.release();
+    }
+    // A changed: the f_a table and the pool were relative to the old A
+    void a_changed() {
+        fa_tags.drop();
+        drop_pool();
+    }
+    // the trapdoor's (A_bar, R) changed: the samp_p table and the pool were relative to the old one
+    void trapdoor_changed() {
+        samp_tags.drop();
+        drop_pool();
     }
 };
 
@@ -831,11 +857,12 @@ qf_status pert_finish(qf_ctx* ctx, int Bc, uint64_t seed, uint64_t first, int32_
     if (dTidx) {
         // per-target tag H_t: A_t = A + [0 | (H_t - H_0) G], so v'_t = H_t^-1 (u - A_t p) = H_t^-1 (v + H_0 y) - y with
         // y = G p_bot (DESIGN 4.4): the same v' as after qf_set_tag(H_t)
+        const TagTable& t = ctx->samp_tags;
         CK(ctx->dTagU.ensure((size_t)C * ctx->n * 8));
-        LAUNCH(qf_launch_tag_syndrome(V, ctx->n, P, ldm, (int)ctx->m_bar, dTidx, (int)ctx->tag_count, ctx->dTagTab.p,
-                                      ctx->key_tagged ? ctx->dTagH0.p : nullptr, ctx->tag_word, ctx->dTagGpow.as<uint64_t>(),
+        LAUNCH(qf_launch_tag_syndrome(V, ctx->n, P, ldm, (int)ctx->m_bar, dTidx, (int)t.count, t.tab.p,
+                                      ctx->key_tagged ? t.h0.p : nullptr, t.word, t.gpow.as<uint64_t>(),
                                       ctx->prm.q, (int)ctx->n, (int)ctx->k, Bc, ctx->dTagU.as<int64_t>(), ctx->n,
-                                      ctx->dFlag.as<int>(), ctx->stream, ctx->tag_poly ? ctx->dTagXr.p : nullptr));
+                                      ctx->dFlag.as<int>(), ctx->stream, t.poly ? t.xr.p : nullptr));
         Vg = ctx->dTagU.as<int64_t>();
     } else if (ctx->key_tagged) {
         QF_TRY(tag_targets(ctx, V, Bc, &Vg));
@@ -1347,9 +1374,10 @@ qf_status np2_finish(qf_ctx* ctx, const int64_t* H, int Bc, uint64_t seed, uint6
 // Per-target tag (dTidx): h_t = H_t^-1 w for w = u - A_bar z2 in dTagU (any installed tag), written to H (w[0])
 qf_status np2_tag_syndrome(qf_ctx* ctx, const int32_t* dTidx, int Bc) {
     const long n = ctx->n;
-    LAUNCH(qf_launch_tag_syndrome(ctx->dTagU.as<int64_t>(), n, nullptr, 0, 0, dTidx, (int)ctx->tag_count, ctx->dTagTab.p,
-                                  nullptr, ctx->tag_word, nullptr, ctx->prm.q, (int)n, (int)ctx->k, Bc, ctx->w[0].as<int64_t>(), n,
-                                  ctx->dFlag.as<int>(), ctx->stream, ctx->tag_poly ? ctx->dTagXr.p : nullptr));
+    const TagTable& t = ctx->samp_tags;
+    LAUNCH(qf_launch_tag_syndrome(ctx->dTagU.as<int64_t>(), n, nullptr, 0, 0, dTidx, (int)t.count, t.tab.p, nullptr, t.word,
+                                  nullptr, ctx->prm.q, (int)n, (int)ctx->k, Bc, ctx->w[0].as<int64_t>(), n,
+                                  ctx->dFlag.as<int>(), ctx->stream, t.poly ? t.xr.p : nullptr));
     return QF_OK;
 }
 
@@ -1658,6 +1686,31 @@ qf_status gso_device(qf_ctx* ctx, const double* dS, double* dG) {
     return QF_OK;
 }
 
+// caller words as residues mod q, as MatZq takes them: -1 becomes q - 1
+std::vector<uint64_t> residues(const int64_t* v, size_t count, uint64_t q) {
+    std::vector<uint64_t> r(count);
+    for (size_t i = 0; i < count; ++i) {
+        const int64_t x = v[i] % (int64_t)q;
+        r[i] = (uint64_t)(x < 0 ? x + (int64_t)q : x);
+    }
+    return r;
+}
+
+// an n x n tag (NULL: I) as residues mod q into h; true when H = I
+bool tag_residues(const qf_ctx* ctx, const int64_t* tag, std::vector<uint64_t>& h) {
+    const long n = ctx->n;
+    if (tag) {
+        h = residues(tag, (size_t)n * n, ctx->prm.q);
+    } else {
+        h.assign((size_t)n * n, 0);
+        for (long i = 0; i < n; ++i) h[(size_t)i * n + i] = 1;
+    }
+    for (long i = 0; i < n; ++i)
+        for (long j = 0; j < n; ++j)
+            if (h[(size_t)i * n + j] != (i == j ? 1u : 0u)) return false;
+    return true;
+}
+
 // H^-1 mod q on the device (qf_launch_mat_inverse_mod) for the n x n residues h; *ok = false when some column has no
 // unit pivot (first row at or below the diagonal whose entry is a unit mod q), and hinv is then left empty
 qf_status tag_inverse(qf_ctx* ctx, const uint64_t* h, std::vector<int64_t>& hinv, bool* ok) {
@@ -1736,6 +1789,151 @@ std::vector<uint64_t> gadget_powers(const qf_ctx* ctx) {
     u128 pwt = 1;
     for (long t = 0; t < ctx->k; ++t) { gpow[t] = (uint64_t)(pwt % ctx->prm.q); pwt = pwt * (uint64_t)ctx->prm.base % ctx->prm.q; }
     return gpow;
+}
+
+// A = [A_bar | H G - A_bar R] (n x m, host) for the key's tag H becomes A + [0 | (H' - H) G] mod q for the tag residues h2
+void add_tag_change(const qf_ctx* ctx, const std::vector<uint64_t>& h2, std::vector<int64_t>& a) {
+    const long n = ctx->n, k = ctx->k, mb = ctx->m_bar, m = ctx->m;
+    const uint64_t q = ctx->prm.q;
+    const std::vector<uint64_t> gpow = gadget_powers(ctx);
+    for (long i = 0; i < n; ++i)
+        for (long j = 0; j < n; ++j) {
+            const uint64_t d = (h2[(size_t)i * n + j] + q - ctx->key_tag[(size_t)i * n + j]) % q;
+            if (!d) continue;
+            for (long t = 0; t < k; ++t) {
+                int64_t& x = a[(size_t)i * m + mb + j * k + t];
+                x = (int64_t)(((u128)(uint64_t)x + mulmod_h(d, gpow[t], q)) % q);
+            }
+        }
+}
+
+// S_k (gadget_classical.rs:248-272), k x k: base on the diagonal, -1 below it and, unless base^k = q (*exact_pow; then S' is
+// I (x) S_k with its columns reversed, short_basis_classical.rs:80-82), the base-b digits of q in the last column.  False
+// when base^k < q.
+bool gadget_sk(const qf_ctx* ctx, std::vector<int64_t>& sk, bool* exact_pow) {
+    const long k = ctx->k;
+    const uint64_t q = ctx->prm.q, base = (uint64_t)ctx->prm.base;
+    u128 pw = 1;
+    for (long i = 0; i < k; ++i) pw *= base;
+    if (pw < q) return false;
+    *exact_pow = pw == (u128)q;
+    sk.assign((size_t)k * k, 0);
+    for (long j = 0; j < k; ++j) sk[j * k + j] = (int64_t)base;
+    for (long i = 0; i + 1 < k; ++i) sk[(i + 1) * k + i] = -1;
+    if (!*exact_pow) {
+        uint64_t qq = q;
+        for (long i = 0; i < k; ++i) { sk[i * k + (k - 1)] = (int64_t)(qq % base); qq /= base; }
+    }
+    return true;
+}
+
+// W = base-b digits of -A_bar' mod q (short_basis_classical.rs:105-110), nk x m_bar: W[j k + t][c] = digit t of
+// (q - A_bar'[j][c]) mod q, for A_bar' given transposed (abt, m_bar x n, tag_abar) or, for abt == NULL, the first m_bar
+// columns of the installed A
+std::vector<int64_t> w_digits(const qf_ctx* ctx, const std::vector<int64_t>* abt) {
+    const long n = ctx->n, k = ctx->k, mb = ctx->m_bar, m = ctx->m;
+    const uint64_t q = ctx->prm.q, base = (uint64_t)ctx->prm.base;
+    std::vector<int64_t> w((size_t)n * k * mb);
+    for (long j = 0; j < n; ++j)
+        for (long c = 0; c < mb; ++c) {
+            uint64_t v = (q - (uint64_t)(abt ? (*abt)[(size_t)c * n + j] : ctx->hA[(size_t)j * m + c])) % q;
+            for (long t = 0; t < k; ++t) {
+                w[(size_t)(j * k + t) * mb + c] = (int64_t)(v % base);
+                v /= base;
+            }
+        }
+    return w;
+}
+
+// R W (m_bar x m_bar, exact int32) on the tensor cores for R (m_bar x nk, one s8 plane, left in dRl) and the digits W
+// (nk x m_bar, w_digits)
+qf_status r_times_w(qf_ctx* ctx, const int8_t* r, const std::vector<int64_t>& w, Dev& dRl, std::vector<int32_t>& rw) {
+    const long mb = ctx->m_bar, nk = ctx->nk, ldk = ctx->ldk_nk;
+    std::vector<int64_t> r64((size_t)mb * nk), wt((size_t)mb * nk);
+    for (size_t i = 0; i < r64.size(); ++i) r64[i] = r[i];
+    for (long row = 0; row < nk; ++row)
+        for (long c = 0; c < mb; ++c) wt[(size_t)c * nk + row] = w[(size_t)row * mb + c];
+    Dev dWt, dOut;
+    QF_TRY(upload_limbs(ctx, r64.data(), mb, nk, ldk, 1, true, dRl));
+    QF_TRY(upload_limbs(ctx, wt.data(), mb, nk, ldk, 1, false, dWt));
+    CK(dOut.ensure((size_t)mb * mb * 4));
+    I8GemmArgs g{};
+    g.x = dRl.as<int8_t>(); g.ldx = ldk; g.x_plane = mb * ldk;
+    g.w = dWt.p; g.ldw = ldk; g.w_plane = mb * ldk;
+    g.LX = 1; g.LW = 1; g.w_signed = 0;
+    g.B = (int)mb; g.N = (int)mb; g.K = (int)nk;
+    g.out_kind = 1; g.sign = 1; g.q = 0; g.out = dOut.p; g.ldout = mb;
+    g.flag = ctx->dFlag.as<int>();
+    LAUNCH(ctx_gemm_i8(ctx, g));
+    rw.resize((size_t)mb * mb);
+    CK(cudaMemcpyAsync(rw.data(), dOut.p, rw.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return QF_OK;
+}
+
+// the key operand of u' = H^-1 u beside dHinvl: A_bar' = H^-1 A_bar (given transposed, tag_abar) as u8 digit planes
+qf_status install_abar(qf_ctx* ctx, const std::vector<int64_t>& abt) {
+    const long n = ctx->n, mb = ctx->m_bar;
+    std::vector<int64_t> ab((size_t)n * mb);
+    for (long i = 0; i < n; ++i)
+        for (long c = 0; c < mb; ++c) ab[(size_t)i * mb + c] = abt[(size_t)c * n + i];
+    QF_TRY(upload_limbs(ctx, ab.data(), n, mb, ctx->ldk_mb, ctx->a_limbs, false, ctx->dAbpl));
+    ctx->tag_ulimbs = limbs_for((double)(ctx->prm.q - 1));
+    return QF_OK;
+}
+
+// The short basis S = [[R S', I + R W], [S', W]] (m x m) of A = [A_bar | H G - A_bar R] for R (m_bar x nk) and A_bar' =
+// H^-1 A_bar given transposed (abt, tag_abar; NULL: H = I).  Needs base <= 256 and base^k >= q.
+qf_status short_basis(qf_ctx* ctx, const int8_t* r, const std::vector<int64_t>* abt, int64_t* s_out) {
+    const long k = ctx->k, mb = ctx->m_bar, nk = ctx->nk, m = ctx->m;
+    std::vector<int64_t> sk;
+    bool exact_pow = false;
+    gadget_sk(ctx, sk, &exact_pow);
+    // column c of S' = column (exact_pow ? nk-1-c : c) of I_n (x) S_k
+    auto sprime = [&](long row, long c) -> int64_t {
+        const long cc = exact_pow ? nk - 1 - c : c;
+        return (row / k == cc / k) ? sk[(row % k) * k + (cc % k)] : 0;
+    };
+    std::fill(s_out, s_out + (size_t)m * m, (int64_t)0);
+    // bottom-left S', top-left R S' (each column of S' has at most k non-zeros, all inside one k-block)
+    for (long c = 0; c < nk; ++c) {
+        const long cc = exact_pow ? nk - 1 - c : c, blk = cc / k;
+        for (long t = 0; t < k; ++t) {
+            const long row = blk * k + t;
+            const int64_t v = sprime(row, c);
+            if (!v) continue;
+            s_out[(size_t)(mb + row) * m + c] = v;
+            for (long i = 0; i < mb; ++i) s_out[(size_t)i * m + c] += (int64_t)r[i * nk + row] * v;
+        }
+    }
+    // bottom-right W, top-right I + R W
+    const std::vector<int64_t> w = w_digits(ctx, abt);
+    for (long row = 0; row < nk; ++row)
+        for (long c = 0; c < mb; ++c) s_out[(size_t)(mb + row) * m + nk + c] = w[(size_t)row * mb + c];
+    Dev dRl;
+    std::vector<int32_t> rw;
+    QF_TRY(r_times_w(ctx, r, w, dRl, rw));
+    for (long i = 0; i < mb; ++i)
+        for (long c = 0; c < mb; ++c) s_out[(size_t)i * m + nk + c] = (int64_t)rw[(size_t)i * mb + c] + (i == c ? 1 : 0);
+    return check_flag(ctx);
+}
+
+// an n x n matrix of residues (row-major, host) into dst column-major in words of `word` bytes: H_0 of a tag table
+qf_status upload_h0_words(qf_ctx* ctx, const std::vector<uint64_t>& h, int word, Dev& dst) {
+    const long n = ctx->n;
+    std::vector<uint64_t> ht((size_t)n * n);
+    std::vector<uint32_t> ht32;
+    for (long i = 0; i < n; ++i)
+        for (long j = 0; j < n; ++j) ht[(size_t)j * n + i] = h[(size_t)i * n + j];
+    const void* src = ht.data();
+    if (word == 4) {
+        ht32.assign(ht.begin(), ht.end());
+        src = ht32.data();
+    }
+    CK(dst.ensure((size_t)n * n * word));
+    CK(cudaMemcpyAsync(dst.p, src, (size_t)n * n * word, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return QF_OK;
 }
 
 // Form of the installed key A for a trapdoor R (m_bar x nk): a G-trapdoor A = [A_bar | H G - A_bar R] (gadget_classical.rs:56-68)
@@ -1820,17 +2018,9 @@ qf_status detect_gpv_structure(qf_ctx* ctx, const int64_t* s, const std::vector<
     const long n = ctx->n, k = ctx->k, mb = ctx->m_bar, nk = ctx->nk, m = ctx->m;
     const uint64_t q = ctx->prm.q, base = (uint64_t)ctx->prm.base;
     if (nk % 128 != 0 || mb < nk || base > 256) return QF_OK;  // plane offsets / zero-tile map need 128-column alignment
-    u128 pw = 1;
-    for (long i = 0; i < k; ++i) pw *= base;
-    if (pw < q) return QF_OK;
-    const bool exact_pow = pw == (u128)q;
-    std::vector<int64_t> sk((size_t)k * k, 0), qd(k, 0);
-    for (long j = 0; j < k; ++j) sk[j * k + j] = (int64_t)base;
-    for (long i = 0; i + 1 < k; ++i) sk[(i + 1) * k + i] = -1;
-    if (!exact_pow) {
-        uint64_t qq = q;
-        for (long i = 0; i < k; ++i) { qd[i] = (int64_t)(qq % base); sk[i * k + (k - 1)] = qd[i]; qq /= base; }
-    }
+    std::vector<int64_t> sk;
+    bool exact_pow = false;
+    if (!gadget_sk(ctx, sk, &exact_pow)) return QF_OK;
     auto colmap = [&](long cc) { return exact_pow ? nk - 1 - cc : cc; };  // column of I (x) S_k -> column of S'
     // bottom-left block must be S', bottom-right block W must hold base-b digits
     for (long row = 0; row < nk; ++row) {
@@ -1864,7 +2054,7 @@ qf_status detect_gpv_structure(qf_ctx* ctx, const int64_t* s, const std::vector<
                 P[0] = 0;
                 for (long t = 0; t + 1 < k; ++t) P[t + 1] = (i128)base * P[t] + Y(t);
                 i128 acc = Y(k - 1);
-                for (long t = 0; t < k; ++t) acc += (i128)qd[t] * P[t];
+                for (long t = 0; t < k; ++t) acc += (i128)sk[t * k + (k - 1)] * P[t];  // the digits of q
                 if (acc % (i128)q) return QF_OK;
                 const i128 x0 = acc / (i128)q;
                 i128 pwt = 1;
@@ -1877,33 +2067,12 @@ qf_status detect_gpv_structure(qf_ctx* ctx, const int64_t* s, const std::vector<
         }
     }
     // top-right block must be I + R W: the product on the tensor cores, compared exactly
-    const long ldk = ctx->ldk_nk;
     ctx->ldk_mb = (mb + 127) / 128 * 128;
-    std::vector<int64_t> r64((size_t)mb * nk), wt((size_t)mb * nk), w64((size_t)nk * mb);
-    for (size_t i = 0; i < r64.size(); ++i) r64[i] = R[i];
+    std::vector<int64_t> w64((size_t)nk * mb);
     for (long row = 0; row < nk; ++row)
-        for (long c = 0; c < mb; ++c) {
-            const int64_t d = s[(size_t)(mb + row) * m + nk + c];
-            wt[(size_t)c * nk + row] = d;
-            w64[(size_t)row * mb + c] = d;
-        }
-    Dev dWt, dOut;
-    QF_TRY(upload_limbs(ctx, r64.data(), mb, nk, ldk, 1, true, ctx->dRl));
-    QF_TRY(upload_limbs(ctx, wt.data(), mb, nk, ldk, 1, false, dWt));
-    CK(dOut.ensure((size_t)mb * mb * 4));
-    {
-        I8GemmArgs g{};
-        g.x = ctx->dRl.as<int8_t>(); g.ldx = ldk; g.x_plane = mb * ldk;
-        g.w = dWt.p; g.ldw = ldk; g.w_plane = mb * ldk;
-        g.LX = 1; g.LW = 1; g.w_signed = 0;
-        g.B = (int)mb; g.N = (int)mb; g.K = (int)nk;
-        g.out_kind = 1; g.sign = 1; g.q = 0; g.out = dOut.p; g.ldout = mb;
-        g.flag = ctx->dFlag.as<int>();
-        LAUNCH(ctx_gemm_i8(ctx, g));
-    }
-    std::vector<int32_t> rw((size_t)mb * mb);
-    CK(cudaMemcpyAsync(rw.data(), dOut.p, rw.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
+        for (long c = 0; c < mb; ++c) w64[(size_t)row * mb + c] = s[(size_t)(mb + row) * m + nk + c];
+    std::vector<int32_t> rw;
+    QF_TRY(r_times_w(ctx, R.data(), w64, ctx->dRl, rw));
     for (long i = 0; i < mb; ++i)
         for (long c = 0; c < mb; ++c)
             if (s[(size_t)i * m + nk + c] != (int64_t)rw[(size_t)i * mb + c] + (i == c ? 1 : 0)) return QF_OK;
@@ -1938,11 +2107,7 @@ qf_status detect_gpv_structure(qf_ctx* ctx, const int64_t* s, const std::vector<
                     if (gw % q != 0) { tag_ok = false; break; }
                 }
             if (tag_ok) {
-                std::vector<int64_t> ab((size_t)n * mb);
-                for (long i = 0; i < n; ++i)
-                    for (long c = 0; c < mb; ++c) ab[(size_t)i * mb + c] = abt[(size_t)c * n + i];
-                QF_TRY(upload_limbs(ctx, ab.data(), n, mb, ctx->ldk_mb, ctx->a_limbs, false, ctx->dAbpl));
-                ctx->tag_ulimbs = limbs_for((double)(q - 1));
+                QF_TRY(install_abar(ctx, abt));
                 ctx->key_tagged = true;
                 ctx->gadget_key_ok = true;
             } else {
@@ -1985,23 +2150,24 @@ qf_status f_a_dev_chunks(qf_ctx* ctx, int64_t batch, F&& run) {
 // grouped by tag on the device (no host round trip).  dTidx: device tag indices of the chunk.
 qf_status f_a_tagged_chunk(qf_ctx* ctx, const int32_t* dSigma, const int32_t* dTidx, int Bc, int64_t* dU, uint8_t* dFlags) {
     QF_TRY(f_a_chunk(ctx, dSigma, Bc, dU, dFlags));
-    const int T = (int)ctx->fa_tag_count;
-    if (ctx->fa_poly) {  // n words per tag: one CTA per target, no grouping
-        LAUNCH(qf_launch_f_a_tag_poly(dSigma, ctx->dim, (int)ctx->m_bar, dTidx, T, ctx->dFaTab.p, ctx->dFaXr.p, ctx->dFaH0.p,
-                                      ctx->fa_h0_kind, ctx->fa_tag_word, ctx->dFaGpow.as<uint64_t>(), ctx->prm.q, (int)ctx->n,
-                                      (int)ctx->k, Bc, dU, ctx->n, ctx->dFlag.as<int>(), ctx->stream));
+    TagTable& t = ctx->fa_tags;
+    const int T = (int)t.count;
+    if (t.poly) {  // n words per tag: one CTA per target, no grouping
+        LAUNCH(qf_launch_f_a_tag_poly(dSigma, ctx->dim, (int)ctx->m_bar, dTidx, T, t.tab.p, t.xr.p, t.h0.p, t.h0_kind, t.word,
+                                      t.gpow.as<uint64_t>(), ctx->prm.q, (int)ctx->n, (int)ctx->k, Bc, dU, ctx->n,
+                                      ctx->dFlag.as<int>(), ctx->stream));
         return QF_OK;
     }
-    int* hist = ctx->dFaSort.as<int>();
+    int* hist = t.sort.as<int>();
     int *off = hist + (T + 1), *gstart = off + (T + 1), *perm = nullptr;
     if (QF_F_A_TAG_GROUP > 1) {  // always in the library; 1 only in the benchmark's comparison build (kernels.h)
-        CK(ctx->dFaPerm.ensure((size_t)Bc * sizeof(int)));
-        perm = ctx->dFaPerm.as<int>();
+        CK(t.perm.ensure((size_t)Bc * sizeof(int)));
+        perm = t.perm.as<int>();
         LAUNCH(qf_launch_f_a_tag_sort(dTidx, Bc, T, hist, off, gstart, perm, ctx->dFlag.as<int>(), ctx->stream));
     }
-    LAUNCH(qf_launch_f_a_tag_correct(dSigma, ctx->dim, (int)ctx->m_bar, dTidx, T, perm, off, gstart, ctx->dFaTab.p,
-                                     ctx->fa_tag_word, ctx->dFaGpow.as<uint64_t>(), ctx->prm.q, (int)ctx->n, (int)ctx->k, Bc,
-                                     dU, ctx->n, ctx->dFlag.as<int>(), ctx->stream));
+    LAUNCH(qf_launch_f_a_tag_correct(dSigma, ctx->dim, (int)ctx->m_bar, dTidx, T, perm, off, gstart, t.tab.p, t.word,
+                                     t.gpow.as<uint64_t>(), ctx->prm.q, (int)ctx->n, (int)ctx->k, Bc, dU, ctx->n,
+                                     ctx->dFlag.as<int>(), ctx->stream));
     return QF_OK;
 }
 
@@ -2012,9 +2178,8 @@ qf_status install_a(qf_ctx* ctx, const int64_t* a) {
     ctx->has_a = false; ctx->has_np = false; ctx->has_pert = false;
     ctx->key_tagged = false; ctx->pert_gadget_key = false;
     ctx->dHinvl.release(); ctx->dAbpl.release();
-    ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release(); ctx->dTagXr.release();
-    ctx->fa_tag_count = 0; ctx->dFaTab.release(); ctx->dFaXr.release(); ctx->dFaH0.release();
-    ctx->drop_pool();
+    ctx->a_changed();
+    ctx->trapdoor_changed();
     const long n = ctx->n, m = ctx->m;
     for (long i = 0; i < n * m; ++i)
         if (a[i] < 0 || (uint64_t)a[i] >= ctx->prm.q) return ctx->fail(QF_ERR_INVALID, "A entry outside [0,q)");
@@ -2082,26 +2247,13 @@ qf_status upload_ainv(qf_ctx* ctx, const std::vector<int64_t>& ainv) {
     return upload_chunks(ctx, ainv.data(), ctx->n, ctx->n, ctx->ld_piv, nch, wb, ctx->dAinv);
 }
 
-// the installed key's tag H_0 into dTagH0 (column-major, tag_word words) for the per-target tag kernel; none for H_0 = I
-qf_status upload_tag_h0(qf_ctx* ctx) {
+// the installed key's tag H_0 into the samp_p table t for the per-target tag kernel; none for H_0 = I
+qf_status upload_tag_h0(qf_ctx* ctx, TagTable& t) {
     if (!ctx->key_tagged) {
-        ctx->dTagH0.release();
+        t.h0.release();
         return QF_OK;
     }
-    const long n = ctx->n;
-    std::vector<uint64_t> h((size_t)n * n);
-    for (long i = 0; i < n; ++i)
-        for (long j = 0; j < n; ++j) h[(size_t)j * n + i] = ctx->key_tag[(size_t)i * n + j];
-    std::vector<uint32_t> h32;
-    const void* src = h.data();
-    if (ctx->tag_word == 4) {
-        h32.assign(h.begin(), h.end());
-        src = h32.data();
-    }
-    CK(ctx->dTagH0.ensure((size_t)n * n * ctx->tag_word));
-    CK(cudaMemcpyAsync(ctx->dTagH0.p, src, (size_t)n * n * ctx->tag_word, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    return QF_OK;
+    return upload_h0_words(ctx, ctx->key_tag, t.word, t.h0);
 }
 
 // ---- tags in polynomial form (qf_set_tag_table_poly, qf_set_f_a_tags_poly)
@@ -2162,19 +2314,115 @@ bool prime_power(uint64_t q, uint64_t* p, int* e) {
     return false;
 }
 
-// f mod q on the device and the rows X^{n+j} mod (f, q) of the product (qf_launch_poly_xpow)
-qf_status poly_modulus(qf_ctx* ctx, const int64_t* f, int word, Dev& dF, Dev& xr) {
+// f mod q on the device (dF), and the table t in polynomial form with the rows X^{n+j} mod (f, q) of the product
+// (qf_launch_poly_xpow)
+qf_status poly_modulus(qf_ctx* ctx, const int64_t* f, TagTable& t, Dev& dF) {
     const long n = ctx->n;
     const uint64_t q = ctx->prm.q;
-    std::vector<uint64_t> fq((size_t)n);
-    for (long i = 0; i < n; ++i) {
-        const int64_t v = f[i] % (int64_t)q;
-        fq[i] = (uint64_t)(v < 0 ? v + (int64_t)q : v);
-    }
+    const std::vector<uint64_t> fq = residues(f, (size_t)n, q);
+    t.poly = true;
     CK(dF.ensure((size_t)n * 8));
-    CK(xr.ensure((size_t)std::max(1L, n - 1) * n * word));
+    CK(t.xr.ensure((size_t)std::max(1L, n - 1) * n * t.word));
     CK(cudaMemcpyAsync(dF.p, fq.data(), (size_t)n * 8, cudaMemcpyHostToDevice, ctx->stream));
-    LAUNCH(qf_launch_poly_xpow(dF.as<uint64_t>(), (int)n, q, word, xr.p, ctx->stream));
+    LAUNCH(qf_launch_poly_xpow(dF.as<uint64_t>(), (int)n, q, t.word, t.xr.p, ctx->stream));
+    return QF_OK;
+}
+
+qf_status samp_p_ready(qf_ctx* ctx) {
+    if (ctx->prm.kind == QF_PSF_PERTURBATION) {
+        if (!ctx->has_a || !ctx->has_pert) return ctx->fail(QF_ERR_NO_KEY, "PSFPerturbation: key or trapdoor missing");
+    } else {
+        if (!ctx->has_np) return ctx->fail(QF_ERR_NO_KEY, "GPV: trapdoor missing (qf_set_trapdoor_gpv)");
+    }
+    return QF_OK;
+}
+
+// samp_p takes a tag per target on PSFPerturbation and on PSFGPV's two-phase recursion, with key and trapdoor installed.
+// bad_args: why a table install refuses its arguments, reported after the context kind; NULL when they are fine.
+qf_status samp_tags_ready(qf_ctx* ctx, const char* bad_args) {
+    if (ctx->prm.kind == QF_PSF_GPV) QF_TRY(gpv_tags_ready(ctx));
+    else if (ctx->prm.kind != QF_PSF_PERTURBATION) return ctx->fail(QF_ERR_INVALID, "not a PSFGPV or PSFPerturbation context");
+    if (bad_args) return ctx->fail(QF_ERR_INVALID, bad_args);
+    return samp_p_ready(ctx);
+}
+
+// the checks both samp_p table installs start with: the tags are relative to a G-trapdoor key
+qf_status samp_table_ready(qf_ctx* ctx, const char* bad_args) {
+    QF_TRY(samp_tags_ready(ctx, bad_args));
+    if (ctx->prm.kind == QF_PSF_PERTURBATION && !ctx->pert_gadget_key)
+        return ctx->fail(QF_ERR_INVALID, "the installed key is not [A_bar | H G - A_bar R] for the installed R");
+    return QF_OK;
+}
+
+// f_a takes a tag per target on a classical context with its key installed; bad_args as for samp_tags_ready
+qf_status f_a_tags_ready(qf_ctx* ctx, const char* bad_args) {
+    if (ctx->prm.kind == QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "f_a tag table: not a classical context");
+    if (bad_args) return ctx->fail(QF_ERR_INVALID, bad_args);
+    if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "no key installed");
+    return QF_OK;
+}
+
+qf_status upload_gpow(qf_ctx* ctx, TagTable& t) {
+    const std::vector<uint64_t> gpow = gadget_powers(ctx);
+    CK(t.gpow.ensure(gpow.size() * 8));
+    CK(cudaMemcpyAsync(t.gpow.p, gpow.data(), gpow.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return QF_OK;
+}
+
+// A samp_p table install after the entry point's checks.  The caller's tags, per_tag words each, are copied in slices of at
+// most slice_cap tags; launch(dTags, cnt, out, dFail) writes the table words of one slice at out and a failure flag per tag,
+// and the first tag that failed is refused by its index ("tag <i> <what>").  t, whose word size and form are set, then
+// gets the gadget powers and, on PSFPerturbation, H_0 (PSFGPV's h_t does not involve it), and replaces the installed table
+// of either form.  A refusal or an error leaves the installed table as it was.
+template <typename Launch>
+qf_status build_samp_table(qf_ctx* ctx, TagTable& t, const int64_t* tags, int64_t ntags, size_t per_tag, int64_t slice_cap,
+                           const char* what, Launch&& launch) {
+    const int64_t slice = std::max<int64_t>(1, std::min<int64_t>(ntags, slice_cap));
+    Dev dTags, dFail;
+    CK(t.tab.ensure((size_t)ntags * per_tag * t.word));
+    CK(dTags.ensure((size_t)slice * per_tag * 8));
+    CK(dFail.ensure((size_t)slice * sizeof(int)));
+    std::vector<int> fail((size_t)slice);
+    for (int64_t t0 = 0; t0 < ntags; t0 += slice) {
+        const int cnt = (int)std::min<int64_t>(slice, ntags - t0);
+        CK(cudaMemcpyAsync(dTags.p, tags + (size_t)t0 * per_tag, (size_t)cnt * per_tag * 8, cudaMemcpyHostToDevice, ctx->stream));
+        QF_TRY(launch(dTags.as<int64_t>(), cnt, t.tab.as<char>() + (size_t)t0 * per_tag * t.word, dFail.as<int>()));
+        CK(cudaMemcpyAsync(fail.data(), dFail.p, (size_t)cnt * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        for (int i = 0; i < cnt; ++i)
+            if (fail[i]) {
+                char buf[128];
+                snprintf(buf, sizeof buf, "tag %lld %s", (long long)(t0 + i), what);
+                return ctx->fail(QF_ERR_INVALID, buf);
+            }
+    }
+    QF_TRY(upload_gpow(ctx, t));
+    if (ctx->prm.kind == QF_PSF_PERTURBATION) QF_TRY(upload_tag_h0(ctx, t));
+    t.count = ntags;
+    ctx->samp_tags.swap(t);
+    return QF_OK;
+}
+
+// An f_a table install after the entry point's checks.  The caller's tags, per_tag words each, are copied in slices of at
+// most 1 GB; launch(dTags, cnt, out) writes the table words of one slice at out.  t, whose word size and form (and for
+// the poly form H_0) are set, then gets the gadget powers and replaces the installed table of either form.
+template <typename Launch>
+qf_status build_f_a_table(qf_ctx* ctx, TagTable& t, const int64_t* tags, int64_t ntags, size_t per_tag, Launch&& launch) {
+    const int64_t slice = std::max<int64_t>(1, std::min<int64_t>(ntags, (int64_t)((1ull << 30) / (8 * per_tag))));
+    Dev dTags;
+    CK(t.tab.ensure((size_t)ntags * per_tag * t.word));
+    CK(dTags.ensure((size_t)slice * per_tag * 8));
+    if (!t.poly) CK(t.sort.ensure((size_t)3 * (ntags + 1) * sizeof(int)));
+    for (int64_t t0 = 0; t0 < ntags; t0 += slice) {
+        const int cnt = (int)std::min<int64_t>(slice, ntags - t0);
+        CK(cudaMemcpyAsync(dTags.p, tags + (size_t)t0 * per_tag, (size_t)cnt * per_tag * 8, cudaMemcpyHostToDevice, ctx->stream));
+        QF_TRY(launch(dTags.as<int64_t>(), cnt, t.tab.as<char>() + (size_t)t0 * per_tag * t.word));
+        CK(cudaStreamSynchronize(ctx->stream));  // dTags is refilled by the next slice
+    }
+    QF_TRY(upload_gpow(ctx, t));
+    t.count = ntags;
+    ctx->fa_tags.swap(t);
     return QF_OK;
 }
 }  // namespace
@@ -2342,8 +2590,7 @@ qf_status qf_set_trapdoor_perturbation(qf_ctx* ctx, const int8_t* r, const doubl
     if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "install A first (qf_set_a / qf_trap_gen)");
     ctx->has_pert = false;
     ctx->key_tagged = false; ctx->pert_gadget_key = false;
-    ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release(); ctx->dTagXr.release();
-    ctx->drop_pool();
+    ctx->trapdoor_changed();
     CK(cudaSetDevice(ctx->device));
     QF_TRY(upload_as_f64(ctx, r, ctx->m_bar, ctx->nk, ctx->ld_nk, ctx->dR));
     {
@@ -2390,22 +2637,11 @@ qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out) {
     if (!ctx->has_a || !ctx->has_pert) return ctx->fail(QF_ERR_NO_KEY, "PSFPerturbation: key or trapdoor missing");
     if (!ctx->pert_gadget_key) return ctx->fail(QF_ERR_INVALID, "the installed key is not [A_bar | H G - A_bar R] for the installed R");
     CK(cudaSetDevice(ctx->device));
-    const long n = ctx->n, k = ctx->k, mb = ctx->m_bar, m = ctx->m;
-    const uint64_t q = ctx->prm.q;
+    const long n = ctx->n, mb = ctx->m_bar, m = ctx->m;
     // the new tag H' as MatZq (entries reduced mod q); H'^-1 before anything changes, so that a tag without a unit pivot
     // leaves the key, its tag and the outputs as they were
-    std::vector<uint64_t> h2((size_t)n * n);
-    bool ident = true;
-    for (long i = 0; i < n; ++i)
-        for (long j = 0; j < n; ++j) {
-            uint64_t v = i == j ? 1 : 0;
-            if (tag) {
-                const int64_t t = tag[i * n + j] % (int64_t)q;
-                v = (uint64_t)(t < 0 ? t + (int64_t)q : t);
-            }
-            h2[(size_t)i * n + j] = v;
-            ident = ident && v == (i == j ? 1u : 0u);
-        }
+    std::vector<uint64_t> h2;
+    const bool ident = tag_residues(ctx, tag, h2);
     std::vector<int64_t> hinv;
     if (!ident) {
         bool ok = false;
@@ -2416,25 +2652,14 @@ qf_status qf_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out) {
     // device copies are consistent again the context has no key (a CUDA error on the way leaves it so).
     ctx->has_a = false;
     ctx->has_pert = false;
-    // the f_a table is relative to A, which changes here
-    ctx->fa_tag_count = 0; ctx->dFaTab.release(); ctx->dFaXr.release(); ctx->dFaH0.release();
-    ctx->drop_pool();
-    const std::vector<uint64_t> gpow = gadget_powers(ctx);
-    for (long i = 0; i < n; ++i)
-        for (long j = 0; j < n; ++j) {
-            const uint64_t d = (h2[(size_t)i * n + j] + q - ctx->key_tag[(size_t)i * n + j]) % q;
-            if (!d) continue;
-            for (long t = 0; t < k; ++t) {
-                int64_t& a = ctx->hA[(size_t)i * m + mb + j * k + t];
-                a = (int64_t)(((u128)(uint64_t)a + mulmod_h(d, gpow[t], q)) % q);
-            }
-        }
+    ctx->a_changed();
+    add_tag_change(ctx, h2, ctx->hA);
     QF_TRY(upload_a_cols(ctx, mb));
     if (ident) ctx->dHinvl.release();
     else QF_TRY(tag_planes(ctx, hinv, ctx->dHinvl));
     ctx->key_tagged = !ident;
     ctx->key_tag = std::move(h2);
-    if (ctx->tag_count) QF_TRY(upload_tag_h0(ctx));  // the tag table stays: it is relative to (A_bar, R)
+    if (ctx->samp_tags.count) QF_TRY(upload_tag_h0(ctx, ctx->samp_tags));  // the table stays: it is relative to (A_bar, R)
     ctx->has_a = true;
     ctx->has_pert = true;
     if (a_out) memcpy(a_out, ctx->hA.data(), (size_t)n * m * sizeof(int64_t));
@@ -2450,43 +2675,24 @@ qf_status qf_gpv_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out, int64_
     if (ctx->prm.kind != QF_PSF_GPV) return ctx->fail(QF_ERR_INVALID, "not a PSFGPV context (PSFPerturbation: qf_set_tag)");
     QF_TRY(gpv_tags_ready(ctx));
     CK(cudaSetDevice(ctx->device));
-    const long n = ctx->n, k = ctx->k, mb = ctx->m_bar, nk = ctx->nk, m = ctx->m;
-    const uint64_t q = ctx->prm.q, base = (uint64_t)ctx->prm.base;
+    const long n = ctx->n, mb = ctx->m_bar, nk = ctx->nk, m = ctx->m;
+    const uint64_t q = ctx->prm.q;
     // everything that can refuse runs before the context changes: H'^-1, the pivots of A', the basis for the caller
-    std::vector<uint64_t> h2((size_t)n * n);
-    std::vector<int64_t> h2w((size_t)n * n);
-    bool ident = true;
-    for (long i = 0; i < n; ++i)
-        for (long j = 0; j < n; ++j) {
-            uint64_t v = i == j ? 1 : 0;
-            if (tag) {
-                const int64_t t = tag[i * n + j] % (int64_t)q;
-                v = (uint64_t)(t < 0 ? t + (int64_t)q : t);
-            }
-            h2[(size_t)i * n + j] = v;
-            h2w[(size_t)i * n + j] = (int64_t)v;
-            ident = ident && v == (i == j ? 1u : 0u);
-        }
-    std::vector<int64_t> hinv;
+    std::vector<uint64_t> h2;
+    const bool ident = tag_residues(ctx, tag, h2);
+    // H'^-1 and A_bar' = H'^-1 A_bar (reads the unchanged first m_bar columns of hA)
+    std::vector<int64_t> hinv, abt;
     Dev dHl;
     if (!ident) {
         bool ok = false;
         QF_TRY(tag_inverse(ctx, h2.data(), hinv, &ok));
         if (!ok) return ctx->fail(QF_ERR_INVALID, "tag is not invertible mod q (no unit pivot)");
         QF_TRY(tag_planes(ctx, hinv, dHl));
+        QF_TRY(tag_abar(ctx, dHl, abt));
     }
-    // A' = A + [0 | (H' - H) G] mod q
+    const std::vector<int64_t>* abar = ident ? nullptr : &abt;
     std::vector<int64_t> a2 = ctx->hA;
-    const std::vector<uint64_t> gpow = gadget_powers(ctx);
-    for (long i = 0; i < n; ++i)
-        for (long j = 0; j < n; ++j) {
-            const uint64_t d = (h2[(size_t)i * n + j] + q - ctx->key_tag[(size_t)i * n + j]) % q;
-            if (!d) continue;
-            for (long t = 0; t < k; ++t) {
-                int64_t& a = a2[(size_t)i * m + mb + j * k + t];
-                a = (int64_t)(((u128)(uint64_t)a + mulmod_h(d, gpow[t], q)) % q);
-            }
-        }
+    add_tag_change(ctx, h2, a2);
     // The pivot search walks the columns in order and stops at n pivots: when all of them lie in A_bar, which H' leaves
     // unchanged, the search over A' makes the same choices.  Otherwise it runs again.
     std::vector<int> piv((size_t)ctx->npiv);
@@ -2496,28 +2702,15 @@ qf_status qf_gpv_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out, int64_
     if (repivot && !find_unit_pivots(a2.data(), n, m, q, piv, ainv))
         return ctx->fail(QF_ERR_UNSUPPORTED, "A has no n columns invertible over Z_q by unit pivoting");
     if (s_out) {
-        // the basis reads A_bar only (the first m_bar columns of the installed A) and R, read back from its s8 plane
+        // the basis reads A_bar' and R, read back from its s8 plane
         std::vector<int8_t> r((size_t)mb * nk);
         CK(cudaMemcpy2D(r.data(), (size_t)nk, ctx->dRl.p, (size_t)ctx->ldk_nk, (size_t)nk, (size_t)mb, cudaMemcpyDeviceToHost));
-        QF_TRY(qf_gen_short_basis_tagged(ctx, r.data(), ident ? nullptr : h2w.data(), s_out));
+        QF_TRY(short_basis(ctx, r.data(), abar, s_out));
     }
-    // A_bar' = H'^-1 A_bar (reads the unchanged first m_bar columns of hA) and W = digits(-A_bar'), nk x m_bar
-    std::vector<int64_t> abt;
-    if (!ident) QF_TRY(tag_abar(ctx, dHl, abt));
-    std::vector<int64_t> w64((size_t)nk * mb), ab;
-    for (long j = 0; j < n; ++j)
-        for (long c = 0; c < mb; ++c) {
-            uint64_t v = (q - (uint64_t)(ident ? ctx->hA[(size_t)j * m + c] : abt[(size_t)c * n + j])) % q;
-            for (long t = 0; t < k; ++t) {
-                w64[(size_t)(j * k + t) * mb + c] = (int64_t)(v % base);
-                v /= base;
-            }
-        }
+    const std::vector<int64_t> w = w_digits(ctx, abar);
     // commit.  Until the device copies are consistent again the context has no trapdoor (a CUDA error on the way leaves it so).
     ctx->has_np = false;
-    // the f_a table is relative to A; the samp_p table to (A_bar, R): kept
-    ctx->fa_tag_count = 0; ctx->dFaTab.release(); ctx->dFaXr.release(); ctx->dFaH0.release();
-    ctx->drop_pool();
+    ctx->a_changed();  // the samp_p table is relative to (A_bar, R): kept
     ctx->hA.swap(a2);
     QF_TRY(upload_a_cols(ctx, mb));
     if (repivot) {
@@ -2527,18 +2720,13 @@ qf_status qf_gpv_set_tag(qf_ctx* ctx, const int64_t* tag, int64_t* a_out, int64_
         for (int pc : piv) piv_low = piv_low || pc >= mb;
         ctx->i2_limbs = limbs_for(8.0 * ctx->prm.s + 64.0 + (piv_low ? (double)q : 0.0));
     }
-    QF_TRY(upload_limbs(ctx, w64.data(), nk, mb, ctx->ldk_mb, 1, false, ctx->dWl));
+    QF_TRY(upload_limbs(ctx, w.data(), nk, mb, ctx->ldk_mb, 1, false, ctx->dWl));
     if (ident) {
         ctx->dHinvl.release();
         ctx->dAbpl.release();
     } else {
-        std::swap(ctx->dHinvl.p, dHl.p);
-        std::swap(ctx->dHinvl.cap, dHl.cap);
-        ab.resize((size_t)n * mb);
-        for (long i = 0; i < n; ++i)
-            for (long c = 0; c < mb; ++c) ab[(size_t)i * mb + c] = abt[(size_t)c * n + i];
-        QF_TRY(upload_limbs(ctx, ab.data(), n, mb, ctx->ldk_mb, ctx->a_limbs, false, ctx->dAbpl));
-        ctx->tag_ulimbs = limbs_for((double)(q - 1));
+        ctx->dHinvl.swap(dHl);
+        QF_TRY(install_abar(ctx, abt));
     }
     ctx->key_tagged = !ident;
     ctx->key_tag = std::move(h2);
@@ -2551,70 +2739,38 @@ constexpr int64_t TAG_SLICE = 256;  // tags inverted per launch: 2 CTAs of 1024 
 
 // H_t^-1 for every tag on the device: [H_t | I] built from the caller's words (reduced mod q there), Gauss-Jordan with unit
 // pivots one CTA per tag, packed column-major.  Slices of at most TAG_SLICE tags and 1 GB bound the scratch ([H | I] is
-// 16 n^2 bytes per tag, 4 MB at n = 512).  The new table replaces the old one only when every tag has been inverted.
+// 16 n^2 bytes per tag, 4 MB at n = 512).
 qf_status qf_set_tag_table(qf_ctx* ctx, const int64_t* tags, int64_t ntags) {
     if (!ctx) return QF_ERR_INVALID;
-    if (ctx->prm.kind == QF_PSF_GPV) {
-        QF_TRY(gpv_tags_ready(ctx));
-    } else if (ctx->prm.kind != QF_PSF_PERTURBATION) {
-        return ctx->fail(QF_ERR_INVALID, "not a PSFGPV or PSFPerturbation context");
-    }
-    if (!tags || ntags < 1) return ctx->fail(QF_ERR_INVALID, "tag table: at least one tag needed");
-    if (ctx->prm.kind == QF_PSF_PERTURBATION) {
-        if (!ctx->has_a || !ctx->has_pert) return ctx->fail(QF_ERR_NO_KEY, "PSFPerturbation: key or trapdoor missing");
-        if (!ctx->pert_gadget_key) return ctx->fail(QF_ERR_INVALID, "the installed key is not [A_bar | H G - A_bar R] for the installed R");
-    }
+    QF_TRY(samp_table_ready(ctx, tags && ntags >= 1 ? nullptr : "tag table: at least one tag needed"));
     const long n = ctx->n;
     if (ctx->k > 64 || 16 * n > 227 * 1024) return ctx->fail(QF_ERR_UNSUPPORTED, "tag table: needs k <= 64 and n <= 14528");
     if (ntags > INT32_MAX) return ctx->fail(QF_ERR_INVALID, "tag table: more than 2^31 - 1 tags");
     CK(cudaSetDevice(ctx->device));
     const uint64_t q = ctx->prm.q;
-    const int word = q <= (1ull << 32) ? 4 : 8;
     const size_t nn = (size_t)n * n;
-    const int64_t slice = std::max<int64_t>(1, std::min<int64_t>({ntags, TAG_SLICE, (int64_t)((1ull << 30) / (16 * nn))}));
-    Dev tab, dTags, dM, dF, dFail;
-    CK(tab.ensure((size_t)ntags * nn * word));
-    CK(dTags.ensure((size_t)slice * nn * 8));
-    CK(dM.ensure((size_t)slice * nn * 16));
-    CK(dF.ensure((size_t)slice * n * 8));
-    CK(dFail.ensure((size_t)slice * sizeof(int)));
-    std::vector<int> fail((size_t)slice);
-    for (int64_t t0 = 0; t0 < ntags; t0 += slice) {
-        const int cnt = (int)std::min<int64_t>(slice, ntags - t0);
-        CK(cudaMemcpyAsync(dTags.p, tags + (size_t)t0 * nn, (size_t)cnt * nn * 8, cudaMemcpyHostToDevice, ctx->stream));
-        LAUNCH(qf_launch_tag_build(dTags.as<int64_t>(), cnt, (int)n, q, dM.as<uint64_t>(), ctx->stream));
-        LAUNCH(qf_launch_mat_inverse_mod_batched(dM.as<uint64_t>(), dF.as<uint64_t>(), (int)n, q, dFail.as<int>(), cnt, ctx->stream));
-        LAUNCH(qf_launch_tag_pack(dM.as<uint64_t>(), cnt, (int)n, word, tab.as<char>() + (size_t)t0 * nn * word, ctx->stream));
-        CK(cudaMemcpyAsync(fail.data(), dFail.p, (size_t)cnt * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-        for (int i = 0; i < cnt; ++i)
-            if (fail[i]) {
-                char buf[128];
-                snprintf(buf, sizeof buf, "tag %lld is not invertible mod q (no unit pivot)", (long long)(t0 + i));
-                return ctx->fail(QF_ERR_INVALID, buf);
-            }
-    }
-    const std::vector<uint64_t> gpow = gadget_powers(ctx);
-    CK(ctx->dTagGpow.ensure(gpow.size() * 8));
-    CK(cudaMemcpyAsync(ctx->dTagGpow.p, gpow.data(), gpow.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
-    ctx->tag_word = word;
-    if (ctx->prm.kind == QF_PSF_PERTURBATION) QF_TRY(upload_tag_h0(ctx));  // PSFGPV's h_t does not involve H_0
-    std::swap(ctx->dTagTab.p, tab.p);
-    std::swap(ctx->dTagTab.cap, tab.cap);
-    ctx->tag_poly = false;
-    ctx->dTagXr.release();
-    ctx->tag_count = ntags;
-    return QF_OK;
+    TagTable t(q);
+    Dev dM, dF;
+    return build_samp_table(ctx, t, tags, ntags, nn, std::min<int64_t>(TAG_SLICE, (int64_t)((1ull << 30) / (16 * nn))),
+                            "is not invertible mod q (no unit pivot)",
+                            [&](const int64_t* dTags, int cnt, char* out, int* dFail) -> qf_status {
+                                CK(dM.ensure((size_t)cnt * nn * 16));
+                                CK(dF.ensure((size_t)cnt * n * 8));
+                                LAUNCH(qf_launch_tag_build(dTags, cnt, (int)n, q, dM.as<uint64_t>(), ctx->stream));
+                                LAUNCH(qf_launch_mat_inverse_mod_batched(dM.as<uint64_t>(), dF.as<uint64_t>(), (int)n, q, dFail, cnt,
+                                                                         ctx->stream));
+                                LAUNCH(qf_launch_tag_pack(dM.as<uint64_t>(), cnt, (int)n, t.word, out, ctx->stream));
+                                return QF_OK;
+                            });
 }
 
-// D_t = H_t - H_0 mod q for every tag, built on the device from the caller's words in slices of at most 1 GB of int64 tags.
-// No trapdoor is needed and no tag is inverted.  The new table replaces the old one only when it is complete.
+// D_t = H_t - H_0 mod q for every tag, built on the device from the caller's words.  No trapdoor is needed and no tag is
+// inverted.
 qf_status qf_set_f_a_tags(qf_ctx* ctx, const int64_t* tags, int64_t ntags, const int64_t* h0) {
     if (!ctx) return QF_ERR_INVALID;
-    if (ctx->prm.kind == QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "f_a tag table: not a classical context");
-    if (!tags || ntags < 1) return ctx->fail(QF_ERR_INVALID, "f_a tag table: at least one tag needed");
-    if (ntags >= INT32_MAX) return ctx->fail(QF_ERR_INVALID, "f_a tag table: more than 2^31 - 2 tags");
-    if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "no key installed");
+    QF_TRY(f_a_tags_ready(ctx, !tags || ntags < 1       ? "f_a tag table: at least one tag needed"
+                               : ntags >= INT32_MAX ? "f_a tag table: more than 2^31 - 2 tags"
+                                                    : nullptr));
     const long n = ctx->n;
     CK(cudaSetDevice(ctx->device));
     int supported = 0;
@@ -2622,62 +2778,28 @@ qf_status qf_set_f_a_tags(qf_ctx* ctx, const int64_t* tags, int64_t ntags, const
     if (!supported)
         return ctx->fail(QF_ERR_UNSUPPORTED, "f_a tag table: needs k <= 64 and the group's shared memory within one block's limit");
     const uint64_t q = ctx->prm.q;
-    const int word = q <= (1ull << 32) ? 4 : 8;
     const size_t nn = (size_t)n * n;
-    const int64_t slice = std::max<int64_t>(1, std::min<int64_t>(ntags, (int64_t)((1ull << 30) / (8 * nn))));
-    Dev tab, dTags, dH0, sort;
-    CK(tab.ensure((size_t)ntags * nn * word));
-    CK(dTags.ensure((size_t)slice * nn * 8));
-    CK(sort.ensure((size_t)3 * (ntags + 1) * sizeof(int)));
+    Dev dH0;  // H_0 mod q in 8-byte words, row-major; none for H_0 = I
     if (h0) {
-        std::vector<uint64_t> h((size_t)nn);
-        for (size_t x = 0; x < nn; ++x) {
-            const int64_t v = h0[x] % (int64_t)q;
-            h[x] = (uint64_t)(v < 0 ? v + (int64_t)q : v);
-        }
+        const std::vector<uint64_t> h = residues(h0, nn, q);
         CK(dH0.ensure(nn * 8));
         CK(cudaMemcpyAsync(dH0.p, h.data(), nn * 8, cudaMemcpyHostToDevice, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
     }
-    for (int64_t t0 = 0; t0 < ntags; t0 += slice) {
-        const int cnt = (int)std::min<int64_t>(slice, ntags - t0);
-        CK(cudaMemcpyAsync(dTags.p, tags + (size_t)t0 * nn, (size_t)cnt * nn * 8, cudaMemcpyHostToDevice, ctx->stream));
-        LAUNCH(qf_launch_tag_diff_pack(dTags.as<int64_t>(), cnt, (int)n, q, dH0.as<uint64_t>(), word,
-                                       tab.as<char>() + (size_t)t0 * nn * word, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));  // dTags is refilled by the next slice
-    }
-    const std::vector<uint64_t> gpow = gadget_powers(ctx);
-    CK(ctx->dFaGpow.ensure(gpow.size() * 8));
-    CK(cudaMemcpyAsync(ctx->dFaGpow.p, gpow.data(), gpow.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    std::swap(ctx->dFaTab.p, tab.p);
-    std::swap(ctx->dFaTab.cap, tab.cap);
-    std::swap(ctx->dFaSort.p, sort.p);
-    std::swap(ctx->dFaSort.cap, sort.cap);
-    ctx->fa_tag_word = word;
-    ctx->fa_poly = false;
-    ctx->dFaXr.release();
-    ctx->dFaH0.release();
-    ctx->fa_tag_count = ntags;
-    return QF_OK;
+    TagTable t(q);
+    return build_f_a_table(ctx, t, tags, ntags, nn, [&](const int64_t* dTags, int cnt, char* out) -> qf_status {
+        LAUNCH(qf_launch_tag_diff_pack(dTags, cnt, (int)n, q, dH0.as<uint64_t>(), t.word, out, ctx->stream));
+        return QF_OK;
+    });
 }
 
 // ---- tags in polynomial form: H_t = rot_f(h_t), column c = coeffs(h_t X^c mod f) (DESIGN 4.10) -------------------------
 
 // h_t^-1 mod (f, q) for every tag on the device (qf_launch_poly_tag_inverse, one CTA per tag), for q = p^e.  Tags are
-// copied in slices of at most 1 GB.  The new table replaces the old one, of either form, only when every tag is a unit.
+// copied in slices of at most 1 GB.
 qf_status qf_set_tag_table_poly(qf_ctx* ctx, const int64_t* f, const int64_t* tags, int64_t ntags) {
     if (!ctx) return QF_ERR_INVALID;
-    if (ctx->prm.kind == QF_PSF_GPV) {
-        QF_TRY(gpv_tags_ready(ctx));
-    } else if (ctx->prm.kind != QF_PSF_PERTURBATION) {
-        return ctx->fail(QF_ERR_INVALID, "not a PSFGPV or PSFPerturbation context");
-    }
-    if (!f || !tags || ntags < 1) return ctx->fail(QF_ERR_INVALID, "tag table: f and at least one tag needed");
-    if (ctx->prm.kind == QF_PSF_PERTURBATION) {
-        if (!ctx->has_a || !ctx->has_pert) return ctx->fail(QF_ERR_NO_KEY, "PSFPerturbation: key or trapdoor missing");
-        if (!ctx->pert_gadget_key) return ctx->fail(QF_ERR_INVALID, "the installed key is not [A_bar | H G - A_bar R] for the installed R");
-    }
+    QF_TRY(samp_table_ready(ctx, f && tags && ntags >= 1 ? nullptr : "tag table: f and at least one tag needed"));
     if (ntags > INT32_MAX) return ctx->fail(QF_ERR_INVALID, "tag table: more than 2^31 - 1 tags");
     const long n = ctx->n;
     const uint64_t q = ctx->prm.q;
@@ -2692,51 +2814,24 @@ qf_status qf_set_tag_table_poly(qf_ctx* ctx, const int64_t* f, const int64_t* ta
         return ctx->fail(QF_ERR_UNSUPPORTED, "tag table in polynomial form: needs k <= 64 and the shared memory within one block's limit");
     int lifts = 0;
     while ((1 << lifts) < e) ++lifts;
-    const int word = q <= (1ull << 32) ? 4 : 8;
-    const int64_t slice = std::max<int64_t>(1, std::min<int64_t>(ntags, (int64_t)((1ull << 30) / (8 * n))));
-    Dev tab, xr, dF, dTags, dFail;
-    QF_TRY(poly_modulus(ctx, f, word, dF, xr));
-    CK(tab.ensure((size_t)ntags * n * word));
-    CK(dTags.ensure((size_t)slice * n * 8));
-    CK(dFail.ensure((size_t)slice * sizeof(int)));
-    std::vector<int> fail((size_t)slice);
-    for (int64_t t0 = 0; t0 < ntags; t0 += slice) {
-        const int cnt = (int)std::min<int64_t>(slice, ntags - t0);
-        CK(cudaMemcpyAsync(dTags.p, tags + (size_t)t0 * n, (size_t)cnt * n * 8, cudaMemcpyHostToDevice, ctx->stream));
-        LAUNCH(qf_launch_poly_tag_inverse(dTags.as<int64_t>(), cnt, (int)n, dF.as<uint64_t>(), xr.p, word, q, p, lifts,
-                                          tab.as<char>() + (size_t)t0 * n * word, dFail.as<int>(), ctx->stream));
-        CK(cudaMemcpyAsync(fail.data(), dFail.p, (size_t)cnt * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-        for (int i = 0; i < cnt; ++i)
-            if (fail[i]) {
-                char buf[128];
-                snprintf(buf, sizeof buf, "tag %lld is not a unit mod (f, q)", (long long)(t0 + i));
-                return ctx->fail(QF_ERR_INVALID, buf);
-            }
-    }
-    const std::vector<uint64_t> gpow = gadget_powers(ctx);
-    CK(ctx->dTagGpow.ensure(gpow.size() * 8));
-    CK(cudaMemcpyAsync(ctx->dTagGpow.p, gpow.data(), gpow.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
-    ctx->tag_word = word;
-    if (ctx->prm.kind == QF_PSF_PERTURBATION) QF_TRY(upload_tag_h0(ctx));  // PSFGPV's h_t does not involve H_0
-    CK(cudaStreamSynchronize(ctx->stream));
-    std::swap(ctx->dTagTab.p, tab.p);
-    std::swap(ctx->dTagTab.cap, tab.cap);
-    std::swap(ctx->dTagXr.p, xr.p);
-    std::swap(ctx->dTagXr.cap, xr.cap);
-    ctx->tag_poly = true;
-    ctx->tag_count = ntags;
-    return QF_OK;
+    TagTable t(q);
+    Dev dF;
+    QF_TRY(poly_modulus(ctx, f, t, dF));
+    return build_samp_table(ctx, t, tags, ntags, n, (int64_t)((1ull << 30) / (8 * n)), "is not a unit mod (f, q)",
+                            [&](const int64_t* dTags, int cnt, char* out, int* dFail) -> qf_status {
+                                LAUNCH(qf_launch_poly_tag_inverse(dTags, cnt, (int)n, dF.as<uint64_t>(), t.xr.p, t.word, q, p,
+                                                                  lifts, out, dFail, ctx->stream));
+                                return QF_OK;
+                            });
 }
 
 // h_t mod q as n words per tag and H_0 (NULL: I; all zero: 0; otherwise dense, column-major).  Nothing is inverted: every
-// q < 2^62, singular tags and H_0 = 0 work.  The new table replaces the old one, of either form, only when it is complete.
+// q < 2^62, singular tags and H_0 = 0 work.
 qf_status qf_set_f_a_tags_poly(qf_ctx* ctx, const int64_t* f, const int64_t* tags, int64_t ntags, const int64_t* h0) {
     if (!ctx) return QF_ERR_INVALID;
-    if (ctx->prm.kind == QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "f_a tag table: not a classical context");
-    if (!f || !tags || ntags < 1) return ctx->fail(QF_ERR_INVALID, "f_a tag table: f and at least one tag needed");
-    if (ntags >= INT32_MAX) return ctx->fail(QF_ERR_INVALID, "f_a tag table: more than 2^31 - 2 tags");
-    if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "no key installed");
+    QF_TRY(f_a_tags_ready(ctx, !f || !tags || ntags < 1 ? "f_a tag table: f and at least one tag needed"
+                               : ntags >= INT32_MAX     ? "f_a tag table: more than 2^31 - 2 tags"
+                                                        : nullptr));
     const long n = ctx->n;
     const uint64_t q = ctx->prm.q;
     CK(cudaSetDevice(ctx->device));
@@ -2744,61 +2839,20 @@ qf_status qf_set_f_a_tags_poly(qf_ctx* ctx, const int64_t* f, const int64_t* tag
     CK(qf_poly_tag_supported((int)std::min<long>(n, INT32_MAX), (int)std::min<long>(ctx->k, INT32_MAX), 0, &supported));
     if (!supported)
         return ctx->fail(QF_ERR_UNSUPPORTED, "f_a tag table in polynomial form: needs k <= 64 and the shared memory within one block's limit");
-    const int word = q <= (1ull << 32) ? 4 : 8;
-    const size_t nn = (size_t)n * n;
-    int kind = 1;
-    std::vector<uint64_t> h;
+    TagTable t(q);
     if (h0) {
-        h.resize(nn);
-        bool zero = true, ident = true;
-        for (long i = 0; i < n; ++i)
-            for (long j = 0; j < n; ++j) {
-                const int64_t v = h0[(size_t)i * n + j] % (int64_t)q;
-                const uint64_t r = (uint64_t)(v < 0 ? v + (int64_t)q : v);
-                h[(size_t)j * n + i] = r;
-                zero = zero && r == 0;
-                ident = ident && r == (i == j ? 1 % q : 0);
-            }
-        kind = ident ? 1 : zero ? 0 : 2;
+        std::vector<uint64_t> h;
+        const bool ident = tag_residues(ctx, h0, h);
+        const bool zero = std::all_of(h.begin(), h.end(), [](uint64_t v) { return v == 0; });
+        t.h0_kind = ident ? 1 : zero ? 0 : 2;
+        if (t.h0_kind == 2) QF_TRY(upload_h0_words(ctx, h, t.word, t.h0));
     }
-    const int64_t slice = std::max<int64_t>(1, std::min<int64_t>(ntags, (int64_t)((1ull << 30) / (8 * n))));
-    Dev tab, xr, dF, dTags, dH0;
-    QF_TRY(poly_modulus(ctx, f, word, dF, xr));
-    CK(tab.ensure((size_t)ntags * n * word));
-    CK(dTags.ensure((size_t)slice * n * 8));
-    if (kind == 2) {
-        std::vector<uint32_t> h32;
-        const void* src = h.data();
-        if (word == 4) {
-            h32.assign(h.begin(), h.end());
-            src = h32.data();
-        }
-        CK(dH0.ensure(nn * word));
-        CK(cudaMemcpyAsync(dH0.p, src, nn * word, cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-    }
-    for (int64_t t0 = 0; t0 < ntags; t0 += slice) {
-        const int cnt = (int)std::min<int64_t>(slice, ntags - t0);
-        CK(cudaMemcpyAsync(dTags.p, tags + (size_t)t0 * n, (size_t)cnt * n * 8, cudaMemcpyHostToDevice, ctx->stream));
-        LAUNCH(qf_launch_poly_tag_pack(dTags.as<int64_t>(), (long)cnt * n, q, word, tab.as<char>() + (size_t)t0 * n * word,
-                                       ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));  // dTags is refilled by the next slice
-    }
-    const std::vector<uint64_t> gpow = gadget_powers(ctx);
-    CK(ctx->dFaGpow.ensure(gpow.size() * 8));
-    CK(cudaMemcpyAsync(ctx->dFaGpow.p, gpow.data(), gpow.size() * 8, cudaMemcpyHostToDevice, ctx->stream));
-    CK(cudaStreamSynchronize(ctx->stream));
-    std::swap(ctx->dFaTab.p, tab.p);
-    std::swap(ctx->dFaTab.cap, tab.cap);
-    std::swap(ctx->dFaXr.p, xr.p);
-    std::swap(ctx->dFaXr.cap, xr.cap);
-    std::swap(ctx->dFaH0.p, dH0.p);
-    std::swap(ctx->dFaH0.cap, dH0.cap);
-    ctx->fa_tag_word = word;
-    ctx->fa_h0_kind = kind;
-    ctx->fa_poly = true;
-    ctx->fa_tag_count = ntags;
-    return QF_OK;
+    Dev dF;
+    QF_TRY(poly_modulus(ctx, f, t, dF));
+    return build_f_a_table(ctx, t, tags, ntags, n, [&](const int64_t* dTags, int cnt, char* out) -> qf_status {
+        LAUNCH(qf_launch_poly_tag_pack(dTags, (long)cnt * n, q, t.word, out, ctx->stream));
+        return QF_OK;
+    });
 }
 
 // gen_short_basis_for_trapdoor_ring (short_basis_ring.rs:64-166) in the coefficient embedding: D x D, D = n (k + 2),
@@ -2814,18 +2868,10 @@ qf_status qf_ring_gen_short_basis(qf_ctx* ctx, const int32_t* r, const int32_t* 
     CK(cudaSetDevice(ctx->device));
     const long n = ctx->n, k = ctx->k, D = n * (k + 2);
     const uint64_t q = ctx->prm.q, base = (uint64_t)ctx->prm.base;
-    u128 pw = 1;
-    for (long i = 0; i < k; ++i) pw *= base;
-    if (pw < q) return ctx->fail(QF_ERR_INVALID, "base^k < q");
-    const bool exact_pow = pw == (u128)q;
-    // S_k (gadget_classical.rs:248-272), columns reversed when base^k == q (short_basis_ring.rs, as the classical :80-82)
-    std::vector<int64_t> sk0((size_t)k * k, 0), sk((size_t)k * k, 0);
-    for (long j = 0; j < k; ++j) sk0[j * k + j] = (int64_t)base;
-    for (long i = 0; i + 1 < k; ++i) sk0[(i + 1) * k + i] = -1;
-    if (!exact_pow) {
-        uint64_t qq = q;
-        for (long i = 0; i < k; ++i) { sk0[i * k + (k - 1)] = (int64_t)(qq % base); qq /= base; }
-    }
+    // S_k, columns reversed when base^k == q (short_basis_ring.rs, as the classical :80-82)
+    std::vector<int64_t> sk0, sk((size_t)k * k, 0);
+    bool exact_pow = false;
+    if (!gadget_sk(ctx, sk0, &exact_pow)) return ctx->fail(QF_ERR_INVALID, "base^k < q");
     for (long j = 0; j < k; ++j)
         for (long c = 0; c < k; ++c) sk[j * k + c] = sk0[j * k + (exact_pow ? k - 1 - c : c)];
     // w[c][j][t] = digit j of coefficient t of -a_c mod q
@@ -2889,47 +2935,15 @@ qf_status qf_gen_short_basis_tagged(qf_ctx* ctx, const int8_t* r, const int64_t*
     if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "install A first (qf_set_a / qf_trap_gen)");
     if (!ctx->use_i8) return ctx->fail(QF_ERR_UNSUPPORTED, "needs the int8 tensor path");
     CK(cudaSetDevice(ctx->device));
-    const long n = ctx->n, k = ctx->k, mb = ctx->m_bar, nk = ctx->nk, m = ctx->m;
-    const uint64_t q = ctx->prm.q, base = (uint64_t)ctx->prm.base;
-    if (base > 256) return ctx->fail(QF_ERR_UNSUPPORTED, "gadget base > 256");
-    // S_k (gadget_classical.rs:248-272) and whether base^k == q (then S' = S with its columns reversed, :80-82)
-    u128 pw = 1;
-    for (long i = 0; i < k; ++i) pw *= base;
-    if (pw < q) return ctx->fail(QF_ERR_INVALID, "base^k < q");
-    const bool exact_pow = pw == (u128)q;
-    std::vector<int64_t> sk((size_t)k * k, 0);
-    for (long j = 0; j < k; ++j) sk[j * k + j] = (int64_t)base;
-    for (long i = 0; i + 1 < k; ++i) sk[(i + 1) * k + i] = -1;
-    if (!exact_pow) {
-        uint64_t qq = q;
-        for (long i = 0; i < k; ++i) { sk[i * k + (k - 1)] = (int64_t)(qq % base); qq /= base; }
-    }
-    // column c of S' = column (exact_pow ? nk-1-c : c) of I_n (x) S_k
-    auto sprime = [&](long row, long c) -> int64_t {
-        const long cc = exact_pow ? nk - 1 - c : c;
-        return (row / k == cc / k) ? sk[(row % k) * k + (cc % k)] : 0;
-    };
-    std::fill(s_out, s_out + (size_t)m * m, (int64_t)0);
-    // bottom-left S', top-left R S' (each column of S' has at most k non-zeros, all inside one k-block)
-    for (long c = 0; c < nk; ++c) {
-        const long cc = exact_pow ? nk - 1 - c : c, blk = cc / k;
-        for (long t = 0; t < k; ++t) {
-            const long row = blk * k + t;
-            const int64_t v = sprime(row, c);
-            if (!v) continue;
-            s_out[(size_t)(mb + row) * m + c] = v;
-            for (long i = 0; i < mb; ++i) s_out[(size_t)i * m + c] += (int64_t)r[i * nk + row] * v;
-        }
-    }
+    if (ctx->prm.base > 256) return ctx->fail(QF_ERR_UNSUPPORTED, "gadget base > 256");
+    std::vector<int64_t> sk;
+    bool exact_pow = false;
+    if (!gadget_sk(ctx, sk, &exact_pow)) return ctx->fail(QF_ERR_INVALID, "base^k < q");
     // A_bar' = H^-1 A[:, :m_bar] mod q (short_basis_classical.rs:106-107), transposed; the tag as MatZq: entries reduced mod q
-    std::vector<int64_t> abt;
-    if (tag) {
-        std::vector<uint64_t> h((size_t)n * n);
-        for (long i = 0; i < n * n; ++i) {
-            const int64_t v = tag[i] % (int64_t)q;
-            h[i] = (uint64_t)(v < 0 ? v + (int64_t)q : v);
-        }
-        std::vector<int64_t> hinv;
+    std::vector<uint64_t> h;
+    std::vector<int64_t> hinv, abt;
+    const bool ident = tag_residues(ctx, tag, h);
+    if (!ident) {
         bool ok = false;
         QF_TRY(tag_inverse(ctx, h.data(), hinv, &ok));
         if (!ok) return ctx->fail(QF_ERR_INVALID, "tag is not invertible mod q (no unit pivot)");
@@ -2937,43 +2951,7 @@ qf_status qf_gen_short_basis_tagged(qf_ctx* ctx, const int8_t* r, const int64_t*
         QF_TRY(tag_planes(ctx, hinv, dHl));
         QF_TRY(tag_abar(ctx, dHl, abt));
     }
-    // W = base-b digits of -A_bar' mod q (short_basis_classical.rs:105-110), stored transposed for the device:
-    // Wt[c][j k + t] = digit t of (q - A_bar'[j][c]) mod q
-    std::vector<int64_t> wt((size_t)mb * nk);
-    for (long j = 0; j < n; ++j)
-        for (long c = 0; c < mb; ++c) {
-            uint64_t v = (q - (uint64_t)(tag ? abt[(size_t)c * n + j] : ctx->hA[(size_t)j * m + c])) % q;
-            for (long t = 0; t < k; ++t) {
-                const int64_t d = (int64_t)(v % base);
-                v /= base;
-                wt[(size_t)c * nk + j * k + t] = d;
-                s_out[(size_t)(mb + j * k + t) * m + nk + c] = d;  // bottom-right W
-            }
-        }
-    // top-right I + R W: R (m_bar x nk, one s8 digit) times W on the tensor cores, exact int32
-    {
-        const long ldk = ctx->ldk_nk;
-        Dev dX, dW, dOut;
-        std::vector<int64_t> r64((size_t)mb * nk);
-        for (size_t i = 0; i < r64.size(); ++i) r64[i] = r[i];
-        QF_TRY(upload_limbs(ctx, r64.data(), mb, nk, ldk, 1, true, dX));
-        QF_TRY(upload_limbs(ctx, wt.data(), mb, nk, ldk, 1, false, dW));
-        CK(dOut.ensure((size_t)mb * mb * 4));
-        I8GemmArgs g{};
-        g.x = dX.as<int8_t>(); g.ldx = ldk; g.x_plane = mb * ldk;
-        g.w = dW.p; g.ldw = ldk; g.w_plane = mb * ldk;
-        g.LX = 1; g.LW = 1; g.w_signed = 0;
-        g.B = (int)mb; g.N = (int)mb; g.K = (int)nk;
-        g.out_kind = 1; g.sign = 1; g.q = 0; g.out = dOut.p; g.ldout = mb;
-        g.flag = ctx->dFlag.as<int>();
-        LAUNCH(ctx_gemm_i8(ctx, g));
-        std::vector<int32_t> rw((size_t)mb * mb);
-        CK(cudaMemcpyAsync(rw.data(), dOut.p, rw.size() * 4, cudaMemcpyDeviceToHost, ctx->stream));
-        CK(cudaStreamSynchronize(ctx->stream));
-        for (long i = 0; i < mb; ++i)
-            for (long c = 0; c < mb; ++c) s_out[(size_t)i * m + nk + c] = (int64_t)rw[(size_t)i * mb + c] + (i == c ? 1 : 0);
-    }
-    return check_flag(ctx);
+    return short_basis(ctx, r, ident ? nullptr : &abt, s_out);
 }
 
 qf_status qf_gen_short_basis(qf_ctx* ctx, const int8_t* r, int64_t* s_out) { return qf_gen_short_basis_tagged(ctx, r, nullptr, s_out); }
@@ -3019,9 +2997,7 @@ qf_status qf_set_trapdoor_gpv(qf_ctx* ctx, const int64_t* s, const double* sg) {
     if (ctx->prm.kind == QF_PSF_PERTURBATION) return ctx->fail(QF_ERR_INVALID, "not a GPV context");
     ctx->has_np = false;  // stays false if anything below fails half-way (pivots / A^-1 / U are overwritten in place)
     ctx->two_phase = false;
-    // the tag table is relative to the old (A_bar, R)
-    ctx->tag_count = 0; ctx->dTagTab.release(); ctx->dTagH0.release(); ctx->dTagXr.release();
-    ctx->drop_pool();
+    ctx->trapdoor_changed();
     ctx->u_limbs = 7;
     CK(cudaSetDevice(ctx->device));
     const long D = ctx->dim, ld = ctx->ld_dim;
@@ -3359,17 +3335,14 @@ qf_status qf_trap_gen_from(qf_ctx* ctx, const int64_t* a_bar, const int8_t* r, c
     CK(cudaMemcpyAsync(art.data(), dOut.p, art.size() * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
     // A = [A_bar | tag*G - A_bar R]
-    std::vector<uint64_t> gpow(k);
-    {
-        u128 pw = 1;
-        for (long t = 0; t < k; ++t) { gpow[t] = (uint64_t)(pw % q); pw = pw * (uint64_t)ctx->prm.base; }
-    }
+    const std::vector<uint64_t> gpow = gadget_powers(ctx);
+    std::vector<uint64_t> h;
+    tag_residues(ctx, tag, h);
     for (long i = 0; i < n; ++i) {
         for (long j = 0; j < mb; ++j) a_out[i * m + j] = a_bar[i * mb + j];
         for (long j = 0; j < nk; ++j) {
             long blk = j / k, t = j % k;
-            uint64_t h = tag ? ((uint64_t)tag[i * n + blk] % q) : (i == blk ? 1 : 0);
-            uint64_t hg = mulmod_h(h, gpow[t], q);
+            uint64_t hg = mulmod_h(h[(size_t)i * n + blk], gpow[t], q);
             uint64_t ar = (uint64_t)art[(size_t)j * n + i];
             a_out[i * m + mb + j] = (int64_t)((hg + q - ar) % q);
         }
@@ -3521,9 +3494,8 @@ static qf_status check_tag_idx(qf_ctx* ctx, const int32_t* tag_idx, int64_t batc
 }
 
 static qf_status f_a_tagged_ready(qf_ctx* ctx) {
-    if (ctx->prm.kind == QF_PSF_GPV_RING) return ctx->fail(QF_ERR_INVALID, "f_a tag table: not a classical context");
-    if (!ctx->has_a) return ctx->fail(QF_ERR_NO_KEY, "no key installed");
-    if (!ctx->fa_tag_count) return ctx->fail(QF_ERR_NO_KEY, "no f_a tag table installed (qf_set_f_a_tags)");
+    QF_TRY(f_a_tags_ready(ctx, nullptr));
+    if (!ctx->fa_tags.count) return ctx->fail(QF_ERR_NO_KEY, "no f_a tag table installed (qf_set_f_a_tags)");
     return QF_OK;
 }
 
@@ -3533,7 +3505,7 @@ qf_status qf_f_a_tagged(qf_ctx* ctx, const int32_t* sigma, const int32_t* tag_id
     if (batch == 0) return QF_OK;
     CK(cudaSetDevice(ctx->device));
     QF_TRY(f_a_tagged_ready(ctx));
-    QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->fa_tag_count, "f_a tag table"));
+    QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->fa_tags.count, "f_a tag table"));
     const long C = ctx->chunk;
     CK(ctx->io_a.ensure((size_t)C * ctx->dim * 4));
     CK(ctx->io_b.ensure((size_t)C * ctx->n * 8));
@@ -3757,15 +3729,6 @@ qf_status qf_samp_d(qf_ctx* ctx, int64_t batch, uint64_t seed, uint64_t first, i
 }
 
 // ---- samp_p ------------------------------------------------------------------
-static qf_status samp_p_ready(qf_ctx* ctx) {
-    if (ctx->prm.kind == QF_PSF_PERTURBATION) {
-        if (!ctx->has_a || !ctx->has_pert) return ctx->fail(QF_ERR_NO_KEY, "PSFPerturbation: key or trapdoor missing");
-    } else {
-        if (!ctx->has_np) return ctx->fail(QF_ERR_NO_KEY, "GPV: trapdoor missing (qf_set_trapdoor_gpv)");
-    }
-    return QF_OK;
-}
-
 qf_status qf_samp_p_dev(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t seed, uint64_t first, int32_t* e_out) {
     if (!ctx || batch < 0 || (batch > 0 && (!u || !e_out))) return QF_ERR_INVALID;
     if (batch == 0) return QF_OK;
@@ -3921,10 +3884,8 @@ qf_status qf_samp_p_i16(qf_ctx* ctx, const int64_t* u, int64_t batch, uint64_t s
 
 // ---- samp_p with a tag per target (PSFPerturbation, PSFGPV on the two-phase recursion; installed tag table) -----------
 static qf_status samp_p_tagged_ready(qf_ctx* ctx) {
-    if (ctx->prm.kind == QF_PSF_GPV) QF_TRY(gpv_tags_ready(ctx));
-    else if (ctx->prm.kind != QF_PSF_PERTURBATION) return ctx->fail(QF_ERR_INVALID, "not a PSFGPV or PSFPerturbation context");
-    QF_TRY(samp_p_ready(ctx));
-    if (!ctx->tag_count) return ctx->fail(QF_ERR_NO_KEY, "no tag table installed (qf_set_tag_table)");
+    QF_TRY(samp_tags_ready(ctx, nullptr));
+    if (!ctx->samp_tags.count) return ctx->fail(QF_ERR_NO_KEY, "no tag table installed (qf_set_tag_table)");
     return QF_OK;
 }
 
@@ -3933,7 +3894,7 @@ qf_status qf_samp_p_tagged(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx
     if (!ctx || batch < 0 || (batch > 0 && (!u || !tag_idx || !e_out))) return QF_ERR_INVALID;
     if (batch == 0) return QF_OK;
     QF_TRY(samp_p_tagged_ready(ctx));
-    QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->tag_count, "tag table"));
+    QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->samp_tags.count, "tag table"));
     return samp_p_host(ctx, u, batch, seed, first, e_out, SampOut{}, tag_idx);
 }
 
@@ -4020,7 +3981,7 @@ static qf_status samp_p_online_accept(qf_ctx* ctx, const int32_t* tag_idx, int64
                  (long long)(ctx->pool_count - ctx->pool_next));
         return ctx->fail(QF_ERR_INVALID, buf);
     }
-    if (tag_idx && host_idx && batch > 0) QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->tag_count, "tag table"));
+    if (tag_idx && host_idx && batch > 0) QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->samp_tags.count, "tag table"));
     *slot0 = ctx->pool_next;
     if (first_index_out) *first_index_out = ctx->pool_first + (uint64_t)ctx->pool_next;
     ctx->pool_next += batch;
@@ -4106,7 +4067,7 @@ qf_status qf_samp_p_packed(qf_ctx* ctx, const int64_t* u, const int32_t* tag_idx
     if (batch == 0) return QF_OK;
     if (tag_idx) {
         QF_TRY(samp_p_tagged_ready(ctx));
-        QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->tag_count, "tag table"));
+        QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->samp_tags.count, "tag table"));
     }
     SampOut f;
     f.kind = SampOut::PACKED;
@@ -4127,7 +4088,7 @@ qf_status qf_f_a_packed(qf_ctx* ctx, const uint8_t* packed, const int32_t* tag_i
     const bool ring = ctx->prm.kind == QF_PSF_GPV_RING;
     if (tag_idx) {
         QF_TRY(f_a_tagged_ready(ctx));
-        QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->fa_tag_count, "f_a tag table"));
+        QF_TRY(check_tag_idx(ctx, tag_idx, batch, ctx->fa_tags.count, "f_a tag table"));
     } else if (ring ? !ctx->has_ring : !ctx->has_a) {
         return ctx->fail(QF_ERR_NO_KEY, "no key installed");
     }
