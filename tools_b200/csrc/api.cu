@@ -214,6 +214,7 @@ struct qf_ctx {
     int sol_limbs = 0;
     bool np_fuse_split = true;  // the diagonal-block kernel writes the digit planes of z itself (no split pass over Z)
     bool np_fuse64 = true; // the rank-64 updates inside a 256-block run in the tail of the diagonal-block kernel
+    bool np_right = false; // right-looking tensor-core updates inside a 4096-block (np_block; A/B measurements and tests)
     int np_dlo = 2;        // digit sums below 256^np_dlo are dropped from the fixed-point updates (error budget: np_block)
     Dev dUl, dUscale, dNz, dMma;
     // highest non-zero digit plane of z per 256-block [0, n256), per 1024-block [n256, n256 + n1024), per 4096-block
@@ -907,11 +908,11 @@ qf_status samp_p_pert_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t s
 // gpv_ring.rs:160-212)
 // ---------------------------------------------------------------------------
 // Block sizes of the recursion: 64-wide diagonal blocks are sequential per target (np_diag, which also applies the rank-64
-// updates inside its 256-block); the updates between 256-blocks inside a 1024-block, between 1024-blocks inside a
-// 4096-block and between 4096-blocks run on tcgen05 (fixed-point digits); fp64 GEMMs (gemm_f64) remain for dimensions
-// below the tensor-core threshold.  The top level contracts K = 4096 coordinates per launch: its epilogue
-// (a read-modify-write of T, serialised with the MMAs because TMEM holds one tile) is paid once per 4096 instead of
-// once per 1024 coordinates.
+// updates inside its 256-block); the updates between 256-blocks run on tcgen05 (fixed-point digits), left-looking inside a
+// 4096-block and right-looking between 4096-blocks (np_block); fp64 GEMMs (gemm_f64) remain for dimensions below the
+// tensor-core threshold.  The 1024 level only places the rejection-sampling proposals (and, in the right-looking order,
+// the updates between its blocks).  The epilogue of an update (a read-modify-write of T, serialised with the MMAs because
+// TMEM holds one tile) is paid once per column of T and 4096-block, so most MACs run in launches of long K.
 constexpr long NP_SIZES[4] = {64, 256, 1024, 4096};
 constexpr int NP_TOP = 4;
 constexpr long NP_SCALE_BLOCK = NP_SIZES[3];  // column block over which the digits of U share one scale per row
@@ -953,11 +954,58 @@ static inline int np_block_index(long col, long D, long S) {
     return (int)(std::min(col, np_last_block_start(D, S)) / S);
 }
 
+// T[:, r0:r1] -= Z[:, c0:c1] U[r0:r1, c0:c1]^t for rows r1 <= c0 in earlier 256-blocks than every column, [c0, c1) inside one
+// NP_SCALE_BLOCK column block: the digit planes of z (written block by block during the recursion) against the fixed-point
+// digits of U, one scale per row; in fp64 below K = 256 (a thin block: per-tile overheads dominate the tensor-core path).
+// gate: the highest non-zero digit plane of z over [c0, c1) (or a device int that bounds it).
+// Exactness: K = c1 - c0 < NP_SCALE_BLOCK + NP_THIN < 2^13 (the longest left-looking launch at C2: 3904), so one digit pair sums to
+// < 2^13 * 2^14 = 2^27 and a digit sum of at most min(LX, LW) <= 3 pairs (z digits x U digits) to < 2^28.6: int32 holds it
+// exactly.  The digit sums are linear in the K range, so the integer V of one launch over [c0, c1) equals the sum of launches
+// over any partition of it; only the fp64 roundings of T -= V * scale depend on how the columns are grouped.
+static qf_status np_update(qf_ctx* ctx, double* T, const double* Z, int Bc, long r0, long r1, long c0, long c1, const int* gate) {
+    const long D = ctx->dim, ldD = ctx->ld_dim;
+    if (c1 - c0 < NP_SIZES[1]) {
+        const double* U = ctx->dU.as<double>();
+        LAUNCH(ctx_gemm(ctx, Z + c0, ldD, U + r0 * ldD + c0, ldD, T + r0, ldD, Bc, (int)(r1 - r0), (int)(c1 - c0), -1.0, 1.0, 0));
+        return QF_OK;
+    }
+    const long ldk = ctx->ldk_dim, plane = (long)ctx->chunk * ldk;
+    I8GemmArgs g{};
+    g.x = ctx->w[8].as<int8_t>() + c0; g.ldx = ldk; g.x_plane = plane;
+    // (two-phase recursion: only the top planes of U that the phase's error budget needs)
+    const int wdrop = ctx->np_wdrop_cur;
+    g.w = ctx->dUl.as<int8_t>() + (size_t)wdrop * D * ldk + r0 * ldk + c0; g.ldw = ldk; g.w_plane = D * ldk;
+    g.LX = ctx->z_limbs; g.LW = ctx->u_limbs - wdrop; g.w_signed = 1;
+    g.scale_mul = std::ldexp(1.0, 8 * wdrop);
+    g.B = Bc; g.N = (int)(r1 - r0); g.K = (int)(c1 - c0);
+    g.out_kind = 3; g.sign = 1; g.q = 0; g.base = nullptr; g.ldbase = 0; g.out = T + r0; g.ldout = ldD;
+    g.flag = ctx->dFlag.as<int>();
+    // (the merged partition: a ragged top column block shares the scales of the block below it)
+    g.scale = ctx->dUscale.as<double>() + np_block_index(c0, D, NP_SCALE_BLOCK) * D + r0;
+    g.x_nz = ctx->dNz.as<uint8_t>(); g.nz_m_tiles = (int)((ctx->chunk + 127) / 128); g.nz_kb_total = (int)(ldk / 128);
+    g.nz_kb_off = (int)(c0 / 128); g.nz_m_off = 0;
+    // Dropped digit sums d < np_dlo: per launch |error| <= K 2^14 256^(d_lo - 1) d_lo scale_row (scale_row =
+    // row maximum of |U| / (127 256^6)), i.e. < 2^-27 |U|max K^(1/2) typically at d_lo = 2 -- four orders
+    // below the 2^-12 the centres need (the widths s / ||b~_i|| are >= 2.3), and below the fp64 rounding of T
+    // at |T| ~ 2^24.
+    g.d_lo = ctx->np_dlo_cur;
+    return gemm_i8_gated(ctx, g, gate, ctx->np_lx_min);
+}
+
 // Process coordinates [lo, hi) in descending order.  Precondition: T[:, lo:hi] already carries the
 // updates of every coordinate >= hi.  level 0 = one sequential diagonal block.  prop0 = first coordinate of the
-// enclosing 1024-level block (origin of the pre-generated proposals).
-qf_status np_block(qf_ctx* ctx, double* T, double* Z, int Bc, long lo, long hi, int level, long prop0, uint64_t seed,
-                   uint64_t first) {
+// enclosing 1024-level block (origin of the pre-generated proposals), q_hi = top of the enclosing 4096-level block.
+//
+// Order of the tensor-core updates.  The 4096 level is right-looking: after each finished 4096-block, one launch updates
+// every coordinate below it.  Inside a 4096-block the updates are left-looking: before the diagonal kernel samples 256-block
+// [sub_lo, sub_hi), one launch applies everything still pending from the finished coordinates of the same 4096-block,
+//   T[:, sub_lo:sub_hi] -= Z[:, sub_hi:q_hi] U[sub_lo:sub_hi, sub_hi:q_hi]^t   (N = 256, K = 256 .. 3840 in a full block),
+// so every column of T is read and written once per 4096-block, and most MACs run at long K.  The right-looking order
+// (ctx->np_right) launches after each finished 256-block (rows of the rest of its 1024-block, K = 256) and after each
+// finished 1024-block (rows of the rest of its 4096-block, K = 1024): the same entries of U and the same MACs, but
+// each column of T takes 1.5 passes at each of the two levels.
+qf_status np_block(qf_ctx* ctx, double* T, double* Z, int Bc, long lo, long hi, int level, long prop0, long q_hi,
+                   uint64_t seed, uint64_t first) {
     const long D = ctx->dim, ldD = ctx->ld_dim;
     const double* U = ctx->dU.as<double>();
     if (level == 0) {
@@ -983,9 +1031,10 @@ qf_status np_block(qf_ctx* ctx, double* T, double* Z, int Bc, long lo, long hi, 
     }
     if (level == 1 && ctx->np_fuse64 && (lo & 63) == 0)
         // a whole 256-block in one launch: its diagonal blocks and the rank-64 updates between them (lattice.cu)
-        return np_block(ctx, T, Z, Bc, lo, hi, 0, prop0, seed, first);
+        return np_block(ctx, T, Z, Bc, lo, hi, 0, prop0, q_hi, seed, first);
     const long step = NP_SIZES[level - 1];
     const bool i8_level = level >= 2 && ctx->use_ozaki;
+    const bool left = i8_level && !ctx->np_right;
     for (long sub_hi = hi; sub_hi > lo;) {
         long sub_lo = std::max(lo, (sub_hi - 1) / step * step);
         // tensor-core levels: the ragged top of the whole recursion joins the block below it (the digit planes of U are
@@ -999,50 +1048,28 @@ qf_status np_block(qf_ctx* ctx, double* T, double* Z, int Bc, long lo, long hi, 
                                         seed, first, ctx->stream));
             prop0 = sub_lo;
         }
-        QF_TRY(np_block(ctx, T, Z, Bc, sub_lo, sub_hi, level - 1, prop0, seed, first));
+        int* gates = ctx->dGate.as<int>();
+        // running maximum of the digit counts over the finished 256-blocks of the enclosing 4096-block (np_diag)
+        int* gate4 = i8_level ? gates + ctx->gate_n256 + ctx->gate_n1024 + np_block_index(sub_lo, D, NP_SIZES[3]) : nullptr;
+        // left-looking: everything pending from [sub_hi, q_hi) before this 256-block is sampled (none for the top block)
+        if (left && level == 2 && sub_hi < q_hi) QF_TRY(np_update(ctx, T, Z, Bc, sub_lo, sub_hi, sub_hi, q_hi, gate4));
+        QF_TRY(np_block(ctx, T, Z, Bc, sub_lo, sub_hi, level - 1, prop0, level == NP_TOP ? sub_hi : q_hi, seed, first));
         if (i8_level) {
-            const long ldk = ctx->ldk_dim, plane = (long)ctx->chunk * ldk;
-            const int nz_m = (int)((ctx->chunk + 127) / 128), nz_kb = (int)(ldk / 128);
-            int8_t* zp = ctx->w[8].as<int8_t>();
-            int* gates = ctx->dGate.as<int>();
             int* gate0 = gates + np_block_index(sub_lo, D, NP_SIZES[1]);
             int* gate1 = gates + ctx->gate_n256 + np_block_index(sub_lo, D, NP_SIZES[2]);
-            int* gate4 = gates + ctx->gate_n256 + ctx->gate_n1024 + np_block_index(sub_lo, D, NP_SIZES[3]);
-            int* gate_z2 = gates + ctx->gate_n256 + ctx->gate_n1024 + ctx->gate_n4096;
-            // digits of the finished 256-block of z (kept: the levels above and the final S z reuse them) -- unless the
+            // digits of the finished 256-block of z (kept: the later updates and the final S z reuse them) -- unless the
             // diagonal-block kernels have written them already
-            if (level == 2 && !ctx->np_fuse_split)
-                LAUNCH(qf_launch_split_f64_limbs(Z + sub_lo, ldD, zp + sub_lo, plane, ldk, Bc, (int)(sub_hi - sub_lo), ctx->z_limbs,
-                                                 ctx->dFlag.as<int>(), ctx->dNz.as<uint8_t>(), nz_m, nz_kb, (int)sub_lo,
-                                                 ctx->stream, gate0, gate1, gate4,
-                                                 (ctx->gpv_struct && sub_hi > ctx->nk) ? gate_z2 : nullptr));
-            // the update of the rows above it (within the enclosing block) on the tensor cores:
-            //   T[:, lo:sub_lo] -= (z digits) x (fixed-point digits of U) * 2^-e
-            if (sub_lo > lo && sub_hi - sub_lo < NP_SIZES[1]) {
-                // a thin block: per-tile overheads dominate the tensor-core path, use fp64
-                LAUNCH(ctx_gemm(ctx, Z + sub_lo, ldD, U + lo * ldD + sub_lo, ldD, T + lo, ldD, Bc, (int)(sub_lo - lo),
-                                (int)(sub_hi - sub_lo), -1.0, 1.0, 0));
-            } else if (sub_lo > lo) {
-                I8GemmArgs g{};
-                g.x = zp + sub_lo; g.ldx = ldk; g.x_plane = plane;
-                // (two-phase recursion: only the top planes of U that the phase's error budget needs)
-                const int wdrop = ctx->np_wdrop_cur;
-                g.w = ctx->dUl.as<int8_t>() + (size_t)wdrop * D * ldk + lo * ldk + sub_lo; g.ldw = ldk; g.w_plane = D * ldk;
-                g.LX = ctx->z_limbs; g.LW = ctx->u_limbs - wdrop; g.w_signed = 1;
-                g.scale_mul = std::ldexp(1.0, 8 * wdrop);
-                g.B = Bc; g.N = (int)(sub_lo - lo); g.K = (int)(sub_hi - sub_lo);
-                g.out_kind = 3; g.sign = 1; g.q = 0; g.base = nullptr; g.ldbase = 0; g.out = T + lo; g.ldout = ldD;
-                g.flag = ctx->dFlag.as<int>();
-                g.scale = ctx->dUscale.as<double>() + (sub_lo / NP_SCALE_BLOCK) * D + lo;
-                g.x_nz = ctx->dNz.as<uint8_t>(); g.nz_m_tiles = nz_m; g.nz_kb_total = nz_kb;
-                g.nz_kb_off = (int)(sub_lo / 128); g.nz_m_off = 0;
-                // Dropped digit sums d < np_dlo: per launch |error| <= K 2^14 256^(d_lo - 1) d_lo scale_row (scale_row =
-                // row maximum of |U| / (127 256^6)), i.e. < 2^-27 |U|max K^(1/2) typically at d_lo = 2 -- four orders
-                // below the 2^-12 the centres need (the widths s / ||b~_i|| are >= 2.3), and below the fp64 rounding of T
-                // at |T| ~ 2^24.
-                g.d_lo = ctx->np_dlo_cur;
-                QF_TRY(gemm_i8_gated(ctx, g, level == 2 ? gate0 : level == 3 ? gate1 : gate4, ctx->np_lx_min));
+            if (level == 2 && !ctx->np_fuse_split) {
+                const long ldk = ctx->ldk_dim, plane = (long)ctx->chunk * ldk;
+                int* gate_z2 = gates + ctx->gate_n256 + ctx->gate_n1024 + ctx->gate_n4096;
+                LAUNCH(qf_launch_split_f64_limbs(Z + sub_lo, ldD, ctx->w[8].as<int8_t>() + sub_lo, plane, ldk, Bc, (int)(sub_hi - sub_lo),
+                                                 ctx->z_limbs, ctx->dFlag.as<int>(), ctx->dNz.as<uint8_t>(),
+                                                 (int)((ctx->chunk + 127) / 128), (int)(ldk / 128), (int)sub_lo, ctx->stream, gate0,
+                                                 gate1, gate4, (ctx->gpv_struct && sub_hi > ctx->nk) ? gate_z2 : nullptr));
             }
+            // right-looking: the update of the rows below it within the enclosing block
+            if (sub_lo > lo && (level == NP_TOP || !left))
+                QF_TRY(np_update(ctx, T, Z, Bc, lo, sub_lo, sub_lo, sub_hi, level == 2 ? gate0 : level == 3 ? gate1 : gate4));
         } else if (sub_lo > lo) {
             LAUNCH(ctx_gemm(ctx, Z + sub_lo, ldD, U + lo * ldD + sub_lo, ldD, T + lo, ldD, Bc, (int)(sub_lo - lo),
                             (int)(sub_hi - sub_lo), -1.0, 1.0, 0));
@@ -1119,7 +1146,7 @@ qf_status samp_p_np1_chunk(qf_ctx* ctx, const int64_t* dUin, int Bc, uint64_t se
         CK(cudaMemsetAsync(ctx->dGate.p, 0, gb, ctx->stream));
     }
     ctx->np_wdrop_cur = 0; ctx->np_dlo_cur = ctx->np_dlo; ctx->np_lx_min = 3;
-    QF_TRY(np_block(ctx, T, Z, Bc, 0, D, NP_TOP, 0, seed, first));
+    QF_TRY(np_block(ctx, T, Z, Bc, 0, D, NP_TOP, 0, D, seed, first));
     // e = sol + S z   (exact integers)
     if (ctx->use_i8) {
         // z -> balanced base-256 digits, S z on the tensor cores, then add sol on its pivot columns
@@ -1262,7 +1289,7 @@ qf_status np2_phase1(qf_ctx* ctx, int Bc, uint64_t seed, uint64_t first) {
     double* T = ctx->w[2].as<double>();
     CK(cudaMemset2DAsync(T + nk, (size_t)ldD * 8, 0, (size_t)ctx->m_bar * 8, (size_t)Bc, ctx->stream));
     ctx->np_wdrop_cur = ctx->u_limbs - ctx->u22_limbs; ctx->np_dlo_cur = ctx->u22_dlo; ctx->np_lx_min = 3;
-    return np_block(ctx, T, ctx->w[3].as<double>(), Bc, nk, D, NP_TOP, 0, seed, first);
+    return np_block(ctx, T, ctx->w[3].as<double>(), Bc, nk, D, NP_TOP, 0, D, seed, first);
 }
 
 // out = (base - A_bar z2) mod q, exact (base == nullptr: -A_bar z2 mod q).  A_bar = the first m_bar columns of the installed
@@ -1340,8 +1367,13 @@ qf_status np2_finish(qf_ctx* ctx, const int64_t* H, int Bc, uint64_t seed, uint6
     else
         QF_TRY(np2_mt1_z2(ctx, Bc, T, ldD, ctx->dMt1scale.as<double>(), 0));
     // ---- phase 2: coordinates nk-1 .. 0
+    // The digit-count gates of the 256-, 1024- and 4096-blocks are indexed by column block of the whole dimension: a block
+    // of phase 2 may share its slot with one of phase 1 (C2: [4096, 8192) holds phase 1's [6144, 8192) and phase 2's
+    // [4096, 6144)), whose three-digit z2 would select the three-digit variant of every phase-2 launch reading it.  Phase 2
+    // starts from zero; the gate of z2 behind them is kept.
+    CK(cudaMemsetAsync(ctx->dGate.p, 0, (size_t)(ctx->gate_n256 + ctx->gate_n1024 + ctx->gate_n4096) * sizeof(int), ctx->stream));
     ctx->np_wdrop_cur = ctx->u_limbs - ctx->u11_limbs; ctx->np_dlo_cur = ctx->u11_dlo; ctx->np_lx_min = 2;
-    QF_TRY(np_block(ctx, T, Z, Bc, 0, nk, NP_TOP, 0, seed, first));
+    QF_TRY(np_block(ctx, T, Z, Bc, 0, nk, NP_TOP, 0, nk, seed, first));
 
     // ---- e_bot = g3 + S' z1,  e_top = z2 + R e_bot
     const long plane2 = C * ldk_nk;
@@ -2474,6 +2506,8 @@ qf_status qf_ctx_create(const qf_params* p, int device, qf_ctx** out) {
         ctx->np_fuse64 = !(envu && envu[0] == '1');
         const char* envs = getenv("QF_DISABLE_NP_FUSE_SPLIT");  // test switch: separate digit-split launches
         ctx->np_fuse_split = !(envs && envs[0] == '1');
+        const char* envo = getenv("QF_NP_ORDER");  // test switch: "right" = the right-looking update order inside a 4096-block
+        ctx->np_right = envo && strcmp(envo, "right") == 0;
         const char* envv = getenv("QF_NP_DIAG_V1");  // test switch: the quad-per-two-targets diagonal-block kernel
         ctx->np_diag_variant = (envv && envv[0] == '1') ? 1 : 0;
         if (const char* envc = getenv("QF_CHUNK")) ctx->chunk_env = atol(envc);  // experiments: targets per internal chunk
