@@ -253,11 +253,29 @@ qf_status qf_ring_set_key_table(qf_ctx* ctx, const int64_t* keys, int64_t nkeys)
  * host before any launch (QF_ERR_INVALID outside [0, nkeys)), in_domain may be NULL, QF_ERR_NOT_IN_DOMAIN when a flag is
  * 0.  qf_ring_f_a_keyed_dev takes device pointers and is asynchronous (in_domain mandatory): an index outside the table
  * is never used to address it, its row is unspecified and the next qf_synchronize returns QF_ERR_INVALID.  QF_ERR_NO_KEY
- * without a table.  An empty batch is valid.  For int16 or packed sigma, decode first (qf_domain_decode_dev). */
+ * without a table.  An empty batch is valid.  For sigma in the packed code of qf_domain_code_params, use
+ * qf_ring_f_a_keyed_packed[_dev] below; int16 sigma is widened first. */
 qf_status qf_ring_f_a_keyed(qf_ctx* ctx, const int32_t* sigma, const int32_t* key_idx, int64_t batch, int64_t* u_out,
                             uint8_t* in_domain);
 qf_status qf_ring_f_a_keyed_dev(qf_ctx* ctx, const int32_t* sigma, const int32_t* key_idx, int64_t batch, int64_t* u_out,
                                 uint8_t* in_domain);
+/* qf_ring_f_a_keyed on packed sigma: packed is batch x slot_bytes, slot b the code (parameter k) of sigma[b] as
+ * qf_f_a_packed reads it.  For a slot that decodes to a row in the domain, u[b] is bit-identical to qf_ring_f_a_keyed on
+ * that row; in_domain[b] = check_domain(sigma[b]) AND slot b is canonical (a non-canonical slot has an unspecified u), for
+ * any split into calls and chunks.  Checks in this order: NULL pointers or batch < 0 (QF_ERR_INVALID), a classical context
+ * (QF_ERR_INVALID), k / slot_bytes as for qf_f_a_packed (QF_ERR_INVALID before any launch), an empty batch (QF_OK), no
+ * table (QF_ERR_NO_KEY).  The ring_small (n <= 512) and Goldilocks kernels decode the slots themselves; the schoolbook
+ * family and n = 1024 decode into an int32 staging buffer first.
+ * qf_ring_f_a_keyed_packed: host pointers.  Key indices are checked on the host before any launch; u_out is mandatory,
+ * in_domain may be NULL, and a 0 flag returns QF_ERR_NOT_IN_DOMAIN.  The slots and indices of chunk i+1 go in, and the
+ * results of chunk i-1 come out, while chunk i is computed: pin packed, key_idx, u_out (cudaHostRegister) or the copies
+ * serialise.
+ * qf_ring_f_a_keyed_packed_dev: device pointers, asynchronous, in_domain mandatory, packed 16-byte aligned (else
+ * QF_ERR_INVALID).  A bad key index is reported at the next qf_synchronize, as for qf_ring_f_a_keyed_dev. */
+qf_status qf_ring_f_a_keyed_packed(qf_ctx* ctx, const uint8_t* packed, const int32_t* key_idx, int64_t batch, int k,
+                                   int64_t slot_bytes, int64_t* u_out, uint8_t* in_domain);
+qf_status qf_ring_f_a_keyed_packed_dev(qf_ctx* ctx, const uint8_t* packed, const int32_t* key_idx, int64_t batch, int k,
+                                       int64_t slot_bytes, int64_t* u_out, uint8_t* in_domain);
 /* count ring TrapGen keys at once (host pointers): a_bar count x n residues in [0, q) (QF_ERR_INVALID otherwise), r and e
  * count x k x n small coefficients; a_out count x (k+2) x n.  Key t is bit-identical to qf_ring_trap_gen_from(a_bar_t,
  * r_t, e_t).  Unlike that call it installs nothing: the context key, its trapdoor and the key table stay as they were.

@@ -73,6 +73,8 @@ extern "C" {
     pub fn qf_ring_set_key_table(ctx: *mut qf_ctx, keys: *const i64, nkeys: i64) -> i32;
     pub fn qf_ring_f_a_keyed(ctx: *mut qf_ctx, sigma: *const i32, key_idx: *const i32, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
     pub fn qf_ring_f_a_keyed_dev(ctx: *mut qf_ctx, sigma: *const i32, key_idx: *const i32, batch: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
+    pub fn qf_ring_f_a_keyed_packed(ctx: *mut qf_ctx, packed: *const u8, key_idx: *const i32, batch: i64, k: i32, slot_bytes: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
+    pub fn qf_ring_f_a_keyed_packed_dev(ctx: *mut qf_ctx, packed: *const u8, key_idx: *const i32, batch: i64, k: i32, slot_bytes: i64, u_out: *mut i64, in_domain: *mut u8) -> i32;
     pub fn qf_ring_trap_gen_batch_from(ctx: *mut qf_ctx, count: i64, a_bar: *const i64, r: *const i32, e: *const i32, a_out: *mut i64) -> i32;
     pub fn qf_samp_d(ctx: *mut qf_ctx, batch: i64, seed: u64, first_index: u64, out: *mut i32) -> i32;
     pub fn qf_samp_d_dev(ctx: *mut qf_ctx, batch: i64, seed: u64, first_index: u64, out: *mut i32) -> i32;

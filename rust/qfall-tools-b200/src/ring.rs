@@ -278,15 +278,7 @@ impl PSFGPVRingB200 {
     /// back; the installed key of `f_a` / `samp_p` is not touched.  Panics like `f_a` when a sigma is outside D_n.
     pub fn f_a_keyed_batch(&self, keys: &[MatPolynomialRingZq], sigmas: &[MatPolyOverZ], key_of: &[usize]) -> Vec<MatPolynomialRingZq> {
         assert_eq!(sigmas.len(), key_of.len(), "one key index per sigma");
-        let mut kw = Vec::with_capacity(keys.len() * self.n() * (self.k() + 2));
-        for a in keys {
-            kw.extend(self.key_words(a));
-        }
-        if self.installed_keys.borrow().as_ref() != Some(&kw) {
-            let st = unsafe { qf_ring_set_key_table(self.ctx.raw, kw.as_ptr(), keys.len() as i64) };
-            self.ctx.check(st, "qf_ring_set_key_table");
-            *self.installed_keys.borrow_mut() = Some(kw);
-        }
+        self.install_key_table(keys);
         let (n, d) = (self.n(), self.n() * (self.k() + 2));
         let mut sg = Vec::with_capacity(sigmas.len() * d);
         for sigma in sigmas {
@@ -301,6 +293,44 @@ impl PSFGPVRingB200 {
         assert!(st != QF_ERR_NOT_IN_DOMAIN && ok.iter().all(|f| *f == 1), "sigma is not in D_n");
         self.ctx.check(st, "qf_ring_f_a_keyed");
         u.chunks(n).map(|row| self.range_from_words(row)).collect()
+    }
+
+    /// `f_a_keyed_batch` on packed signatures (qf_ring_f_a_keyed_packed): row b of `packed` is the code of sigma b, as
+    /// `samp_p_batch_packed` returns it, decoded on the device inside the keyed kernels.  Panics like `f_a` when a sigma is
+    /// outside D_n or its code is not canonical.
+    pub fn f_a_keyed_batch_packed(&self, keys: &[MatPolynomialRingZq], packed: &PackedDomain, key_of: &[usize]) -> Vec<MatPolynomialRingZq> {
+        assert_eq!(packed.rows.len(), key_of.len(), "one key index per sigma");
+        self.install_key_table(keys);
+        let (n, slot) = (self.n(), packed.slot_bytes as usize);
+        let mut buf = vec![0u8; packed.rows.len() * slot];
+        for (dst, row) in buf.chunks_mut(slot).zip(&packed.rows) {
+            assert!(row.len() <= slot, "a packed row is longer than its slot");
+            dst[..row.len()].copy_from_slice(row);
+        }
+        let idx: Vec<i32> = key_of.iter().map(|&t| i32::try_from(t).expect("key index below 2^31")).collect();
+        let b = packed.rows.len();
+        let mut u = vec![0i64; b * n];
+        let mut ok = vec![0u8; b];
+        let st = unsafe {
+            qf_ring_f_a_keyed_packed(self.ctx.raw, buf.as_ptr(), idx.as_ptr(), b as i64, packed.k, packed.slot_bytes,
+                                     u.as_mut_ptr(), ok.as_mut_ptr())
+        };
+        assert!(st != QF_ERR_NOT_IN_DOMAIN && ok.iter().all(|f| *f == 1), "sigma is not in D_n");
+        self.ctx.check(st, "qf_ring_f_a_keyed_packed");
+        u.chunks(n).map(|row| self.range_from_words(row)).collect()
+    }
+
+    // the key table of the keyed calls: uploaded once and kept while the same keys come back
+    fn install_key_table(&self, keys: &[MatPolynomialRingZq]) {
+        let mut kw = Vec::with_capacity(keys.len() * self.n() * (self.k() + 2));
+        for a in keys {
+            kw.extend(self.key_words(a));
+        }
+        if self.installed_keys.borrow().as_ref() != Some(&kw) {
+            let st = unsafe { qf_ring_set_key_table(self.ctx.raw, kw.as_ptr(), keys.len() as i64) };
+            self.ctx.check(st, "qf_ring_set_key_table");
+            *self.installed_keys.borrow_mut() = Some(kw);
+        }
     }
 
     /// gen_trapdoor_ring_lwe (gadget_ring.rs:62-81) for many (a_bar, r, e) in one call (qf_ring_trap_gen_batch_from): key t

@@ -70,6 +70,8 @@ SIGNATURES = {
     "qf_ring_set_key_table": (_i32, [_vp, _vp, _i64]),
     "qf_ring_f_a_keyed": (_i32, [_vp, _vp, _vp, _i64, _vp, _vp]),
     "qf_ring_f_a_keyed_dev": (_i32, [_vp, _vp, _vp, _i64, _vp, _vp]),
+    "qf_ring_f_a_keyed_packed": (_i32, [_vp, _vp, _vp, _i64, _i32, _i64, _vp, _vp]),
+    "qf_ring_f_a_keyed_packed_dev": (_i32, [_vp, _vp, _vp, _i64, _i32, _i64, _vp, _vp]),
     "qf_ring_trap_gen_batch_from": (_i32, [_vp, _i64, _vp, _vp, _vp, _vp]),
     "qf_samp_d": (_i32, [_vp, _i64, _u64, _u64, _vp]),
     "qf_samp_d_dev": (_i32, [_vp, _i64, _u64, _u64, _vp]),

@@ -748,6 +748,35 @@ qf_status ring_f_a_keyed_chunk(qf_ctx* ctx, const int32_t* dSigma, const int32_t
     return QF_OK;
 }
 
+// The same on packed rows (qf_ring_f_a_keyed_packed): dPacked holds Bc slots of slot_bytes.  The ring_small (n <= 512) and
+// Goldilocks kernels decode the slots themselves and write the canonical byte of every row into dFlags; the schoolbook
+// family (and ring_small at n = 1024) decodes into the int32 staging buffer io_a first.  The domain check is then ANDed in.
+qf_status ring_f_a_keyed_packed_chunk(qf_ctx* ctx, const uint8_t* dPacked, const int32_t* dKidx, int Bc, int k,
+                                      int64_t slot_bytes, int64_t* dU, uint8_t* dFlags) {
+    CK(ctx->dNorm.ensure((size_t)std::max<int64_t>(ctx->chunk, Bc) * 8));
+    unsigned long long* norm2 = ctx->dNorm.as<unsigned long long>();
+    const int n = (int)ctx->n, npoly = (int)(ctx->k + 2), family = ctx->key_family;
+    const unsigned long long q = ctx->prm.q;
+    if (family == 1 || (family == 2 && qf_ring_small_packed_fused(n))) {
+        const PackedRows pk{dPacked, slot_bytes, qf_domain_h0(ctx->dim, k), (int)ctx->dim, k, dFlags};
+        int* flag = ctx->dFlag.as<int>();
+        if (family == 2)
+            LAUNCH(qf_launch_ring_small(nullptr, ctx->dKeyTab.as<uint32_t>(), dU, norm2, Bc, npoly, n, ctx->key_d, q,
+                                        ctx->key_np_inv, ctx->dKeyTw.as<uint32_t>(), ctx->stream, dKidx, (int)ctx->key_count,
+                                        flag, &pk));
+        else
+            LAUNCH(qf_launch_ring_f_a(nullptr, ctx->dKeyTab.as<uint64_t>(), dU, norm2, Bc, npoly, n, q,
+                                      ctx->dKeyTw.as<uint64_t>(), ctx->stream, dKidx, (int)ctx->key_count, flag, &pk));
+    } else {
+        CK(ctx->io_a.ensure((size_t)std::max<int64_t>(ctx->chunk, Bc) * ctx->dim * 4));
+        LAUNCH(qf_launch_domain_decode(dPacked, Bc, (int)ctx->dim, k, slot_bytes, ctx->io_a.as<int32_t>(), dFlags, ctx->stream));
+        QF_TRY(ring_keyed_launch(ctx, family, ctx->key_d, ctx->key_np_inv, ctx->dKeyTw, ctx->dKeyTab, ctx->key_count,
+                                 ctx->io_a.as<int32_t>(), dKidx, Bc, npoly, dU, norm2));
+    }
+    LAUNCH(qf_launch_domain_flags_and(norm2, ctx->bound, dFlags, Bc, ctx->stream));
+    return QF_OK;
+}
+
 // ---------------------------------------------------------------------------
 // PSFPerturbation::samp_p on one chunk (mp_perturbation.rs:304-336)
 // ---------------------------------------------------------------------------
@@ -3625,13 +3654,8 @@ static qf_status ring_keyed_ready(qf_ctx* ctx) {
     return QF_OK;
 }
 
-qf_status qf_ring_f_a_keyed(qf_ctx* ctx, const int32_t* sigma, const int32_t* key_idx, int64_t batch, int64_t* u_out,
-                            uint8_t* in_domain) {
-    if (!ctx || batch < 0 || (batch > 0 && (!sigma || !key_idx || !u_out))) return QF_ERR_INVALID;
-    if (ctx->prm.kind != QF_PSF_GPV_RING) return ring_keyed_ready(ctx);
-    if (batch == 0) return QF_OK;
-    CK(cudaSetDevice(ctx->device));
-    QF_TRY(ring_keyed_ready(ctx));
+// key indices of a host batch, checked before any launch
+static qf_status check_key_idx(qf_ctx* ctx, const int32_t* key_idx, int64_t batch) {
     for (int64_t b = 0; b < batch; ++b)
         if (key_idx[b] < 0 || key_idx[b] >= ctx->key_count) {
             char buf[128];
@@ -3639,6 +3663,17 @@ qf_status qf_ring_f_a_keyed(qf_ctx* ctx, const int32_t* sigma, const int32_t* ke
                      (int)key_idx[b]);
             return ctx->fail(QF_ERR_INVALID, buf);
         }
+    return QF_OK;
+}
+
+qf_status qf_ring_f_a_keyed(qf_ctx* ctx, const int32_t* sigma, const int32_t* key_idx, int64_t batch, int64_t* u_out,
+                            uint8_t* in_domain) {
+    if (!ctx || batch < 0 || (batch > 0 && (!sigma || !key_idx || !u_out))) return QF_ERR_INVALID;
+    if (ctx->prm.kind != QF_PSF_GPV_RING) return ring_keyed_ready(ctx);
+    if (batch == 0) return QF_OK;
+    CK(cudaSetDevice(ctx->device));
+    QF_TRY(ring_keyed_ready(ctx));
+    QF_TRY(check_key_idx(ctx, key_idx, batch));
     const long C = ctx->chunk;
     CK(ctx->io_a.ensure((size_t)C * ctx->dim * 4));
     CK(ctx->io_b.ensure((size_t)C * ctx->n * 8));
@@ -3785,6 +3820,19 @@ struct SampOut {
     size_t row_bytes(long dim) const { return kind == I32 ? (size_t)dim * 4 : kind == I16 ? (size_t)dim * 2 : (size_t)slot_bytes; }
 };
 
+// the second stream and the events of the host calls that overlap their copies with the computation (created once)
+static qf_status ensure_copy_stream(qf_ctx* ctx) {
+    if (ctx->copy_stream) return QF_OK;
+    CK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+    for (int i = 0; i < 2; ++i) {
+        CK(cudaEventCreateWithFlags(&ctx->ev_done[i], cudaEventDisableTiming));
+        CK(cudaEventCreateWithFlags(&ctx->ev_copied[i], cudaEventDisableTiming));
+        CK(cudaEventCreateWithFlags(&ctx->ev_u_in[i], cudaEventDisableTiming));
+        CK(cudaEventCreateWithFlags(&ctx->ev_u_used[i], cudaEventDisableTiming));
+    }
+    return QF_OK;
+}
+
 // host-buffer samp_p in one of the SampOut forms
 // tidx (optional, host): tag index of every target in the installed tag table (qf_samp_p_tagged), copied with the targets
 // pool_slot0 >= 0: the online half of the pool entries from that slot on (qf_samp_p_online; seed and first unused)
@@ -3817,15 +3865,7 @@ static qf_status samp_p_host(qf_ctx* ctx, const int64_t* u, int64_t batch, uint6
         } else CK(ctx->io_a2.ensure((size_t)C * ctx->dim * 4));
         CK(ctx->io_b2.ensure((size_t)C * ctx->n * 8));
         if (tidx) CK(ctx->io_t[1].ensure((size_t)C * 4));
-        if (!ctx->copy_stream) {
-            CK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
-            for (int i = 0; i < 2; ++i) {
-                CK(cudaEventCreateWithFlags(&ctx->ev_done[i], cudaEventDisableTiming));
-                CK(cudaEventCreateWithFlags(&ctx->ev_copied[i], cudaEventDisableTiming));
-                CK(cudaEventCreateWithFlags(&ctx->ev_u_in[i], cudaEventDisableTiming));
-                CK(cudaEventCreateWithFlags(&ctx->ev_u_used[i], cudaEventDisableTiming));
-            }
-        }
+        QF_TRY(ensure_copy_stream(ctx));
     }
     // chunk boundaries (the same balanced split as for_chunks)
     const int64_t nch = std::max<int64_t>(1, (batch + C - 1) / C);
@@ -4161,6 +4201,109 @@ qf_status qf_f_a_packed(qf_ctx* ctx, const uint8_t* packed, const int32_t* tag_i
     if (in_domain) memcpy(in_domain, flags.data(), (size_t)batch);
     if (!all) return ctx->fail(QF_ERR_NOT_IN_DOMAIN, "f_a: a packed sigma is not canonical or not in the domain D_n");
     return QF_OK;
+}
+
+// ---- ring f_a with a key per target on packed sigma (DESIGN 4.13) ---------------------------------------------------------
+static const char* kPackedArgsMsg =
+    "packed Domain code: k outside [0, 30] or slot_bytes not a multiple of 16 of at least H0 + ceil(dim / 8)";
+
+// Host buffers.  Chunk i's slots and key indices go to the device (io_p[i & 1], io_n[i & 1]) and chunk i's u and flags come
+// back (io_b / io_b2, io_c halves) on the second stream while the kernels of the neighbouring chunk run, as in samp_p_host;
+// only the first chunk's input and the last chunk's output are exposed.  Pageable host memory serialises these copies.
+qf_status qf_ring_f_a_keyed_packed(qf_ctx* ctx, const uint8_t* packed, const int32_t* key_idx, int64_t batch, int k,
+                                   int64_t slot_bytes, int64_t* u_out, uint8_t* in_domain) {
+    if (!ctx || batch < 0 || (batch > 0 && (!packed || !key_idx || !u_out))) return QF_ERR_INVALID;
+    if (ctx->prm.kind != QF_PSF_GPV_RING) return ring_keyed_ready(ctx);
+    if (!packed_args_ok(ctx->dim, k, slot_bytes)) return ctx->fail(QF_ERR_INVALID, kPackedArgsMsg);
+    if (batch == 0) return QF_OK;
+    CK(cudaSetDevice(ctx->device));
+    QF_TRY(ring_keyed_ready(ctx));
+    QF_TRY(check_key_idx(ctx, key_idx, batch));
+    const long C = ctx->chunk, n = ctx->n;
+    const bool overlap = batch > C;
+    // chunk boundaries (the same balanced split as for_chunks); buffers of per rows, not of the context's chunk: slots of a
+    // small k are long
+    const int64_t nch = std::max<int64_t>(1, (batch + C - 1) / C);
+    const int64_t per = std::min<int64_t>(C, ((batch + nch - 1) / nch + 127) / 128 * 128);
+    for (int s = 0; s < (overlap ? 2 : 1); ++s) {
+        CK(ctx->io_p[s].ensure((size_t)(per * slot_bytes)));
+        CK(ctx->io_n[s].ensure((size_t)per * 4));
+    }
+    CK(ctx->io_b.ensure((size_t)per * n * 8));
+    if (overlap) CK(ctx->io_b2.ensure((size_t)per * n * 8));
+    CK(ctx->io_c.ensure((size_t)per * 2));
+    if (overlap) QF_TRY(ensure_copy_stream(ctx));
+    auto copy_in = [&](int64_t i, cudaStream_t st) -> qf_status {
+        const int64_t b0 = i * per, Bc = std::min<int64_t>(per, batch - b0);
+        const int s = overlap ? (int)(i & 1) : 0;
+        CK(cudaMemcpyAsync(ctx->io_p[s].p, packed + b0 * slot_bytes, (size_t)(Bc * slot_bytes), cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(ctx->io_n[s].p, key_idx + b0, (size_t)Bc * 4, cudaMemcpyHostToDevice, st));
+        return QF_OK;
+    };
+    std::vector<uint8_t> flags((size_t)batch);
+    int64_t idx = 0;
+    qf_status st = QF_OK;
+    if (overlap) {
+        st = copy_in(0, ctx->copy_stream);
+        if (st == QF_OK && cudaEventRecord(ctx->ev_u_in[0], ctx->copy_stream) != cudaSuccess)
+            st = ctx->fail(QF_ERR_CUDA, "cudaEventRecord failed");
+    }
+    if (st == QF_OK)
+        st = for_chunks(ctx, batch, [&](int64_t b0, int Bc) -> qf_status {
+            const int s = overlap ? (int)(idx & 1) : 0;
+            if (overlap) {
+                if (idx >= 2) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_copied[s], 0));  // output buffers free again
+                CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_u_in[s], 0));                  // this chunk's input is in
+                if (b0 + Bc < batch) {  // the next chunk's input, once the kernels that read that buffer are done
+                    if (idx >= 1) CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_u_used[s ^ 1], 0));
+                    QF_TRY(copy_in(idx + 1, ctx->copy_stream));
+                    CK(cudaEventRecord(ctx->ev_u_in[s ^ 1], ctx->copy_stream));
+                }
+            } else {
+                QF_TRY(copy_in(idx, ctx->stream));
+            }
+            int64_t* du = s ? ctx->io_b2.as<int64_t>() : ctx->io_b.as<int64_t>();
+            uint8_t* df = ctx->io_c.as<uint8_t>() + (size_t)s * per;
+            QF_TRY(ring_f_a_keyed_packed_chunk(ctx, ctx->io_p[s].as<uint8_t>(), ctx->io_n[s].as<int32_t>(), Bc, k, slot_bytes,
+                                               du, df));
+            cudaStream_t cs = ctx->stream;
+            if (overlap) {
+                CK(cudaEventRecord(ctx->ev_u_used[s], ctx->stream));
+                CK(cudaEventRecord(ctx->ev_done[s], ctx->stream));
+                CK(cudaStreamWaitEvent(ctx->copy_stream, ctx->ev_done[s], 0));
+                cs = ctx->copy_stream;
+            }
+            CK(cudaMemcpyAsync(u_out + b0 * n, du, (size_t)Bc * n * 8, cudaMemcpyDeviceToHost, cs));
+            CK(cudaMemcpyAsync(flags.data() + b0, df, (size_t)Bc, cudaMemcpyDeviceToHost, cs));
+            if (overlap) CK(cudaEventRecord(ctx->ev_copied[s], ctx->copy_stream));
+            else CK(cudaStreamSynchronize(ctx->stream));
+            ++idx;
+            return QF_OK;
+        });
+    // no copy into flags or u_out may outlive the call, also when it failed
+    const cudaError_t e = overlap ? cudaStreamSynchronize(ctx->copy_stream) : cudaSuccess;
+    QF_TRY(st);
+    CK(e);
+    bool all = true;
+    for (int64_t b = 0; b < batch; ++b) all = all && flags[b];
+    if (in_domain) memcpy(in_domain, flags.data(), (size_t)batch);
+    if (!all) return ctx->fail(QF_ERR_NOT_IN_DOMAIN, "f_a: a packed sigma is not canonical or not in the domain D_n");
+    return QF_OK;
+}
+
+qf_status qf_ring_f_a_keyed_packed_dev(qf_ctx* ctx, const uint8_t* packed, const int32_t* key_idx, int64_t batch, int k,
+                                       int64_t slot_bytes, int64_t* u_out, uint8_t* in_domain) {
+    if (!ctx || batch < 0 || (batch > 0 && (!packed || !key_idx || !u_out || !in_domain))) return QF_ERR_INVALID;
+    if (ctx->prm.kind != QF_PSF_GPV_RING) return ring_keyed_ready(ctx);
+    if (!packed_args_ok(ctx->dim, k, slot_bytes)) return ctx->fail(QF_ERR_INVALID, kPackedArgsMsg);
+    if (batch == 0) return QF_OK;
+    if (((uintptr_t)packed) & 15) return ctx->fail(QF_ERR_INVALID, "packed sigma: the slot pointer is not 16-byte aligned");
+    CK(cudaSetDevice(ctx->device));
+    QF_TRY(ring_keyed_ready(ctx));
+    return for_chunks(ctx, batch, [&](int64_t b0, int Bc) {
+        return ring_f_a_keyed_packed_chunk(ctx, packed + b0 * slot_bytes, key_idx + b0, Bc, k, slot_bytes, u_out + b0 * ctx->n,
+                                           in_domain + b0);
+    });
 }
 
 qf_status qf_domain_encode_dev(const int32_t* in, int64_t rows, int64_t dim, int k, int64_t slot_bytes, uint8_t* out,

@@ -70,6 +70,13 @@ __global__ void domain_flags_kernel(const unsigned long long* __restrict__ norm2
         flags[b] = norm2[b] <= bound ? 1 : 0;
 }
 
+// flags[b] already holds a per-row ok byte (a canonical packed slot): the domain check is ANDed in
+__global__ void domain_flags_and_kernel(const unsigned long long* __restrict__ norm2, unsigned long long bound,
+                                        uint8_t* __restrict__ flags, int B) {
+    for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x)
+        flags[b] = (flags[b] && norm2[b] <= bound) ? 1 : 0;
+}
+
 // ---- recombination of exact fp64 partial products --------------------------
 template <typename OutT>
 __global__ void combine_kernel(CombineArgs a, OutT* __restrict__ out, long ldout, int B, int N) {
@@ -261,6 +268,12 @@ cudaError_t qf_launch_domain_flags(const unsigned long long* norm2, unsigned lon
                                    cudaStream_t stream) {
     if (B <= 0) return cudaSuccess;
     domain_flags_kernel<<<grid_for(B, TPB), TPB, 0, stream>>>(norm2, bound, flags, B);
+    return cudaGetLastError();
+}
+cudaError_t qf_launch_domain_flags_and(const unsigned long long* norm2, unsigned long long bound, uint8_t* flags, int B,
+                                       cudaStream_t stream) {
+    if (B <= 0) return cudaSuccess;
+    domain_flags_and_kernel<<<grid_for(B, TPB), TPB, 0, stream>>>(norm2, bound, flags, B);
     return cudaGetLastError();
 }
 cudaError_t qf_launch_combine_i64(const CombineArgs& a, int64_t* out, long ldout, int B, int N, cudaStream_t stream) {

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "common.cuh"
+#include "domain_code.cuh"
 
 // ---- gemm_f64.cu ----------------------------------------------------------
 cudaError_t qf_launch_gemm_f64(const double* X, long ldx, const double* W, long ldw, double* C, long ldc,
@@ -21,6 +22,9 @@ cudaError_t qf_launch_f64_to_i32(const double* in, long ldin, int32_t* out, long
 // in_domain[b] = norm2[b] <= bound
 cudaError_t qf_launch_domain_flags(const unsigned long long* norm2, unsigned long long bound, uint8_t* flags,
                                    int B, cudaStream_t stream);
+// flags[b] &= norm2[b] <= bound: flags already holds a per-row ok byte (a canonical packed slot) that the domain check ANDs in
+cudaError_t qf_launch_domain_flags_and(const unsigned long long* norm2, unsigned long long bound, uint8_t* flags,
+                                       int B, cudaStream_t stream);
 
 struct CombineArgs {
     const double* acc[4];   // exact-integer fp64 partial products, B x N each, leading dim ldacc
@@ -155,7 +159,10 @@ cudaError_t qf_launch_ring_prepare(const int64_t* a, uint64_t* a_hat, long npoly
 // and norm2 = ~0 (not in the domain).  The same holds for the keyed forms of the two launchers below.
 cudaError_t qf_launch_ring_f_a(const int32_t* sigma, const uint64_t* a_hat, int64_t* out, unsigned long long* norm2,
                                int B, int npoly, int n, unsigned long long q, const uint64_t* tw,
-                               cudaStream_t stream, const int32_t* key_idx = nullptr, int nkeys = 0, int* flag = nullptr);
+                               cudaStream_t stream, const int32_t* key_idx = nullptr, int nkeys = 0, int* flag = nullptr,
+                               const PackedRows* packed = nullptr);
+// packed != NULL (keyed only, n >= 64): sigma is unused and row b is decoded from slot b of *packed inside the kernel;
+// packed->ok[b] = 1 when the slot is canonical.  The same for qf_launch_ring_small.
 // Schoolbook fallback for degrees that are not a power of two (or < 64): a is the raw key, npoly x n in [0,q).
 cudaError_t qf_launch_ring_f_a_schoolbook(const int32_t* sigma, const int64_t* a, int64_t* out,
                                           unsigned long long* norm2, int B, int npoly, int n, unsigned long long q,
@@ -380,7 +387,9 @@ void qf_ring_small_key(const int64_t* a, int npoly, int n, int d, unsigned long 
 cudaError_t qf_launch_ring_small(const int32_t* sigma, const uint32_t* a_hat, int64_t* out, unsigned long long* norm2,
                                  int B, int npoly, int n, int d, unsigned long long q, uint32_t np_inv,
                                  const uint32_t* tw, cudaStream_t stream, const int32_t* key_idx = nullptr, int nkeys = 0,
-                                 int* flag = nullptr);
+                                 int* flag = nullptr, const PackedRows* packed = nullptr);
+// whether qf_launch_ring_small takes packed rows at degree n (the others decode first, qf_launch_domain_decode)
+bool qf_ring_small_packed_fused(int n);
 // qf_ring_small_key on the device for npolys polynomials (one warp each): bit-identical words
 cudaError_t qf_launch_ring_small_key(const int64_t* a, uint32_t* a_hat, long npolys, int n, int d, unsigned long long q,
                                      const uint32_t* tw, cudaStream_t stream);

@@ -11,6 +11,7 @@
 // in the transform domain and ONE inverse NTT.  ||sigma||^2 for check_domain
 // (gpv_ring.rs:274-283) is reduced in the same pass.
 #include "common.cuh"
+#include "domain_code.cuh"
 #include "kernels.h"
 
 namespace {
@@ -109,11 +110,15 @@ __global__ void ring_prepare_kernel(const int64_t* __restrict__ a, uint64_t* __r
 
 // KEYED: target b reads the key at a_hat + key_idx[b] npoly n (a table of nkeys keys); an index outside [0, nkeys) sets
 // *flag |= QF_FLAG_KEY_INDEX and gives a zero row that is not in the domain, without reading the table.
-template <bool KEYED>
+// PACKED (keyed only): sigma is unused and target b is the slot b of pk (DESIGN 4.11).  In each round warp 0 reads the high
+// parts of the round's PP polynomials, in entry order, into their work slices (packed_high); each thread then joins its
+// entries with their fixed fields in place.  pk.ok[b] = 1 when the slot is canonical (0 for a bad index).
+template <bool KEYED, bool PACKED = false>
 __global__ void ring_f_a_kernel(const int32_t* __restrict__ sigma, const uint64_t* __restrict__ a_hat,
                                 int64_t* __restrict__ out, unsigned long long* __restrict__ norm2, int B, int npoly,
                                 int n, unsigned long long q, const uint64_t* __restrict__ tw,
-                                const int32_t* __restrict__ key_idx, int nkeys, int* flag) {
+                                const int32_t* __restrict__ key_idx, int nkeys, int* flag, PackedRows pk = {}) {
+    static_assert(!PACKED || KEYED, "the packed form is keyed");
     extern __shared__ uint64_t sm[];
     const int PP = blockDim.y, nh = n >> 1;
     const int t_id = threadIdx.x, y = threadIdx.y;
@@ -121,8 +126,10 @@ __global__ void ring_f_a_kernel(const int32_t* __restrict__ sigma, const uint64_
     uint64_t* acc = sm + (size_t)PP * n + (size_t)y * n;  // PP x n
     __shared__ unsigned long long nrm_s;
     __shared__ unsigned int nrm_ovf;
+    __shared__ PackedCursor cur;
     const uint64_t* psi_rev = tw;
     const uint64_t* psi_inv_rev = tw + n;
+    const bool warp0 = y == 0 && t_id < 32;  // (n >= 64: warp 0 is the first 32 threads of slice 0)
     for (int b = blockIdx.x; b < B; b += gridDim.x) {
         const uint64_t* key = a_hat;
         if (KEYED) {  // block-uniform branch
@@ -133,6 +140,7 @@ __global__ void ring_f_a_kernel(const int32_t* __restrict__ sigma, const uint64_
                     if (t_id == 0) {
                         if (flag) atomicOr(flag, QF_FLAG_KEY_INDEX);
                         if (norm2) norm2[b] = ~0ull;
+                        if (PACKED) pk.ok[b] = 0;
                     }
                 }
                 continue;
@@ -140,6 +148,7 @@ __global__ void ring_f_a_kernel(const int32_t* __restrict__ sigma, const uint64_
             key = a_hat + (long)t * npoly * n;
         }
         if (t_id == 0 && y == 0) { nrm_s = 0; nrm_ovf = 0; }
+        if (PACKED && warp0) packed_begin(&cur, t_id);
         for (int i = t_id; i < n; i += nh) acc[i] = 0;
         NormAcc nrm;  // saturating squared norm (common.cuh)
         nrm.clear();
@@ -148,7 +157,20 @@ __global__ void ring_f_a_kernel(const int32_t* __restrict__ sigma, const uint64_
             const int j = rd * PP + y;
             const bool active = j < npoly;
             __syncthreads();
-            if (active) {
+            if (PACKED) {
+                if (warp0)
+                    for (int yy = 0; yy < PP && rd * PP + yy < npoly; ++yy) packed_high(pk, b, &cur, sm + (size_t)yy * n, n, t_id);
+                __syncthreads();
+                if (active) {
+                    bool bad = false;
+                    for (int i = t_id; i < n; i += nh) {
+                        const int32_t v = packed_value(pk, b, (long long)j * n + i, (uint32_t)work[i], bad);
+                        nrm.add_sq(v);
+                        work[i] = gl_from_i64(v);
+                    }
+                    if (bad) cur.bad = 1;
+                }
+            } else if (active) {
                 const int32_t* src = sigma + ((long)b * npoly + j) * n;
                 for (int i = t_id; i < n; i += nh) {
                     long long v = src[i];
@@ -162,6 +184,10 @@ __global__ void ring_f_a_kernel(const int32_t* __restrict__ sigma, const uint64_
                 const uint64_t* ah = key + (long)j * n;
                 for (int i = t_id; i < n; i += nh) acc[i] = gl_add(acc[i], gl_mul(work[i], ah[i]));
             }
+        }
+        if (PACKED && warp0) {  // (every packed_value of the row is behind the barriers of the last forward transform)
+            const bool canon = packed_finish(pk, b, &cur, t_id);
+            if (t_id == 0) pk.ok[b] = canon ? 1 : 0;
         }
         __syncthreads();
         // reduce the PP partial accumulators into slice 0's work buffer
@@ -322,9 +348,10 @@ cudaError_t qf_launch_ring_prepare(const int64_t* a, uint64_t* a_hat, long npoly
 
 cudaError_t qf_launch_ring_f_a(const int32_t* sigma, const uint64_t* a_hat, int64_t* out, unsigned long long* norm2,
                                int B, int npoly, int n, unsigned long long q, const uint64_t* tw,
-                               cudaStream_t stream, const int32_t* key_idx, int nkeys, int* flag) {
+                               cudaStream_t stream, const int32_t* key_idx, int nkeys, int* flag, const PackedRows* packed) {
     if (B <= 0) return cudaSuccess;
     if (n < 2 || n > 2048 || (n & (n - 1))) return cudaErrorInvalidValue;
+    if (packed && (!key_idx || n < 64)) return cudaErrorInvalidValue;
     int nh = n / 2;
     int pp = 256 / nh;
     if (pp < 1) pp = 1;
@@ -332,16 +359,20 @@ cudaError_t qf_launch_ring_f_a(const int32_t* sigma, const uint64_t* a_hat, int6
     if (pp > 8) pp = 8;
     dim3 block(nh, pp);
     size_t smem = (size_t)2 * pp * n * 8;
-    static size_t configured_dev[QF_MAX_DEVICES][2] = {};
-    size_t& configured = configured_dev[qf_device_slot()][key_idx ? 1 : 0];
+    static size_t configured_dev[QF_MAX_DEVICES][3] = {};
+    size_t& configured = configured_dev[qf_device_slot()][packed ? 2 : key_idx ? 1 : 0];
     if (smem > 48 * 1024 && smem > configured) {
-        cudaError_t e = key_idx ? cudaFuncSetAttribute(ring_f_a_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                                : cudaFuncSetAttribute(ring_f_a_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = packed    ? cudaFuncSetAttribute(ring_f_a_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                        : key_idx ? cudaFuncSetAttribute(ring_f_a_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
+                                  : cudaFuncSetAttribute(ring_f_a_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
         configured = smem;
     }
     int grid = B < 148 * 8 ? B : 148 * 8;
-    if (key_idx)
+    if (packed)
+        ring_f_a_kernel<true, true><<<grid, block, smem, stream>>>(nullptr, a_hat, out, norm2, B, npoly, n, q, tw, key_idx, nkeys,
+                                                                   flag, *packed);
+    else if (key_idx)
         ring_f_a_kernel<true><<<grid, block, smem, stream>>>(sigma, a_hat, out, norm2, B, npoly, n, q, tw, key_idx, nkeys, flag);
     else
         ring_f_a_kernel<false><<<grid, block, smem, stream>>>(sigma, a_hat, out, norm2, B, npoly, n, q, tw, nullptr, 0, nullptr);

@@ -12,6 +12,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "domain_code.cuh"
 #include "kernels.h"
 
 namespace {
@@ -98,15 +99,23 @@ __device__ __forceinline__ void ntt_inv(uint32_t (&v)[EPL], const uint32_t* __re
 // KEYED: row b reads the key at a_hat + key_idx[b] npoly n (a table of nkeys keys); an index outside [0, nkeys) sets
 // *flag |= QF_FLAG_KEY_INDEX and gives a zero row that is not in the domain, without reading the table.  The keyed form
 // asks for 4 blocks per SM at 128-point tiles (the 3329 / n = 256 case): without that bound ptxas spills a register.
-template <int EPL, int D, bool KEYED = false>
-__global__ void __launch_bounds__(128, (KEYED && EPL * D == 8) ? 4 : 0)
+// PACKED (keyed only): sigma is unused and row b is the slot b of pk (DESIGN 4.11).  The warp reads the high parts of one
+// polynomial into its tile of n words of dynamic shared memory (packed_high, in entry order across the row; the cursor sits
+// after the tile), then each lane joins the entries it owns with their fixed fields; pk.ok[b] = 1 when the slot is
+// canonical (0 for a bad index).  The packed complete 256-point tile (D = 1) asks for 3 blocks per SM: at 4 it spills.
+template <int EPL, int D, bool KEYED = false, bool PACKED = false>
+__global__ void __launch_bounds__(128, (KEYED && EPL * D == 8) ? ((PACKED && D == 1) ? 3 : 4) : 0)
 ring_small_kernel(const int32_t* __restrict__ sigma, const uint32_t* __restrict__ a_hat, int64_t* __restrict__ out,
                   unsigned long long* __restrict__ norm2, int B, int npoly, SmallRing R, const uint32_t* __restrict__ tw,
-                  const int32_t* __restrict__ key_idx = nullptr, int nkeys = 0, int* flag = nullptr) {
+                  const int32_t* __restrict__ key_idx = nullptr, int nkeys = 0, int* flag = nullptr, PackedRows pk = {}) {
+    static_assert(!PACKED || KEYED, "the packed form is keyed");
+    extern __shared__ uint32_t rs_tiles[];
     const int lane = threadIdx.x & 31;
     const int wpb = blockDim.x >> 5;
     constexpr int NP = EPL * 32;
     const int n = NP * D;
+    uint32_t* tile = rs_tiles + (threadIdx.x >> 5) * (n + 4);
+    PackedCursor* cur = reinterpret_cast<PackedCursor*>(tile + n);
     for (long b = (long)blockIdx.x * wpb + (threadIdx.x >> 5); b < B; b += (long)gridDim.x * wpb) {
         int t = 0;
         if (KEYED) {
@@ -116,10 +125,12 @@ ring_small_kernel(const int32_t* __restrict__ sigma, const uint32_t* __restrict_
                 if (lane == 0) {
                     if (flag) atomicOr(flag, QF_FLAG_KEY_INDEX);
                     if (norm2) norm2[b] = ~0ull;
+                    if (PACKED) pk.ok[b] = 0;
                 }
                 continue;
             }
         }
+        if (PACKED) packed_begin(cur, lane);
         uint32_t acc[D][EPL];
 #pragma unroll
         for (int c = 0; c < D; ++c)
@@ -129,12 +140,17 @@ ring_small_kernel(const int32_t* __restrict__ sigma, const uint32_t* __restrict_
         nrm.clear();
         for (int j = 0; j < npoly; ++j) {
             const int32_t* src = sigma + ((long)b * npoly + j) * n;
+            if (PACKED) packed_high(pk, b, cur, tile, n, lane);
+            bool bad = false;
             uint32_t v[D][EPL];
 #pragma unroll
             for (int r = 0; r < EPL; ++r) {
                 const int e = r * 32 + lane;
                 int32_t x[D];
-                if (D == 2) {
+                if (PACKED) {
+#pragma unroll
+                    for (int c = 0; c < D; ++c) x[c] = packed_value(pk, b, (long long)j * n + D * e + c, tile[D * e + c], bad);
+                } else if (D == 2) {
                     const int2 t = *reinterpret_cast<const int2*>(src + 2 * e);
                     x[0] = t.x;
                     x[D - 1] = t.y;
@@ -148,6 +164,7 @@ ring_small_kernel(const int32_t* __restrict__ sigma, const uint32_t* __restrict_
                     v[c][r] = (uint32_t)(m < 0 ? m + (int32_t)R.q : m);
                 }
             }
+            if (PACKED && bad) cur->bad = 1;
 #pragma unroll
             for (int c = 0; c < D; ++c) ntt_fwd<EPL>(v[c], tw, lane, R);
             // (the largest tile re-reads its index from L1 instead of keeping it live: no spill at 255 registers)
@@ -188,6 +205,10 @@ ring_small_kernel(const int32_t* __restrict__ sigma, const uint32_t* __restrict_
         if (norm2) {
             nrm.warp_reduce();
             if (lane == 0) norm2[b] = nrm.value();
+        }
+        if (PACKED) {
+            const bool canon = packed_finish(pk, b, cur, lane);
+            if (lane == 0) pk.ok[b] = canon ? 1 : 0;
         }
     }
 }
@@ -317,24 +338,32 @@ SmallRing small_ring(int n, int d, unsigned long long q, uint32_t np_inv) {
 
 cudaError_t qf_launch_ring_small(const int32_t* sigma, const uint32_t* a_hat, int64_t* out, unsigned long long* norm2,
                                  int B, int npoly, int n, int d, unsigned long long q, uint32_t np_inv,
-                                 const uint32_t* tw, cudaStream_t stream, const int32_t* key_idx, int nkeys, int* flag) {
+                                 const uint32_t* tw, cudaStream_t stream, const int32_t* key_idx, int nkeys, int* flag,
+                                 const PackedRows* packed) {
     if (B <= 0) return cudaSuccess;
+    if (packed && (!key_idx || !qf_ring_small_packed_fused(n))) return cudaErrorInvalidValue;
     const SmallRing R = small_ring(n, d, q, np_inv);
     const int wpb = 4;
     long long g = ((long long)B + wpb - 1) / wpb;
     if (g > 148 * 16) g = 148 * 16;
     const int epl = R.np / 32;
-#define QF_RS(E, DD)                                                                                                    \
+    const size_t tiles = packed ? (size_t)wpb * (n + 4) * 4 : 0;  // a tile and a cursor per warp: at most 8.06 KB (n <= 512)
+#define QF_RS_I32(E, DD)                                                                                                \
     (key_idx ? ring_small_kernel<E, DD, true><<<(int)g, 32 * wpb, 0, stream>>>(sigma, a_hat, out, norm2, B, npoly, R, tw, \
                                                                                 key_idx, nkeys, flag)                  \
              : ring_small_kernel<E, DD><<<(int)g, 32 * wpb, 0, stream>>>(sigma, a_hat, out, norm2, B, npoly, R, tw))
+#define QF_RS(E, DD)                                                                                                    \
+    (packed ? ring_small_kernel<E, DD, true, true><<<(int)g, 32 * wpb, tiles, stream>>>(nullptr, a_hat, out, norm2, B,  \
+                                                                                        npoly, R, tw, key_idx, nkeys,   \
+                                                                                        flag, *packed)                  \
+            : QF_RS_I32(E, DD))
     if (d == 1) {
         switch (epl) {
             case 2: QF_RS(2, 1); break;
             case 4: QF_RS(4, 1); break;
             case 8: QF_RS(8, 1); break;
             case 16: QF_RS(16, 1); break;
-            case 32: QF_RS(32, 1); break;
+            case 32: QF_RS_I32(32, 1); break;
             default: return cudaErrorInvalidValue;
         }
     } else {
@@ -343,13 +372,18 @@ cudaError_t qf_launch_ring_small(const int32_t* sigma, const uint32_t* a_hat, in
             case 2: QF_RS(2, 2); break;
             case 4: QF_RS(4, 2); break;
             case 8: QF_RS(8, 2); break;
-            case 16: QF_RS(16, 2); break;
+            case 16: QF_RS_I32(16, 2); break;
             default: return cudaErrorInvalidValue;
         }
     }
 #undef QF_RS
+#undef QF_RS_I32
     return cudaGetLastError();
 }
+
+// The packed form spills at n = 1024 (255 registers hold the int32 tile with nothing to spare), so there the caller
+// decodes into an int32 staging buffer and launches the int32 keyed form.
+bool qf_ring_small_packed_fused(int n) { return n <= 512; }
 
 cudaError_t qf_launch_ring_small_key(const int64_t* a, uint32_t* a_hat, long npolys, int n, int d, unsigned long long q,
                                      const uint32_t* tw, cudaStream_t stream) {

@@ -705,6 +705,34 @@ class PSFGPVRing(_PSFBase):
             raise NotInDomain(_ffi.QF_ERR_NOT_IN_DOMAIN, "sigma is not in the domain D_n")
         return u, ok
 
+    def f_a_keyed_packed_batch(self, keys, packed: np.ndarray, key_idx, k=None, strict: bool = True):
+        """f_a_keyed_batch on packed Domain values (qf_ring_f_a_keyed_packed): packed is B x slot_bytes, one slot per
+        signature in the code of f_a_packed_batch; the table is installed as in f_a_keyed_batch.  k defaults to
+        domain_code_params().  Returns (u, in_domain), in_domain[b] False also when slot b is not a canonical code; rows in
+        the domain equal f_a_keyed_batch on the decoded sigma, bit for bit.  Pin `packed` (and the outputs) for the copies
+        to overlap the computation."""
+        if self._keys_id is not keys:
+            kk = np.ascontiguousarray(keys, dtype=np.int64)
+            assert kk.ndim == 3 and kk.shape[1:] == self._domain_shape and kk.shape[0] >= 1
+            self.ctx.call("qf_ring_set_key_table", _ffi.ptr(kk), kk.shape[0])
+            self._keys_id = keys
+        p = np.ascontiguousarray(packed, dtype=np.uint8)
+        assert p.ndim == 2
+        b, slot_bytes = p.shape
+        k, _ = self._code_params(k, slot_bytes)
+        ki = np.ascontiguousarray(key_idx, dtype=np.int32)
+        assert ki.shape == (b,)
+        u = np.empty((b, self.n), dtype=np.int64)
+        flags = np.empty(b, dtype=np.uint8)
+        st = self.ctx.status("qf_ring_f_a_keyed_packed", _ffi.ptr(p), _ffi.ptr(ki), b, k, slot_bytes, _ffi.ptr(u),
+                             _ffi.ptr(flags))
+        if st not in (_ffi.QF_OK, _ffi.QF_ERR_NOT_IN_DOMAIN):
+            raise QfError(st, self.ctx._lib.qf_last_error(self.ctx._h).decode())
+        ok = flags.astype(bool)
+        if strict and not ok.all():
+            raise NotInDomain(_ffi.QF_ERR_NOT_IN_DOMAIN, "sigma is not canonical or not in the domain D_n")
+        return u, ok
+
     def gen_trapdoor_ring_lwe_batch(self, a_bars, rs, es) -> np.ndarray:
         """gen_trapdoor_ring_lwe for T keys in one call (qf_ring_trap_gen_batch_from): a_bars T x n residues in [0, q),
         rs and es T x k x n.  Key t equals gen_trapdoor_ring_lwe(a_bars[t], rs[t], es[t]) bit for bit; nothing is
